@@ -2,6 +2,7 @@
 """Benchmark of the RHMC leapfrog hot path (BASELINE.json: "RHMC star-gradient evals/sec").
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload all|c2|c4|c5]
+                    [--dump-outputs DIR]
 
 One unit of the metric = one star advanced by one RHMC_single_step (reference sampler_RHMC.py:522-566).
 One "step" = one resident pass of the hot path over one batch of synthetic input (every chain of the batch runs
@@ -25,6 +26,11 @@ other BASELINE configs under "workloads":
 Per record: `value` (inputs resident, device time from CUDA events on the launching stream), `e2e` (public API with
 pinned HOST buffers, copies inside the timed region), `roofline`, `clocks`, `gpu_launches`, and at N = 1 `cpu_baseline`
 (the NumPy oracle port of the reference on the box's host cores; the Python-2 reference itself cannot travel).
+
+--dump-outputs DIR: after the timed steps of the headline record, rank 0 writes what the timed path computed in its last
+step as DIR/<name>.npy (see dump_outputs), so that two builds run with the same arguments -- hence the same inputs and
+seeds -- can be compared output for output.  With N > 1 GPUs that is rank 0's share of the work only.  DIR must lie
+outside the repository: bench.py writes nothing inside it.
 """
 from __future__ import annotations
 
@@ -292,6 +298,30 @@ class ClockSampler:
                 "power_w_max": max(power), "samples": len(sm)}
 
 
+DUMP_LIMIT_BYTES = 64 * 10**6   # array data written by --dump-outputs (plus one 128-byte .npy header per file)
+
+
+def dump_outputs(path, rows, whole=None):
+    """Write each array as <path>/<name>.npy: flags (uint8) as float32, everything else as float64.
+    `rows` maps names to arrays sharing a leading axis (chains, fields or stars); when they would exceed DUMP_LIMIT_BYTES,
+    a fixed seeded sample of that axis is kept in increasing order.  sample_index.npy holds the kept indices.
+    `whole` maps names to small arrays written in full."""
+    def conv(a):
+        a = np.asarray(a)
+        return a.astype(np.float32) if a.dtype in (np.uint8, np.bool_) else a.astype(np.float64)
+
+    out = {k: conv(v) for k, v in (whole or {}).items()}
+    n = len(next(iter(rows.values())))
+    per_row = 8 + sum(conv(v[:1]).nbytes for v in rows.values())
+    keep = min(n, max(0, DUMP_LIMIT_BYTES - sum(v.nbytes for v in out.values())) // per_row)
+    idx = np.arange(n) if keep == n else np.sort(np.random.RandomState(0).choice(n, keep, replace=False))
+    out["sample_index"] = conv(idx)
+    out.update({k: conv(np.asarray(v)[idx]) for k, v in rows.items()})
+    os.makedirs(path, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(path, k + ".npy"), v)
+
+
 def measured_peaks():
     path = os.path.join(ROOT, "MEASURED_PEAKS.json")
     if os.path.isfile(path):
@@ -383,10 +413,11 @@ class Env:
 
 # ----------------------------------------------------------------------------------------------- independent chains / fields
 def bench_chains(env, wl, *, niter, steps, warmup, e2e_steps, want, precision, scaling, seed_base, field_id_base=0,
-                 device_data_seed=None, parallelism="", min_seconds=0.0):
+                 device_data_seed=None, parallelism="", min_seconds=0.0, dump_dir=None):
     """C2 / C4: F independent fields per rank in one RHMCContext, one resident launch per step.
     min_seconds (sub-records only): lengthen the timed region to at least this, so that the clock sampler (50 ms period) sees
-    it -- `steps` in the record is the number actually timed."""
+    it -- `steps` in the record is the number actually timed.
+    dump_dir: write the chains, final states and acceptance rates of the last timed launch there (dump_outputs)."""
     torch = env.torch
     from hmc_stellar_toy_model_b200 import RHMCContext, _capi
 
@@ -452,6 +483,9 @@ def bench_chains(env, wl, *, niter, steps, warmup, e2e_steps, want, precision, s
     clocks = sampler.stop() if sampler else None
     total_ms = float(sum(kernel_ms))
     region_ms = ev0.elapsed_time(ev1)
+    if dump_dir is not None and rank == 0:
+        ctx.run_download(a)   # the last timed launch's results, copied back after the timed region
+        dump_outputs(dump_dir, out_arrays)
 
     # ---- e2e: public API, host buffers, copies inside the timed region
     e2e_steps = max(1, min(steps, e2e_steps))
@@ -619,9 +653,11 @@ def tiled_parity_check(env, stream):
 
 
 def bench_bigfield(env, *, rows, cols, nstars, weak, niter, steps, warmup, e2e_steps, comm_kind, with_parity, precision=64,
-                   replicas=False, label="c5_tiled_field", dt=None, fixed_point_mode=0, min_seconds=0.0):
+                   replicas=False, label="c5_tiled_field", dt=None, fixed_point_mode=0, min_seconds=0.0, dump_dir=None):
     """C5: ONE large field, row strips over the ranks (strong), or one rows x cols strip per rank (weak).
-    replicas=True (C3): every rank runs its own copy of the whole field, no communication."""
+    replicas=True (C3): every rank runs its own copy of the whole field, no communication.
+    dump_dir: write the chain scalars of the last timed run and the final (q, p, dV/dq) of this rank's stars, in global
+    star-id order, there (dump_outputs)."""
     torch = env.torch
     from hmc_stellar_toy_model_b200 import _capi
     from hmc_stellar_toy_model_b200 import bigfield as bf
@@ -686,6 +722,11 @@ def bench_bigfield(env, *, rows, cols, nstars, weak, niter, steps, warmup, e2e_s
         launches += strip.launch_count - l0 + eng.replayed_launches
         acc = out["accept_rate"]
     clocks = sampler.stop() if sampler else None
+    if dump_dir is not None and env.rank == 0:
+        q, p, g = strip.get_stars()
+        order = np.argsort(strip.ids)
+        dump_outputs(dump_dir, {"star_id": strip.ids[order], "q_final": q[order], "p_final": p[order], "grad_final": g[order]},
+                     {k: out[k] for k in ("E_chain", "V_chain", "T_chain", "A_chain", "accept_rate")})
     # e2e: host buffers in (data window + stars), final stars and the chain scalars out
     e2e_steps = max(1, min(steps, e2e_steps))
     t_e2e = 0.0
@@ -790,13 +831,14 @@ def run_ours(args):
         cpu["c4"] = cpu_baseline_record("c4", 6.0) if which in ("all", "c4") else None
         cpu["c5"] = cpu_baseline_record("c5", 6.0) if which in ("all", "c5") else None
 
-    def c2():
+    def c2(dump_dir=None):
         wl = workload_c2(args.chains_per_mag, 77 + rank)
         return bench_chains(env, wl, niter=args.niter, steps=args.steps, warmup=args.warmup, e2e_steps=args.e2e_steps,
                             want=("q", "p", "E", "V", "T", "A"), precision=args.precision, scaling="weak", seed_base=0,
-                            parallelism="independent chains sharded across %d GPU(s), no communication" % world)
+                            parallelism="independent chains sharded across %d GPU(s), no communication" % world,
+                            dump_dir=dump_dir)
 
-    def c4(precision=None):
+    def c4(precision=None, dump_dir=None):
         total = args.fields
         per = max(1, total // world)
         wl = workload_c4(per, 5000 + rank, host_data=False)
@@ -807,32 +849,33 @@ def run_ours(args):
                             precision=args.precision if precision is None else precision, scaling="strong", seed_base=17,
                             field_id_base=rank * per, min_seconds=0.6 if which == "all" else 0.0,
                             device_data_seed=4, parallelism="%d independent fields split over %d GPU(s) (contiguous "
-                            "blocks), no communication" % (per * world, world))
+                            "blocks), no communication" % (per * world, world), dump_dir=dump_dir)
 
-    def c5(weak, precision=None, fixed_point_mode=0):
+    def c5(weak, precision=None, fixed_point_mode=0, dump_dir=None):
         return bench_bigfield(env, rows=args.rows, cols=args.cols, nstars=args.stars, weak=weak, niter=args.c5_niter,
                               steps=max(10, args.sub_steps) if which == "all" else args.steps, warmup=3, e2e_steps=2,
                               comm_kind=args.comm, with_parity=not weak and precision is None and not fixed_point_mode,
                               precision=args.precision if precision is None else precision,
                               fixed_point_mode=fixed_point_mode or args.fixed_point_mode,
-                              min_seconds=0.6 if which == "all" else 0.0)
+                              min_seconds=0.6 if which == "all" else 0.0, dump_dir=dump_dir)
 
-    def c3():
+    def c3(dump_dir=None):
         # BASELINE configs[2]: "RHMC-big-sim2/3/4 crowded field: hundreds to thousands of stars in one large image with the
         # full RHMC leapfrog loop" -- one 256 x 256 field at the sim4 / configs[3] density (0.05 stars per pixel: 3277 stars)
         return bench_bigfield(env, rows=256, cols=256, nstars=3277, weak=False, niter=args.c5_niter,
                               steps=max(10, args.sub_steps) if which == "all" else args.steps, warmup=3, e2e_steps=2,
                               comm_kind=args.comm, with_parity=False, precision=args.precision, replicas=True,
-                              label="c3_crowded_field", min_seconds=0.6 if which == "all" else 0.0)
+                              label="c3_crowded_field", min_seconds=0.6 if which == "all" else 0.0, dump_dir=dump_dir)
 
+    dump = args.dump_outputs
     if which == "c4":
-        out = c4()
+        out = c4(dump_dir=dump)
     elif which == "c3":
-        out = c3()
+        out = c3(dump_dir=dump)
     elif which == "c5":
-        out = c5(args.weak)
+        out = c5(args.weak, dump_dir=dump)
     else:
-        out = c2()
+        out = c2(dump_dir=dump)
     if rank == 0 and out is not None:
         out["cpu_baseline"] = cpu.get("c2" if which == "all" else which)
     def c2_fp32():
@@ -925,7 +968,21 @@ def main():
     ap.add_argument("--precision", type=int, default=64, choices=[64, 32])
     ap.add_argument("--e2e-steps", type=int, default=3)
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the headline record's timed path computed in its last step as DIR/<name>.npy "
+                         "(float32 / float64, at most 64 MB: a fixed seeded sample of the chains when larger); DIR "
+                         "must lie outside the repository.  With N > 1 GPUs only rank 0 writes, and only its own share: "
+                         "its chains or fields (c2, c4) or the stars of its strip (c5)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs:
+        if args.impl != "ours":
+            ap.error("--dump-outputs writes the outputs of the CUDA path: use it with --impl ours")
+        args.dump_outputs = os.path.realpath(args.dump_outputs)
+        root = os.path.realpath(ROOT)
+        if os.path.commonpath([args.dump_outputs, root]) == root:
+            ap.error("--dump-outputs: %s is inside the repository; bench.py writes nothing there" % args.dump_outputs)
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3  # timing rule: W >= 3
     if args.impl == "reference":

@@ -1,4 +1,4 @@
-"""Import-time Python-3 shim for the UNMODIFIED reference at /root/reference.
+"""Import-time Python-3 shim for the UNMODIFIED reference, a checkout named by $SRHMC_REFERENCE_DIR.
 
 TEST INFRASTRUCTURE ONLY.  Nothing in the product package imports this file.
 
@@ -12,8 +12,8 @@ this repository) after three mechanical, semantics-preserving rewrites:
   * `np.infty`, `np.product` aliases for NumPy >= 2
 
 and with stub `matplotlib*` modules registered so the import-time rcParams
-writes in utils.py:2-16,22 succeed.  The reference directory only exists in the
-build container, never on the GPU box, so callers must gate on `available()`.
+writes in utils.py:2-16,22 succeed.  The reference is not part of this
+repository, so callers must gate on `available()`.
 
 Used by: tests/golden/make_golden.py (fixture generator) and the CPU tests that
 pin oracle/stellar_oracle.py against the live reference.
@@ -27,14 +27,14 @@ import types
 
 import numpy as np
 
-REFERENCE_DIR = os.environ.get("SRHMC_REFERENCE_DIR", "/root/reference")
+REFERENCE_DIR = os.environ.get("SRHMC_REFERENCE_DIR", "")
 
 _PRINT_RE = re.compile(r"^(\s*)print\s+(?!\()(.*?)\s*$", re.M)
 _loaded: dict[str, types.ModuleType] = {}
 
 
 def available() -> bool:
-    return os.path.isfile(os.path.join(REFERENCE_DIR, "sampler_RHMC.py"))
+    return bool(REFERENCE_DIR) and os.path.isfile(os.path.join(REFERENCE_DIR, "sampler_RHMC.py"))
 
 
 class _Anything(types.ModuleType):
@@ -108,7 +108,8 @@ def _load(name: str) -> types.ModuleType:
 def load():
     """Return (utils, sampler_RHMC, samplers) modules of the live reference."""
     if not available():
-        raise RuntimeError("reference checkout not present at %s" % REFERENCE_DIR)
+        raise RuntimeError("reference checkout not present: set SRHMC_REFERENCE_DIR to a checkout of the reference "
+                           "(now %r)" % REFERENCE_DIR)
     _install_stubs()
     utils = _load("utils")
     sampler_rhmc = _load("sampler_RHMC")

@@ -12,7 +12,7 @@ unpinned" upstream, SURVEY.md section 4), so this oracle is pinned against the
 reference itself executed in the build container through oracle/ref_shim.py:
 tests/golden/make_golden.py records the reference's outputs as fixtures and
 tests/test_oracle_golden.py checks this file against them (and against the live
-reference when /root/reference is present).  The arithmetic follows the
+reference when SRHMC_REFERENCE_DIR names a checkout).  The arithmetic follows the
 reference's operation order so agreement is at the 1e-15 level, not just 1e-10.
 
 Conventions (SURVEY.md section 8 / appendix A): q is a flat float64 array

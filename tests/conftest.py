@@ -11,4 +11,4 @@ for p in (ROOT, os.path.join(ROOT, "oracle"), os.path.dirname(os.path.abspath(__
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
-    config.addinivalue_line("markers", "reference: needs the read-only reference checkout at /root/reference")
+    config.addinivalue_line("markers", "reference: needs a checkout of the upstream reference, named by SRHMC_REFERENCE_DIR")

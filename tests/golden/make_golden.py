@@ -1,9 +1,9 @@
 #!/usr/bin/env python
 """Generate the golden fixtures in this directory from the UNMODIFIED reference.
 
-Run in the build container only (needs /root/reference):
+Needs a checkout of the reference (jaekor91/HMC-stellar-toy-model):
 
-    python tests/golden/make_golden.py
+    SRHMC_REFERENCE_DIR=<checkout> python tests/golden/make_golden.py
 
 Every array written here is an output of the reference's own code
 (sampler_RHMC.py / samplers.py / utils.py loaded through oracle/ref_shim.py),

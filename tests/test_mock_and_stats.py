@@ -8,10 +8,9 @@ import os
 import numpy as np
 import pytest
 
+import ref_shim
 import stellar_oracle as so
 from helpers import GOLDEN_DIR, relerr
-
-REF = "/root/reference"
 
 
 def _ar1_chains(seed, nchain, niter, d, phi):
@@ -33,10 +32,9 @@ def test_convergence_stats_golden():
             assert relerr(neff, z["neff_" + tag]) < 1e-10
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout not present")
+@pytest.mark.reference
+@pytest.mark.skipif(not ref_shim.available(), reason="reference checkout not present")
 def test_convergence_stats_matches_live_reference():
-    import ref_shim
-
     utils = ref_shim.load()[0]
     x = _ar1_chains(5, 6, 400, 3, 0.6)
     for thin, warm in ((5, 0), (1, 37), (3, 100)):
@@ -302,11 +300,10 @@ def test_find_peaks_descent_matches_oracle_per_seed():
     assert relerr(q[alive], want[alive]) < 1e-6
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout not present")
+@pytest.mark.reference
+@pytest.mark.skipif(not ref_shim.available(), reason="reference checkout not present")
 def test_find_peaks_oracle_matches_live_reference():
     """A second configuration (24x40 image, two stars, coarser grid, larger steps) straight against the reference."""
-    import ref_shim
-
     utils, _, smp = ref_shim.load()
     np.random.seed(123)
     gym = smp.lightsource_gym()
