@@ -284,9 +284,9 @@ class TorchDistComm:
 
 class PeerComm:
     """The library's own collectives: exchange kernels over peer-mapped memory (NVLink P2P / CUDA IPC) enqueued by the
-    phases themselves (PFIX_QFIX, QFIX_KICK: max of the fixed-point counts; PACK: boundary lists into the neighbours'
-    buffers; RECORD_E0 / ACCEPT: sum of the energy partials) -- no NCCL call on the path, and one strip per process can
-    replay a captured CUDA graph of an iteration.
+    phases themselves (KICK1, PFIX_QFIX, EVAL_KICK2_KICK1: max of the fixed-point counts they produce; PACK: boundary lists
+    into the neighbours' buffers; RECORD_E0 / ACCEPT: sum of the energy partials) -- no NCCL call on the path, and one
+    strip per process can replay a captured CUDA graph of an iteration.
 
     PeerComm(strips)            all strips of the tiling live in this process (each on its OWN stream: the exchange kernels
                                 wait for each other), mailboxes shared by raw device pointers;

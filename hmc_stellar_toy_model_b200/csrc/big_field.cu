@@ -296,34 +296,15 @@ __device__ __forceinline__ bool peer_wait_word(const PeerSlot* s, unsigned long 
     return true;
 }
 
-// The field-wide maximum of a fixed-point count taken INSIDE the kernel that consumes it (no separate exchange kernel):
-// block 0 sends this rank's count to every rank's mailbox, every block waits for the world's contributions in its OWN
-// rank's mailbox (local memory) and takes the maximum; the last block to leave the kernel advances the epoch, so every
-// block of the launch sees the same one.
+// What the kernels that produce a fixed-point count need for its all-reduce (all zero without peer exchange)
 struct PeerX {
     PeerPtrs peers;
-    int rank, world, on;
-    int prod;   // the kernel that PRODUCES a fixed-point count all-reduces it in its last block (peer_max_epilogue)
+    int rank, world;
+    int prod;   // peer exchange is on: the kernel's last block all-reduces the count (peer_max_epilogue)
     unsigned long long* epoch;
     unsigned int* ticket;
     int* err;
 };
-
-__device__ __forceinline__ int peer_max_in_kernel(const PeerX& X, int local) {
-    __shared__ int s_max;
-    const unsigned long long e = X.epoch[0] + 1;
-    const int par = (int)(e & 1), t = threadIdx.x;
-    if (t == 0) s_max = local;
-    __syncthreads();
-    if (t < X.world) {
-        if (blockIdx.x == 0) peer_send_word(&reinterpret_cast<PeerHeader*>(X.peers.box[t])->ar[par][X.rank], e, local);
-        const PeerSlot* mine = &reinterpret_cast<const PeerHeader*>(X.peers.box[X.rank])->ar[par][t];
-        int got = 0;
-        if (peer_wait_word(mine, e, X.err, got)) atomicMax(&s_max, got);
-    }
-    __syncthreads();
-    return s_max;
-}
 
 // all-reduce(max) of *word over the ranks by the LAST block to leave the kernel that produced it: the word is complete (every
 // block's atomicMax precedes its ticket), one block polls the mailbox, and the consumer kernel just reads the word.
@@ -353,17 +334,6 @@ __device__ __forceinline__ void peer_max_epilogue(const PeerX& X, int* word) {
         *word = s_max;
         X.epoch[0] = e;
         *X.ticket = 0u;
-    }
-}
-
-__device__ __forceinline__ void peer_epoch_advance(const PeerX& X) {
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        __threadfence();
-        if (atomicAdd(X.ticket, 1u) == gridDim.x - 1) {
-            X.epoch[0] += 1;
-            *X.ticket = 0u;
-        }
     }
 }
 
@@ -416,7 +386,7 @@ __global__ void big_kick1_kernel(const BigParams P, const BigStep S, int n, cons
 // p fixed point phase B (continue to the global count), then (3) q fixed point phase A
 __global__ void big_pfix_qfix_kernel(const BigParams P, const BigStep S, int n, double* q, double* p, double* a1, double* a2,
                                      const int* cnt_p, int* cnt_q, const PeerX X) {
-    const int target = S.per_star ? 0 : (X.on ? peer_max_in_kernel(X, *cnt_p) : *cnt_p);
+    const int target = S.per_star ? 0 : *cnt_p;
     int local_max = 0;
     for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += gridDim.x * blockDim.x) {
         double pf = p[3 * k];
@@ -443,27 +413,23 @@ __global__ void big_pfix_qfix_kernel(const BigParams P, const BigStep S, int n, 
         a1[3 * k] = sf; a1[3 * k + 1] = sx; a1[3 * k + 2] = sy;   // sigma
         a2[3 * k] = bf; a2[3 * k + 1] = bx; a2[3 * k + 2] = by;   // p/H(sigma)
         q[3 * k] = qf; q[3 * k + 1] = qx; q[3 * k + 2] = qy;
-        // own count rides in the sign-free spare: store in g-independent slot via a2? keep it in a separate array
-        // (written below through cnt_own)
         local_max = max(local_max, c);
-        // stash own count in the low bits of nothing: use p-array neighbour? -> dedicated array in launcher (a3)
-        reinterpret_cast<int*>(a2 + 3 * (size_t)n)[k] = c;
+        reinterpret_cast<int*>(a2 + 3 * (size_t)n)[k] = c;   // own count, past the 3n doubles of a2
     }
     if (local_max) atomicMax(cnt_q, local_max);
-    if (X.on && !S.per_star) peer_epoch_advance(X);
     if (X.prod && !S.per_star) peer_max_epilogue(X, cnt_q);
 }
 
 // q fixed point phase B, then (4) p -= h dtau/dq at the new q
 // and -- tile path -- the pair records of the star's final position for the coming evaluation (bin_star, big_tile.cuh)
 __global__ void big_qfix_kick_kernel(const BigParams P, const BigStep S, int n, double* q, double* p, const double* a1,
-                                     const double* a2, const int* cnt_q, int ntx, int* tcnt, PairRec* tlist, int* err, const PeerX X,
+                                     const double* a2, const int* cnt_q, int ntx, int* tcnt, PairRec* tlist, int* err,
                                      int2* pack_counts, double lo_edge, double hi_edge, double* Lfill, size_t npix) {
     // star-parallel evaluation path: the model image of the COMING evaluation is reset to the background here (nobody reads
     // it between the last gather and the next scatter), which saves that path a launch per leapfrog step
     if (Lfill)
         for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < npix; i += (size_t)gridDim.x * blockDim.x) Lfill[i] = P.F.B;
-    const int target = S.per_star ? 0 : (X.on ? peer_max_in_kernel(X, *cnt_q) : *cnt_q);
+    const int target = S.per_star ? 0 : *cnt_q;
     for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += gridDim.x * blockDim.x) {
         const double sf = a1[3 * k], sx = a1[3 * k + 1], sy = a1[3 * k + 2];
         const double bf = a2[3 * k], bx = a2[3 * k + 1], by = a2[3 * k + 2];
@@ -485,7 +451,6 @@ __global__ void big_qfix_kick_kernel(const BigParams P, const BigStep S, int n, 
             if (qx >= hi_edge) atomicAdd(&pack_counts[k >> 10].y, 1);
         }
     }
-    if (X.on && !S.per_star) peer_epoch_advance(X);
 }
 
 // (5) p -= h dphi/dq at the new q; (6) reflections
@@ -757,8 +722,9 @@ __global__ void big_pack_count_kernel(int n, const double* q, double lo_edge, do
     if (threadIdx.x == 0) counts[blockIdx.x] = make_int2(c[0], c[1]);
 }
 
-__global__ void big_pack_kernel(int n, const double* q, double lo_edge, double hi_edge, const int2* counts, double* send, int cap,
-                                int* err) {
+// the compaction of the ordered packing (big_pack_kernel, big_pack_xchg_kernel); the last block writes the two list lengths
+__device__ __forceinline__ void pack_chunk(int n, const double* q, double lo_edge, double hi_edge, const int2* counts, double* send,
+                                           int cap, int* err) {
     __shared__ int base[2];
     __shared__ int wcount[2][32];
     // exclusive prefix of the block counts
@@ -811,9 +777,14 @@ __global__ void big_pack_kernel(int n, const double* q, double lo_edge, double h
     }
 }
 
-// all-reduce of a small vector: op 0 = max of n ints (in place), op 1 = sum of n doubles (in -> out), rank order
-__global__ void big_xchg_small_kernel(const PeerPtrs peers, int rank, int world, int op, int n, int* ivals, const double* din,
-                                      double* dout, unsigned long long* epoch, int* err) {
+__global__ void big_pack_kernel(int n, const double* q, double lo_edge, double hi_edge, const int2* counts, double* send, int cap,
+                                int* err) {
+    pack_chunk(n, q, lo_edge, hi_edge, counts, send, cap, err);
+}
+
+// all-reduce(sum) of n doubles (in -> out), summed in rank order on every rank
+__global__ void big_xchg_small_kernel(const PeerPtrs peers, int rank, int world, int n, const double* din, double* dout,
+                                      unsigned long long* epoch, int* err) {
     __shared__ int ok;
     const unsigned long long e = epoch[0] + 1;
     const int par = (int)(e & 1);
@@ -822,7 +793,7 @@ __global__ void big_xchg_small_kernel(const PeerPtrs peers, int rank, int world,
     __syncthreads();
     if (t < world) {
         PeerSlot* s = &reinterpret_cast<PeerHeader*>(peers.box[t])->ar[par][rank];
-        for (int k = 0; k < n; ++k) s->v[k] = op == 0 ? (double)ivals[k] : din[k];
+        for (int k = 0; k < n; ++k) s->v[k] = din[k];
         peer_publish_tag(&s->tag, e);
         const PeerSlot* mine = &reinterpret_cast<const PeerHeader*>(peers.box[rank])->ar[par][t];
         if (!peer_wait_tag(&mine->tag, e, err)) ok = 0;
@@ -833,11 +804,8 @@ __global__ void big_xchg_small_kernel(const PeerPtrs peers, int rank, int world,
         if (ok) {
             for (int k = 0; k < n; ++k) {
                 double acc = __ldcv(&h->ar[par][0].v[k]);
-                for (int r = 1; r < world; ++r) {
-                    const double x = __ldcv(&h->ar[par][r].v[k]);
-                    acc = op == 0 ? fmax(acc, x) : acc + x;
-                }
-                if (op == 0) ivals[k] = (int)acc; else dout[k] = acc;
+                for (int r = 1; r < world; ++r) acc += __ldcv(&h->ar[par][r].v[k]);
+                dout[k] = acc;
             }
         }
         epoch[0] = e;
@@ -896,12 +864,6 @@ __device__ void ghost_exchange_body(const PeerPtrs peers, int rank, int world, c
     }
 }
 
-__global__ void big_xchg_ghost_kernel(const PeerPtrs peers, int rank, int world, const double* send, double* recv, size_t list,
-                                      unsigned long long* epoch, int* err, const BigParams P, int ntx, int n_own, int cap, int* tcnt,
-                                      PairRec* tlist) {
-    ghost_exchange_body(peers, rank, world, send, recv, list, epoch, err, P, ntx, n_own, cap, tcnt, tlist);
-}
-
 // Ordered ghost packing, the exchange and the binning of the received ghosts in ONE kernel: every block compacts its chunk
 // (as big_pack_kernel), the last block to finish runs the exchange body.  The chunk counts come from the position-update
 // kernel (big_qfix_kick_kernel) and are zeroed here for the next step.
@@ -919,55 +881,8 @@ struct GhostX {
 
 __global__ void big_pack_xchg_kernel(int n, const double* q, double lo_edge, double hi_edge, int2* counts, double* send, int cap,
                                      int* err, const BigParams P, const GhostX G) {
-    __shared__ int base[2];
-    __shared__ int wcount[2][32];
     __shared__ int s_last;
-    int plo = 0, phi = 0;
-    for (int b = threadIdx.x; b < (int)blockIdx.x; b += blockDim.x) {
-        const int2 c = counts[b];
-        plo += c.x;
-        phi += c.y;
-    }
-    if (threadIdx.x == 0) base[0] = base[1] = 0;
-    __syncthreads();
-    if (plo) atomicAdd(&base[0], plo);
-    if (phi) atomicAdd(&base[1], phi);
-    __syncthreads();
-    const int k_begin = blockIdx.x * kPackChunk, k_end = min(n, k_begin + kPackChunk);
-    for (int k0 = k_begin; k0 < k_end; k0 += blockDim.x) {
-        const int k = k0 + threadIdx.x;
-        bool lo = false, hi = false;
-        double f = 0, x = 0, y = 0;
-        if (k < k_end) {
-            f = q[3 * k]; x = q[3 * k + 1]; y = q[3 * k + 2];
-            lo = x < lo_edge;
-            hi = x >= hi_edge;
-        }
-        const int lane = threadIdx.x & 31, w = threadIdx.x >> 5, nw = blockDim.x >> 5;
-        const unsigned blo = __ballot_sync(0xffffffffu, lo), bhi = __ballot_sync(0xffffffffu, hi);
-        if (lane == 0) { wcount[0][w] = __popc(blo); wcount[1][w] = __popc(bhi); }
-        __syncthreads();
-        int off_lo = base[0], off_hi = base[1];
-        for (int i = 0; i < w; ++i) { off_lo += wcount[0][i]; off_hi += wcount[1][i]; }
-        const unsigned lt = (1u << lane) - 1u;
-        if (lo) {
-            const int o = off_lo + __popc(blo & lt);
-            if (o < cap) { double* d = send + 1 + 3 * (size_t)o; d[0] = f; d[1] = x; d[2] = y; } else atomicExch(err, 2);
-        }
-        if (hi) {
-            const int o = off_hi + __popc(bhi & lt);
-            if (o < cap) { double* d = send + (1 + 3 * (size_t)cap) + 1 + 3 * (size_t)o; d[0] = f; d[1] = x; d[2] = y; } else atomicExch(err, 2);
-        }
-        __syncthreads();
-        if (threadIdx.x == 0) {
-            for (int i = 0; i < nw; ++i) { base[0] += wcount[0][i]; base[1] += wcount[1][i]; }
-        }
-        __syncthreads();
-    }
-    if (threadIdx.x == 0 && blockIdx.x == gridDim.x - 1) {
-        send[0] = (double)min(base[0], cap);
-        send[1 + 3 * (size_t)cap] = (double)min(base[1], cap);
-    }
+    pack_chunk(n, q, lo_edge, hi_edge, counts, send, cap, err);
     // last block out: every chunk (and the two list lengths) is in `send`
     __syncthreads();
     if (threadIdx.x == 0) {
@@ -1000,8 +915,6 @@ struct BBuf {
 
 }  // namespace
 
-#include "big_tile.cuh"
-
 struct srhmc_big {
     srhmc_big_config cfg;
     BigParams P;
@@ -1016,14 +929,9 @@ struct srhmc_big {
     // peer exchange (our own collectives over P2P / IPC mapped memory)
     BBuf peerbox, xepoch, packcnt, xticket;
     bool ghosts_binned = false;   // the ghost exchange kernel has already put the received ghosts into the tile lists
-    // Measured on 2 x B200 (8192^2 split in two strips): taking the fixed-point maxima inside their consumer kernels is
-    // SLOWER than the separate one-block exchange kernels (451 against 496 M star-steps/s: every block of the consumer polls
-    // the mailbox line the peer is writing), binning the ghosts in the exchange kernel is neutral and saves a launch.
-    bool fuse_max = false, fuse_bin = true;   // SRHMC_PEER_FUSE_MAX=1 / SRHMC_PEER_FUSE_BIN=0 switch them
-    // Producer-side fusion (SRHMC_PEER_FUSE_PROD=0 switches it off): the kernel that produces a fixed-point count all-reduces
-    // it in its last block, the position-update kernel counts the boundary stars, and packing + ghost exchange + ghost
-    // binning are one kernel: 5 kernels per leapfrog step on N ranks instead of 9.
-    bool fuse_prod = true;
+    // With peer exchange the kernel that produces a fixed-point count all-reduces it in its last block, the position-update
+    // kernel counts the boundary stars, and packing + ghost exchange + ghost binning are one kernel: 5 kernels per leapfrog
+    // step on N ranks.
     bool pack_counted = false;   // big_qfix_kick_kernel has left this step's chunk counts in packcnt
     PeerPtrs peers{};
     void* ipc_opened[kMaxWorld] = {};
@@ -1035,7 +943,6 @@ struct srhmc_big {
     BBuf D32;
     CUtensorMap tmapD32{};
     bool tma = false;          // a tensor map over the data window exists: the tile kernels load their tile by TMA
-    bool tile2 = false;        // persistent variant (big_tile2_kernel, SRHMC_TILE_V2=1) instead of one CTA per tile
     bool L_filled = false;     // star-parallel path: the position-update kernel has already reset the model image
     int star_mode = -1;        // gradient-only FP64 evaluations by big_star_kernel: -1 = when the tile lists are short (sparse
                                // field), 0 = never, 1 = always (SRHMC_BIG_STAR)
@@ -1152,23 +1059,8 @@ int srhmc_big_create(const srhmc_big_config* cfg, srhmc_big** out) {
     }
     if (!rc && b->use_tiles) {
         // 2-D tensor map over the FP64 data window [nrows, C] with 64 x 64 boxes for the TMA tile loads
-        bool want = (cfg->cols % 2) == 0;   // global row stride must be a multiple of 16 bytes
-        if (const char* e = std::getenv("SRHMC_TILE_TMA"))
-            if (e[0] == '0') want = false;   // A/B: cp.async staging
-        // Measured on 8192^2 / 1e5 stars: one CTA per tile 323 M star-steps/s, persistent variant 308 -- the persistent
-        // kernel is kept selectable, the default is the faster one.
-        bool want2 = false;
-        if (const char* e = std::getenv("SRHMC_TILE_V2")) want2 = e[0] == '1';
-        if (want) {
-            b->tma = encode_tile_map(&b->tmapD, b->D.ptr, cfg->nrows, cfg->cols, 8);
-            b->tile2 = b->tma && want2;
-            if (b->tile2 &&
-                (cudaFuncSetAttribute(big_tile2_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Tile2Smem)) != cudaSuccess ||
-                 cudaFuncSetAttribute(big_tile2_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Tile2Smem)) != cudaSuccess)) {
-                cudaGetLastError();
-                b->tile2 = false;
-            }
-        }
+        // (global row stride must be a multiple of 16 bytes; otherwise, or without the driver's encoder, cp.async staging)
+        if ((cfg->cols % 2) == 0) b->tma = encode_tile_map(&b->tmapD, b->D.ptr, cfg->nrows, cfg->cols, 8);
     }
     rc |= b->q.ensure(S * 8); rc |= b->p.ensure(S * 8); rc |= b->g.ensure(S * 8);
     rc |= b->a1.ensure(S * 8); rc |= b->a2.ensure(S * 8 + (size_t)cfg->max_stars * 4 + 8);
@@ -1424,10 +1316,6 @@ int srhmc_big_comm_import(srhmc_big* b, const void* ipc_handles, void* const* ra
         }
     }
     b->peer_enabled = true;
-    if (const char* e = std::getenv("SRHMC_PEER_FUSE_MAX")) b->fuse_max = e[0] == '1';
-    if (const char* e = std::getenv("SRHMC_PEER_FUSE_BIN")) b->fuse_bin = e[0] != '0';
-    if (const char* e = std::getenv("SRHMC_PEER_FUSE_PROD")) b->fuse_prod = e[0] != '0';
-    if (b->fuse_max || !b->fuse_bin) b->fuse_prod = false;
     BCU(cudaMemset(b->packcnt.ptr, 0, b->packcnt.cap));
     return 0;
 }
@@ -1526,10 +1414,9 @@ int srhmc_big_phase(srhmc_big* b, int32_t phase, const srhmc_big_step* s) {
     PeerX X;
     std::memset(&X, 0, sizeof(X));
     const bool peer_multi = b->peer_enabled && b->world > 1;
-    if (peer_multi && (b->fuse_max || b->fuse_prod)) {
+    if (peer_multi) {
         X.peers = b->peers; X.rank = b->rank; X.world = b->world;
-        X.on = b->fuse_max ? 1 : 0;
-        X.prod = b->fuse_prod ? 1 : 0;
+        X.prod = 1;
         X.epoch = b->xepoch.as<unsigned long long>(); X.ticket = b->xticket.as<unsigned int>(); X.err = b->err.as<int>();
     }
     // per-star stop rule: the whole advance between two evaluations in one kernel (big_perstar_kernel)
@@ -1538,14 +1425,13 @@ int srhmc_big_phase(srhmc_big* b, int32_t phase, const srhmc_big_step* s) {
             BCU(cudaMemsetAsync(b->tcnt.ptr, 0, (size_t)b->nty * b->ntx * 4, st));
             b->ghosts_binned = false;
         }
-        const bool count_here = peer_multi && b->fuse_prod;
-        if (count_here && b->pack_counted) BCU(cudaMemsetAsync(b->packcnt.ptr, 0, b->packcnt.cap, st));
+        if (peer_multi && b->pack_counted) BCU(cudaMemsetAsync(b->packcnt.ptr, 0, b->packcnt.cap, st));
         const double reach_k = (double)(b->cfg.nrows_halo + P.rad + 1);
         const double lo_edge_k = (b->rank > 0) ? (double)P.own_lo + reach_k : -1e300;
         const double hi_edge_k = (b->rank < b->world - 1) ? (double)P.own_hi - reach_k : 1e300;
         int* tc = b->use_tiles ? b->tcnt.as<int>() : nullptr;
         PairRec* tl = b->use_tiles ? b->tlist.as<PairRec>() : nullptr;
-        int2* pc = count_here ? b->packcnt.as<int2>() : nullptr;
+        int2* pc = peer_multi ? b->packcnt.as<int2>() : nullptr;
         double* lf = (!b->use_tiles && n > 0) ? b->L.as<double>() : nullptr;
         if (from_eval)
             big_perstar_kernel<true><<<gs, tb, 0, st>>>(P, S, n, b->q.as<double>(), b->p.as<double>(), b->g.as<double>(), gpart_in,
@@ -1554,7 +1440,7 @@ int srhmc_big_phase(srhmc_big* b, int32_t phase, const srhmc_big_step* s) {
             big_perstar_kernel<false><<<gs, tb, 0, st>>>(P, S, n, b->q.as<double>(), b->p.as<double>(), b->g.as<double>(), nullptr,
                                                          b->ntx, tc, tl, b->err.as<int>(), pc, lo_edge_k, hi_edge_k, lf, npix);
         b->L_filled = lf != nullptr;
-        b->pack_counted = count_here;
+        b->pack_counted = peer_multi;
         b->own_binned = b->use_tiles;
         b->launches += 1;
         return 0;
@@ -1569,7 +1455,7 @@ int srhmc_big_phase(srhmc_big* b, int32_t phase, const srhmc_big_step* s) {
             const double lo_edge = (b->rank > 0) ? (double)P.own_lo + reach : -1e300;
             const double hi_edge = (b->rank < b->world - 1) ? (double)P.own_hi - reach : 1e300;
             const int pb = std::max(1, (n + kPackChunk - 1) / kPackChunk);
-            if (peer_multi && b->fuse_prod) {
+            if (peer_multi) {
                 if (!b->pack_counted) {   // a PACK that does not follow a position update (first evaluation of a run)
                     big_pack_count_kernel<<<pb, 256, 0, st>>>(n, b->q.as<double>(), lo_edge, hi_edge, b->packcnt.as<int2>());
                     b->launches += 1;
@@ -1591,15 +1477,6 @@ int srhmc_big_phase(srhmc_big* b, int32_t phase, const srhmc_big_step* s) {
             big_pack_kernel<<<pb, 256, 0, st>>>(n, b->q.as<double>(), lo_edge, hi_edge, b->packcnt.as<int2>(), b->send.as<double>(),
                                                  std::max(1, b->cfg.max_ghosts), b->err.as<int>());
             b->launches += 2;
-            if (b->peer_enabled && b->world > 1) {  // the exchange itself: our own kernel over peer memory
-                // ... which also puts the received ghosts into the tile lists (no separate binning kernel before the evaluation)
-                big_xchg_ghost_kernel<<<1, 256, 0, st>>>(b->peers, b->rank, b->world, b->send.as<double>(), b->recv.as<double>(), list,
-                                                         b->xepoch.as<unsigned long long>(), b->err.as<int>(), P, b->ntx, n,
-                                                         std::max(1, b->cfg.max_ghosts), (b->use_tiles && b->fuse_bin) ? b->tcnt.as<int>() : nullptr,
-                                                         b->use_tiles ? b->tlist.as<PairRec>() : nullptr);
-                b->ghosts_binned = b->use_tiles && b->fuse_bin;
-                b->launches += 1;
-            }
             break;
         }
         case SRHMC_BIG_EVAL:
@@ -1635,20 +1512,6 @@ int srhmc_big_phase(srhmc_big* b, int32_t phase, const srhmc_big_step* s) {
                 if (b->precision == 32 && !want_V) {
                     big_tile32_kernel<<<ntiles, kTileThreads, sizeof(TileSmemF), st>>>(P, S, b->ntx, b->tcnt.as<int>(), b->tlist.as<PairRec>(),
                                                                                        b->gpart.as<double>(), cnt, b->tmapD32);
-                } else if (b->tile2) {
-                    int grid2 = std::min(ntiles, 4 * b->sm_count);   // persistent: 4 CTAs per SM walk the tiles
-                    if (const char* e = std::getenv("SRHMC_TILE_GRID")) {   // experiments: CTAs per SM, 0 = one CTA per tile
-                        const int k = std::atoi(e);
-                        grid2 = k <= 0 ? ntiles : std::min(ntiles, k * b->sm_count);
-                    }
-                    if (want_V)
-                        big_tile2_kernel<true><<<grid2, kTileThreads, sizeof(Tile2Smem), st>>>(P, S, b->tmapD, b->ntx, ntiles, b->tcnt.as<int>(),
-                            b->tlist.as<PairRec>(), b->gpart.as<double>(), b->vpart.as<double>(), b->tickets.as<unsigned int>() + 1,
-                            b->scalars.as<double>(), cnt);
-                    else
-                        big_tile2_kernel<false><<<grid2, kTileThreads, sizeof(Tile2Smem), st>>>(P, S, b->tmapD, b->ntx, ntiles, b->tcnt.as<int>(),
-                            b->tlist.as<PairRec>(), b->gpart.as<double>(), b->vpart.as<double>(), b->tickets.as<unsigned int>() + 1,
-                            b->scalars.as<double>(), cnt);
                 } else if (!want_V && n > 0 && P.rad <= 15 &&
                            (b->star_mode == 1 || (b->star_mode < 0 && 2.0 * n <= 3.0 * ntiles))) {
                     // very sparse field (mean tile list below ~1.5 records): one warp per owned star, neighbours from the tile lists
@@ -1715,40 +1578,29 @@ int srhmc_big_phase(srhmc_big* b, int32_t phase, const srhmc_big_step* s) {
             b->launches += 1;
             break;
         case SRHMC_BIG_PFIX_QFIX:
-            if (peer_multi && !b->fuse_max && !b->fuse_prod && !S.per_star) {
-                big_xchg_small_kernel<<<1, 32, 0, st>>>(b->peers, b->rank, b->world, 0, 2, cnt, nullptr, nullptr,
-                                                        b->xepoch.as<unsigned long long>(), b->err.as<int>());
-                b->launches += 1;
-            }
             // tiled over peers: the field-wide maximum of the p fixed-point counts was all-reduced by the last block of the
-            // kernel that produced it (fuse_prod), or is taken inside this kernel (fuse_max), or by the exchange kernel above
+            // kernel that produced it
             big_pfix_qfix_kernel<<<gs, tb, 0, st>>>(P, S, n, b->q.as<double>(), b->p.as<double>(), b->a1.as<double>(),
                                                     b->a2.as<double>(), cnt, cnt + 1, X);
             b->launches += 1;
             break;
         case SRHMC_BIG_QFIX_KICK: {
-            if (peer_multi && !b->fuse_max && !b->fuse_prod && !S.per_star) {
-                big_xchg_small_kernel<<<1, 32, 0, st>>>(b->peers, b->rank, b->world, 0, 2, cnt, nullptr, nullptr,
-                                                        b->xepoch.as<unsigned long long>(), b->err.as<int>());
-                b->launches += 1;
-            }
             if (b->use_tiles && (b->own_binned || b->ghosts_binned)) {  // records nobody consumed (two position updates without an evaluation)
                 BCU(cudaMemsetAsync(b->tcnt.ptr, 0, (size_t)b->nty * b->ntx * 4, st));
                 b->ghosts_binned = false;
             }
-            const bool count_here = peer_multi && b->fuse_prod;
-            if (count_here && b->pack_counted)   // counts nobody consumed (two position updates without a PACK)
+            if (peer_multi && b->pack_counted)   // counts nobody consumed (two position updates without a PACK)
                 BCU(cudaMemsetAsync(b->packcnt.ptr, 0, b->packcnt.cap, st));
             const double reach_k = (double)(b->cfg.nrows_halo + P.rad + 1);
             const double lo_edge_k = (b->rank > 0) ? (double)P.own_lo + reach_k : -1e300;
             const double hi_edge_k = (b->rank < b->world - 1) ? (double)P.own_hi - reach_k : 1e300;
             big_qfix_kick_kernel<<<gs, tb, 0, st>>>(P, S, n, b->q.as<double>(), b->p.as<double>(), b->a1.as<double>(),
                                                     b->a2.as<double>(), cnt + 1, b->ntx, b->use_tiles ? b->tcnt.as<int>() : nullptr,
-                                                    b->use_tiles ? b->tlist.as<PairRec>() : nullptr, b->err.as<int>(), X,
-                                                    count_here ? b->packcnt.as<int2>() : nullptr, lo_edge_k, hi_edge_k,
+                                                    b->use_tiles ? b->tlist.as<PairRec>() : nullptr, b->err.as<int>(),
+                                                    peer_multi ? b->packcnt.as<int2>() : nullptr, lo_edge_k, hi_edge_k,
                                                     (!b->use_tiles && n > 0) ? b->L.as<double>() : nullptr, npix);
             b->L_filled = !b->use_tiles && n > 0;
-            b->pack_counted = count_here;
+            b->pack_counted = peer_multi;
             b->own_binned = b->use_tiles;
             b->launches += 1;
             break;
@@ -1779,7 +1631,7 @@ int srhmc_big_phase(srhmc_big* b, int32_t phase, const srhmc_big_step* s) {
             if (b->world == 1) {
                 BCU(cudaMemcpyAsync(b->gscalars.ptr, b->scalars.ptr, kScalars * 8, cudaMemcpyDeviceToDevice, st));
             } else if (b->peer_enabled) {  // sum of the energy partials over the ranks, in rank order on every rank
-                big_xchg_small_kernel<<<1, 32, 0, st>>>(b->peers, b->rank, b->world, 1, kScalars, nullptr, b->scalars.as<double>(),
+                big_xchg_small_kernel<<<1, 32, 0, st>>>(b->peers, b->rank, b->world, kScalars, b->scalars.as<double>(),
                                                         b->gscalars.as<double>(), b->xepoch.as<unsigned long long>(), b->err.as<int>());
                 b->launches += 1;
             }

@@ -218,15 +218,16 @@ __device__ __forceinline__ void tma_load_2d(void* dst, const void* tmap, int x, 
     asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
                  ::"r"(smem_u32(dst)), "l"(tmap), "r"(smem_u32(bar)), "r"(x), "r"(y) : "memory");
 }
-__device__ __forceinline__ void tma_prefetch_l2_2d(const void* tmap, int x, int y) {
-    asm volatile("cp.async.bulk.prefetch.tensor.2d.L2.global [%0, {%1, %2}];" ::"l"(tmap), "r"(x), "r"(y) : "memory");
-}
 __device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 
 // 16-byte asynchronous copy global -> shared (LDGSTS): no registers held while the data are in flight
 __device__ __forceinline__ void cp_async16(void* smem, const void* gmem) {
     const unsigned s = (unsigned)__cvta_generic_to_shared(smem);
     asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(s), "l"(gmem) : "memory");
+}
+// 8-byte asynchronous copy global -> shared
+__device__ __forceinline__ void cp_async8(void* smem, const void* gmem) {
+    asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(smem_u32(smem)), "l"(gmem) : "memory");
 }
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
 __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_group 0;" ::: "memory"); }
@@ -640,318 +641,6 @@ big_tile32_kernel(const BigParams P, const TileSrc S, int ntx, int* __restrict__
 
 __global__ void big_to_float_kernel(const double* __restrict__ src, float* __restrict__ dst, size_t n) {
     for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) dst[i] = (float)src[i];
-}
-
-// ------------------------------------------------------------------------------------------------ persistent TMA variant
-// Same sums per tile as big_tile_kernel<0|1> (fixed summation orders: results are bit-reproducible run to run),
-// reorganised for Blackwell:
-//   * the grid is persistent (4 CTAs per SM), each CTA walks tiles blockIdx.x, blockIdx.x + gridDim.x, ...;
-//   * the 64x64 FP64 data tile arrives by TMA (cp.async.bulk.tensor.2d -> the shared rho buffer, completion on an
-//     mbarrier; tiles cut by the image edge are zero-filled by the copy engine) while the CTA builds tables and renders;
-//     the NEXT tile's data are prefetched into L2 at the same time;
-//   * the next tile's pair list is fetched during the current tile (count at its start, records behind the render, star
-//     records behind the residual), so the three dependent L2 round trips that used to open every CTA are hidden;
-//   * the list is ranked from shared memory (no nl^2 global loads), the gather takes two pairs per warp trip with one
-//     16-byte residual load + one {ex, ex dx} load per row for 4 FMAs, the reciprocal of Lambda is seeded in FP32.
-constexpr int kT2List = 96;     // sorted records held in shared memory per pass (denser tiles take several passes)
-constexpr int kT2Chunk = 16;    // table slots: render chunk = 16 pairs; the gather uses slots 2 warp, 2 warp + 1
-
-struct PairTab2 {
-    double2 rowp[kTabLen];      // {ex, ex dx} of row ia + k at [kTabPad + k]; zero outside the box
-    double colf[kTabLen];       // f ey / (2 pi s^2) of column ja + k at [kTabPad + k]; zero outside the box
-    double dy0, pad;
-};
-
-struct Tile2Smem {
-    double rho[kTile][kTile];               // 32 KB, TMA destination (128-byte aligned: first member)
-    PairTab2 tab[kT2Chunk];
-    PairRec list[2][kT2List];               // records of the current / the next tile, in arrival order
-    unsigned char order[2][kT2List];        // order[b][r] = index in list[b] of the record with the r-th smallest star id
-    int box[kT2Chunk][4];
-    double red[32];
-    double2 ltab[kLogTableSize];
-    unsigned long long mbar;
-    int nl[2];                              // list lengths of the current / the next tile (capped)
-    bool is_last;
-};
-
-// 1/a for a in the float range: FP32 seed (MUFU.RCP) + two Newton steps in FP64 (2^-23 -> 2^-46 -> 2^-92 before rounding)
-__device__ __forceinline__ double rcp_seed32(double a) {
-    float xf;
-    asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(xf) : "f"((float)a));
-    const double x0 = (double)xf;
-    const double x1 = fma(x0, fma(-a, x0, 1.0), x0);
-    return fma(x1, fma(-a, x1, 1.0), x1);
-}
-
-__device__ __forceinline__ void build_pair_tab2(const BigParams& P, const PairRec& rec, int r0, int c0, int lane, PairTab2& T,
-                                                int* box) {
-    const int ia = rec.box & 63, ib = (rec.box >> 6) & 63, ja = (rec.box >> 12) & 63, jb = (rec.box >> 18) & 63;
-    const double dx = ((double)(r0 + ia + lane) + 0.5) - rec.x, dy = ((double)(c0 + ja + lane) + 0.5) - rec.y;
-    const double e = (ia + lane <= ib) ? exp_neg(-(dx * dx) * P.inv2s2) : 0.0;
-    T.rowp[kTabPad + lane] = make_double2(e, e * dx);
-    T.colf[kTabPad + lane] = (ja + lane <= jb) ? exp_neg(-(dy * dy) * P.inv2s2) * (P.norm * rec.f) : 0.0;
-    if (lane == 0) {
-        T.dy0 = dy;
-        if (box) {
-            box[0] = ia; box[1] = ib; box[2] = ja; box[3] = jb;
-        }
-    }
-}
-
-// 8-byte asynchronous copy global -> shared
-__device__ __forceinline__ void cp_async8(void* smem, const void* gmem) {
-    asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(smem_u32(smem)), "l"(gmem) : "memory");
-}
-
-#ifndef SRHMC_T2_RCP
-#define SRHMC_T2_RCP rcp_fast   // measured: 305 M star-steps/s against 301 with the FP32-seeded rcp_seed32
-#endif
-
-template <bool WANT_V>
-__global__ void __launch_bounds__(kTileThreads, 4)
-big_tile2_kernel(const BigParams P, const TileSrc S, const __grid_constant__ CUtensorMap tmapD, int ntx, int ntiles,
-                 int* __restrict__ cnt, const PairRec* __restrict__ glist, double* __restrict__ gpart, double* vpart,
-                 unsigned int* ticket, double* scalars, int* fp_counters) {
-    extern __shared__ __align__(128) unsigned char tile2_smem_raw[];
-    Tile2Smem& sm = *reinterpret_cast<Tile2Smem*>(tile2_smem_raw);
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    constexpr int kWarps = kTileThreads / 32;
-
-    if (tid == 0) mbar_init(&sm.mbar, 1);
-    if (fp_counters && blockIdx.x == 0 && tid < 2) fp_counters[tid] = 0;
-    for (int k = tid; k < kT2Chunk * 4 * kTabPad; k += kTileThreads) {   // table guards stay zero for the whole launch
-        const int pair = k / (4 * kTabPad), e = k % (4 * kTabPad), side = e / kTabPad, g = e % kTabPad;
-        const int at = (side & 2) ? kTabPad + 32 + g : g;
-        if (side & 1) sm.tab[pair].colf[at] = 0.0; else sm.tab[pair].rowp[at] = make_double2(0.0, 0.0);
-    }
-    if (WANT_V && tid < kLogTableSize) {
-        const double rc = 1.0 / (1.0 + ((double)tid + 0.5) / (double)kLogTableSize);
-        sm.ltab[tid] = make_double2(rc, -log(rc));
-    }
-
-    // The three dependent trips that fetch a tile's pair list, each asynchronous (global -> shared, no registers held):
-    //   fetch_records: (star id, box) of record tid;  fetch_stars: (f, x, y) of that star, once the id has landed;
-    //   rank_list: order[] by star id (fixed summation order).  Lists longer than kT2List go pass by pass (dense_pass).
-    auto fetch_records = [&](int buf, int nl, const PairRec* gl) {
-        if (nl <= kT2List && tid < nl) {   // the whole 32-byte record (id, box, star) in two 16-byte asynchronous copies
-            cp_async16(&sm.list[buf][tid], &gl[tid]);
-            cp_async16(reinterpret_cast<char*>(&sm.list[buf][tid]) + 16, reinterpret_cast<const char*>(&gl[tid]) + 16);
-        }
-        cp_async_commit();
-    };
-    auto fetch_stars = [&](int buf, int nl) {   // nothing left to fetch: the records carry (f, x, y)
-        (void)buf; (void)nl;
-    };
-    auto rank_list = [&](int buf, int nl) {   // after a barrier that follows every thread's cp_async_wait_all
-        if (nl <= kT2List && tid < nl) {
-            const int mine = sm.list[buf][tid].sid;
-            int r = 0;
-            for (int m = 0; m < nl; ++m) r += sm.list[buf][m].sid < mine;
-            sm.order[buf][r] = (unsigned char)tid;
-        }
-        if (tid == 0) sm.nl[buf] = nl;
-    };
-    auto dense_pass = [&](int buf, int nl_total, int base, const PairRec* gl) {
-        // dense tile: every record is ranked against the whole global list; this pass keeps ranks [base, base + kT2List)
-        for (int k = tid; k < nl_total; k += kTileThreads) {
-            const int mine = __ldcg(&gl[k].sid);
-            int r = 0;
-            for (int m = 0; m < nl_total; ++m) r += __ldcg(&gl[m].sid) < mine;
-            if (r >= base && r < base + kT2List) {
-                sm.list[buf][r - base] = ld_rec(&gl[k]);
-                sm.order[buf][r - base] = (unsigned char)(r - base);
-            }
-        }
-    };
-
-    int tile = blockIdx.x;
-    int cur = 0;
-    unsigned phase = 0;
-    // prologue: the first tile's list (latency exposed once per CTA)
-    if (tile < ntiles) {
-        const int nl0 = min(__ldcg(&cnt[tile]), kTileMaxList);
-        const PairRec* gl = glist + (size_t)tile * kTileMaxList;
-        fetch_records(cur, nl0, gl);
-        fetch_stars(cur, nl0);
-        cp_async_wait_all();
-        __syncthreads();   // guards / mbarrier / records visible; every thread has read cnt[tile]
-        rank_list(cur, nl0);
-        if (tid == 0) cnt[tile] = 0;
-    }
-    for (; tile < ntiles; tile += gridDim.x) {
-        const int ti = tile / ntx, tj = tile % ntx;
-        const int r0 = P.row0 + ti * kTile, c0 = tj * kTile;  // global pixel of the tile origin
-        const int next = tile + gridDim.x;
-        const bool has_next = next < ntiles;
-        __syncthreads();   // order[cur] published; every reader of rho (previous gather) is done
-        const int nl_total = sm.nl[cur];
-        if (tid == 0) {
-            fence_proxy_async_smem();   // generic-proxy accesses of rho (previous tile) before the async-proxy write
-            mbar_expect_tx(&sm.mbar, kTile * kTile * 8);
-            tma_load_2d(&sm.rho[0][0], &tmapD, c0, r0 - P.row0, &sm.mbar);
-            if (has_next) tma_prefetch_l2_2d(&tmapD, (next % ntx) * kTile, (next / ntx) * kTile);
-        }
-        // the next tile's count: every thread reads it (one broadcast L2 load per warp), first used behind the render
-        int nl_next_raw = 0;
-        if (has_next) asm volatile("ld.global.cg.s32 %0, [%1];" : "=r"(nl_next_raw) : "l"(cnt + next));   // consumed after the render
-
-        const int ty = tid >> 4, tx = tid & 15;
-        const int pr = 4 * ty, pc = 4 * tx;  // thread owns the 4x4 pixel block at (pr, pc)
-        // ---- passes over the ordered list (one pass unless more than kT2List stars touch the tile)
-        double lam[4][4];
-#pragma unroll
-        for (int a = 0; a < 4; ++a)
-#pragma unroll
-            for (int b = 0; b < 4; ++b) lam[a][b] = P.F.B;
-        const int npass = nl_total > kT2List ? (nl_total + kT2List - 1) / kT2List : 1;
-        for (int pass = 0; pass < npass; ++pass) {
-            const int base0 = pass * kT2List;
-            const int nl = min(kT2List, nl_total - base0);
-            if (npass > 1) {
-                __syncthreads();
-                dense_pass(cur, nl_total, base0, glist + (size_t)tile * kTileMaxList);
-                __syncthreads();
-            }
-            for (int base = 0; base < nl; base += kT2Chunk) {
-                const int nc = min(kT2Chunk, nl - base);
-                for (int s = warp; s < nc; s += kWarps)
-                    build_pair_tab2(P, sm.list[cur][sm.order[cur][base + s]], r0, c0, lane, sm.tab[s], sm.box[s]);
-                __syncthreads();
-                for (int s = 0; s < nc; ++s) {
-                    const int ia = sm.box[s][0], ja = sm.box[s][2];
-                    if (pr + 3 < ia || pr > sm.box[s][1] || pc + 3 < ja || pc > sm.box[s][3]) continue;
-                    const double2* te = &sm.tab[s].rowp[kTabPad + pr - ia];  // pr - ia in [-3, 31]: inside the padded table
-                    const double* tf = &sm.tab[s].colf[kTabPad + pc - ja];
-                    const double ex[4] = {te[0].x, te[1].x, te[2].x, te[3].x}, fy[4] = {tf[0], tf[1], tf[2], tf[3]};
-#pragma unroll
-                    for (int a = 0; a < 4; ++a)
-#pragma unroll
-                        for (int b = 0; b < 4; ++b) lam[a][b] = fma(ex[a], fy[b], lam[a][b]);
-                }
-                if (base + kT2Chunk < nl || pass + 1 < npass) __syncthreads();  // the tables are rewritten by the next chunk
-            }
-        }
-        // ---- next tile's records: first trip, in flight behind the residual
-        const int nl_next = min(nl_next_raw, kTileMaxList);
-        if (has_next) fetch_records(cur ^ 1, nl_next, glist + (size_t)next * kTileMaxList);
-
-        // ---- residual into the shared tile; pixel potential of the owned rows
-        mbar_wait(&sm.mbar, phase);
-        phase ^= 1u;
-        {
-            const int vr = min(kTile, P.row0 + P.nrows - r0), vc = min(kTile, P.C - c0);   // valid rows / columns
-            double v = 0.0;
-#pragma unroll
-            for (int a = 0; a < 4; ++a) {
-                const int li = pr + a, gi = r0 + li;
-                const bool own = WANT_V && li < vr && gi >= P.own_lo && gi < P.own_hi;
-                const double2 d0 = *reinterpret_cast<const double2*>(&sm.rho[li][pc]);
-                const double2 d1 = *reinterpret_cast<const double2*>(&sm.rho[li][pc + 2]);
-                const double d[4] = {d0.x, d0.y, d1.x, d1.y};
-                double rho[4];
-#pragma unroll
-                for (int b = 0; b < 4; ++b) {
-                    const bool in = li < vr && pc + b < vc;
-                    rho[b] = in ? fma(d[b], SRHMC_T2_RCP(lam[a][b]), -1.0) : 0.0;
-                    if (WANT_V && own && pc + b < vc) v += lam[a][b] - d[b] * (lam[a][b] >= 2.3e-308 ? log_pos(lam[a][b], sm.ltab) : CUDART_NAN);
-                }
-                *reinterpret_cast<double2*>(&sm.rho[li][pc]) = make_double2(rho[0], rho[1]);
-                *reinterpret_cast<double2*>(&sm.rho[li][pc + 2]) = make_double2(rho[2], rho[3]);
-            }
-            if (WANT_V) {
-                double a1[1] = {v};
-                block_sum<1>(a1, sm.red);
-                if (tid == 0) vpart[tile] = a1[0];
-            }
-        }
-        // second trip of the next list (star records), in flight behind the gather
-        if (has_next) fetch_stars(cur ^ 1, nl_next);
-        __syncthreads();
-
-        // ---- gather: two owned pairs per warp trip, one per half-warp; lane hl owns the columns jae + 2 hl, jae + 2 hl + 1
-        //      (jae = ja rounded down to even: 16-byte aligned residual pairs)
-        for (int pass = npass - 1; pass >= 0; --pass) {
-            // multi-pass lists: the last render pass is still in shared memory, earlier ones are fetched again
-            const int base0 = pass * kT2List;
-            const int nl = min(kT2List, nl_total - base0);
-            if (pass != npass - 1) {
-                __syncthreads();
-                dense_pass(cur, nl_total, base0, glist + (size_t)tile * kTileMaxList);
-                __syncthreads();
-            }
-            const bool keep = npass == 1 && nl <= kT2Chunk;   // the render's tables are still valid
-            const int half = lane >> 4, hl = lane & 15;
-            for (int s0 = 2 * warp; s0 < nl; s0 += 2 * kWarps) {
-                const int s = min(s0 + half, nl - 1);
-                const bool live = s0 + half < nl;
-                const PairRec& rec = sm.list[cur][sm.order[cur][s]];
-                PairTab2& T = sm.tab[keep ? s : 2 * warp + half];
-                if (!keep) {
-                    __syncwarp();
-                    build_pair_tab2(P, sm.list[cur][sm.order[cur][min(s0, nl - 1)]], r0, c0, lane, sm.tab[2 * warp], nullptr);
-                    build_pair_tab2(P, sm.list[cur][sm.order[cur][min(s0 + 1, nl - 1)]], r0, c0, lane, sm.tab[2 * warp + 1], nullptr);
-                    __syncwarp();
-                }
-                const int ia = rec.box & 63, ib = (rec.box >> 6) & 63, ja = (rec.box >> 12) & 63;
-                const int jae = ja & ~1;
-                const int cofs = min(2 * hl + (jae - ja), 27);            // column index relative to ja: -1 .. 27 (zero guards)
-                const double fy0 = T.colf[kTabPad + cofs], fy1 = T.colf[kTabPad + cofs + 1];
-                const int col = min(jae + 2 * hl, kTile - 2);
-                const double2* rp = &T.rowp[kTabPad];
-                const double* rho = &sm.rho[ia][col];
-                double a0 = 0.0, a1 = 0.0, b0 = 0.0, b1 = 0.0;
-                const int nr = (live && rec.sid < S.n_own) ? ib - ia + 1 : 0;   // ghosts are rendered only
-#pragma unroll 4
-                for (int k = 0; k < nr; ++k) {
-                    const double2 e = rp[k];
-                    const double2 w = *reinterpret_cast<const double2*>(rho + k * kTile);
-                    a0 = fma(w.x, e.x, a0);
-                    a1 = fma(w.x, e.y, a1);
-                    b0 = fma(w.y, e.x, b0);
-                    b1 = fma(w.y, e.y, b1);
-                }
-                const double dyl = T.dy0 + (double)cofs;
-                double sf = fy0 * a0 + fy1 * b0;
-                double sx = fy0 * a1 + fy1 * b1;
-                double sy = (fy0 * dyl) * a0 + (fy1 * (dyl + 1.0)) * b0;
-                if (2 * hl + (jae - ja) > 26) sf = sx = sy = 0.0;   // lanes past the box read a clamped column
-                const bool h8 = hl & 8;
-                const double k0 = h8 ? sy : sf, k1 = h8 ? 0.0 : sx, t0 = h8 ? sf : sy, t1 = h8 ? sx : 0.0;
-                const double x0 = k0 + __shfl_xor_sync(0xffffffffu, t0, 8), x1 = k1 + __shfl_xor_sync(0xffffffffu, t1, 8);
-                const bool h4 = hl & 4;
-                double yv = (h4 ? x1 : x0) + __shfl_xor_sync(0xffffffffu, h4 ? x0 : x1, 4);
-                yv += __shfl_xor_sync(0xffffffffu, yv, 2);
-                yv += __shfl_xor_sync(0xffffffffu, yv, 1);
-                // lanes 0-3 of the half: sum sf, 4-7: sum sx, 8-11: sum sy
-                if (nr > 0 && (hl & 3) == 0 && hl < 12) gpart[((size_t)rec.sid * 4 + (rec.box >> 24)) * 3 + (hl >> 2)] = yv;
-            }
-        }
-        cp_async_wait_all();   // own star records of the next list
-        __syncthreads();       // every reader of list[cur] / rho / tables is done; the next list is complete
-        // ---- third step: order the next tile's list
-        if (has_next) {
-            if (nl_next <= kT2List) {
-                rank_list(cur ^ 1, nl_next);
-            } else {
-                if (tid == 0) sm.nl[cur ^ 1] = nl_next;   // dense tile: its passes are fetched when it is processed
-            }
-            if (tid == 0) cnt[next] = 0;
-        }
-        cur ^= 1;
-    }
-    // ---- pixel potential: the last CTA to finish sums the per-tile partials in tile order -> scalars[0]
-    if (WANT_V) {
-        if (last_block_ticket(ticket, &sm.is_last)) {
-            double w[1] = {0.0};
-            for (int b = tid; b < ntiles; b += kTileThreads) w[0] += __ldcg(vpart + b);
-            block_sum<1>(w, sm.red);
-            if (tid == 0) {
-                scalars[0] = w[0];
-                *ticket = 0u;
-            }
-        }
-    }
 }
 
 // g = scaled sum of the footprint slots of star k, in slot order (sampler_RHMC.py:404-406)

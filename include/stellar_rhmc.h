@@ -389,11 +389,11 @@ int srhmc_big_buffers(srhmc_big* b, srhmc_big_buffers_t* out);
  * between the GPUs of one node) instead of by the caller.  Every rank exports its mailbox (a 64-byte CUDA IPC handle for
  * other processes and/or the raw device pointer for strips hosted by the same process), the caller distributes the
  * handles (any transport: they are plain bytes) and every rank imports all `world_size` of them (ipc_handles: world x 64
- * bytes, or raw_ptrs: world pointers; the own entry is ignored).  From then on PFIX_QFIX and QFIX_KICK all-reduce(max) the
- * fixed-point counters themselves, PACK also delivers the boundary lists into the neighbours' ghost_recv, and RECORD_E0 /
- * ACCEPT sum the scalars over the ranks (rank order, identical on every rank): the caller issues no collective, and a
- * captured CUDA graph of an iteration can be replayed on every rank.  A peer that never arrives raises error flag 4
- * after ~10 s instead of hanging the device. */
+ * bytes, or raw_ptrs: world pointers; the own entry is ignored).  From then on the phases that produce the fixed-point
+ * counters (KICK1, PFIX_QFIX, EVAL_KICK2_KICK1) all-reduce(max) them themselves, PACK also delivers the boundary lists
+ * into the neighbours' ghost_recv, and RECORD_E0 / ACCEPT sum the scalars over the ranks (rank order, identical on every
+ * rank): the caller issues no collective, and a captured CUDA graph of an iteration can be replayed on every rank.  A peer
+ * that never arrives raises error flag 4 after ~10 s instead of hanging the device. */
 int srhmc_big_comm_export(srhmc_big* b, void* ipc_handle_64 /* may be NULL */, void** raw_ptr /* may be NULL */);
 int srhmc_big_comm_import(srhmc_big* b, const void* ipc_handles, void* const* raw_ptrs);
 /* Parity mode: normals [n_iters, n, 3] for the owned stars and/or lnu [n_iters]; NULL -> device Philox (seed). */
