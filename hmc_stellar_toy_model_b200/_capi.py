@@ -216,6 +216,9 @@ SIGNATURES = {
                                         C.POINTER(C.c_double), C.POINTER(C.c_int32)]),
     "srhmc_big_read_scalars": (C.c_int, [C.c_void_p, c_double_p]),
     "srhmc_big_phase": (C.c_int, [C.c_void_p, C.c_int32, C.POINTER(BigStep)]),
+    "srhmc_big_set_recording": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32]),
+    "srhmc_big_read_samples": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, c_double_p, c_double_p]),
+    "srhmc_big_convergence_stats": (C.c_int, [C.POINTER(C.c_void_p), C.c_int32, C.c_int32, C.c_int32, c_double_p, c_double_p]),
 }
 
 

@@ -75,6 +75,29 @@ def ghost_mask(x, lo: int, hi: int, reach: int, rank: int, world: int):
     return to_lo, to_hi
 
 
+# ----------------------------------------------------------------------------------------------- sample rows
+def record_want(want):
+    """The chains a run records: a subset of ("q", "p") -> the canonical tuple (empty: recording off)."""
+    want = (want,) if isinstance(want, str) else tuple(want)
+    bad = set(want) - {"q", "p"}
+    if bad:
+        raise ValueError("want must be a subset of ('q', 'p'), got %r" % (sorted(bad),))
+    return tuple(w for w in ("q", "p") if w in want)
+
+
+def record_rows(n_iters: int, stride: int):
+    """Rows kept of n_iters iterations at chain_stride `stride`: ceil(n_iters / stride) (row r = iteration r * stride)."""
+    if stride < 1:
+        raise ValueError("chain_stride must be >= 1")
+    return -(-int(n_iters) // int(stride))
+
+
+def slot_ids(ids):
+    """Global ids of a strip's stars in slot order: the column order of its recorded rows and statistics (ascending id,
+    independent of the tile order the stars are stored in)."""
+    return np.sort(np.asarray(ids, dtype=np.int64))
+
+
 class _DevView:
     """Zero-copy torch view of a device buffer owned by the library."""
 
@@ -112,6 +135,7 @@ class BigFieldStrip:
         self._h = C.c_void_p()
         check(self._lib.srhmc_big_create(C.byref(cfg), C.byref(self._h)))
         self.n = 0
+        self.n_global = 0
         self.ids = np.zeros(0, dtype=np.int64)
         self._views = None
 
@@ -171,7 +195,7 @@ class BigFieldStrip:
         order = tile_order(q, self.cols)
         mine, q = mine[order], np.ascontiguousarray(q[order])
         check(self._lib.srhmc_big_set_stars(self._h, _capi.dptr(q), mine.ctypes.data_as(C.POINTER(C.c_int64)), len(mine)))
-        self.n, self.ids = len(mine), mine
+        self.n, self.ids, self.n_global = len(mine), mine, len(q_global)
 
     def get_stars(self):
         q, p, g = (np.zeros((self.n, 3)) for _ in range(3))
@@ -207,6 +231,19 @@ class BigFieldStrip:
         if err.value == 4:
             raise RuntimeError("peer exchange timed out: a rank of the tiling never delivered its contribution")
         return dict(E_chain=E, V_chain=V, T_chain=T, A_chain=A, n_accepted=float(nacc.value))
+
+    def set_recording(self, n_iters, stride=1, want=()):
+        """Record the sample rows of the coming run (see srhmc_big_set_recording); want=() turns recording off."""
+        want = record_want(want)
+        check(self._lib.srhmc_big_set_recording(self._h, int(n_iters), int(stride), int("q" in want), int("p" in want)))
+
+    def read_samples(self, row0, nrows, want=("q",)):
+        """{name: [nrows, n, 3]} of recorded rows [row0, row0 + nrows), stars in slot order (`slot_ids(self.ids)`)."""
+        want = record_want(want)
+        out = {w: np.empty((int(nrows), self.n, 3)) for w in want}
+        check(self._lib.srhmc_big_read_samples(self._h, int(row0), int(nrows), _capi.dptr(out.get("q")),
+                                               _capi.dptr(out.get("p"))))
+        return out
 
     def read_scalars(self):
         s = np.zeros(8)
@@ -457,18 +494,31 @@ class BigFieldRHMC:
         self._all("ACCEPT", st)
 
     def run(self, niter, nsteps, dt, delta=1e-6, counter_max=1000, f_pos=True, g_ff2=1.0, seed=0, normals=None, lnu=None,
-            schedule_g_ff2=None, use_graph=None):
+            schedule_g_ff2=None, use_graph=None, want=(), chain_stride=1):
         """Move-0 leg of multi_gym.run_RHMC (sampler_RHMC.py:1009-1083) for iterations 0..niter, all enqueued on
         the stream; `normals` [niter+1, N_global, 3] / `lnu` [niter+1] inject the reference's draws (parity mode),
         otherwise device Philox keyed by global star id.
+
+        want: a subset of ("q", "p"): the samples recorded on the device and returned as out["q_chain"] / out["p_chain"],
+        [ceil((niter+1) / chain_stride), N_global, 3] in global-id order, NaN for stars hosted elsewhere.  Row r is the state
+        at the start of iteration r * chain_stride (q before the trajectory, p as drawn), as in multi_gym.run_RHMC.  The
+        rows stay on the device for `convergence_stats` until the next run.
 
         use_graph: capture ONE Metropolis iteration (all its phases and, when tiled, its NCCL collectives) into a CUDA
         graph and replay it niter+1 times -- the chain row and RNG counter then come from a device-side iteration
         counter.  Default: on for an untiled field without a g_ff2 schedule."""
         L = niter + 1
+        want = record_want(want)
+        Ls = record_rows(L, chain_stride)
+        # a change of the recording set-up may move its buffers: no graph captured before it may be replayed after it
+        rec = (want, int(chain_stride), L, tuple(s.n for s in self.strips))
+        if rec != getattr(self, "_rec", None):
+            self._graph_key = None
         for s in self.strips:
             s.set_draws(None if normals is None else np.asarray(normals)[:, s.ids, :], lnu, L)
             s.alloc_chains(L)
+            s.set_recording(L, chain_stride, want)
+        self._rec = rec
         st0 = self._step_struct(dt, delta, g_ff2, counter_max, f_pos, 0, seed)
         if self.multi:
             self._all("PACK", st0)
@@ -495,7 +545,7 @@ class BigFieldRHMC:
             # one captured iteration serves every later run with the same launch parameters (the chain row and the RNG
             # counter come from the device-side iteration counter; the buffers are owned by the strips and never move)
             key = (int(nsteps), float(dt), float(delta), float(g_ff2), int(counter_max), bool(f_pos), int(seed), L,
-                   tuple(s.n for s in self.strips), int(getattr(self, "fixed_point_mode", 0)))
+                   tuple(s.n for s in self.strips), int(getattr(self, "fixed_point_mode", 0)), want, int(chain_stride))
             if normals is not None or lnu is not None:
                 key = None  # injected draws live in buffers that are re-allocated per run: always capture afresh
             if key is None or getattr(self, "_graph_key", None) != key:
@@ -526,6 +576,20 @@ class BigFieldRHMC:
         for s in self.strips[1:]:
             s.read_chains(L)  # synchronises and surfaces per-strip errors
         out["accept_rate"] = out["n_accepted"] / float(L)
+        for w in want:
+            out[w + "_chain"] = self._samples(w, Ls)
+        return out
+
+    def _samples(self, name, rows, chunk_bytes=256 << 20):
+        """Recorded rows of every strip hosted here in global-id order, downloaded in pieces of about `chunk_bytes`."""
+        n_global = self.strips[0].n_global
+        out = np.full((rows, n_global, 3), np.nan)
+        for s in self.strips:
+            cols = slot_ids(s.ids)
+            step = max(1, chunk_bytes // max(1, 24 * s.n))
+            for r0 in range(0, rows, step):
+                nr = min(step, rows - r0)
+                out[r0:r0 + nr, cols, :] = s.read_samples(r0, nr, (name,))[name]
         return out
 
     def energies(self):
@@ -543,3 +607,30 @@ class BigFieldRHMC:
             a, b, c = s.get_stars()
             q[s.ids], p[s.ids], g[s.ids] = a, b, c
         return q, p, g
+
+
+def convergence_stats(engines, thin_rate=5, warm_up_num=0):
+    """utils.convergence_stats (split-chain R-hat and n_eff, the reference's quirks kept) over the q rows that K >= 2 runs of
+    the same field recorded on the device (`run(..., want=("q",))`): each engine is one chain, all hosted on one device with
+    the same tiling and row count (different seeds or starts).  One variable-parallel kernel per strip; returns (R, n_eff),
+    each [N_global, 3] in global-id order, NaN for stars hosted by other processes."""
+    engines = list(engines)
+    if len(engines) < 2:
+        raise ValueError("convergence statistics need at least two chains (utils.py:94)")
+    nstrips = len(engines[0].strips)
+    if any(len(e.strips) != nstrips for e in engines):
+        raise ValueError("every chain must host the same strips")
+    n_global = engines[0].strips[0].n_global
+    R = np.full((n_global, 3), np.nan)
+    n_eff = np.full((n_global, 3), np.nan)
+    lib = _capi.load_library()
+    for i in range(nstrips):
+        strips = [e.strips[i] for e in engines]
+        s0 = strips[0]
+        handles = (C.c_void_p * len(strips))(*[s._h.value for s in strips])
+        r, ne = np.empty(3 * s0.n), np.empty(3 * s0.n)
+        check(lib.srhmc_big_convergence_stats(handles, len(strips), int(thin_rate), int(warm_up_num), _capi.dptr(r),
+                                              _capi.dptr(ne)))
+        cols = slot_ids(s0.ids)
+        R[cols], n_eff[cols] = r.reshape(-1, 3), ne.reshape(-1, 3)
+    return R, n_eff

@@ -30,9 +30,12 @@
 #include <cstdlib>
 #include <cstring>
 #include <new>
+#include <numeric>
+#include <vector>
 
 #include "../../include/stellar_rhmc.h"
 #include "common.cuh"
+#include "kernels_api.h"
 #include "fastmath.cuh"
 #include "poisson.cuh"
 
@@ -698,6 +701,23 @@ __global__ void big_restore_v_kernel(double* local_scalars, const double* state,
     if (iter_dev) *iter_dev += 1;  // the next replay of a captured iteration works on the next chain row
 }
 
+// Sample row of the iteration (RECORD_E0: q before the trajectory, p just drawn by MOMENTUM) when the iteration is a multiple of
+// the stride: row iter / stride, stars in ascending global-id order (slot = rank of the star's id within the strip), so the rows
+// do not depend on the storage order.  One thread per coordinate: coalesced reads, the three coordinates of a star together.
+__global__ void big_record_kernel(int n, const double* q, const double* p, const int* slot, int iter_host, const int* iter_dev,
+                                  int stride, int rows, double* rec_q, double* rec_p) {
+    const int iter = iter_dev ? *iter_dev : iter_host;
+    if (iter < 0 || iter % stride) return;
+    const int r = iter / stride;
+    if (r >= rows) return;
+    const size_t row = (size_t)r * 3 * n;
+    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < 3 * n; i += gridDim.x * blockDim.x) {
+        const size_t o = row + 3 * (size_t)slot[i / 3] + i % 3;
+        if (rec_q) rec_q[o] = q[i];
+        if (rec_p) rec_p[o] = p[i];
+    }
+}
+
 // boundary stars for the neighbours: list 0 = stars with x < lo_edge (for the rank below), list 1 = x >= hi_edge.
 // Layout per list: [0] = count, then triples.  Order follows the star index (deterministic): block b owns the stars
 // [b kPackChunk, (b+1) kPackChunk); a first kernel counts its matches, the second one starts at the sum of the counts of
@@ -937,6 +957,10 @@ struct srhmc_big {
     void* ipc_opened[kMaxWorld] = {};
     bool peer_enabled = false;  // the pair records of the owned stars' current positions are already in the tile lists
     BBuf epart, tickets;  // per-block energy partials; last-block tickets [0] energy, [1] tile potential
+    // sample recording (srhmc_big_set_recording): rows [rec_rows][n][3] of q and/or p in slot order, written at RECORD_E0
+    BBuf slot, recq, recp;
+    std::vector<int64_t> sorted_ids;   // the owned global ids in slot order (ascending)
+    int rec_rows = 0, rec_stride = 1, rec_n = 0;
     int nty = 0, ntx = 0;
     bool use_tiles = false;
     int precision = 64;        // 32: gradient-only evaluations run the FP32 tile kernel on a float copy of the data
@@ -1065,6 +1089,7 @@ int srhmc_big_create(const srhmc_big_config* cfg, srhmc_big** out) {
     rc |= b->q.ensure(S * 8); rc |= b->p.ensure(S * 8); rc |= b->g.ensure(S * 8);
     rc |= b->a1.ensure(S * 8); rc |= b->a2.ensure(S * 8 + (size_t)cfg->max_stars * 4 + 8);
     rc |= b->q0.ensure(S * 8); rc |= b->g0.ensure(S * 8); rc |= b->gid.ensure((size_t)cfg->max_stars * 8);
+    rc |= b->slot.ensure((size_t)cfg->max_stars * 4);
     rc |= b->vpart.ensure(std::max<size_t>(kVBlocks, ntiles) * 8); rc |= b->scalars.ensure(kScalars * 8); rc |= b->gscalars.ensure(kScalars * 8); rc |= b->state.ensure(8 * 8);
     rc |= b->counters.ensure(4 * 4); rc |= b->err.ensure(4);
     rc |= b->epart.ensure(kEnergyBlocks * 4 * 8); rc |= b->tickets.ensure(2 * 4);
@@ -1095,7 +1120,8 @@ int srhmc_big_destroy(srhmc_big* b) {
     if (b->stream) cudaStreamSynchronize(b->stream);
     BBuf* all[] = {&b->D, &b->L, &b->q, &b->p, &b->g, &b->a1, &b->a2, &b->q0, &b->g0, &b->gid, &b->vpart, &b->scalars, &b->gscalars, &b->state,
                    &b->counters, &b->send, &b->recv, &b->err, &b->normals, &b->lnu, &b->E, &b->V, &b->T, &b->A,
-                   &b->tcnt, &b->tlist, &b->gpart, &b->epart, &b->tickets, &b->xepoch, &b->packcnt, &b->xticket, &b->D32};
+                   &b->tcnt, &b->tlist, &b->gpart, &b->epart, &b->tickets, &b->xepoch, &b->packcnt, &b->xticket, &b->D32,
+                   &b->slot, &b->recq, &b->recp};
     for (BBuf* x : all) x->release();
     for (int r = 0; r < kMaxWorld; ++r)
         if (b->ipc_opened[r]) cudaIpcCloseMemHandle(b->ipc_opened[r]);
@@ -1217,9 +1243,19 @@ int srhmc_big_set_stars(srhmc_big* b, const double* q, const int64_t* global_ids
     if (!b || (n > 0 && (!q || !global_ids))) return bfail(SRHMC_ERR_INVALID, "null argument");
     if (n < 0 || n > b->cfg.max_stars) return bfail(SRHMC_ERR_INVALID, "%d stars exceed max_stars = %d", n, b->cfg.max_stars);
     BCU(cudaSetDevice(b->cfg.device));
+    // slot of a star = rank of its id among the strip's ids: the position of its column in a recorded sample row
+    std::vector<int32_t> order(n), slots(n);
+    std::iota(order.begin(), order.end(), 0);
+    std::stable_sort(order.begin(), order.end(), [&](int32_t a, int32_t c) { return global_ids[a] < global_ids[c]; });
+    std::vector<int64_t> sorted(n);
+    for (int32_t r = 0; r < n; ++r) {
+        slots[order[r]] = r;
+        sorted[r] = global_ids[order[r]];
+    }
     if (n) {
         BCU(cudaMemcpyAsync(b->q.ptr, q, (size_t)n * 24, cudaMemcpyHostToDevice, b->stream));
         BCU(cudaMemcpyAsync(b->gid.ptr, global_ids, (size_t)n * 8, cudaMemcpyHostToDevice, b->stream));
+        BCU(cudaMemcpyAsync(b->slot.ptr, slots.data(), (size_t)n * 4, cudaMemcpyHostToDevice, b->stream));
     }
     BCU(cudaMemsetAsync(b->p.ptr, 0, 3 * (size_t)b->cfg.max_stars * 8, b->stream));
     if (b->own_binned || b->ghosts_binned) {  // records of the previous positions
@@ -1233,6 +1269,7 @@ int srhmc_big_set_stars(srhmc_big* b, const double* q, const int64_t* global_ids
     }
     BCU(cudaStreamSynchronize(b->stream));
     b->n = n;
+    b->sorted_ids.swap(sorted);
     return 0;
 }
 
@@ -1391,6 +1428,96 @@ int srhmc_big_read_scalars(srhmc_big* b, double* scalars /* [8] local partial su
     BCU(cudaSetDevice(b->cfg.device));
     BCU(cudaMemcpyAsync(scalars, b->scalars.ptr, kScalars * 8, cudaMemcpyDeviceToHost, b->stream));
     BCU(cudaStreamSynchronize(b->stream));
+    return 0;
+}
+
+int srhmc_big_set_recording(srhmc_big* b, int32_t n_iters, int32_t stride, int32_t want_q, int32_t want_p) {
+    if (!b) return bfail(SRHMC_ERR_INVALID, "null context");
+    BCU(cudaSetDevice(b->cfg.device));
+    if (!want_q && !want_p) {
+        if (b->recq.ptr || b->recp.ptr) BCU(cudaStreamSynchronize(b->stream));   // rows a queued RECORD_E0 may still write
+        b->recq.release();
+        b->recp.release();
+        b->rec_rows = 0;
+        return 0;
+    }
+    if (n_iters < 1 || stride < 1) return bfail(SRHMC_ERR_INVALID, "n_iters and stride must be >= 1");
+    if (std::adjacent_find(b->sorted_ids.begin(), b->sorted_ids.end()) != b->sorted_ids.end())
+        return bfail(SRHMC_ERR_STATE, "an owned global id appears twice: the sample rows need distinct ids");
+    const int rows = (int)((n_iters + (int64_t)stride - 1) / stride);
+    const size_t bytes = std::max<size_t>(1, (size_t)rows * b->n * 24);
+    BCU(cudaStreamSynchronize(b->stream));
+    BBuf* want[2] = {want_q ? &b->recq : nullptr, want_p ? &b->recp : nullptr};
+    BBuf* drop[2] = {want_q ? nullptr : &b->recq, want_p ? nullptr : &b->recp};
+    for (BBuf* x : drop)
+        if (x) x->release();
+    for (BBuf* x : want) {
+        if (x && x->ensure(bytes) != 0) {
+            cudaGetLastError();   // the failed cudaMalloc must not surface as a launch error of a later phase
+            b->recq.release();
+            b->recp.release();
+            b->rec_rows = 0;
+            return bfail(SRHMC_ERR_CUDA, "cannot allocate %zu bytes for %d sample rows of %d stars", bytes, rows, b->n);
+        }
+    }
+    b->rec_rows = rows;
+    b->rec_stride = stride;
+    b->rec_n = b->n;
+    return 0;
+}
+
+int srhmc_big_read_samples(srhmc_big* b, int32_t row0, int32_t nrows, double* q, double* p) {
+    if (!b) return bfail(SRHMC_ERR_INVALID, "null context");
+    if (row0 < 0 || nrows < 0 || (int64_t)row0 + nrows > b->rec_rows)
+        return bfail(SRHMC_ERR_INVALID, "rows [%d, %d) outside the %d recorded rows", row0, row0 + nrows, b->rec_rows);
+    if ((q && !b->recq.ptr) || (p && !b->recp.ptr)) return bfail(SRHMC_ERR_STATE, "%s was not recorded", (q && !b->recq.ptr) ? "q" : "p");
+    BCU(cudaSetDevice(b->cfg.device));
+    const size_t row = (size_t)b->rec_n * 24, off = (size_t)row0 * row, bytes = (size_t)nrows * row;
+    if (q && bytes) BCU(cudaMemcpyAsync(q, b->recq.as<unsigned char>() + off, bytes, cudaMemcpyDeviceToHost, b->stream));
+    if (p && bytes) BCU(cudaMemcpyAsync(p, b->recp.as<unsigned char>() + off, bytes, cudaMemcpyDeviceToHost, b->stream));
+    BCU(cudaStreamSynchronize(b->stream));
+    return 0;
+}
+
+int srhmc_big_convergence_stats(srhmc_big* const* chains, int32_t k, int32_t thin_rate, int32_t warm_up_num, double* R,
+                                double* n_eff) {
+    if (!chains || !R || !n_eff) return bfail(SRHMC_ERR_INVALID, "null argument");
+    if (k < 2) return bfail(SRHMC_ERR_INVALID, "convergence statistics need at least two chains (utils.py:94), got %d", k);
+    if (k > kMaxStatsChains) return bfail(SRHMC_ERR_INVALID, "at most %d chains, got %d", kMaxStatsChains, k);
+    const srhmc_big* c0 = chains[0];
+    for (int32_t c = 0; c < k; ++c) {
+        const srhmc_big* b = chains[c];
+        if (!b) return bfail(SRHMC_ERR_INVALID, "chain %d is null", c);
+        if (!b->recq.ptr || b->rec_rows == 0) return bfail(SRHMC_ERR_STATE, "chain %d has no recorded q rows", c);
+        if (b->cfg.device != c0->cfg.device) return bfail(SRHMC_ERR_INVALID, "chain %d is on device %d, chain 0 on %d", c, b->cfg.device, c0->cfg.device);
+        if (b->rec_rows != c0->rec_rows || b->rec_stride != c0->rec_stride)
+            return bfail(SRHMC_ERR_INVALID, "chain %d holds %d rows at stride %d, chain 0 %d rows at stride %d", c, b->rec_rows,
+                         b->rec_stride, c0->rec_rows, c0->rec_stride);
+        if (b->rec_n != (int)b->sorted_ids.size() || b->sorted_ids != c0->sorted_ids)
+            return bfail(SRHMC_ERR_INVALID, "chain %d does not own the same stars as chain 0", c);
+    }
+    const int d = 3 * c0->rec_n;
+    if (int rc = check_stats_args(k, c0->rec_rows, d, 1, thin_rate, warm_up_num)) return bfail(rc, "%s", srhmc_last_error());
+    BCU(cudaSetDevice(c0->cfg.device));
+    const double* x[kMaxStatsChains];
+    for (int32_t c = 0; c < k; ++c) {
+        BCU(cudaStreamSynchronize(chains[c]->stream));   // every chain's rows are complete
+        x[c] = chains[c]->recq.as<double>();
+    }
+    BBuf out;
+    if (int rc = out.ensure(2 * (size_t)d * 8)) {
+        cudaGetLastError();
+        return bfail(rc, "cannot allocate the statistics output (%d variables)", d);
+    }
+    cudaStream_t st = c0->stream;
+    cudaError_t e = (cudaError_t)conv_stats_var_launch(st, x, k, c0->rec_rows, d, thin_rate, warm_up_num, out.as<double>(),
+                                                       out.as<double>() + d);
+    chains[0]->launches += 1;
+    if (e == cudaSuccess) e = cudaMemcpyAsync(R, out.ptr, (size_t)d * 8, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(n_eff, out.as<double>() + d, (size_t)d * 8, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+    out.release();
+    if (e != cudaSuccess) return bfail(SRHMC_ERR_CUDA, "chain statistics failed: %s", cudaGetErrorString(e));
     return 0;
 }
 
@@ -1646,6 +1773,15 @@ int srhmc_big_phase(srhmc_big* b, int32_t phase, const srhmc_big_step* s) {
                 big_restore_v_kernel<<<1, 1, 0, st>>>(b->scalars.as<double>(), b->state.as<double>(),
                                                       s->iteration < 0 ? cnt + 2 : nullptr);
             b->launches += 1 + ph;
+            if (ph == 0 && b->rec_rows > 0) {   // sample row of this iteration (srhmc_big_set_recording)
+                if (b->rec_n != n) return bfail(SRHMC_ERR_STATE, "the stars changed since srhmc_big_set_recording");
+                if (n > 0) {
+                    big_record_kernel<<<std::max(1, std::min((3 * n + 255) / 256, 4 * b->sm_count)), 256, 0, st>>>(
+                        n, b->q.as<double>(), b->p.as<double>(), b->slot.as<int>(), s->iteration, s->iteration < 0 ? cnt + 2 : nullptr,
+                        b->rec_stride, b->rec_rows, b->recq.as<double>(), b->recp.as<double>());
+                    b->launches += 1;
+                }
+            }
             break;
         }
         default:

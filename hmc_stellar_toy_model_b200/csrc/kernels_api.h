@@ -3,6 +3,7 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <stddef.h>
+#include <stdint.h>
 
 #include "common.cuh"
 
@@ -56,6 +57,12 @@ int poisson_launch(cudaStream_t stream, const double* lam, double* D, size_t n, 
 size_t conv_stats_scratch_doubles(long long rows, int d, int n_groups, int cpg, int thin, int warm);
 int conv_stats_launch(cudaStream_t stream, const double* X, long long rows, int d, int n_groups, int cpg, int thin, int warm,
                       double* scratch, double* R, double* neff);
+// variable-parallel form for a few chains held in separate buffers (the large-field engine): one thread per variable
+constexpr int kMaxStatsChains = 16;
+int conv_stats_var_launch(cudaStream_t stream, const double* const* chains, int k, long long rows, int d, int thin, int warm,
+                          double* R, double* neff);
+// argument checks shared by every statistics entry point (message through srhmc_last_error)
+int check_stats_args(int64_t n_chains, int64_t rows, int32_t d, int32_t n_groups, int32_t thin, int32_t warm);
 
 // gradient-descent leg of lightsource_gym.find_peaks (peaks_kernels.cu): one warp per seed, image 0 of the context
 int peaks_launch(cudaStream_t stream, const FieldParams& P, const double* D, int n, int nstep, double dt_f_coeff,

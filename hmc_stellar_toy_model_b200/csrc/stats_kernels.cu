@@ -32,6 +32,31 @@ __device__ __forceinline__ const double* sample_ptr(const double* X, const Stats
     return X + (chain * G.rows + first) * G.d + v;
 }
 
+// Sum of the autocorrelations that enters n_eff (utils.py:137-165) from the variogram at lag t, `vario(t)`: rho_t = 1 - V_t / (2 var);
+// nothing when rho_1 < 0.05, otherwise the sum of rho_1 .. rho_t up to the first odd t with rho_{t+1} + rho_{t+2} < 0 (or
+// t = n - 2), clamped at 0.  The reference's rho_t list index i holds lag i + 1.  Every caller thread follows the same control
+// flow.  Shared by conv_stats_final_kernel and conv_stats_var_kernel.
+template <class Vario>
+__device__ __forceinline__ double ess_sum_rho(int n, double var, const Vario& vario) {
+    const double rho1 = 1.0 - vario(1) / (2.0 * var);
+    const double rho2 = 1.0 - vario(2) / (2.0 * var);
+    double sum_rho = 0.0;
+    if (!(rho1 < 5e-2)) {
+        // loop invariant: prefix = sum(rho_t[:t]), cur = rho_t[t]
+        double prefix = rho1, cur = rho2;
+        int t = 1;
+        while (t < n - 2) {
+            const double next = 1.0 - vario(t + 2) / (2.0 * var);  // appended as rho_t[t + 1]
+            if ((t & 1) && (cur + next) < 0.0) break;
+            prefix += cur;
+            cur = next;
+            ++t;
+        }
+        sum_rho = prefix < 0.0 ? 0.0 : prefix;
+    }
+    return sum_rho;
+}
+
 __global__ void __launch_bounds__(256) conv_stats_kernel(const double* __restrict__ X, const StatsGeom G, double* __restrict__ means,
                                                          double* __restrict__ R_out, double* __restrict__ neff_out) {
     __shared__ double red[2 * 32];
@@ -211,25 +236,69 @@ conv_stats_final_kernel(const StatsGeom G, int blocks_per_group, const double* _
     }
     __syncthreads();
     if (threadIdx.x == 0) {
-        // effective sample size (utils.py:137-165): rho_t list index i holds lag i + 1
-        const double rho1 = 1.0 - V[0] / (2.0 * var);
-        const double rho2 = 1.0 - V[1] / (2.0 * var);
-        double sum_rho = 0.0;
-        if (!(rho1 < 5e-2)) {
-            double prefix = rho1, cur = rho2;
-            int t = 1;
-            while (t < n - 2) {
-                const double next = 1.0 - V[t + 1] / (2.0 * var);   // lag t + 2
-                if ((t & 1) && (cur + next) < 0.0) break;
-                prefix += cur;
-                cur = next;
-                ++t;
-            }
-            sum_rho = prefix < 0.0 ? 0.0 : prefix;
-        }
+        // effective sample size (utils.py:137-165)
+        const double sum_rho = ess_sum_rho(n, var, [&](int lag) { return V[lag - 1]; });
         R_out[blockIdx.x] = R;
         neff_out[blockIdx.x] = (double)m * (double)n / (1.0 + 2.0 * sum_rho);
     }
+}
+
+
+// ---- variable-parallel variant: few chains, many variables (the chains of the large-field engine) -------------------------
+// One thread per variable; the K chains are separate row-major buffers [rows][d] (X[c] in the parameter struct), so a warp
+// reads 32 consecutive variables of one row per load.  Every thread loops over the split chains and samples in a fixed
+// order (reproducible run to run) and runs its own lag loop to its own cut-off.  Same formulas as conv_stats_kernel.
+struct ChainSet {
+    const double* x[kMaxStatsChains];
+};
+
+__global__ void __launch_bounds__(128) conv_stats_var_kernel(const ChainSet X, const StatsGeom G, double* __restrict__ R_out,
+                                                             double* __restrict__ neff_out) {
+    const int v = blockIdx.x * blockDim.x + threadIdx.x;
+    if (v >= G.d) return;
+    const int m = 2 * G.cpg, n = G.n;
+    const long long stride = (long long)G.thin * G.d;
+    auto sample0 = [&](int j) {   // first sample of split chain j (j = 2 * chain + half)
+        const long long first = (long long)G.warm + (long long)G.thin * ((j & 1) ? n : 0);
+        return X.x[j >> 1] + first * G.d + v;
+    };
+    double mu[2 * kMaxStatsChains];
+    double sd_sum = 0.0, mu_sum = 0.0;
+    for (int j = 0; j < m; ++j) {
+        const double* x = sample0(j);
+        double s = 0.0;
+        for (int k = 0; k < n; ++k) s += x[k * stride];
+        const double mean = s / (double)n;
+        double ss = 0.0;
+        for (int k = 0; k < n; ++k) {
+            const double dlt = x[k * stride] - mean;
+            ss += dlt * dlt;
+        }
+        mu[j] = mean;
+        sd_sum += sqrt(ss / (double)(n - 1));
+        mu_sum += mean;
+    }
+    const double W = sd_sum / (double)m, mean_all = mu_sum / (double)m;
+    double b = 0.0;
+    for (int j = 0; j < m; ++j) {
+        const double dlt = mu[j] - mean_all;
+        b += dlt * dlt;
+    }
+    const double B = b * (double)n / (double)(m - 1);
+    const double var = W * (double)(n - 1) / (double)n + B / (double)n;
+    const double sum_rho = ess_sum_rho(n, var, [&](int t) {
+        double a = 0.0;
+        for (int j = 0; j < m; ++j) {
+            const double* x = sample0(j);
+            for (int k = 0; k + t < n; ++k) {
+                const double dlt = x[(k + t) * stride] - x[k * stride];
+                a += dlt * dlt;
+            }
+        }
+        return a / ((double)m * (double)(n - t));
+    });
+    R_out[v] = sqrt(var / W);
+    neff_out[v] = (double)m * (double)n / (1.0 + 2.0 * sum_rho);
 }
 
 }  // namespace
@@ -272,6 +341,17 @@ int conv_stats_launch(cudaStream_t stream, const double* X, long long rows, int 
     if (e != cudaSuccess) return (int)e;
     conv_stats_chain_kernel<<<n_groups * bpg, 32 * kStatsChainsPerBlock, smem, stream>>>(X, G, bpg, mu, sd, lagpart);
     conv_stats_final_kernel<<<n_groups * d, 256, 0, stream>>>(G, bpg, mu, sd, lagpart, vario, R, neff);
+    return (int)cudaGetLastError();
+}
+
+// K (2..kMaxStatsChains) chains, each its own device buffer [rows][d]; R, n_eff [d] on the device.
+int conv_stats_var_launch(cudaStream_t stream, const double* const* chains, int k, long long rows, int d, int thin, int warm,
+                          double* R, double* neff) {
+    if (k < 2 || k > kMaxStatsChains) return (int)cudaErrorInvalidValue;
+    ChainSet X{};
+    for (int c = 0; c < k; ++c) X.x[c] = chains[c];
+    const StatsGeom G = stats_geom(rows, d, k, thin, warm);
+    conv_stats_var_kernel<<<(d + 127) / 128, 128, 0, stream>>>(X, G, R, neff);
     return (int)cudaGetLastError();
 }
 

@@ -264,6 +264,16 @@ bool all_one_star(const srhmc_ctx* c, const int32_t* nstars) {
 
 }  // namespace
 
+int srhmc::check_stats_args(int64_t n_chains, int64_t rows, int32_t d, int32_t n_groups, int32_t thin, int32_t warm) {
+    if (n_chains < 1 || rows < 1 || d < 1 || n_groups < 1 || thin < 1 || warm < 0) return fail(SRHMC_ERR_INVALID, "bad chain statistics argument");
+    if (n_chains % n_groups) return fail(SRHMC_ERR_INVALID, "%lld chains do not split into %d equal groups", (long long)n_chains, n_groups);
+    if (n_chains / n_groups < 2) return fail(SRHMC_ERR_INVALID, "convergence statistics need at least two chains per group (utils.py:94)");
+    const int64_t Lw = rows - warm, Lc = Lw > 0 ? (Lw + thin - 1) / thin : 0;
+    if (Lc / 2 < 2) return fail(SRHMC_ERR_INVALID, "fewer than two samples per split chain after warm-up and thinning");
+    if (n_chains / n_groups > (1 << 24)) return fail(SRHMC_ERR_INVALID, "too many chains per group");
+    return 0;
+}
+
 extern "C" {
 
 int srhmc_abi_version(void) { return SRHMC_ABI_VERSION; }
@@ -1111,16 +1121,6 @@ int srhmc_hessian(srhmc_ctx* c, const double* q, const double* p, const int32_t*
     return 0;
 }
 
-
-static int check_stats_args(int64_t n_chains, int64_t rows, int32_t d, int32_t n_groups, int32_t thin, int32_t warm) {
-    if (n_chains < 1 || rows < 1 || d < 1 || n_groups < 1 || thin < 1 || warm < 0) return fail(SRHMC_ERR_INVALID, "bad chain statistics argument");
-    if (n_chains % n_groups) return fail(SRHMC_ERR_INVALID, "%lld chains do not split into %d equal groups", (long long)n_chains, n_groups);
-    if (n_chains / n_groups < 2) return fail(SRHMC_ERR_INVALID, "convergence statistics need at least two chains per group (utils.py:94)");
-    const int64_t Lw = rows - warm, Lc = Lw > 0 ? (Lw + thin - 1) / thin : 0;
-    if (Lc / 2 < 2) return fail(SRHMC_ERR_INVALID, "fewer than two samples per split chain after warm-up and thinning");
-    if (n_chains / n_groups > (1 << 24)) return fail(SRHMC_ERR_INVALID, "too many chains per group");
-    return 0;
-}
 
 int srhmc_convergence_stats(int32_t device, const double* q_chain, int64_t n_chains, int64_t n_iter, int32_t d, int32_t n_groups,
                             int32_t thin_rate, int32_t warm_up_num, double* R, double* n_eff) {

@@ -330,7 +330,7 @@ typedef enum srhmc_big_phase_id {
     SRHMC_BIG_KICK2 = 6,      /* p -= h dphi/dq at the new q; reflections (a7 steps 5-6) */
     SRHMC_BIG_MOMENTUM = 7,   /* p = z sqrt(H); remember the iteration's start state (a8) */
     SRHMC_BIG_ENERGY = 8,     /* scalars[1..3] = T, #stars outside the support, prior potential (a3, a5) */
-    SRHMC_BIG_RECORD_E0 = 9,  /* E0 from global_scalars; chain row */
+    SRHMC_BIG_RECORD_E0 = 9,  /* E0 from global_scalars; chain row; sample row while recording (srhmc_big_set_recording) */
     SRHMC_BIG_ACCEPT = 10,    /* Metropolis test on global_scalars; restore on rejection; chain row (a8) */
     SRHMC_BIG_RESET_ITER = 11, /* zero the device-side iteration counter used when step.iteration < 0 */
     /* fused forms (same arithmetic in the same order, fewer launches): */
@@ -404,6 +404,22 @@ int srhmc_big_read_chains(srhmc_big* b, int32_t n_iters, double* E, double* V, d
                                                     3: tile list overflow; 4: peer exchange timed out */);
 int srhmc_big_read_scalars(srhmc_big* b, double* scalars);
 int srhmc_big_phase(srhmc_big* b, int32_t phase, const srhmc_big_step* step);
+/* Sample recording (the q_chain / p_chain of multi_gym.run_RHMC): from the next RECORD_E0 on, the phase also stores the owned
+ * stars' q (before the trajectory) and/or p (just drawn by MOMENTUM) of iteration l as row l / stride when stride divides l:
+ * ceil(n_iters / stride) rows of [n][3] doubles on the device, stars in ascending global-id order (slot order, independent of
+ * the storage order).  The iteration index is step.iteration, or the device counter when it is < 0, so eager runs and replays
+ * of a captured iteration record alike.  One extra kernel per RECORD_E0 while recording; nothing changes while it is off.
+ * want_q = want_p = 0 turns recording off and frees the rows.  Call it after srhmc_big_set_stars and outside graph capture: it
+ * may move the buffers. */
+int srhmc_big_set_recording(srhmc_big* b, int32_t n_iters, int32_t stride, int32_t want_q, int32_t want_p);
+/* Rows [row0, row0 + nrows) of the recorded samples, each [n][3] in slot order (q or p may be NULL): a long chain can be
+ * fetched in pieces. */
+int srhmc_big_read_samples(srhmc_big* b, int32_t row0, int32_t nrows, double* q, double* p);
+/* utils.convergence_stats over k (2..16) chains of the same field: k contexts on one device that own the same global ids and
+ * recorded q with the same row count and stride.  thin_rate / warm_up_num apply to the recorded rows.  R, n_eff [3 n] in slot
+ * order.  One thread per variable over the resident rows (variable-parallel: few chains, many variables). */
+int srhmc_big_convergence_stats(srhmc_big* const* chains, int32_t k, int32_t thin_rate, int32_t warm_up_num, double* R,
+                                double* n_eff);
 
 /* Roofline denominator measured on the device itself: a register-resident FMA chain (8 independent chains per
  * thread, all SMs filled) in the given precision (64 or 32).  Returns TFLOP/s (2 flop per FMA) and the launch time. */
