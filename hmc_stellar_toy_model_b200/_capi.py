@@ -12,7 +12,7 @@ import os
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-LIB_PATH = os.environ.get("SRHMC_LIB") or os.path.join(_HERE, "libstellar_rhmc.so")  # SRHMC_LIB: experimental builds
+LIB_PATH = os.path.join(_HERE, "libstellar_rhmc.so")
 ABI_VERSION = 3
 
 c_double_p = C.POINTER(C.c_double)

@@ -44,24 +44,6 @@ def _stale(obj, src):
     return any(os.path.getmtime(d) > t for d in heads + [src])
 
 
-def build_variant(tag: str, defines) -> str:
-    """Experimental build with extra -D flags -> libstellar_rhmc_<tag>.so (selected at run time by SRHMC_LIB)."""
-    nvcc = shutil.which("nvcc") or "/usr/local/cuda/bin/nvcc"
-    out = os.path.join(HERE, "libstellar_rhmc_%s.so" % tag)
-    odir = os.path.join(OBJ_DIR, tag)
-    os.makedirs(odir, exist_ok=True)
-    procs = []
-    for name in SOURCES:
-        obj = os.path.join(odir, name[:-3] + ".o")
-        cmd = [nvcc] + COMPILE_FLAGS + ["-D" + d for d in defines] + ["-o", obj, os.path.join(CSRC, name)]
-        procs.append((obj, subprocess.Popen(cmd, stdout=subprocess.DEVNULL, stderr=subprocess.STDOUT)))
-    for obj, pr in procs:
-        if pr.wait() != 0:
-            raise RuntimeError("variant build failed for " + obj)
-    subprocess.check_call([nvcc] + LINK_FLAGS + ["-o", out] + [o for o, _ in procs])
-    return out
-
-
 def build(force: bool = False, verbose: bool = False) -> str:
     """Compile every translation unit for sm_100a (in parallel) and link libstellar_rhmc.so in-tree."""
     if not force and up_to_date():

@@ -117,15 +117,6 @@ __global__ void big_bin_kernel(const BigParams P, const TileSrc S, int ntx, int 
     }
 }
 
-// Data loads before (1) or after (0) the render phase: early loads overlap HBM latency with the render inside one CTA
-// but hold 32 more registers per thread.
-#ifndef SRHMC_TILE_EARLY_LOAD
-#define SRHMC_TILE_EARLY_LOAD 0
-#endif
-#ifndef SRHMC_TILE_MIN_CTAS
-#define SRHMC_TILE_MIN_CTAS 4
-#endif
-
 constexpr int kTabPad = 4;                 // zero guard entries on each side of a 32-entry factor table
 constexpr int kTabLen = 32 + 2 * kTabPad;  // a thread reads 4 consecutive entries starting anywhere in [-3, 31]
 
@@ -235,7 +226,7 @@ __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wai
 // MODE 0: gradient; 1: gradient + pixel potential; 2: mock data -- the rendered model of the tile is Poisson-sampled
 // (poisson.cuh, counter = global pixel index) into Dout and nothing else happens
 template <int MODE>
-__global__ void __launch_bounds__(kTileThreads, SRHMC_TILE_MIN_CTAS) big_tile_kernel(const BigParams P, const TileSrc S, int ntx,
+__global__ void __launch_bounds__(kTileThreads, 4) big_tile_kernel(const BigParams P, const TileSrc S, int ntx,
                                                                 const double* __restrict__ D,
                                                                 int* __restrict__ cnt,
                                                                 const PairRec* __restrict__ list, double* __restrict__ gpart,

@@ -103,53 +103,39 @@ __device__ __forceinline__ float rcp_pixf(float a) {
 // (Measured and not adopted: the product-tree reciprocal (rcp_row) in the FP32 loop: 1725 against 1738 M star-steps/s.)
 // (Measured and not adopted: feeding the count as the double 2^52 + d with fma(X, r, -2^52 r) = round(d r) removes the
 // I2F from the pixel loop but costs three integer instructions per pixel: 1422 against 1472 M star-steps/s.)
-#ifdef SRHMC_EXP_NEWTON2
-// EXPERIMENT (not adopted): one quadratic Newton step is 8% faster but its 2^-40 error grows to 1e-8 in q over 30
-// Metropolis iterations, beyond the 1e-9 trajectory tolerance of the parity tests
-__device__ __forceinline__ double rcp_pix(double a) {
-    double x0;
-    asm("rcp.approx.ftz.f64 %0, %1;" : "=d"(x0) : "d"(a));
-    return fma(x0, fma(-a, x0, 1.0), x0);
-}
-#else
-__device__ __forceinline__ double rcp_pix(double a) { return rcp_fast(a); }
-#endif
+// (Measured and not adopted: one quadratic Newton step instead of rcp_fast's cubic one is 8% faster, but its 2^-40 error
+// grows to 1e-8 in q over 30 Metropolis iterations, beyond the 1e-9 trajectory tolerance of the parity tests.)
 
 // Reciprocals of N pixels from ONE MUFU.RCP64H: 1/a_k = (product of the others) / (product of all).  The FP64 instruction
 // count is the same as N separate cubic Newton reciprocals (3 per pixel: products down, one Newton step, products up), but the
 // pixel loop was bound by the XU pipe (MUFU.RCP64H + I2F per pixel, 8 issue cycles each per scheduler against 14 cycles of
 // DFMA): this leaves one MUFU per 3 (4) pixels.  Each result carries <= 4 roundings (~2^-51 relative).  Lambda = 0 in a group
 // gives NaN for its neighbours as well (the reference gives inf at that pixel and a non-finite gradient either way).
-#ifndef SRHMC_RCP_TREE
-#define SRHMC_RCP_TREE 1
-#endif
 template <int N>
 __device__ __forceinline__ void rcp_group(const double (&a)[N], double (&r)[N]) {
-    if (SRHMC_RCP_TREE && N == 3) {
+    static_assert(N == 3 || N == 4, "reciprocal groups are triples or quadruples");
+    if constexpr (N == 3) {
         const double p01 = a[0] * a[1];
-        const double ip = rcp_pix(p01 * a[2]);
+        const double ip = rcp_fast(p01 * a[2]);
         const double r01 = a[2] * ip;
         r[2] = p01 * ip;
         r[0] = a[1] * r01;
         r[1] = a[0] * r01;
-    } else if (SRHMC_RCP_TREE && N == 4) {
+    } else {
         const double p01 = a[0] * a[1], p23 = a[2] * a[3];
-        const double ip = rcp_pix(p01 * p23);
+        const double ip = rcp_fast(p01 * p23);
         const double r01 = p23 * ip, r23 = p01 * ip;
         r[0] = a[1] * r01;
         r[1] = a[0] * r01;
         r[2] = a[3] * r23;
         r[3] = a[2] * r23;
-    } else {
-#pragma unroll
-        for (int k = 0; k < N; ++k) r[k] = rcp_pix(a[k]);
     }
 }
 // reciprocals of the NCS pixels a lane owns in one image row: triples when NCS is a multiple of 3 (24-column window: 6 slots),
 // quadruples for the full-width variant (8 slots)
 template <int NCS>
 __device__ __forceinline__ void rcp_row(const double (&lam)[NCS], double (&r)[NCS]) {
-    constexpr int GS = (NCS % 3 == 0) ? 3 : (NCS % 4 == 0) ? 4 : 1;
+    constexpr int GS = (NCS % 3 == 0) ? 3 : 4;
 #pragma unroll
     for (int g = 0; g < NCS / GS; ++g) {
         double a[GS], o[GS];
@@ -364,11 +350,7 @@ __device__ __forceinline__ void chain_eval(const FieldParams& P, const DT* __res
     } else if (!WANT_V) {
         // rows per trip of the gradient-only loop.  With the product-tree reciprocal (one MUFU per three pixels) and a 255-register
         // budget (still 8 single-warp blocks per SM) four rows measured best: x2 1533, x3 1543, x4 1556 M star-steps/s
-#ifndef SRHMC_MAIN_UNROLL
-#define SRHMC_MAIN_UNROLL (kChainLPC <= 4 ? 4 : 2)
-#endif
-        constexpr int kMainUnroll = SRHMC_MAIN_UNROLL;
-#pragma unroll kMainUnroll
+#pragma unroll 4
         for (int i = i_lo; i < i_hi; ++i) {
             const double2 re = rt[i];
             double lam[CPL], il[CPL];
@@ -538,10 +520,8 @@ __device__ __forceinline__ void chain_step(const FieldParams& P, const ChainCons
     if ((s.y < 0.0) || (s.y > P.C - 1.0)) s.py = -s.py;
 }
 
-#ifndef SRHMC_CHAIN_MAXREG
-#define SRHMC_CHAIN_MAXREG (kChainLPC <= 4 ? 255 : 168)
-#endif
-constexpr int kChainMaxReg = SRHMC_CHAIN_MAXREG;
+// register budget: the 255-register maximum (the kernel uses 240 and still keeps 8 single-warp blocks per SM resident)
+constexpr int kChainMaxReg = 255;
 template <int LPC, typename DT, int MODE, int NCS, int MAXREG = kChainMaxReg, typename PT = double>
 __global__ void __maxnreg__(MAXREG) chain_kernel(const __grid_constant__ FieldParams P, const __grid_constant__ LaunchArgs A) {
     extern __shared__ __align__(16) unsigned char smem_raw[];

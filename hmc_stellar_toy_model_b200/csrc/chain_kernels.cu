@@ -11,44 +11,36 @@ namespace srhmc {
 namespace {
 
 constexpr int kLPC = kChainLPC;  // lanes per chain: 4 -> 8 chains per warp (measured: 16 lanes 734, 8 lanes 1104, 4 lanes 1210 M star-steps/s)
-#ifndef SRHMC_CHAIN_WARPS_PER_BLOCK
-#define SRHMC_CHAIN_WARPS_PER_BLOCK 1
-#endif
-constexpr int kWarpsPerBlock = SRHMC_CHAIN_WARPS_PER_BLOCK;
 // Column slots per lane: the full 32-column image, or a 24-column window around the star when the PSF weight of
 // every dropped column is below 2^-46 of its peak (sigma <= 1.50 px: |dy| >= 12 px).  SRHMC_CHAIN_WINDOW=0 at run time
-// forces the full width (A/B measurements).
+// forces the full width, so that the tests can compare the two.
 constexpr int kSlotsFull = 32 / kLPC;
-#ifndef SRHMC_CHAIN_WIN_COLS
-#define SRHMC_CHAIN_WIN_COLS 24
-#endif
-constexpr int kWinCols = SRHMC_CHAIN_WIN_COLS;
-constexpr int kSlotsWin = (kWinCols % kLPC == 0 && kWinCols / kLPC < kSlotsFull) ? kWinCols / kLPC : kSlotsFull;
+constexpr int kWinCols = 24;
+constexpr int kSlotsWin = kWinCols / kLPC;
 
 bool use_column_window(const FieldParams& P) {
-    if (kSlotsWin == kSlotsFull) return false;
     if (const char* env = std::getenv("SRHMC_CHAIN_WINDOW"))
         if (std::atoi(env) == 0) return false;
     const double half = 0.5 * kWinCols;
     return half * half * P.inv2s2 >= 46.0 * M_LN2;
 }
 
-size_t chain_smem_bytes(const FieldParams& P, int lpc, int nw, size_t elem, bool f32 = false) {
-    const size_t gpw = 32 / lpc;
+// one single-warp block: the log table and kChainGroup chains of image copy and row tables
+size_t chain_smem_bytes(const FieldParams& P, size_t elem, bool f32) {
     const size_t rowtab = sizeof(double2) + (f32 ? sizeof(float2) : 0);
-    const size_t per_warp = gpw * (((size_t)P.R * kChainCS + lpc) * elem + (size_t)P.R * rowtab + kChainTabPad);
-    return kLogTableSize * sizeof(double2) + (size_t)nw * per_warp;
+    return kLogTableSize * sizeof(double2) +
+           (size_t)kChainGroup * (((size_t)P.R * kChainCS + kLPC) * elem + (size_t)P.R * rowtab + kChainTabPad);
 }
 
 template <typename DT, int MODE, int NCS, typename PT = double>
-int configure_mode(size_t smem, int nw, int& blocks_per_sm) {
+int configure_mode(size_t smem, int& blocks_per_sm) {
     auto fn = chain_kernel<kLPC, DT, MODE, NCS, kChainMaxReg, PT>;
     cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return (int)e;
     e = cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
     if (e != cudaSuccess) return (int)e;
     int nb = 0;
-    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, fn, 32 * nw, smem);
+    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, fn, kWarp, smem);
     if (e != cudaSuccess) return (int)e;
     if (nb < 1) return (int)cudaErrorInvalidConfiguration;
     blocks_per_sm = blocks_per_sm == 0 ? nb : std::min(blocks_per_sm, nb);
@@ -56,51 +48,42 @@ int configure_mode(size_t smem, int nw, int& blocks_per_sm) {
 }
 
 template <typename DT, int NCS, typename PT = double>
-int configure_slots(size_t smem, int nw, int& blocks_per_sm) {
-    if (int rc = configure_mode<DT, MODE_EVAL, NCS, PT>(smem, nw, blocks_per_sm)) return rc;
-    if (int rc = configure_mode<DT, MODE_STEP, NCS, PT>(smem, nw, blocks_per_sm)) return rc;
-    if (int rc = configure_mode<DT, MODE_RUN, NCS, PT>(smem, nw, blocks_per_sm)) return rc;
-    return configure_mode<DT, MODE_SINGLE, NCS, PT>(smem, nw, blocks_per_sm);
+int configure_slots(size_t smem, int& blocks_per_sm) {
+    if (int rc = configure_mode<DT, MODE_EVAL, NCS, PT>(smem, blocks_per_sm)) return rc;
+    if (int rc = configure_mode<DT, MODE_STEP, NCS, PT>(smem, blocks_per_sm)) return rc;
+    if (int rc = configure_mode<DT, MODE_RUN, NCS, PT>(smem, blocks_per_sm)) return rc;
+    return configure_mode<DT, MODE_SINGLE, NCS, PT>(smem, blocks_per_sm);
 }
 
 template <typename DT, typename PT = double>
-int configure_one(const FieldParams& P, int nw, size_t& smem, int& blocks_per_sm) {
-    smem = chain_smem_bytes(P, kLPC, nw, sizeof(DT), sizeof(PT) == 4);
+int configure_one(const FieldParams& P, size_t& smem, int& blocks_per_sm) {
+    smem = chain_smem_bytes(P, sizeof(DT), sizeof(PT) == 4);
     blocks_per_sm = 0;
-    const int rc = use_column_window(P) ? configure_slots<DT, kSlotsWin, PT>(smem, nw, blocks_per_sm)
-                                        : configure_slots<DT, kSlotsFull, PT>(smem, nw, blocks_per_sm);
-    if (const char* env = std::getenv("SRHMC_CHAIN_MAX_RESIDENT")) {   // occupancy experiments: cap the resident blocks per SM
-        const int k = std::atoi(env);
-        if (rc == 0 && k >= 1) blocks_per_sm = std::min(blocks_per_sm, k);
-    }
-    return rc;
+    return use_column_window(P) ? configure_slots<DT, kSlotsWin, PT>(smem, blocks_per_sm)
+                                : configure_slots<DT, kSlotsFull, PT>(smem, blocks_per_sm);
 }
 
 template <typename DT, int NCS, typename PT = double>
-void launch_slots(int grid, int threads, size_t smem, cudaStream_t stream, const FieldParams& P, const LaunchArgs& A) {
+void launch_slots(int grid, size_t smem, cudaStream_t stream, const FieldParams& P, const LaunchArgs& A) {
     switch (A.mode) {
-        case MODE_EVAL: chain_kernel<kLPC, DT, MODE_EVAL, NCS, kChainMaxReg, PT><<<grid, threads, smem, stream>>>(P, A); break;
-        case MODE_STEP: chain_kernel<kLPC, DT, MODE_STEP, NCS, kChainMaxReg, PT><<<grid, threads, smem, stream>>>(P, A); break;
-        case MODE_SINGLE: chain_kernel<kLPC, DT, MODE_SINGLE, NCS, kChainMaxReg, PT><<<grid, threads, smem, stream>>>(P, A); break;
-        default: chain_kernel<kLPC, DT, MODE_RUN, NCS, kChainMaxReg, PT><<<grid, threads, smem, stream>>>(P, A); break;
+        case MODE_EVAL: chain_kernel<kLPC, DT, MODE_EVAL, NCS, kChainMaxReg, PT><<<grid, kWarp, smem, stream>>>(P, A); break;
+        case MODE_STEP: chain_kernel<kLPC, DT, MODE_STEP, NCS, kChainMaxReg, PT><<<grid, kWarp, smem, stream>>>(P, A); break;
+        case MODE_SINGLE: chain_kernel<kLPC, DT, MODE_SINGLE, NCS, kChainMaxReg, PT><<<grid, kWarp, smem, stream>>>(P, A); break;
+        default: chain_kernel<kLPC, DT, MODE_RUN, NCS, kChainMaxReg, PT><<<grid, kWarp, smem, stream>>>(P, A); break;
     }
 }
 
 template <typename DT, typename PT = double>
-void launch_mode(int grid, int threads, size_t smem, cudaStream_t stream, const FieldParams& P, const LaunchArgs& A) {
+void launch_mode(int grid, size_t smem, cudaStream_t stream, const FieldParams& P, const LaunchArgs& A) {
     if (use_column_window(P))
-        launch_slots<DT, kSlotsWin, PT>(grid, threads, smem, stream, P, A);
+        launch_slots<DT, kSlotsWin, PT>(grid, smem, stream, P, A);
     else
-        launch_slots<DT, kSlotsFull, PT>(grid, threads, smem, stream, P, A);
+        launch_slots<DT, kSlotsFull, PT>(grid, smem, stream, P, A);
 }
 
 // Grid = (blocks per SM) x SMs with the per-SM count chosen so that every SM runs the same number of equally long
 // rounds (all chains of one launch run the same number of iterations).
 int balanced_grid(int max_blocks_per_sm, long long blocks_needed, int sms) {
-    if (const char* env = std::getenv("SRHMC_CHAIN_BLOCKS_PER_SM")) {  // tuning / experiments
-        const int k = std::atoi(env);
-        if (k >= 1) return (int)std::min<long long>(blocks_needed, (long long)std::min(k, max_blocks_per_sm) * sms);
-    }
     const long long cap = (long long)max_blocks_per_sm * sms;
     if (blocks_needed <= cap) return (int)std::max<long long>(1, blocks_needed);
     // k resident warps per SM run ceil(needed / (k sms)) rounds; a round costs ~k (throughput-bound) but never less
@@ -156,13 +139,11 @@ void fill_log_table(double* host_table /* [kLogTableSize*2] */) {
 }
 
 int chain_kernel_configure(const FieldParams& P, ChainLaunchPlan& plan) {
-    plan.lpc = kLPC;
-    plan.nw = kWarpsPerBlock;
-    if (int rc = configure_one<double>(P, plan.nw, plan.smem_f64, plan.blocks_per_sm_f64)) return rc;
-    if (int rc = configure_one<unsigned int>(P, plan.nw, plan.smem_u32, plan.blocks_per_sm_u32)) return rc;
-    if (int rc = configure_one<unsigned short>(P, plan.nw, plan.smem_u16, plan.blocks_per_sm_u16)) return rc;
+    if (int rc = configure_one<double>(P, plan.smem_f64, plan.blocks_per_sm_f64)) return rc;
+    if (int rc = configure_one<unsigned int>(P, plan.smem_u32, plan.blocks_per_sm_u32)) return rc;
+    if (int rc = configure_one<unsigned short>(P, plan.smem_u16, plan.blocks_per_sm_u16)) return rc;
     // FP32 pixel arithmetic (precision-32 contexts) on the uint16 count images
-    return configure_one<unsigned short, float>(P, plan.nw, plan.smem_u16_f32, plan.blocks_per_sm_u16_f32);
+    return configure_one<unsigned short, float>(P, plan.smem_u16_f32, plan.blocks_per_sm_u16_f32);
 }
 
 // Iteration chunks per chain for a MODE_RUN launch of `groups` warp-sized work items on `warps` resident warps.
@@ -185,48 +166,47 @@ int pick_chunks(long long groups, long long warps, int L) {
     return valid_chunks(std::min(16, L / 32), L);
 }
 
-long long chain_kernel_resident_warps(const LaunchArgs& A, const ChainLaunchPlan& plan, int sms, int n_fields) {
-    const int chains_per_block = plan.nw * (32 / plan.lpc);
-    const long long blocks = ((long long)n_fields + chains_per_block - 1) / chains_per_block;
+// resident single-warp blocks per SM of the image layout a launch with these arguments uses
+static int max_blocks_per_sm(const LaunchArgs& A, const ChainLaunchPlan& plan) {
     const bool u16 = A.D_int != nullptr && A.D_int_bytes == 2;
-    const int max_k = (u16 && A.pix_f32) ? plan.blocks_per_sm_u16_f32
-                                         : (u16 ? plan.blocks_per_sm_u16 : (A.D_int != nullptr ? plan.blocks_per_sm_u32 : plan.blocks_per_sm_f64));
-    return std::min<long long>(blocks, (long long)max_k * sms) * plan.nw;
+    if (u16) return A.pix_f32 ? plan.blocks_per_sm_u16_f32 : plan.blocks_per_sm_u16;
+    return A.D_int != nullptr ? plan.blocks_per_sm_u32 : plan.blocks_per_sm_f64;
+}
+
+long long chain_kernel_resident_warps(const LaunchArgs& A, const ChainLaunchPlan& plan, int sms, int n_fields) {
+    const long long blocks = ((long long)n_fields + kChainGroup - 1) / kChainGroup;
+    return std::min<long long>(blocks, (long long)max_blocks_per_sm(A, plan) * sms);
 }
 
 int chain_kernel_launch(const FieldParams& P, const LaunchArgs& A_in, const ChainLaunchPlan& plan, int sms, cudaStream_t stream) {
     LaunchArgs A = A_in;
-    const int chains_per_block = plan.nw * (32 / plan.lpc);
     const int n_range = (A.field_end > 0 ? A.field_end : A.n_fields) - A.field_begin;
-    const long long blocks = ((long long)n_range + chains_per_block - 1) / chains_per_block;
+    const long long blocks = ((long long)n_range + kChainGroup - 1) / kChainGroup;
     const bool u16 = A.D_int != nullptr && A.D_int_bytes == 2;
     // 4 lanes per chain: 240 of 255 registers -> 8 resident single-warp blocks per SM (2 per scheduler: the register file is
     // partitioned per scheduler, a third warp would need <= 168 registers and measured slower); residency comes from the
     // occupancy query in chain_kernel_configure.  Register-capped 8-lane builds were measured earlier and are slower
     // (128 registers / 16 warps 1057 M star-steps/s, 112 / 18 warps 892 against 1104 at 168 / 12).
-    const bool f32 = u16 && A.pix_f32;
-    const int max_k = f32 ? plan.blocks_per_sm_u16_f32
-                          : (u16 ? plan.blocks_per_sm_u16 : (A.D_int != nullptr ? plan.blocks_per_sm_u32 : plan.blocks_per_sm_f64));
+    const int max_k = max_blocks_per_sm(A, plan);
+    const int full = (int)std::min<long long>(blocks, (long long)max_k * sms);
     int grid = balanced_grid(max_k, blocks, sms);
     if (!(A.mode == MODE_RUN && A.sched_done != nullptr && A.chunk_count > 0)) A.n_chunks = 1;
     if (A.mode == MODE_RUN && A.sched_done != nullptr && A.chunk_count > 0) {
         // one launch of a run that the host has cut along the iteration axis: the chunking is fixed by the caller
-        grid = (int)std::min<long long>(blocks, (long long)max_k * sms);
+        grid = full;
     } else if (A.mode == MODE_RUN && A.sched_done != nullptr) {
         // with the chunked scheduler a partly filled last round costs little, so run at full residency
-        const int full = (int)std::min<long long>(blocks, (long long)max_k * sms);
-        const int chunks = pick_chunks(blocks, (long long)full * plan.nw, A.niter + 1);
-        if (chunks > 1 && !std::getenv("SRHMC_CHAIN_BLOCKS_PER_SM")) grid = full;
-        A.n_chunks = pick_chunks(blocks, (long long)grid * plan.nw, A.niter + 1);
+        if (pick_chunks(blocks, full, A.niter + 1) > 1) grid = full;
+        A.n_chunks = pick_chunks(blocks, grid, A.niter + 1);
     }
-    if (f32) {
-        launch_mode<unsigned short, float>(grid, 32 * plan.nw, plan.smem_u16_f32, stream, P, A);
+    if (u16 && A.pix_f32) {
+        launch_mode<unsigned short, float>(grid, plan.smem_u16_f32, stream, P, A);
     } else if (u16) {
-        launch_mode<unsigned short>(grid, 32 * plan.nw, plan.smem_u16, stream, P, A);
+        launch_mode<unsigned short>(grid, plan.smem_u16, stream, P, A);
     } else if (A.D_int != nullptr) {
-        launch_mode<unsigned int>(grid, 32 * plan.nw, plan.smem_u32, stream, P, A);
+        launch_mode<unsigned int>(grid, plan.smem_u32, stream, P, A);
     } else {
-        launch_mode<double>(grid, 32 * plan.nw, plan.smem_f64, stream, P, A);
+        launch_mode<double>(grid, plan.smem_f64, stream, P, A);
     }
     return (int)cudaGetLastError();
 }

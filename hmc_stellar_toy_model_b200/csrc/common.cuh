@@ -10,10 +10,7 @@ constexpr int kWarp = 32;
 // Lanes per chain of the one-star kernel.  Measured on the headline workload: 16 lanes 734, 8 lanes 1104, 4 lanes
 // 1210 M star-steps/s -- fewer lanes replicate the per-chain scalar work and the table exponentials less; 2 lanes
 // would need more than 255 registers.
-#ifndef SRHMC_LPC
-#define SRHMC_LPC 4
-#endif
-constexpr int kChainLPC = SRHMC_LPC;
+constexpr int kChainLPC = 4;
 constexpr int kChainGroup = 32 / kChainLPC;   // chains per warp: the unit of its work scheduler
 
 // Problem constants snapshot (host fills it from srhmc_config).

@@ -9,9 +9,9 @@
 
 namespace srhmc {
 
+// Dynamic shared memory and resident blocks per SM of the one-star kernel for each image layout.  A block is one warp
+// holding kChainGroup chains.
 struct ChainLaunchPlan {
-    int lpc = 16;   // lanes per chain
-    int nw = 4;     // warps per block
     size_t smem_f64 = 0, smem_u32 = 0, smem_u16 = 0, smem_u16_f32 = 0;
     int blocks_per_sm_f64 = 0, blocks_per_sm_u32 = 0, blocks_per_sm_u16 = 0, blocks_per_sm_u16_f32 = 0;
 };

@@ -9,7 +9,6 @@
 // One CTA per (group of chains, variable).  Chain layout X[chain][row][d] (the layout of q_chain).  All reductions are
 // fixed-order (block_sum), so the numbers are reproducible run to run.
 #include <algorithm>
-#include <cstdlib>
 
 #include "kernels_api.h"
 
@@ -35,7 +34,7 @@ __device__ __forceinline__ const double* sample_ptr(const double* X, const Stats
 // Sum of the autocorrelations that enters n_eff (utils.py:137-165) from the variogram at lag t, `vario(t)`: rho_t = 1 - V_t / (2 var);
 // nothing when rho_1 < 0.05, otherwise the sum of rho_1 .. rho_t up to the first odd t with rho_{t+1} + rho_{t+2} < 0 (or
 // t = n - 2), clamped at 0.  The reference's rho_t list index i holds lag i + 1.  Every caller thread follows the same control
-// flow.  Shared by conv_stats_final_kernel and conv_stats_var_kernel.
+// flow.  Shared by all three statistics kernels.
 template <class Vario>
 __device__ __forceinline__ double ess_sum_rho(int n, double var, const Vario& vario) {
     const double rho1 = 1.0 - vario(1) / (2.0 * var);
@@ -108,23 +107,8 @@ __global__ void __launch_bounds__(256) conv_stats_kernel(const double* __restric
         block_sum<1>(a, red);
         return a[0] / ((double)m * (double)(n - t));
     };
-    // effective sample size (utils.py:137-165); every thread follows the same control flow
-    const double rho1 = 1.0 - variogram(1) / (2.0 * var);
-    const double rho2 = 1.0 - variogram(2) / (2.0 * var);
-    double sum_rho = 0.0;
-    if (!(rho1 < 5e-2)) {
-        // rho_t list of the reference: index i holds lag i + 1.  Loop invariant: prefix = sum(rho_t[:t]), cur = rho_t[t].
-        double prefix = rho1, cur = rho2;
-        int t = 1;
-        while (t < n - 2) {
-            const double next = 1.0 - variogram(t + 2) / (2.0 * var);  // appended as rho_t[t + 1]
-            if ((t & 1) && (cur + next) < 0.0) break;
-            prefix += cur;
-            cur = next;
-            ++t;
-        }
-        sum_rho = prefix < 0.0 ? 0.0 : prefix;
-    }
+    // effective sample size (utils.py:137-165); every thread calls the variogram, and so block_sum, equally often
+    const double sum_rho = ess_sum_rho(n, var, variogram);
     if (threadIdx.x == 0) {
         R_out[blockIdx.x] = R;
         neff_out[blockIdx.x] = (double)m * (double)n / (1.0 + 2.0 * sum_rho);
@@ -325,8 +309,7 @@ int conv_stats_launch(cudaStream_t stream, const double* X, long long rows, int 
                       double* scratch, double* R, double* neff) {
     const StatsGeom G = stats_geom(rows, d, cpg, thin, warm);
     const size_t nout = (size_t)n_groups * d, m = 2 * (size_t)cpg;
-    const char* old = std::getenv("SRHMC_STATS_SINGLE_CTA");
-    if (G.n > kStatsMaxN || G.n < 3 || (old && old[0] == '1')) {
+    if (G.n > kStatsMaxN || G.n < 3) {
         conv_stats_kernel<<<n_groups * d, 256, 0, stream>>>(X, G, scratch, R, neff);   // one CTA per (group, variable)
         return (int)cudaGetLastError();
     }

@@ -125,10 +125,6 @@ int configure(srhmc_ctx* c) {
     int threads = 256;
     if ((size_t)R * C >= 4096 || N > 256) threads = 512;
     if ((size_t)R * C <= 256 && N <= 64) threads = 128;
-    if (const char* env = std::getenv("SRHMC_FIELD_THREADS")) {  // tuning / experiments
-        const int t = std::atoi(env);
-        if (t == 128 || t == 256 || t == 512) threads = t;
-    }
     c->threads = threads;
     c->kc = pick_kernel(R, C, threads / 32);
     // table strides: rows / columns rounded up to the warp tile, plus 16 bytes so that the tables of consecutive stars
@@ -145,13 +141,8 @@ int configure(srhmc_ctx* c) {
         if (base + per + 64 > budget) return 0;
         return (int)std::min<size_t>((size_t)nwant, (budget - base - 64) / per);
     };
-    size_t budget = 112 * 1024;
-    if (const char* env = std::getenv("SRHMC_FIELD_SMEM_KB")) budget = (size_t)std::max(16, std::atoi(env)) * 1024;
-    int kc = fit(budget, true);
+    int kc = fit(112 * 1024, true);
     bool dsm = true;
-    if (const char* env = std::getenv("SRHMC_FIELD_D_GLOBAL")) {
-        if (env[0] == '1') { dsm = false; kc = fit(budget, false); }
-    }
     if (kc < std::min(nwant, 24)) kc = fit(kSmemMax, true);
     if (kc < std::min(nwant, 8)) {
         const int kg = fit(kSmemMax, false);
@@ -349,9 +340,8 @@ int srhmc_create(const srhmc_config* cfg, srhmc_ctx** out) {
     P.cLh = std::exp(-(double)(kChainLPC * kChainLPC) / (2.0 * sigma * sigma));
     {
         // rows whose Gaussian weight is below 2^-bits of the peak are skipped by the one-star kernel (its 24-column window
-        // cuts at 2^-47 for the default PSF); SRHMC_CHAIN_WCUT_BITS overrides for A/B measurements
-        double bits = 46.0;
-        if (const char* env = std::getenv("SRHMC_CHAIN_WCUT_BITS")) bits = std::max(20.0, std::min(1000.0, std::atof(env)));
+        // cuts at 2^-47 for the default PSF)
+        const double bits = 46.0;
         P.wcut = std::sqrt(bits * M_LN2 * 2.0 * sigma * sigma);
     }
     P.f_lim = cfg->f_lim;
@@ -468,9 +458,7 @@ static int finish_data(srhmc_ctx* c, size_t n) {
         CU_TRY(cudaMemcpyAsync(&flags, c->flag.ptr, 4, cudaMemcpyDeviceToHost, c->stream));
         CU_TRY(cudaStreamSynchronize(c->stream));
         const char* off = std::getenv("SRHMC_DISABLE_U32_IMAGES");   // both integer layouts off
-        const char* off16 = std::getenv("SRHMC_DISABLE_U16_IMAGES");
-        if (!(off && off[0] == '1') && (flags & 1) == 0)
-            c->d_int_bytes = ((flags & 2) == 0 && !(off16 && off16[0] == '1')) ? 2 : 4;
+        if (!(off && off[0] == '1') && (flags & 1) == 0) c->d_int_bytes = (flags & 2) == 0 ? 2 : 4;
     }
     CU_TRY(cudaStreamSynchronize(c->stream));
     c->have_data = true;

@@ -1,6 +1,6 @@
 #!/bin/bash
 # ncu evidence for the headline workload (run under gpurun, one GPU).  Usage: scripts/profile_c2.sh <tag>
-# Environment (SRHMC_CHAIN_LPC, SRHMC_CHAIN_BLOCKS_PER_SM) is inherited by the benchmark processes.
+# Environment is inherited by the benchmark processes.
 set -u
 TAG=${1:-r1}
 CMD="python bench.py --workload c2 --steps 2 --warmup 3 --no-cpu --chains-per-mag 1000 --niter 100 --e2e-steps 1"

@@ -298,20 +298,27 @@ def test_device_math_accuracy():
 
 
 def test_u32_image_path_is_lossless(monkeypatch):
-    """Integer-valued data takes the compact uint32 shared-memory layout; results are bit-identical to the
-    float64 layout, and non-integer data silently uses float64."""
+    """Integer-valued data take a compact integer shared-memory layout; results are bit-identical to the float64
+    layout (SRHMC_DISABLE_U32_IMAGES=1), and non-integer data silently use float64.  The golden image (largest count 46)
+    takes the uint16 layout.  The same image with one corner pixel raised to 70 000 takes the uint32 layout: that pixel
+    sets bit 1 of the flags of to_counts_kernel, and the context then keeps the uint32 copy.  The pixel lies 16 rows and
+    16 columns from the star, where the PSF weight is below 2^-80, so the chain still follows the star."""
     g = golden("chain_one_star_m21")
     S = setup_from(g)
     q0 = so.format_q(S, g["q_model"])
-    outs = []
-    for off in ("0", "1"):
-        monkeypatch.setenv("SRHMC_DISABLE_U32_IMAGES", off)
-        with make_ctx(S, max_stars=1) as ctx:
-            ctx.set_data(S.D)
-            r = ctx.run(q0[None], 20, 10, 0.2, normals=g["normals"][None, :21], lnu=g["lnu"][None, :21], g_ff2=S.g_ff2)
-            outs.append(r)
-    assert np.array_equal(outs[0].q_chain, outs[1].q_chain) and np.array_equal(outs[0].E_chain, outs[1].E_chain)
-    assert np.array_equal(outs[0].A_chain, outs[1].A_chain)
+    assert S.D.max() <= 65535 and min(q0[1], q0[2]) > 12
+    D32 = S.D.copy()
+    D32[0, 0] = 70000.0
+    for D in (S.D, D32):
+        outs = []
+        for off in ("0", "1"):
+            monkeypatch.setenv("SRHMC_DISABLE_U32_IMAGES", off)
+            with make_ctx(S, max_stars=1) as ctx:
+                ctx.set_data(D)
+                r = ctx.run(q0[None], 20, 10, 0.2, normals=g["normals"][None, :21], lnu=g["lnu"][None, :21], g_ff2=S.g_ff2)
+                outs.append(r)
+        assert np.array_equal(outs[0].q_chain, outs[1].q_chain) and np.array_equal(outs[0].E_chain, outs[1].E_chain)
+        assert np.array_equal(outs[0].A_chain, outs[1].A_chain)
 
 
 def test_chunked_scheduler_is_bit_identical(monkeypatch):

@@ -208,11 +208,13 @@ def test_bigfield_mock_data_tiled_equals_untiled():
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("thin,warm", [(5, 0), (1, 37), (3, 100)])
-def test_convergence_stats_device_matches_oracle(thin, warm):
+# rows 1700 (n = 850 samples per split chain) takes the single-CTA kernel, the others the chain-parallel pair
+@pytest.mark.parametrize("thin,warm,rows", [(5, 0, 500), (1, 37, 500), (3, 100, 500), (1, 0, 1700)],
+                         ids=["5-0", "1-37", "3-100", "1-0-1700"])
+def test_convergence_stats_device_matches_oracle(thin, warm, rows):
     from hmc_stellar_toy_model_b200 import utils
 
-    x = _ar1_chains(7, 12, 500, 3, 0.7)
+    x = _ar1_chains(7, 12, rows, 3, 0.7)
     R0, n0 = so.convergence_stats(x, thin, warm)
     R1, n1 = utils.convergence_stats(x, thin_rate=thin, warm_up_num=warm)
     assert relerr(R1, R0) < 1e-12 and relerr(n1, n0) < 1e-9
