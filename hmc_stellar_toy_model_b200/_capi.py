@@ -122,6 +122,14 @@ class RunArgs(C.Structure):
     ]
 
 
+class LaunchPlan(C.Structure):
+    """struct srhmc_launch_plan"""
+
+    _fields_ = [(n, C.c_int32) for n in ("threads", "tile_rows", "tile_cols", "chunk_stars", "image_in_smem",
+                                         "compact_tables", "chain_kernel", "int_image_bytes")] + \
+               [("smem_bytes", C.c_int64)]
+
+
 class BigConfig(C.Structure):
     """struct srhmc_big_config"""
 
@@ -159,6 +167,7 @@ SIGNATURES = {
     "srhmc_synchronize": (C.c_int, [C.c_void_p]),
     "srhmc_last_kernel_ms": (C.c_int, [C.c_void_p, C.POINTER(C.c_float)]),
     "srhmc_launch_count": (C.c_int64, [C.c_void_p]),
+    "srhmc_get_launch_plan": (C.c_int, [C.c_void_p, C.POINTER(LaunchPlan)]),
     "srhmc_host_alloc": (C.c_void_p, [C.c_uint64]),
     "srhmc_host_free": (C.c_int, [C.c_void_p]),
     "srhmc_set_data": (C.c_int, [C.c_void_p, c_double_p, C.c_int64]),

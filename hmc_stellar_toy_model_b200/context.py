@@ -85,6 +85,14 @@ class RHMCContext:
     def launch_count(self):
         return int(self._lib.srhmc_launch_count(self._h))
 
+    def launch_plan(self):
+        """How the CTA-per-field kernel was configured for this context (struct srhmc_launch_plan as a dict):
+        threads, tile_rows, tile_cols, chunk_stars, image_in_smem, compact_tables, chain_kernel, int_image_bytes
+        (meaningful after set_data) and smem_bytes."""
+        plan = _capi.LaunchPlan()
+        check(self._lib.srhmc_get_launch_plan(self._h, C.byref(plan)))
+        return {name: int(getattr(plan, name)) for name, _ in plan._fields_}
+
     def _nstars(self, nstars):
         if nstars is None:
             return None

@@ -27,7 +27,7 @@ struct FieldParams {
     // compact-table evaluation of the CTA-per-field kernel (field_kernel.cuh, "v3"): every star keeps a TL-row table of
     // {ex, ex dx} pairs and a (TL+1)-column table of f ey over a window clamped inside the image, so that all stars of a
     // crowded field fit one table build and the gradient pass needs no bounds handling
-    int v3;            // 1: enabled (patch-limited PSF, rad <= 12, even C, R >= TL, C >= TL+1, all tables fit at once)
+    int v3;            // 1: enabled (patch-limited PSF, rad <= 12, C even (FP64) / C % 4 == 0 (FP32), R >= TL, C >= TL+1, all tables fit)
     int tl;            // TL = 2 rad + 1
     int rs, cs;        // strides: row table in pairs (odd: conflict-free 16-byte stores), column table in entries (odd)
     double inv2s2;     // 1/(2 sigma^2)

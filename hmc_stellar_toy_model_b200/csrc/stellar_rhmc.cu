@@ -161,10 +161,13 @@ int configure(srhmc_ctx* c) {
     c->P_ls = P;
     c->smem_ls = c->smem;
     c->dsm_ls = c->d_in_smem;
-    // compact-table evaluation (field_kernel.cuh "v3") when the PSF is patch-limited and every star's tables fit at once
+    // compact-table evaluation (field_kernel.cuh "v3") when the PSF is patch-limited and every star's tables fit at once.
+    // render_v3 reads four image pixels of a row with one 16-byte load at column offsets that are multiples of 4, so a
+    // float image needs C % 4 == 0 for every row to start on a 16-byte boundary (doubles load as two 16-byte pairs: even C)
     {
         const int TL = 2 * g.patch_radius + 1;
-        bool want = g.patch_radius > 0 && g.patch_radius <= 12 && (C % 2 == 0) && R >= TL && C >= TL + 1 && !P.hess && N >= 1;
+        bool want = g.patch_radius > 0 && g.patch_radius <= 12 && (C % (prec == 64 ? 2 : 4) == 0) && R >= TL && C >= TL + 1 &&
+                    !P.hess && N >= 1;
         if (const char* env = std::getenv("SRHMC_FIELD_V3"))
             if (env[0] == '0') want = false;
         if (want) {
@@ -434,6 +437,20 @@ int srhmc_last_kernel_ms(srhmc_ctx* c, float* ms) {
 }
 
 int64_t srhmc_launch_count(srhmc_ctx* c) { return c ? c->launches : 0; }
+
+int srhmc_get_launch_plan(srhmc_ctx* c, srhmc_launch_plan* out) {
+    if (!c || !out) return fail(SRHMC_ERR_INVALID, "null argument");
+    out->threads = c->threads;
+    out->tile_rows = c->kc.mr;
+    out->tile_cols = c->kc.mc;
+    out->chunk_stars = c->P.Kc;
+    out->image_in_smem = c->d_in_smem;
+    out->compact_tables = c->P.v3;
+    out->chain_kernel = c->chain_ok ? 1 : 0;
+    out->int_image_bytes = c->d_int_bytes;
+    out->smem_bytes = (int64_t)c->smem;
+    return 0;
+}
 
 // after the float64 images are in place on the device (c->D for the FP64 build, c->Dstage for the FP32 build): the
 // reduced-precision / exact-integer copies the kernels read

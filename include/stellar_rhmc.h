@@ -173,6 +173,19 @@ int srhmc_last_kernel_ms(srhmc_ctx* ctx, float* ms);
 /* Number of kernels this context has launched since creation. */
 int64_t srhmc_launch_count(srhmc_ctx* ctx);
 
+/* How srhmc_create configured the CTA-per-field kernel for this context's shape, star count, precision and patch radius
+ * (read-only; lets a caller or test check which kernel variant a shape runs). */
+typedef struct srhmc_launch_plan {
+    int32_t threads, tile_rows, tile_cols; /* threads per CTA; a warp renders (8 tile_rows) x (4 tile_cols) pixels */
+    int32_t chunk_stars;                   /* stars per table chunk of the chunked-table path */
+    int32_t image_in_smem;                 /* 1: the data image is copied to shared memory; 0: read from global memory */
+    int32_t compact_tables;                /* 1: compact-table path (patch-limited PSF, all stars' tables at once) */
+    int32_t chain_kernel;                  /* 1: one-star batches may run on the warp-resident chain kernel */
+    int32_t int_image_bytes;               /* integer image copy the chain kernel reads (2, 4, or 0); valid after set_data */
+    int64_t smem_bytes;                    /* dynamic shared memory per CTA */
+} srhmc_launch_plan;
+int srhmc_get_launch_plan(srhmc_ctx* ctx, srhmc_launch_plan* out);
+
 /* Pinned host memory helpers for callers that want asynchronous copies. */
 void* srhmc_host_alloc(uint64_t bytes);
 int srhmc_host_free(void* p);

@@ -217,9 +217,11 @@ def _inverse_distance(q):
     return 1.0 / R, X, Y
 
 
-def potential(S: Setup, q, f_pos=False):
+def potential(S: Setup, q, f_pos=False, rad=0):
     """V(q): Poisson negative log-likelihood + prior + repulsion
-    (sampler_RHMC.py:294-351).  +inf outside the support."""
+    (sampler_RHMC.py:294-351).  +inf outside the support.  rad > 0: the
+    likelihood and prior come from patch_eval (every PSF cut to (2 rad + 1)^2
+    pixels), the repulsion term is unchanged."""
     n = q.size // 3
     if f_pos:
         for k in range(n):
@@ -229,17 +231,20 @@ def potential(S: Setup, q, f_pos=False):
         x, y = q[3 * k + 1 : 3 * k + 3]
         if (x < -1) or (x > S.num_rows + 1) or (y < -1) or (y > S.num_cols + 1):
             return np.inf
-    v_prior = 0.0
-    vpc = S.prior_const() if (S.V_prior_const is not None or S.fmin is not None) else 0.0
-    lam = np.ones_like(S.D) * S.B_count
-    for k in range(n):
-        f, x, y = q[3 * k : 3 * k + 3]
-        lam += f * gauss_psf(S.num_rows, S.num_cols, x, y, S.PSF_FWHM_pix)
+    if rad > 0:
+        V = patch_eval(S, S.D, q, rad)[0]
+    else:
+        v_prior = 0.0
+        vpc = S.prior_const() if (S.V_prior_const is not None or S.fmin is not None) else 0.0
+        lam = np.ones_like(S.D) * S.B_count
+        for k in range(n):
+            f, x, y = q[3 * k : 3 * k + 3]
+            lam += f * gauss_psf(S.num_rows, S.num_cols, x, y, S.PSF_FWHM_pix)
+            if S.use_prior:
+                v_prior += S.alpha * np.log(f) + vpc
+        V = np.sum(lam - S.D * np.log(lam))
         if S.use_prior:
-            v_prior += S.alpha * np.log(f) + vpc
-    V = np.sum(lam - S.D * np.log(lam))
-    if S.use_prior:
-        V += v_prior
+            V += v_prior
     if S.use_Vc:
         inv_r, _, _ = _inverse_distance(q)
         V += 0.5 * S.beta * np.sum(inv_r**S.Vc_r_pow)
@@ -251,26 +256,33 @@ def kinetic(p, H):
     return (np.sum(p**2 / H) + np.sum(np.log(np.abs(H)))) / 2.0
 
 
-def grad_potential(S: Setup, q):
-    """dV/dq as residual-weighted PSF reductions (sampler_RHMC.py:365-425)."""
+def grad_potential(S: Setup, q, rad=0):
+    """dV/dq as residual-weighted PSF reductions (sampler_RHMC.py:365-425).
+    rad > 0: the pixel part comes from patch_eval (PSFs cut to (2 rad + 1)^2
+    pixels); the prior and repulsion terms are unchanged."""
     n = q.size // 3
-    g = np.zeros(q.size)
-    lam = np.ones_like(S.D) * S.B_count
-    for k in range(n):
-        f, x, y = q[3 * k : 3 * k + 3]
-        lam += f * gauss_psf(S.num_rows, S.num_cols, x, y, S.PSF_FWHM_pix)
-    rho = (S.D / lam) - 1.0
-    li = np.arange(0, S.num_rows)[:, None] * np.ones((1, S.num_cols), dtype=int)
-    mj = np.arange(0, S.num_cols)[None, :] * np.ones((S.num_rows, 1), dtype=int)
-    var = (S.PSF_FWHM_pix / FWHM_TO_SIGMA) ** 2
+    if rad > 0:
+        g = patch_eval(S, S.D, q, rad)[1].ravel()
+    else:
+        g = np.zeros(q.size)
+        lam = np.ones_like(S.D) * S.B_count
+        for k in range(n):
+            f, x, y = q[3 * k : 3 * k + 3]
+            lam += f * gauss_psf(S.num_rows, S.num_cols, x, y, S.PSF_FWHM_pix)
+        rho = (S.D / lam) - 1.0
+        li = np.arange(0, S.num_rows)[:, None] * np.ones((1, S.num_cols), dtype=int)
+        mj = np.arange(0, S.num_cols)[None, :] * np.ones((S.num_rows, 1), dtype=int)
+        var = (S.PSF_FWHM_pix / FWHM_TO_SIGMA) ** 2
+        for k in range(n):
+            f, x, y = q[3 * k : 3 * k + 3]
+            psf = gauss_psf(S.num_rows, S.num_cols, x, y, S.PSF_FWHM_pix)
+            g[3 * k] = -np.sum(rho * psf)
+            g[3 * k + 1] = -np.sum(rho * (li - x + 0.5) * psf) * f / var
+            g[3 * k + 2] = -np.sum(rho * (mj - y + 0.5) * psf) * f / var
     if S.use_Vc:
         inv_r, X, Y = _inverse_distance(q)
     for k in range(n):
         f, x, y = q[3 * k : 3 * k + 3]
-        psf = gauss_psf(S.num_rows, S.num_cols, x, y, S.PSF_FWHM_pix)
-        g[3 * k] = -np.sum(rho * psf)
-        g[3 * k + 1] = -np.sum(rho * (li - x + 0.5) * psf) * f / var
-        g[3 * k + 2] = -np.sum(rho * (mj - y + 0.5) * psf) * f / var
         if S.use_prior:
             g[3 * k] += S.alpha / f
         if S.use_Vc:
@@ -315,9 +327,9 @@ def patch_eval(S: Setup, D, q, rad=12):
     return V, g
 
 
-def dphidq(S: Setup, q):
+def dphidq(S: Setup, q, rad=0):
     """grad V + half the log-det gradient on flux slots (sampler_RHMC.py:448-465)."""
-    g = grad_potential(S, q)
+    g = grad_potential(S, q, rad=rad)
     H, dH = metric(S, q, grad=True)
     for k in range(q.size // 3):
         g[3 * k] += ((dH[3 * k] / H[3 * k]) + (2 * dH[3 * k + 1] / H[3 * k + 1])) / 2.0
@@ -338,31 +350,57 @@ def dtaudp(S: Setup, q, p):
     return p / metric(S, q)
 
 
-def rhmc_step(S: Setup, q, p, delta=1e-6, counter_max=1000, counters=None):
+def _per_star_fixed_point(x, update, delta, counter_max):
+    """x <- update(x) for every star [3 slots] until that star's own max |x - x'| <= delta or counter_max iterations
+    (srhmc_config.fixed_point_mode = 1).  A star's update reads only its own slots, so the stars still iterating see
+    the same values as if each ran alone.  Returns x and the largest per-star iteration count."""
+    n = x.size // 3
+    cnt = np.zeros(n, dtype=int)
+    live = cnt < counter_max
+    while live.any():
+        x_new = update(x)
+        more = np.max(np.abs(x - x_new).reshape(n, 3), axis=1) > delta
+        x = np.where(np.repeat(live, 3), x_new, x)
+        cnt += live
+        live &= more & (cnt < counter_max)
+    return x, int(cnt.max(initial=0))
+
+
+def rhmc_step(S: Setup, q, p, delta=1e-6, counter_max=1000, counters=None, rad=0, per_star=False):
     """One generalised (implicit) leapfrog step with reflections
     (base_class.RHMC_single_step, sampler_RHMC.py:522-566; SURVEY appendix A4).
-    `counters`, if a list, receives the two fixed-point iteration counts."""
+    `counters`, if a list, receives the two fixed-point iteration counts.
+    rad > 0: PSFs cut to (2 rad + 1)^2 pixels (see potential).  per_star: each
+    star's two fixed-point loops stop on their own (fixed_point_mode = 1); the
+    counts are then the maxima over the stars."""
     h = S.dt / 2.0
-    p = p - h * dphidq(S, q)
+    p = p - h * dphidq(S, q, rad=rad)
 
     rho0 = np.copy(p)
-    dp, cnt_p = np.inf, 0
-    while (dp > delta) and (cnt_p < counter_max):
-        p_new = rho0 - h * dtaudq(S, q, p)
-        dp = np.max(np.abs(p - p_new))
-        p = np.copy(p_new)
-        cnt_p += 1
+    if per_star:
+        p, cnt_p = _per_star_fixed_point(p, lambda pp: rho0 - h * dtaudq(S, q, pp), delta, counter_max)
+    else:
+        dp, cnt_p = np.inf, 0
+        while (dp > delta) and (cnt_p < counter_max):
+            p_new = rho0 - h * dtaudq(S, q, p)
+            dp = np.max(np.abs(p - p_new))
+            p = np.copy(p_new)
+            cnt_p += 1
 
     sig0 = np.copy(q)
-    dq, cnt_q = np.inf, 0
-    while (dq > delta) and (cnt_q < counter_max):
-        q_new = sig0 + h * (dtaudp(S, sig0, p) + dtaudp(S, q, p))
-        dq = np.max(np.abs(q - q_new))
-        q = np.copy(q_new)
-        cnt_q += 1
+    if per_star:
+        q, cnt_q = _per_star_fixed_point(q, lambda qq: sig0 + h * (dtaudp(S, sig0, p) + dtaudp(S, qq, p)), delta,
+                                         counter_max)
+    else:
+        dq, cnt_q = np.inf, 0
+        while (dq > delta) and (cnt_q < counter_max):
+            q_new = sig0 + h * (dtaudp(S, sig0, p) + dtaudp(S, q, p))
+            dq = np.max(np.abs(q - q_new))
+            q = np.copy(q_new)
+            cnt_q += 1
 
     p = p - h * dtaudq(S, q, p)
-    p = p - h * dphidq(S, q)
+    p = p - h * dphidq(S, q, rad=rad)
 
     for k in range(q.size // 3):
         f, x, y = q[3 * k : 3 * k + 3]
@@ -389,12 +427,13 @@ class Chains:
 
 
 def run_rhmc(S: Setup, q0_flat, normals, lnu, niter, nsteps, dt, f_pos=True, delta=1e-6,
-             counter_max=1000, schedule_g_ff2=None, schedule_beta=None):
+             counter_max=1000, schedule_g_ff2=None, schedule_beta=None, rad=0):
     """Within-model RHMC chain (multi_gym.run_RHMC move 0, sampler_RHMC.py:1009-1083;
     SURVEY appendix A5) with injected draws: normals[l] replaces
     np.random.randn(3N) of iteration l and lnu[l] replaces log(np.random.random(1)).
     Row l of every chain array is the state at the START of iteration l; there are
-    niter+1 iterations and the outcome of the last is never stored."""
+    niter+1 iterations and the outcome of the last is never stored.  rad > 0: PSFs
+    cut to (2 rad + 1)^2 pixels (see potential)."""
     S = S.clone(dt=dt)
     d = q0_flat.size
     out = Chains(
@@ -409,14 +448,14 @@ def run_rhmc(S: Setup, q0_flat, normals, lnu, niter, nsteps, dt, f_pos=True, del
             S.beta = schedule_beta[l]
         H = metric(S, q)
         p = normals[l] * np.sqrt(H)
-        v0 = potential(S, q, f_pos=f_pos)
+        v0 = potential(S, q, f_pos=f_pos, rad=rad)
         t0 = kinetic(p, H)
         e0 = v0 + t0
         out.q[l], out.p[l], out.V[l], out.E[l], out.T[l] = q, p, v0, e0, t0
         for _ in range(nsteps):
-            q, p = rhmc_step(S, q, p, delta=delta, counter_max=counter_max)
+            q, p = rhmc_step(S, q, p, delta=delta, counter_max=counter_max, rad=rad)
         H = metric(S, q)
-        e1 = potential(S, q, f_pos=f_pos) + kinetic(p, H)
+        e1 = potential(S, q, f_pos=f_pos, rad=rad) + kinetic(p, H)
         dE = e1 - e0
         if (dE < 0) or (lnu[l] < -dE):
             out.A[l] = True
@@ -425,10 +464,11 @@ def run_rhmc(S: Setup, q0_flat, normals, lnu, niter, nsteps, dt, f_pos=True, del
     return out
 
 
-def run_single_rhmc(S: Setup, q0_flat, p0, nsteps, dt, f_pos=False, delta=1e-6, counter_max=100):
+def run_single_rhmc(S: Setup, q0_flat, p0, nsteps, dt, f_pos=False, delta=1e-6, counter_max=100, rad=0):
     """One long implicit-solver trajectory recording V-V0, T-T0 every step
     (single_gym.run_single_RHMC, solver="implicit", sampler_RHMC.py:649-783;
-    SURVEY appendix A6).  Row 0 keeps q0, p0 and zeros for the energies."""
+    SURVEY appendix A6).  Row 0 keeps q0, p0 and zeros for the energies.
+    rad > 0: PSFs cut to (2 rad + 1)^2 pixels (see potential)."""
     S = S.clone(dt=dt)
     d = q0_flat.size
     out = Chains(q=np.zeros((nsteps + 1, d)), p=np.zeros((nsteps + 1, d)), E=np.zeros(nsteps + 1),
@@ -437,13 +477,13 @@ def run_single_rhmc(S: Setup, q0_flat, p0, nsteps, dt, f_pos=False, delta=1e-6, 
     p = np.copy(p0)
     H = metric(S, q)
     out.q[0], out.p[0] = q, p
-    v0 = potential(S, q, f_pos=f_pos)
+    v0 = potential(S, q, f_pos=f_pos, rad=rad)
     t0 = kinetic(p, H)
     for i in range(1, nsteps + 1):
-        q, p = rhmc_step(S, q, p, delta=delta, counter_max=counter_max)
+        q, p = rhmc_step(S, q, p, delta=delta, counter_max=counter_max, rad=rad)
         H = metric(S, q)
         out.q[i], out.p[i] = q, p
-        out.V[i] = potential(S, q, f_pos=f_pos) - v0
+        out.V[i] = potential(S, q, f_pos=f_pos, rad=rad) - v0
         out.T[i] = kinetic(p, H) - t0
         out.E[i] = out.V[i] + out.T[i]
     return out
