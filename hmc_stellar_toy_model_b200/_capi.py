@@ -130,6 +130,19 @@ class LaunchPlan(C.Structure):
                [("smem_bytes", C.c_int64)]
 
 
+class ChainPlan(C.Structure):
+    """struct srhmc_chain_plan"""
+
+    _fields_ = [(n, C.c_int32) for n in ("chain_kernel", "window_cols", "image_bytes", "pixel_f32", "blocks_per_sm",
+                                         "tab_stride")] + [("smem_bytes", C.c_int64)]
+
+
+class ChainLayout(C.Structure):
+    """struct srhmc_chain_layout_t"""
+
+    _fields_ = [(n, C.c_int64) for n in ("log_bytes", "img_stride", "tab_base", "tab_stride", "smem_bytes")]
+
+
 class BigConfig(C.Structure):
     """struct srhmc_big_config"""
 
@@ -168,6 +181,9 @@ SIGNATURES = {
     "srhmc_last_kernel_ms": (C.c_int, [C.c_void_p, C.POINTER(C.c_float)]),
     "srhmc_launch_count": (C.c_int64, [C.c_void_p]),
     "srhmc_get_launch_plan": (C.c_int, [C.c_void_p, C.POINTER(LaunchPlan)]),
+    "srhmc_get_chain_plan": (C.c_int, [C.c_void_p, C.POINTER(ChainPlan)]),
+    "srhmc_chain_layout": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.POINTER(ChainLayout)]),
+    "srhmc_chain_column_exponent": (C.c_double, [C.c_int32, C.c_double, C.c_int32]),
     "srhmc_host_alloc": (C.c_void_p, [C.c_uint64]),
     "srhmc_host_free": (C.c_int, [C.c_void_p]),
     "srhmc_set_data": (C.c_int, [C.c_void_p, c_double_p, C.c_int64]),
@@ -238,6 +254,13 @@ def measure_fma_peak(device=0, precision=64):
     ms = C.c_float()
     check(lib.srhmc_measure_fma_peak(int(device), int(precision), C.byref(tf), C.byref(ms)))
     return float(tf.value), float(ms.value)
+
+def chain_layout(rows, image_bytes, pixel_f32=False):
+    """Shared-memory layout of one block of the one-star kernel (struct srhmc_chain_layout_t as a dict); no device needed."""
+    out = ChainLayout()
+    check(load_library().srhmc_chain_layout(int(rows), int(image_bytes), int(bool(pixel_f32)), C.byref(out)))
+    return {name: int(getattr(out, name)) for name, _ in out._fields_}
+
 
 _lib = None
 

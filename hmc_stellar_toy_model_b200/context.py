@@ -93,6 +93,14 @@ class RHMCContext:
         check(self._lib.srhmc_get_launch_plan(self._h, C.byref(plan)))
         return {name: int(getattr(plan, name)) for name, _ in plan._fields_}
 
+    def chain_plan(self):
+        """What a launch of one-star fields runs now on the warp-resident one-star kernel (struct srhmc_chain_plan as a
+        dict): chain_kernel, window_cols, image_bytes, pixel_f32, blocks_per_sm, tab_stride and smem_bytes; meaningful
+        after set_data."""
+        plan = _capi.ChainPlan()
+        check(self._lib.srhmc_get_chain_plan(self._h, C.byref(plan)))
+        return {name: int(getattr(plan, name)) for name, _ in plan._fields_}
+
     def _nstars(self, nstars):
         if nstars is None:
             return None

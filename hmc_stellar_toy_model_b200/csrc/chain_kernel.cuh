@@ -149,8 +149,24 @@ __device__ __forceinline__ void rcp_row(const double (&lam)[NCS], double (&r)[NC
 
 // Elements of padding after each chain image so that the chains of one warp sit on disjoint shared-memory banks:
 // the LPC lanes of a chain read LPC consecutive pixels, so shifting chain g by g*LPC pixels tiles the banks.
-template <typename DT>
 __host__ __device__ constexpr int chain_pad(int lpc) { return lpc; }
+
+// Dynamic shared memory of one single-warp block (kernel and host both take it from here): the log table, then the
+// kChainGroup chain images, then the kChainGroup row tables.  A row table is a double2 per image row (plus, in the FP32
+// build, a float2 per row after it) and is read and written with 128-bit accesses, so every table must start on a
+// 16-byte boundary: the FP32 stride 24 R + 16 is rounded up (it is 8 bytes short for odd R); the double stride 16 R + 16
+// and the image block before the tables are multiples of 16 already.
+__host__ __device__ constexpr ChainLayout chain_layout(int R, size_t elem, bool f32) {
+    ChainLayout L{};
+    L.log_bytes = kLogTableSize * sizeof(double2);
+    L.img_elems = (size_t)R * kChainCS + chain_pad(kChainLPC);
+    L.img_bytes = L.img_elems * elem;
+    const size_t tab = (size_t)R * (sizeof(double2) + (f32 ? sizeof(float2) : 0)) + kChainTabPad;
+    L.tab_bytes = f32 ? (tab + 15) & ~(size_t)15 : tab;
+    L.tab_base = L.log_bytes + kChainGroup * L.img_bytes;
+    L.smem_bytes = L.tab_base + kChainGroup * L.tab_bytes;
+    return L;
+}
 
 template <int LPC>
 __device__ __forceinline__ double group_sum(double v) {
@@ -529,16 +545,18 @@ __global__ void __maxnreg__(MAXREG) chain_kernel(const __grid_constant__ FieldPa
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
     const int grp = lane / LPC, sub = lane % LPC;
     const int R = P.R, C = P.C;
-    // per-chain image stride padded by LPC elements: the GPW chains of a warp then sit on disjoint shared-memory banks
-    const size_t img_elems = (size_t)R * kChainCS + chain_pad<DT>(LPC);
-    constexpr size_t kRowTab = sizeof(double2) + (sizeof(PT) == 4 ? sizeof(float2) : 0);   // per image row and chain
-    // row tables of the GPW chains of a warp: 16 bytes of padding per chain, so that entry i of chain g sits 4 (g + i) banks
-    // into shared memory and the warp's 8 distinct 16-byte entries of a row fill one 128-byte wavefront (unpadded, the
-    // 512-byte table stride put all eight on the same four banks: an 8-way conflict on every row-table load and store)
-    const size_t tab_bytes = (size_t)R * kRowTab + kChainTabPad;
+    static_assert(GPW == kChainGroup && LPC == kChainLPC, "chain_layout describes kChainGroup chains of kChainLPC lanes");
+    // per-chain image stride padded by LPC elements: the GPW chains of a warp then sit on disjoint shared-memory banks.
+    // Row tables: 16 bytes of padding per chain, so that entry i of chain g sits 4 (g + i) banks into shared memory and the
+    // warp's 8 distinct 16-byte entries of a row fill one 128-byte wavefront (unpadded, the 512-byte table stride put all
+    // eight on the same four banks: an 8-way conflict on every row-table load and store)
+    const ChainLayout lay = chain_layout(R, sizeof(DT), sizeof(PT) == 4);
+    const size_t img_elems = lay.img_elems;
+    const size_t tab_bytes = lay.tab_bytes;
+    // (GPW * img_elems * sizeof(DT) below is GPW * lay.img_bytes, written as the kernel always computed it)
     const size_t warp_bytes = (size_t)GPW * (img_elems * sizeof(DT) + tab_bytes);
     double2* ltab = reinterpret_cast<double2*>(smem_raw);
-    unsigned char* wbase = smem_raw + kLogTableSize * sizeof(double2) + (size_t)warp * warp_bytes;
+    unsigned char* wbase = smem_raw + lay.log_bytes + (size_t)warp * warp_bytes;
     DT* sD = reinterpret_cast<DT*>(wbase) + (size_t)grp * img_elems;
     double2* rt = reinterpret_cast<double2*>(wbase + (size_t)GPW * img_elems * sizeof(DT) + (size_t)grp * tab_bytes);
     const double h = A.dt / 2.0;

@@ -26,11 +26,7 @@ bool use_column_window(const FieldParams& P) {
 }
 
 // one single-warp block: the log table and kChainGroup chains of image copy and row tables
-size_t chain_smem_bytes(const FieldParams& P, size_t elem, bool f32) {
-    const size_t rowtab = sizeof(double2) + (f32 ? sizeof(float2) : 0);
-    return kLogTableSize * sizeof(double2) +
-           (size_t)kChainGroup * (((size_t)P.R * kChainCS + kLPC) * elem + (size_t)P.R * rowtab + kChainTabPad);
-}
+size_t chain_smem_bytes(const FieldParams& P, size_t elem, bool f32) { return chain_layout(P.R, elem, f32).smem_bytes; }
 
 template <typename DT, int MODE, int NCS, typename PT = double>
 int configure_mode(size_t smem, int& blocks_per_sm) {
@@ -137,6 +133,34 @@ void fill_log_table(double* host_table /* [kLogTableSize*2] */) {
         host_table[2 * k + 1] = (double)(-logl((long double)rc));
     }
 }
+
+int chain_kernel_window_cols(const FieldParams& P) { return use_column_window(P) ? kWinCols : kLPC * kSlotsFull; }
+
+ChainLayout chain_kernel_layout(int R, size_t elem, bool f32) { return chain_layout(R, elem, f32); }
+
+// chain_eval starts each lane's column table at its first column jb with e = exp(-arg_c), arg_c = v0^2/2s^2, v0 = jb + .5 - y,
+// and the ratio r_c = exp(-(2 L v0 + L^2)/2s^2), then multiplies its way along the row.  It zeroes the whole table when
+// arg_c >= 690, and exp_neg overflows for arguments above ~709.  The window start jb moves in steps of one column when
+// y - 12.5 crosses an integer, so |v0| is extreme at the support's ends or at such a crossing, all of which lie on the
+// 1/16-pixel grid of y scanned here.
+double chain_column_exponent(const FieldParams& P, int win) {
+    double worst = 0.0;
+    for (int k = 0; k <= 16 * (P.C + 2); ++k) {
+        const double y = -1.0 + k / 16.0;
+        for (int sub = 0; sub < kLPC; ++sub) {
+            int jb = sub;
+            if (win < kChainCS) {
+                const double a = std::ceil(y - (0.5 + 0.5 * win));
+                jb += (int)std::fmin(std::fmax(a, 0.0), (double)std::max(P.C - win, 0));
+            }
+            const double v0 = ((double)jb + 0.5) - y;
+            worst = std::max(worst, std::max(v0 * v0, -(2.0 * kLPC * v0 + kLPC * kLPC)) * P.inv2s2);
+        }
+    }
+    return worst;
+}
+
+bool chain_kernel_psf_ok(const FieldParams& P) { return chain_column_exponent(P, chain_kernel_window_cols(P)) <= kChainExpMax; }
 
 int chain_kernel_configure(const FieldParams& P, ChainLaunchPlan& plan) {
     if (int rc = configure_one<double>(P, plan.smem_f64, plan.blocks_per_sm_f64)) return rc;

@@ -13,6 +13,17 @@ constexpr int kWarp = 32;
 constexpr int kChainLPC = 4;
 constexpr int kChainGroup = 32 / kChainLPC;   // chains per warp: the unit of its work scheduler
 
+// Shared-memory layout of one single-warp block of the one-star kernel (chain_layout, chain_kernel.cuh); byte offsets are
+// from the start of the block's dynamic shared memory.
+struct ChainLayout {
+    size_t log_bytes;   // log table at offset 0
+    size_t img_elems;   // elements of one chain image (R rows of kChainCS, plus the bank padding)
+    size_t img_bytes;   // stride of the chain images, which start at log_bytes
+    size_t tab_base;    // row table of chain 0
+    size_t tab_bytes;   // stride of the row tables (a multiple of 16)
+    size_t smem_bytes;  // the whole block
+};
+
 // Problem constants snapshot (host fills it from srhmc_config).
 struct FieldParams {
     int R, C;          // image rows / cols

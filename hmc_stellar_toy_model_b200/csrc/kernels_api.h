@@ -36,6 +36,17 @@ int convert_image_launch(cudaStream_t stream, const double* src, float* dst, siz
 
 // warp-resident one-star kernel (chain_kernel.cuh), FP64
 int chain_kernel_configure(const FieldParams& P, ChainLaunchPlan& plan);
+// columns a chain's lanes cover in a launch now: 24 (window) or 32 (full width)
+int chain_kernel_window_cols(const FieldParams& P);
+// shared-memory layout of one block for R image rows of elem-byte pixels (f32: FP32 pixel arithmetic)
+ChainLayout chain_kernel_layout(int R, size_t elem, bool f32);
+// Largest exponent from which a lane's column table starts, over star positions in the support y in [-1, C+1], for a
+// window of `window_cols` columns.  chain_eval drops a lane's whole column table at 690 (and exp_neg overflows above ~709),
+// so the host sends a PSF to the kernel only when this stays at or below kChainExpMax, 50 under that cut-off (a star a
+// little outside the support, within a trajectory, then still gets its whole table); other PSFs take the CTA kernel.
+double chain_column_exponent(const FieldParams& P, int window_cols);
+constexpr double kChainExpMax = 640.0;
+bool chain_kernel_psf_ok(const FieldParams& P);
 int chain_kernel_launch(const FieldParams& P, const LaunchArgs& A, const ChainLaunchPlan& plan, int sms, cudaStream_t stream);
 // iteration chunks of the MODE_RUN work scheduler for `groups` warp-sized work items on `warps` resident warps
 int pick_chunks(long long groups, long long warps, int L);

@@ -198,10 +198,13 @@ int configure(srhmc_ctx* c) {
     return 0;
 }
 
+// the one-star kernel runs a batch of one-star fields (launch_field): FP64 on any image, FP32 on uint16 counts only
+bool chain_kernel_runs(const srhmc_ctx* c) { return c->chain_ok && (c->cfg.precision == 64 || c->d_int_bytes == 2); }
+
 int launch_field(srhmc_ctx* c, const LaunchArgs& A_in, bool one_star_everywhere) {
     LaunchArgs A = A_in;
     // the FP32 build of the one-star kernel reads the uint16 count images only
-    const bool chain = c->chain_ok && one_star_everywhere && (c->cfg.precision == 64 || c->d_int_bytes == 2);
+    const bool chain = one_star_everywhere && chain_kernel_runs(c);
     A.pix_f32 = (chain && c->cfg.precision == 32) ? 1 : 0;
     if (chain && A.mode == MODE_RUN) {
         // scheduler state of the chunked chain kernel: completion counters start at 0 for every launch
@@ -242,12 +245,16 @@ int download(srhmc_ctx* c, void* dst, const DevBuf& b, size_t bytes) {
     return 0;
 }
 
-bool chain_kernel_eligible(const srhmc_config& g) {
+bool chain_kernel_eligible(const srhmc_config& g, const FieldParams& P) {
     const char* off = std::getenv("SRHMC_DISABLE_CHAIN_KERNEL");
     if (off && off[0] == '1') return false;
-    // precision 32: FP32 pixel arithmetic on the uint16 count images (data that are not counts < 65536 take the CTA kernel)
-    return g.max_stars == 1 && g.num_cols <= 32 && g.num_rows <= 64 && !g.use_Vc && !g.shared_data && g.patch_radius == 0;
+    // precision 32: FP32 pixel arithmetic on the uint16 count images (data that are not counts < 65536 take the CTA kernel).
+    // A PSF so narrow that a lane's column table would start below the kernel's exponent cut-off somewhere in the support
+    // takes the CTA kernel too (chain_column_exponent).
+    return g.max_stars == 1 && g.num_cols <= 32 && g.num_rows <= 64 && !g.use_Vc && !g.shared_data && g.patch_radius == 0 &&
+           chain_kernel_psf_ok(P);
 }
+
 
 bool all_one_star(const srhmc_ctx* c, const int32_t* nstars) {
     if (!nstars) return c->cfg.max_stars == 1;
@@ -359,7 +366,7 @@ int srhmc_create(const srhmc_config* cfg, srhmc_ctx** out) {
     c->pix_bytes = cfg->precision == 64 ? 8 : 4;
 
     int rc = configure(c);
-    if (rc == 0 && chain_kernel_eligible(*cfg)) {
+    if (rc == 0 && chain_kernel_eligible(*cfg, P)) {
         const int e = chain_kernel_configure(P, c->chain_plan);
         if (e != 0) rc = fail(SRHMC_ERR_CUDA, "chain kernel configuration failed: %s", cudaGetErrorString((cudaError_t)e));
         c->chain_ok = (e == 0);
@@ -450,6 +457,48 @@ int srhmc_get_launch_plan(srhmc_ctx* c, srhmc_launch_plan* out) {
     out->int_image_bytes = c->d_int_bytes;
     out->smem_bytes = (int64_t)c->smem;
     return 0;
+}
+
+int srhmc_get_chain_plan(srhmc_ctx* c, srhmc_chain_plan* out) {
+    if (!c || !out) return fail(SRHMC_ERR_INVALID, "null argument");
+    *out = srhmc_chain_plan{};
+    if (!chain_kernel_runs(c)) return 0;
+    const bool f32 = c->cfg.precision == 32;
+    const int bytes = c->d_int_bytes ? c->d_int_bytes : 8;
+    const ChainLaunchPlan& pl = c->chain_plan;
+    out->chain_kernel = 1;
+    out->window_cols = chain_kernel_window_cols(c->P);
+    out->image_bytes = bytes;
+    out->pixel_f32 = f32 ? 1 : 0;
+    out->blocks_per_sm = f32 ? pl.blocks_per_sm_u16_f32
+                             : (bytes == 2 ? pl.blocks_per_sm_u16 : (bytes == 4 ? pl.blocks_per_sm_u32 : pl.blocks_per_sm_f64));
+    out->tab_stride = (int32_t)chain_kernel_layout(c->P.R, bytes, f32).tab_bytes;
+    out->smem_bytes = (int64_t)(f32 ? pl.smem_u16_f32 : (bytes == 2 ? pl.smem_u16 : (bytes == 4 ? pl.smem_u32 : pl.smem_f64)));
+    return 0;
+}
+
+int srhmc_chain_layout(int32_t rows, int32_t image_bytes, int32_t pixel_f32, srhmc_chain_layout_t* out) {
+    if (!out) return fail(SRHMC_ERR_INVALID, "null argument");
+    if (rows < 1 || rows > 64) return fail(SRHMC_ERR_INVALID, "the one-star kernel takes 1..64 image rows, not %d", rows);
+    if (image_bytes != 8 && image_bytes != 4 && image_bytes != 2)
+        return fail(SRHMC_ERR_INVALID, "image_bytes must be 8, 4 or 2");
+    if (pixel_f32 && image_bytes != 2) return fail(SRHMC_ERR_INVALID, "FP32 pixel arithmetic reads uint16 images only");
+    const ChainLayout L = chain_kernel_layout(rows, image_bytes, pixel_f32 != 0);
+    out->log_bytes = (int64_t)L.log_bytes;
+    out->img_stride = (int64_t)L.img_bytes;
+    out->tab_base = (int64_t)L.tab_base;
+    out->tab_stride = (int64_t)L.tab_bytes;
+    out->smem_bytes = (int64_t)L.smem_bytes;
+    return 0;
+}
+
+double srhmc_chain_column_exponent(int32_t num_cols, double psf_fwhm_pix, int32_t window_cols) {
+    if (num_cols < 1 || num_cols > 32 || !(psf_fwhm_pix > 0.0) || (window_cols != 24 && window_cols != 32)) return -1.0;
+    FieldParams P{};
+    P.C = num_cols;
+    const double sigma = psf_fwhm_pix / 2.354;  // as srhmc_create
+    P.inv2s2 = 1.0 / (2.0 * sigma * sigma);
+    return chain_column_exponent(P, window_cols);
 }
 
 // after the float64 images are in place on the device (c->D for the FP64 build, c->Dstage for the FP32 build): the

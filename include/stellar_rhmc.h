@@ -186,6 +186,35 @@ typedef struct srhmc_launch_plan {
 } srhmc_launch_plan;
 int srhmc_get_launch_plan(srhmc_ctx* ctx, srhmc_launch_plan* out);
 
+/* What a launch of one-star fields of this context runs now on the warp-resident one-star kernel (read-only; valid after
+ * srhmc_set_data, which picks the image copy).  srhmc_create sends a context to that kernel when it has one star slot,
+ * at most 32 columns and 64 rows, no repulsion, no shared data, the full-image PSF, and a PSF wide enough that every
+ * lane's column table starts above the kernel's exponent cut-off for every star position in the support (roughly
+ * FWHM >= 1.6 px on a 32-column image; see DESIGN.md section 4.1).  Precision 32 runs it on uint16 count images only. */
+typedef struct srhmc_chain_plan {
+    int32_t chain_kernel;   /* 1: the one-star kernel; 0: the CTA-per-field kernel (other fields are all 0) */
+    int32_t window_cols;    /* columns a chain's lanes cover: 24 (window around the star) or 32 (full width) */
+    int32_t image_bytes;    /* pixel of the image copy it reads: 8 (float64), 4 (uint32 counts) or 2 (uint16 counts) */
+    int32_t pixel_f32;      /* 1: FP32 pixel arithmetic in the gradient-only evaluations */
+    int32_t blocks_per_sm;  /* resident single-warp blocks per SM for that layout */
+    int32_t tab_stride;     /* bytes between the row tables of consecutive chains */
+    int64_t smem_bytes;     /* dynamic shared memory per block */
+} srhmc_chain_plan;
+int srhmc_get_chain_plan(srhmc_ctx* ctx, srhmc_chain_plan* out);
+
+/* Shared-memory layout of one block of the one-star kernel (host only, no device needed): the log table at offset 0,
+ * then 8 chain images of img_stride bytes, then 8 row tables of tab_stride bytes from tab_base.  rows 1..64,
+ * image_bytes 8 / 4 / 2, pixel_f32 only with image_bytes 2.  The kernel takes its pointers from the same computation. */
+typedef struct srhmc_chain_layout_t {
+    int64_t log_bytes, img_stride, tab_base, tab_stride, smem_bytes;
+} srhmc_chain_layout_t;
+int srhmc_chain_layout(int32_t rows, int32_t image_bytes, int32_t pixel_f32, srhmc_chain_layout_t* out);
+
+/* Host only: the largest exponent from which a lane of the one-star kernel starts its column table, over star positions
+ * y in [-1, num_cols + 1], for a window of window_cols (24 or 32) columns; the kernel is used when it is at most 640.
+ * Returns -1 for arguments outside num_cols 1..32, psf_fwhm_pix > 0. */
+double srhmc_chain_column_exponent(int32_t num_cols, double psf_fwhm_pix, int32_t window_cols);
+
 /* Pinned host memory helpers for callers that want asynchronous copies. */
 void* srhmc_host_alloc(uint64_t bytes);
 int srhmc_host_free(void* p);

@@ -50,7 +50,8 @@ def test_struct_layouts_match_the_header():
 
     for struct, cls in (("srhmc_config", _capi.Config), ("srhmc_run_args", _capi.RunArgs), ("srhmc_ls_args", _capi.LsArgs),
                         ("srhmc_big_config", _capi.BigConfig), ("srhmc_big_step", _capi.BigStep),
-                        ("srhmc_big_buffers_t", _capi.BigBuffers), ("srhmc_launch_plan", _capi.LaunchPlan)):
+                        ("srhmc_big_buffers_t", _capi.BigBuffers), ("srhmc_launch_plan", _capi.LaunchPlan),
+                        ("srhmc_chain_plan", _capi.ChainPlan), ("srhmc_chain_layout_t", _capi.ChainLayout)):
         assert fields(struct) == [f[0] for f in cls._fields_], struct
 
 
