@@ -15,6 +15,7 @@
 // Scalar work (metric, implicit fixed points, reflections; sampler_RHMC.py:229-292, 448-492, 522-566) is one
 // thread per star with a CTA-wide vote per fixed-point iteration (the reference's field-wide stop rule).
 #pragma once
+#include <cfloat>
 #include <math_constants.h>
 
 #include "common.cuh"
@@ -505,6 +506,16 @@ __device__ void gather_v3(const Ctx<T>& c) {
     }
 }
 
+// True in every thread when every star of the field has |f| >= the smallest normal T, so that grad_chunk<T, true> can
+// divide the flux sum by f.  A zero flux (0/0) or a subnormal one (tables underflow) needs the two-pass branch.
+template <typename T>
+__device__ bool fluxes_normal(const Ctx<T>& c) {
+    const double fmin = sizeof(T) == 8 ? (double)DBL_MIN : (double)FLT_MIN;
+    int tiny = 0;
+    for (int k = threadIdx.x; k < c.N; k += blockDim.x) tiny |= !(fabs(c.q[3 * k]) >= fmin);
+    return !__syncthreads_or(tiny);
+}
+
 // Pixel part of V and dV/dq at the current c.q.  Returns sum(Lambda - D ln Lambda) in every thread when want_V.
 // KV3: -1 = follow P.v3 at run time (generic kernels), 1 = the compact-table path only, 0 = the chunked tables only
 template <typename T, int MR, int MC, int KV3 = -1>
@@ -521,7 +532,7 @@ __device__ double eval_pixels(const Ctx<T>& c, bool want_V) {
         __syncthreads();
     } else if (KV3 == 1) {
         // unreachable: the specialised kernel is only launched for compact-table contexts
-    } else if (nchunks == 1 && c.N > 0) {
+    } else if (nchunks == 1 && c.N > 0 && fluxes_normal(c)) {
         // every star's tables fit at once: ONE build serves the render and the gradient pass (flux in the column table)
         build_tables<T>(c, 0, c.N, 2);
         __syncthreads();

@@ -1033,6 +1033,7 @@ static int ls_common(srhmc_ctx* c, LsArgs& A, const double* q0, const double* p0
     if (!c->have_data) return fail(SRHMC_ERR_STATE, "srhmc_set_data has not been called");
     if (c->cfg.precision != 64) return fail(SRHMC_ERR_INVALID, "the lightsource_gym entry points need a precision=64 context");
     if (c->cfg.use_prior || c->cfg.use_Vc) return fail(SRHMC_ERR_INVALID, "lightsource_gym has no prior / repulsion: create the context with use_prior = use_Vc = 0");
+    if (c->cfg.patch_radius != 0) return fail(SRHMC_ERR_INVALID, "lightsource_gym sums over the full image: create the context with patch_radius = 0");
     const size_t F = c->cfg.n_fields, S = 3 * (size_t)c->cfg.max_stars, FS = std::max<size_t>(F * S * 8, 8);
     if (int rc = upload(c, c->q, q0, FS)) return rc;
     if (p0) if (int rc = upload(c, c->p, p0, FS)) return rc;

@@ -656,10 +656,20 @@ def ls_efficient(L: LightSetup, q, p, dVdqq_only=False, parts=False):
 
 @dataclass
 class LsChains:
+    """Chain outputs of the lightsource_gym samplers, plus diagnostics of the branches the chain took.  HMC_random /
+    RHMC_random_diag: `flips` the iterations (1-based) whose trajectory ended in the flip branch, `flip_steps` one
+    (iteration, step, flagged, new) entry per leapfrog step that took the flip branch, with the number of flux momenta
+    flipped (the flags are never cleared inside an iteration) and the number that crossed f_lim in that step.
+    RHMC_random: `breaks` the (iteration, step) pairs where a trajectory stopped on an infinite energy, `abandoned` the
+    iteration at which the chain was given up for its acceptance rate (None if it was not)."""
     q: np.ndarray
     E: np.ndarray
     dE: np.ndarray
     A: np.ndarray
+    flips: list = field(default_factory=list)
+    flip_steps: list = field(default_factory=list)
+    breaks: list = field(default_factory=list)
+    abandoned: int | None = None
 
 
 def ls_hmc_random(L: LightSetup, q0, dt, normals, steps, lnu, niter, f_lim=0.0):
@@ -686,7 +696,7 @@ def ls_hmc_random(L: LightSetup, q0, dt, normals, steps, lnu, niter, f_lim=0.0):
         p_half = p - dt * ls_grad(L, q) / 2.0
         iflip = np.zeros(d, dtype=bool)
         flip = False
-        for _ in range(int(steps[i - 1])):
+        for z in range(int(steps[i - 1])):
             flip = False
             q = q + dt * p_half
             for k in range(n):
@@ -694,12 +704,16 @@ def ls_hmc_random(L: LightSetup, q0, dt, normals, steps, lnu, niter, f_lim=0.0):
                     iflip[3 * k] = True
                     flip = True
             if flip:
+                new = sum(q[3 * k] < L.f_lim for k in range(n))
+                out.flip_steps.append((i, z, int(np.sum(iflip)), int(new)))
                 keep = -p_half[iflip]
                 p_half = p_half - dt * ls_grad(L, q)
                 p_half[iflip] = keep
             else:
                 p_half = p_half - dt * ls_grad(L, q)
-        if not flip:
+        if flip:
+            out.flips.append(i)
+        else:
             p = p_half + dt * ls_grad(L, q) / 2.0
         e1 = ls_energy(L, q, p)
         dE = e1 - e0
@@ -742,7 +756,7 @@ def ls_rhmc_random_diag(L: LightSetup, q0, dt_global, normals, steps, lnu, niter
         p_half = p - dt_global / 2.0 * force(q, p)
         iflip = np.zeros(d, dtype=bool)
         flip = False
-        for _ in range(int(steps[i - 1])):
+        for z in range(int(steps[i - 1])):
             flip = False
             M = ls_mass_matrix(L, q)
             q = q + dt_global * p_half / M
@@ -751,12 +765,16 @@ def ls_rhmc_random_diag(L: LightSetup, q0, dt_global, normals, steps, lnu, niter
                     iflip[3 * k] = True
                     flip = True
             if flip:
+                new = sum(q[3 * k] < L.f_lim for k in range(n))
+                out.flip_steps.append((i, z, int(np.sum(iflip)), int(new)))
                 keep = -p_half[iflip]
                 p_half = p_half - dt_global * force(q, p)
                 p_half[iflip] = keep
             else:
                 p_half = p_half - dt_global * force(q, p)
-        if not flip:
+        if flip:
+            out.flips.append(i)
+        else:
             p = p_half + dt_global * force(q, p) / 2.0
         M = ls_mass_matrix(L, q)
         e1 = ls_energy(L, q, p, M)
@@ -802,6 +820,7 @@ def ls_rhmc_random(L: LightSetup, q0, dt, normals, steps, lnu, niter, f_lim=0.0)
         for z in range(nst):
             dqdt, dpdt, E = ls_efficient(L, q, p_half)
             if E == np.inf:
+                out.breaks.append((i, z))
                 break
             q += dt * dqdt
             for k in range(n):
@@ -823,6 +842,7 @@ def ls_rhmc_random(L: LightSetup, q0, dt, normals, steps, lnu, niter, f_lim=0.0)
             out.A[i - 1] = 1
         out.q[i] = q
         if (i % 100) == 0 and np.sum(out.A[:i]) * 100 / float(i) < 50:
+            out.abandoned = i
             break
     return out
 
