@@ -168,6 +168,15 @@ class BigBuffers(C.Structure):
                 ("n_scalars", C.c_int64), ("counters", C.c_void_p), ("n_counters", C.c_int64)]
 
 
+class BigPeaksArgs(C.Structure):
+    """struct srhmc_big_peaks_args"""
+
+    _fields_ = [("seeds", c_double_p), ("n", C.c_int32), ("nstep", C.c_int32)] + \
+               [(n, C.c_double) for n in ("dt_f_coeff", "dt_xy_coeff", "f_lim", "dr_tol", "dmag_tol", "flux_to_count")] + \
+               [("q", c_double_p), ("alive", c_uint8_p), ("steps", c_int32_p), ("kept", c_uint8_p), ("n_kept", c_int32_p),
+                ("merge_rounds", c_int32_p)]
+
+
 # name -> (restype, argtypes); every symbol declared in include/stellar_rhmc.h
 SIGNATURES = {
     "srhmc_abi_version": (C.c_int, []),
@@ -244,6 +253,7 @@ SIGNATURES = {
     "srhmc_big_set_recording": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32]),
     "srhmc_big_read_samples": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, c_double_p, c_double_p]),
     "srhmc_big_convergence_stats": (C.c_int, [C.POINTER(C.c_void_p), C.c_int32, C.c_int32, C.c_int32, c_double_p, c_double_p]),
+    "srhmc_big_find_peaks": (C.c_int, [C.c_void_p, C.POINTER(BigPeaksArgs)]),
 }
 
 

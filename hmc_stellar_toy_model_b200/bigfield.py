@@ -22,6 +22,7 @@ import numpy as np
 
 from . import _capi
 from ._capi import check_big as check
+from .utils import mag2flux
 
 PHASE = dict(PACK=0, EVAL=1, EVAL_V=2, KICK1=3, PFIX_QFIX=4, QFIX_KICK=5, KICK2=6, MOMENTUM=7, ENERGY=8, RECORD_E0=9,
              ACCEPT=10, RESET_ITER=11, EVAL_KICK2=12, EVAL_V_KICK2=13, EVAL_KICK2_KICK1=14, PS_ADVANCE=15, EVAL_PS_ADVANCE=16)
@@ -73,6 +74,25 @@ def ghost_mask(x, lo: int, hi: int, reach: int, rank: int, world: int):
     to_lo = (x < lo + reach) if rank > 0 else np.zeros(x.shape, bool)
     to_hi = (x >= hi - reach) if rank < world - 1 else np.zeros(x.shape, bool)
     return to_lo, to_hi
+
+
+def peak_seeds(rows, cols, linear_pix_density, jitter, f_seed):
+    """Seed grid of lightsource_gym.find_peaks (samplers.py:163-176): int(density * rows) - 1 rows by
+    int(density * cols) - 1 columns at spacing 1 / density; seed t = i * n_col + j sits at
+    (spacing * (i + 0.5 + 0.1 jitter[t, 0]), spacing * (j + 0.5 + 0.1 jitter[t, 1])) with flux f_seed.  jitter
+    [n_row * n_col, 2] holds the draws in the reference's order.  The reference's flat index i * n_row + j overwrites
+    seeds on a non-square grid; on a square one the two are the same."""
+    n_row = max(0, int(linear_pix_density * rows) - 1)
+    n_col = max(0, int(linear_pix_density * cols) - 1)
+    spacing = 1 / float(linear_pix_density)
+    jitter = np.asarray(jitter, dtype=np.float64).reshape(n_row * n_col, 2)
+    i = np.repeat(np.arange(n_row), n_col)
+    j = np.tile(np.arange(n_col), n_row)
+    q = np.empty((n_row * n_col, 3))
+    q[:, 0] = f_seed
+    q[:, 1] = spacing * (i + 0.5 + 0.1 * jitter[:, 0])
+    q[:, 2] = spacing * (j + 0.5 + 0.1 * jitter[:, 1])
+    return q
 
 
 # ----------------------------------------------------------------------------------------------- sample rows
@@ -243,6 +263,47 @@ class BigFieldStrip:
         out = {w: np.empty((int(nrows), self.n, 3)) for w in want}
         check(self._lib.srhmc_big_read_samples(self._h, int(row0), int(nrows), _capi.dptr(out.get("q")),
                                                _capi.dptr(out.get("p"))))
+        return out
+
+    def find_peaks(self, flux_to_count, mag_lim, linear_pix_density=0.2, dr_tol=1., dmag_tol=0.5, Nstep=1000,
+                   dt_f_coeff=0.1, dt_xy_coeff=0.1, jitter=None, return_all=False):
+        """lightsource_gym.find_peaks (samplers.py:129-254) on this strip's image, which must be the whole field
+        (world_size = 1): seeds on the jittered grid (`peak_seeds`, flux mag_lim - 0.5), descent of every seed on a
+        pure-background model with potential and gradient over its (2 patch_radius + 1)^2 window, and the greedy merge.
+        jitter=None draws np.random.randn in the reference's order from the global stream.  Returns the catalogue [k,3]
+        (f in counts, x, y) in seed order, ready for set_stars; with return_all also the descended seeds (q [n,3],
+        alive [n], steps [n])."""
+        f_lim = mag2flux(mag_lim) * flux_to_count
+        f_seed = mag2flux(mag_lim - 0.5) * flux_to_count
+        n = max(0, int(linear_pix_density * self.rows) - 1) * max(0, int(linear_pix_density * self.cols) - 1)
+        if jitter is None:
+            jitter = np.random.randn(n, 2)
+        seeds = peak_seeds(self.rows, self.cols, linear_pix_density, jitter, f_seed)
+        out = self.descend_seeds(seeds, Nstep, dt_f_coeff, dt_xy_coeff, f_lim, merge=(dr_tol, dmag_tol, flux_to_count))
+        catalogue = out["q"][out["kept"]]
+        return (catalogue, out["q"], out["alive"], out["steps"]) if return_all else catalogue
+
+    def descend_seeds(self, seeds, Nstep, dt_f_coeff, dt_xy_coeff, f_lim, merge=None):
+        """srhmc_big_find_peaks on seeds [n,3]: dict of the descended q, alive and steps; with merge = (dr_tol, dmag_tol,
+        flux_to_count) also the kept mask, n_kept and the number of merge rounds.  Nstep = 0 leaves the seeds alive where
+        they are, so the merge alone runs on a given list."""
+        seeds = np.ascontiguousarray(np.asarray(seeds, dtype=np.float64).reshape(-1, 3))
+        n = len(seeds)
+        q = np.empty((n, 3))
+        alive = np.empty(n, dtype=np.uint8)
+        steps = np.empty(n, dtype=np.int32)
+        kept = np.empty(n, dtype=np.uint8) if merge is not None else None
+        n_kept, rounds = C.c_int32(), C.c_int32()
+        dr_tol, dmag_tol, flux_to_count = merge if merge is not None else (1.0, 0.5, 1.0)
+        args = _capi.BigPeaksArgs(seeds=_capi.dptr(seeds), n=n, nstep=int(Nstep), dt_f_coeff=float(dt_f_coeff),
+                                  dt_xy_coeff=float(dt_xy_coeff), f_lim=float(f_lim), dr_tol=float(dr_tol),
+                                  dmag_tol=float(dmag_tol), flux_to_count=float(flux_to_count), q=_capi.dptr(q),
+                                  alive=_capi.bptr(alive), steps=_capi.iptr(steps), kept=_capi.bptr(kept),
+                                  n_kept=C.pointer(n_kept) if merge is not None else None, merge_rounds=C.pointer(rounds))
+        check(self._lib.srhmc_big_find_peaks(self._h, C.byref(args)))
+        out = dict(q=q, alive=alive.astype(bool), steps=steps)
+        if merge is not None:
+            out.update(kept=kept.astype(bool), n_kept=int(n_kept.value), rounds=int(rounds.value))
         return out
 
     def read_scalars(self):

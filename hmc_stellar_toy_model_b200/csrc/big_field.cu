@@ -112,6 +112,7 @@ __device__ __forceinline__ bool last_block_ticket(unsigned int* ticket, bool* fl
 
 #include "big_tile.cuh"
 #include "big_star.cuh"
+#include "big_peaks.cuh"
 
 namespace {
 
@@ -1519,6 +1520,109 @@ int srhmc_big_convergence_stats(srhmc_big* const* chains, int32_t k, int32_t thi
     out.release();
     if (e != cudaSuccess) return bfail(SRHMC_ERR_CUDA, "chain statistics failed: %s", cudaGetErrorString(e));
     return 0;
+}
+
+int srhmc_big_find_peaks(srhmc_big* b, const srhmc_big_peaks_args* a) {
+    // big_peaks.cuh: windowed descent of every seed, then the exact greedy merge in rounds
+    if (!b || !a) return bfail(SRHMC_ERR_INVALID, "null argument");
+    if (b->world > 1)
+        return bfail(SRHMC_ERR_STATE, "peak finding needs the whole image on one device: this context is a strip of %d", b->world);
+    if (!b->have_data) return bfail(SRHMC_ERR_STATE, "srhmc_big_set_data or srhmc_big_mock_data has not been called");
+    const int n = a->n;
+    if (n < 0 || a->nstep < 0 || (n > 0 && !a->seeds)) return bfail(SRHMC_ERR_INVALID, "bad seed count, nstep or seed pointer");
+    const double coeffs[] = {a->dt_f_coeff, a->dt_xy_coeff, a->f_lim, a->dr_tol, a->dmag_tol, a->flux_to_count};
+    for (double v : coeffs)
+        if (!std::isfinite(v)) return bfail(SRHMC_ERR_INVALID, "step coefficients, f_lim and tolerances must be finite");
+    if (!(a->flux_to_count > 0.0)) return bfail(SRHMC_ERR_INVALID, "flux_to_count must be positive");
+    for (size_t k = 0; k < 3 * (size_t)n; ++k)
+        if (!std::isfinite(a->seeds[k])) return bfail(SRHMC_ERR_INVALID, "seed %zu is not finite", k / 3);
+    if (a->n_kept) *a->n_kept = 0;
+    if (a->merge_rounds) *a->merge_rounds = 0;
+    if (n == 0) return 0;
+    BCU(cudaSetDevice(b->cfg.device));
+    const BigParams& P = b->P;
+    cudaStream_t st = b->stream;
+    const bool merge = a->kept || a->n_kept;
+    // cells of side max(|dr_tol|, 1), widened by one part in 1e12 so that the rounding of the distance test cannot put a
+    // conflicting pair two cells apart
+    const double cell = std::max(std::fabs(a->dr_tol), 1.0) * (1.0 + 1e-12), inv_cell = 1.0 / cell;
+    const int ncx = std::max(1, (int)std::ceil(P.Rg / cell)), ncy = std::max(1, (int)std::ceil(P.C / cell));
+    const size_t nlists = (size_t)ncx * ncy + 1;
+    BBuf dq, dalive, dsteps, dcnt, dmag, dhead, dnext, dst0, dst1;
+    BBuf* bufs[] = {&dq, &dalive, &dsteps, &dcnt, &dmag, &dhead, &dnext, &dst0, &dst1};
+    auto done = [&](int rc) {
+        for (BBuf* x : bufs) x->release();
+        return rc;
+    };
+    int rc = dq.ensure((size_t)n * 24) | dalive.ensure(n) | dsteps.ensure((size_t)n * 4) | dcnt.ensure(16);
+    if (merge)
+        rc |= dmag.ensure((size_t)n * 8) | dhead.ensure(nlists * 4) | dnext.ensure((size_t)n * 4) | dst0.ensure(n) | dst1.ensure(n);
+    if (rc) {
+        cudaGetLastError();
+        return done(bfail(SRHMC_ERR_CUDA, "cannot allocate the peak-finding buffers for %d seeds", n));
+    }
+    cudaError_t e = cudaMemcpyAsync(dq.ptr, a->seeds, (size_t)n * 24, cudaMemcpyHostToDevice, st);
+    if (e == cudaSuccess && a->nstep > 0) {
+        const int smem = kSeedWarps * ((2 * P.rad + 1) * 32 + 64) * 8;
+        e = cudaFuncSetAttribute(big_seed_descent_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+        if (e == cudaSuccess) {
+            big_seed_descent_kernel<<<(n + kSeedWarps - 1) / kSeedWarps, 32 * kSeedWarps, smem, st>>>(
+                P, b->D.as<double>(), n, a->nstep, a->dt_f_coeff, a->dt_xy_coeff, a->f_lim, dq.as<double>(),
+                dalive.as<unsigned char>(), dsteps.as<int>());
+            b->launches += 1;
+            e = cudaGetLastError();
+        }
+    } else if (e == cudaSuccess) {  // no step: every seed stays where it is, alive (the reference's loop does not run)
+        e = cudaMemsetAsync(dalive.ptr, 1, n, st);
+        if (e == cudaSuccess) e = cudaMemsetAsync(dsteps.ptr, 0, (size_t)n * 4, st);
+    }
+    int rounds = 0, counts[4] = {0, 0, 0, 0};   // [0] open seeds, [1] decided in a round, [2] kept
+    unsigned char* sin = dst0.as<unsigned char>();
+    unsigned char* sout = dst1.as<unsigned char>();
+    const int tb = 256, nb = (n + tb - 1) / tb;
+    if (merge && e == cudaSuccess) {
+        e = cudaMemsetAsync(dhead.ptr, 0xFF, nlists * 4, st);
+        if (e == cudaSuccess) e = cudaMemsetAsync(dcnt.ptr, 0, 16, st);
+        if (e == cudaSuccess) {
+            big_merge_bin_kernel<<<nb, tb, 0, st>>>(n, dq.as<double>(), dalive.as<unsigned char>(), a->flux_to_count, inv_cell, ncx, ncy,
+                                                    dmag.as<double>(), dhead.as<int>(), dnext.as<int>(), sin, dcnt.as<int>());
+            b->launches += 1;
+            e = cudaGetLastError();
+        }
+        if (e == cudaSuccess) e = cudaMemcpyAsync(counts, dcnt.ptr, 4, cudaMemcpyDeviceToHost, st);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+        const double dr2 = a->dr_tol * a->dr_tol;
+        for (int open = counts[0]; e == cudaSuccess && open > 0;) {
+            e = cudaMemsetAsync(dcnt.as<int>() + 1, 0, 4, st);
+            if (e != cudaSuccess) break;
+            big_merge_round_kernel<<<nb, tb, 0, st>>>(n, dq.as<double>(), dmag.as<double>(), dhead.as<int>(), dnext.as<int>(), inv_cell,
+                                                      ncx, ncy, dr2, a->dmag_tol, sin, sout, dcnt.as<int>() + 1);
+            b->launches += 1;
+            e = cudaGetLastError();
+            if (e == cudaSuccess) e = cudaMemcpyAsync(counts + 1, dcnt.as<int>() + 1, 4, cudaMemcpyDeviceToHost, st);
+            if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+            if (e != cudaSuccess) break;
+            ++rounds;
+            std::swap(sin, sout);
+            if (counts[1] <= 0) return done(bfail(SRHMC_ERR_CUDA, "merge round %d decided no seed (%d open)", rounds, open));
+            open -= counts[1];
+        }
+        if (e == cudaSuccess) {   // the kept mask goes to the other state buffer
+            big_merge_kept_kernel<<<nb, tb, 0, st>>>(n, sin, sout, dcnt.as<int>() + 2);
+            b->launches += 1;
+            e = cudaGetLastError();
+        }
+        if (e == cudaSuccess) e = cudaMemcpyAsync(counts + 2, dcnt.as<int>() + 2, 4, cudaMemcpyDeviceToHost, st);
+        if (e == cudaSuccess && a->kept) e = cudaMemcpyAsync(a->kept, sout, n, cudaMemcpyDeviceToHost, st);
+    }
+    if (e == cudaSuccess && a->q) e = cudaMemcpyAsync(a->q, dq.ptr, (size_t)n * 24, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess && a->alive) e = cudaMemcpyAsync(a->alive, dalive.ptr, n, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess && a->steps) e = cudaMemcpyAsync(a->steps, dsteps.ptr, (size_t)n * 4, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+    if (e != cudaSuccess) return done(bfail(SRHMC_ERR_CUDA, "peak finding failed: %s", cudaGetErrorString(e)));
+    if (a->n_kept) *a->n_kept = counts[2];
+    if (a->merge_rounds) *a->merge_rounds = rounds;
+    return done(0);
 }
 
 // Enqueue one phase on the context's stream (no synchronisation).  See srhmc_big_phase_id in the header.

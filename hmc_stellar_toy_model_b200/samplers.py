@@ -7,11 +7,14 @@ What runs where
   device (C ABI)  dVdq, V, E, K, dVdq_single, V_single, E_single, RHMC_efficient_computation, and the whole chain loops
                   of HMC_random, RHMC_random_diag and RHMC_random (ONE resident launch per chain); HMC_find_best_dt
                   keeps its search loop on the host (as SURVEY.md 8a says) and runs every acceptance-rate trial
-                  (Niter_per_trial random-length trajectories) as one launch.
+                  (Niter_per_trial random-length trajectories) as one launch; the seed descent of find_peaks is one
+                  launch for all seeds.
   host (set-up)   mock data, Fisher factors, mass_matrix / F / G / dlnDetdq / dpMpdq scalars, random draws -- taken from
                   the global np.random stream in exactly the reference's order (p_sample, then per iteration
-                  p_sample, randint, random; samplers.py:507,520,529,562), so seeded scripts reproduce the reference.
-  not provided    find_peaks (mode finding, SURVEY.md 8f next #2), RHMC_GMM (unrelated toy density), display_data.
+                  p_sample, randint, random; samplers.py:507,520,529,562), so seeded scripts reproduce the reference;
+                  find_peaks' seed grid and greedy merge (bigfield.BigFieldStrip.find_peaks runs both stages on the
+                  device for images too large for this path).
+  not provided    RHMC_GMM (unrelated toy density), display_data.
 
 The reference's behavioural quirks are reproduced on the device (see csrc/ls_kernel.cuh).  No CPU fallback.
 """

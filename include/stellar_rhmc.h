@@ -463,6 +463,26 @@ int srhmc_big_read_samples(srhmc_big* b, int32_t row0, int32_t nrows, double* q,
 int srhmc_big_convergence_stats(srhmc_big* const* chains, int32_t k, int32_t thin_rate, int32_t warm_up_num, double* R,
                                 double* n_eff);
 
+/* lightsource_gym.find_peaks (samplers.py:129-254) on the context's image: every seed descends on a pure-background model
+ * (B_count) with every potential and gradient evaluated over its (2 patch_radius + 1)^2 window, clipped to the image; it
+ * stops when V on the window of its new position changes by less than 1e-9 relative (V at the old position re-evaluated on
+ * that window when the seed changed pixel), dies when f < f_lim, or stops after nstep steps.  Then the exact greedy merge in
+ * seed order: an alive seed is kept unless an earlier kept seed lies within dr_tol pixels AND dmag_tol magnitudes
+ * (mag = 22.5 - 2.5 log10(f / flux_to_count)).  Needs world_size = 1 and data.  Every output may be NULL; without kept and
+ * n_kept the merge is skipped.  Buffers are allocated per call and released before it returns. */
+typedef struct srhmc_big_peaks_args {
+    const double* seeds;         /* [n,3] f (counts), x, y */
+    int32_t n, nstep;
+    double dt_f_coeff, dt_xy_coeff, f_lim, dr_tol, dmag_tol, flux_to_count;
+    double* q;                   /* [n,3] descended seeds */
+    uint8_t* alive;              /* [n] 1 unless the seed fell below f_lim */
+    int32_t* steps;              /* [n] descent steps taken */
+    uint8_t* kept;               /* [n] 1 for the seeds of the catalogue */
+    int32_t* n_kept;
+    int32_t* merge_rounds;       /* rounds of the parallel merge */
+} srhmc_big_peaks_args;
+int srhmc_big_find_peaks(srhmc_big* b, const srhmc_big_peaks_args* a);
+
 /* Roofline denominator measured on the device itself: a register-resident FMA chain (8 independent chains per
  * thread, all SMs filled) in the given precision (64 or 32).  Returns TFLOP/s (2 flop per FMA) and the launch time. */
 int srhmc_measure_fma_peak(int32_t device, int32_t precision, double* tflops, float* ms);
