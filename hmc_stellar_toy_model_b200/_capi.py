@@ -122,6 +122,14 @@ class RunArgs(C.Structure):
     ]
 
 
+class RjArgs(C.Structure):
+    """struct srhmc_rj_args"""
+
+    _fields_ = [("P_move", C.c_double * 3), ("fmin", C.c_double), ("fmax", C.c_double), ("K_split", C.c_double),
+                ("beta_a", C.c_double), ("beta_b", C.c_double), ("draws", c_double_p), ("N_chain", c_int32_p),
+                ("move_chain", c_uint8_p), ("n_final", c_int32_p), ("overflow", c_int32_p)]
+
+
 class LaunchPlan(C.Structure):
     """struct srhmc_launch_plan"""
 
@@ -215,6 +223,9 @@ SIGNATURES = {
     "srhmc_run_upload": (C.c_int, [C.c_void_p, C.POINTER(RunArgs)]),
     "srhmc_run_launch": (C.c_int, [C.c_void_p, C.POINTER(RunArgs)]),
     "srhmc_run_download": (C.c_int, [C.c_void_p, C.POINTER(RunArgs)]),
+    "srhmc_run_rj": (C.c_int, [C.c_void_p, C.POINTER(RunArgs), C.POINTER(RjArgs)]),
+    "srhmc_philox_rj_draws": (C.c_int, [C.c_void_p, C.c_uint64, C.c_int32, C.c_int32, C.c_int32, C.c_double, C.c_double,
+                                        c_double_p]),
     "srhmc_run_single": (C.c_int, [C.c_void_p, c_double_p, c_double_p, c_int32_p, C.c_int32, C.c_double, C.c_double,
                                    C.c_int32, C.c_int32, C.c_double, C.c_double,
                                    c_double_p, c_double_p, c_double_p, c_double_p, c_double_p]),

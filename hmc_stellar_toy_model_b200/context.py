@@ -11,7 +11,7 @@ from dataclasses import dataclass
 import numpy as np
 
 from . import _capi
-from ._capi import Config, LsArgs, RunArgs, as_f64, bptr, check, dptr, iptr
+from ._capi import Config, LsArgs, RjArgs, RunArgs, as_f64, bptr, check, dptr, iptr
 
 
 @dataclass
@@ -25,6 +25,18 @@ class RunResult:
     q_final: np.ndarray
     accept_rate: np.ndarray
     kernel_ms: float
+
+
+@dataclass
+class RjRunResult(RunResult):
+    """RunResult of a reversible-jump run plus its trans-dimensional record."""
+    N_chain: np.ndarray = None      # [F, Ls] int32: star count at the start of each kept iteration
+    move_chain: np.ndarray = None   # [F, Ls] uint8: 0 within, 1 birth, 2 death, 3 split, 4 merge
+    n_final: np.ndarray = None      # [F] int32: star count after the last iteration
+    overflow: np.ndarray = None     # [F] int32: first iteration whose proposal needed more than max_stars stars, or -1
+
+
+RJ_DRAWS = 14  # doubles of one (field, iteration) draw record of run_rj
 
 
 class RHMCContext:
@@ -273,6 +285,33 @@ class RHMCContext:
 
     def run_download(self, a):
         check(self._lib.srhmc_run_download(self._h, C.byref(a)))
+
+    def run_rj(self, q0, niter, nsteps, dt, *, P_move, fmin, fmax, K_split=1.0, beta_a=2.0, beta_b=2.0, draws=None,
+               **run_kw):
+        """Reversible-jump chains (multi_gym.run_RHMC with birth/death and split/merge moves): every iteration of every
+        field in ONE launch, the star counts changing on the device.  run_kw as for run(); nstars gives the start counts
+        (default max_stars).  draws [F, niter+1, 14] replaces the device records (philox_rj_draws).  alpha and
+        V_prior_const are the context's.  Returns RjRunResult; chain rows are zero past 3 * N_chain of their row."""
+        F, L = self.F, int(niter) + 1
+        a, keep = self.make_run_args(q0, niter, nsteps, dt, **run_kw)
+        rows = (L + a.chain_stride - 1) // a.chain_stride
+        dr = None if draws is None else as_f64(draws, (F, L, RJ_DRAWS))
+        out = dict(N_chain=np.zeros((F, rows), dtype=np.int32), move_chain=np.zeros((F, rows), dtype=np.uint8),
+                   n_final=np.zeros(F, dtype=np.int32), overflow=np.zeros(F, dtype=np.int32))
+        rj = RjArgs(P_move=(C.c_double * 3)(*[float(x) for x in P_move]), fmin=float(fmin), fmax=float(fmax),
+                    K_split=float(K_split), beta_a=float(beta_a), beta_b=float(beta_b), draws=dptr(dr),
+                    N_chain=iptr(out["N_chain"]), move_chain=bptr(out["move_chain"]), n_final=iptr(out["n_final"]),
+                    overflow=iptr(out["overflow"]))
+        check(self._lib.srhmc_run_rj(self._h, C.byref(a), C.byref(rj)))
+        return RjRunResult(keep["q_chain"], keep["p_chain"], keep["E_chain"], keep["V_chain"], keep["T_chain"],
+                           keep["A_chain"], keep["q_final"], keep["accept_rate"], self.last_kernel_ms(), **out)
+
+    def philox_rj_draws(self, seed, niter, beta_a=2.0, beta_b=2.0, field_id_base=0, field_id_stride=1):
+        """The draw records [F, niter+1, 14] run_rj consumes for `seed` (see rj_draws.cuh for the layout)."""
+        draws = np.zeros((self.F, int(niter) + 1, RJ_DRAWS))
+        check(self._lib.srhmc_philox_rj_draws(self._h, int(seed), int(niter), int(field_id_base), int(field_id_stride),
+                                              float(beta_a), float(beta_b), dptr(draws)))
+        return draws
 
     # ------------------------------------------------------------------ a9: run_single_RHMC(implicit)
     def run_single(self, q0, p0, nsteps, dt, delta=1e-6, counter_max=100, f_pos=False, g_ff2=1.0, beta=1.0,

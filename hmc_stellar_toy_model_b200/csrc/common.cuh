@@ -54,7 +54,7 @@ struct FieldParams {
     double alpha, Vpc, vc_pow;
 };
 
-enum Mode : int { MODE_EVAL = 0, MODE_STEP = 1, MODE_RUN = 2, MODE_SINGLE = 3 };
+enum Mode : int { MODE_EVAL = 0, MODE_STEP = 1, MODE_RUN = 2, MODE_SINGLE = 3, MODE_RUN_RJ = 4 };
 // samplers.lightsource_gym family (ls_kernel.cuh)
 enum LsVariant : int { LS_HMC = 0, LS_DIAG = 1, LS_HESS = 2, LS_TRIAL = 3, LS_EVAL_HESS = 4, LS_EVAL_BG = 5 };
 
@@ -134,6 +134,22 @@ struct LaunchArgs {
     double* draws_normals;  // philox dump
     double* draws_lnu;
 };
+
+// Reversible-jump chains (field_kernel MODE_RUN_RJ, field_rj.cuh).  The block sits at the start of the launch's scratch
+// buffer, so that LaunchArgs, and with it every other kernel's parameter space, stays as it is.
+constexpr int kRjDraws = 14;   // doubles of one (field, iteration) draw record (rj_draws.cuh)
+struct RjParams {
+    double cdf0, cdf1;          // (P0, P0 + P1) / (P0 + P1 + P2): np.random.choice's cumulative move probabilities
+    double pl_lo, pl_span;      // fmin^(1-alpha) and fmax^(1-alpha) - fmin^(1-alpha) of gen_pow_law_sample
+    double K_split, beta_a, beta_b, ln_beta;   // ln_beta = ln B(beta_a, beta_b)
+    const double* draws;        // [F, L, kRjDraws] injected records, or nullptr (device Philox)
+    int* N_chain;               // [F, n_rows] star count at the start of each kept iteration, or nullptr
+    unsigned char* move_chain;  // [F, n_rows] 0 within, 1 birth, 2 death, 3 split, 4 merge (gym.move_types), or nullptr
+    int* n_final;               // [F] star count after the last iteration
+    int* overflow;              // [F] first iteration whose proposal needed more than Nmax stars, -1 if none
+    long long field_stride;     // doubles of per-field scratch that follow the block
+};
+constexpr size_t kRjHeaderDoubles = (sizeof(RjParams) + 15) / 16 * 2;
 
 // ------------------------------------------------------------------ metric (sampler_RHMC.py:229-292)
 struct Metric {

@@ -611,6 +611,12 @@ struct Energies {
     double V, T;
 };
 
+// One star's share of the two sums of T = (sum p^2/H + sum ln|H|)/2 (sampler_RHMC.py:353-363)
+__device__ __forceinline__ void kinetic_terms(const Metric& m, double pf, double px, double py, double& quad, double& logdet) {
+    quad += pf * pf / m.Hff + px * px / m.Hxx + py * py / m.Hxx;
+    logdet += log(fabs(m.Hff)) + 2.0 * log(fabs(m.Hxx));
+}
+
 // two CTA-wide maxima of the fixed-point iteration counts (rhmc_step): a corner of the reduction scratch that block_sum
 // (at most 7 values wide here) never touches
 template <typename T>
@@ -624,10 +630,7 @@ __device__ Energies energies(const Ctx<T>& c, double Vpix, int f_pos, bool with_
     for (int k = threadIdx.x; k < c.N; k += blockDim.x) {
         const double f = c.q[3 * k], x = c.q[3 * k + 1], y = c.q[3 * k + 2];
         if (with_T) {
-            const Metric m = metric_of(P, f, c.g_ff2);
-            const double pf = c.p[3 * k], px = c.p[3 * k + 1], py = c.p[3 * k + 2];
-            v[0] += pf * pf / m.Hff + px * px / m.Hxx + py * py / m.Hxx;
-            v[1] += log(fabs(m.Hff)) + 2.0 * log(fabs(m.Hxx));
+            kinetic_terms(metric_of(P, f, c.g_ff2), c.p[3 * k], c.p[3 * k + 1], c.p[3 * k + 2], v[0], v[1]);
         }
         if (P.use_prior) v[2] += P.alpha * log(f) + P.Vpc;
         if (P.use_Vc) v[3] += vc_row(c, k);
@@ -807,10 +810,16 @@ __device__ void rhmc_step(const Ctx<T>& c, double delta, int counter_max, bool w
     }
 }
 
+}  // namespace srhmc
+
+#include "field_rj.cuh"
+
+namespace srhmc {
+
 // ---------------------------------------------------------------------------------------------- kernel
 // KMODE: -1 = every mode in one kernel (A.mode decides), otherwise the kernel is compiled for that mode alone; KV3 as in
 // eval_pixels.  The specialised <MODE_RUN, 1> build is the hot path of crowded-field chains: a third of the code of the
-// generic kernel, no spills.
+// generic kernel, no spills.  MODE_RUN_RJ (reversible-jump chains) exists only as its own instantiations.
 template <typename T, int MR, int MC, int KMODE = -1, int KV3 = -1>
 __global__ void __launch_bounds__(512, 1)
 field_kernel(const __grid_constant__ FieldParams P, const __grid_constant__ LaunchArgs A, double* scratch, int d_in_smem) {
@@ -854,7 +863,10 @@ field_kernel(const __grid_constant__ FieldParams P, const __grid_constant__ Laun
         __syncthreads();
 
         const int mode = KMODE >= 0 ? KMODE : A.mode;
-        if (mode == MODE_EVAL) {
+        if constexpr (KMODE == MODE_RUN_RJ) {
+            // compiled into the MODE_RUN_RJ instantiations only (field_rj.cuh)
+            run_rj_field<T, MR, MC, KV3>(c, A, scratch, field);
+        } else if (mode == MODE_EVAL) {
             const double Vpix = eval_pixels<T, MR, MC, KV3>(c, true);
             const Energies e = energies(c, Vpix, A.f_pos, false);
             for (int k = tid; k < c.N; k += nt) {

@@ -27,6 +27,9 @@ int ls_kernel_launch(int mr, int mc, int grid, int threads, size_t smem, cudaStr
                      const LsArgs& A, double* scratch, int dsm);
 int philox_dump_launch(cudaStream_t stream, unsigned long long seed, int n_fields, int L, int Nmax, int fid_base,
                        int fid_stride, double* normals, double* lnu);
+// the draw records of field_kernel MODE_RUN_RJ (rj_draws.cuh): draws [n_fields, L, kRjDraws]
+int rj_dump_launch(cudaStream_t stream, unsigned long long seed, int n_fields, int L, int fid_base, int fid_stride, double beta_a,
+                   double beta_b, double* draws);
 int metric_launch(cudaStream_t stream, const FieldParams& P, size_t n_stars, const double* q, double g_ff2, double* H,
                   double* Hgrad);
 int kinetic_diag_launch(cudaStream_t stream, size_t n, const double* p, const double* H, double* T);

@@ -1,6 +1,7 @@
 // Small utility kernels: Philox dump, image conversion, FMA-chain peak microbenchmark, and the precision
 // dispatch of the CTA-per-field launchers.
 #include "kernels_api.h"
+#include "rj_draws.cuh"
 
 namespace srhmc {
 
@@ -19,6 +20,24 @@ __global__ void philox_dump_kernel(unsigned long long seed, int n_fields, int L,
         o[0] = z[0]; o[1] = z[1]; o[2] = z[2];
         if (k == 0) lnu[(size_t)f * L + l] = philox_lnu(seed, fid, (uint32_t)l);
     }
+}
+
+// Reversible-jump draw records exactly as MODE_RUN_RJ consumes them: one thread per (field, iteration).
+__global__ void rj_dump_kernel(unsigned long long seed, int n_fields, int L, int fid_base, int fid_stride, double beta_a,
+                               double beta_b, double* draws) {
+    const size_t total = (size_t)n_fields * L;
+    for (size_t t = blockIdx.x * (size_t)blockDim.x + threadIdx.x; t < total; t += (size_t)gridDim.x * blockDim.x) {
+        const int l = (int)(t % L), f = (int)(t / L);
+        rj_record(seed, (uint32_t)(fid_base + f * fid_stride), (uint32_t)l, beta_a, beta_b, draws + t * kRjDraws);
+    }
+}
+
+int rj_dump_launch(cudaStream_t stream, unsigned long long seed, int n_fields, int L, int fid_base, int fid_stride, double beta_a,
+                   double beta_b, double* draws) {
+    const size_t total = (size_t)n_fields * L;
+    const int blocks = (int)((total + 127) / 128 < 4096 ? (total + 127) / 128 : 4096);
+    rj_dump_kernel<<<blocks > 0 ? blocks : 1, 128, 0, stream>>>(seed, n_fields, L, fid_base, fid_stride, beta_a, beta_b, draws);
+    return (int)cudaGetLastError();
 }
 
 // Kinetic energy and the tau-part derivatives of one field per block (sampler_RHMC.py:353-363, 467-492):

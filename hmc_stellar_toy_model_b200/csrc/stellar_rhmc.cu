@@ -103,6 +103,7 @@ struct srhmc_ctx {
     bool run_has_nstars = false, run_has_normals = false, run_has_lnu = false, run_one_star = false;
     bool run_has_qchain = false;  // the last launched run recorded q_chain on the device
     DevBuf st_means, st_R, st_neff;  // chain statistics
+    DevBuf rj_draws, rj_N, rj_move, rj_nfinal, rj_overflow;  // reversible-jump runs
 };
 
 namespace {
@@ -256,6 +257,17 @@ bool chain_kernel_eligible(const srhmc_config& g, const FieldParams& P) {
 }
 
 
+bool no_device() {
+    int n = 0;
+    return cudaGetDeviceCount(&n) != cudaSuccess || n == 0;
+}
+
+// a null context: without a device there can be none, so say that rather than "bad argument"
+int null_ctx() {
+    return no_device() ? fail(SRHMC_ERR_NO_DEVICE, "no CUDA device visible: this library has no CPU path")
+                       : fail(SRHMC_ERR_INVALID, "null argument");
+}
+
 bool all_one_star(const srhmc_ctx* c, const int32_t* nstars) {
     if (!nstars) return c->cfg.max_stars == 1;
     for (int f = 0; f < c->cfg.n_fields; ++f)
@@ -406,7 +418,7 @@ int srhmc_destroy(srhmc_ctx* c) {
     cudaStreamSynchronize(c->stream);
     DevBuf* all[] = {&c->ls_dt, &c->ls_steps, &c->ls_bg, &c->ls_scratch, &c->ls_d1, &c->ls_d2, &c->ls_d3, &c->field_ids, &c->sched_done, &c->sched_state, &c->sched_err, &c->D32, &c->D16, &c->logtab, &c->flag, &c->D, &c->Dstage, &c->q, &c->p, &c->nstars, &c->normals, &c->lnu, &c->sg, &c->sb, &c->qchain,
                      &c->pchain, &c->E, &c->V, &c->T, &c->A, &c->acc, &c->scratch, &c->qout, &c->pout, &c->Vout, &c->st_means, &c->st_R, &c->st_neff,
-                     &c->grad, &c->H, &c->Hg, &c->counts};
+                     &c->grad, &c->H, &c->Hg, &c->counts, &c->rj_draws, &c->rj_N, &c->rj_move, &c->rj_nfinal, &c->rj_overflow};
     for (DevBuf* b : all) b->release();
     if (c->ev0) cudaEventDestroy(c->ev0);
     if (c->ev1) cudaEventDestroy(c->ev1);
@@ -972,6 +984,72 @@ int srhmc_run(srhmc_ctx* c, const srhmc_run_args* a) {
     return srhmc_run_download(c, a);
 }
 
+int srhmc_run_rj(srhmc_ctx* c, const srhmc_run_args* a, const srhmc_rj_args* rj) {
+    if (!c) return null_ctx();
+    if (!a || !rj) return fail(SRHMC_ERR_INVALID, "null argument");
+    if (c->cfg.precision != 64) return fail(SRHMC_ERR_INVALID, "reversible-jump runs need a precision-64 context");
+    const double* pm = rj->P_move;
+    for (int i = 0; i < 3; ++i)
+        if (!(pm[i] >= 0.0) || !std::isfinite(pm[i])) return fail(SRHMC_ERR_INVALID, "P_move[%d] = %g is not a finite probability", i, pm[i]);
+    const double psum = (pm[0] + pm[1]) + pm[2];
+    if (!(psum > 0.0)) return fail(SRHMC_ERR_INVALID, "P_move sums to 0");
+    if (!(rj->fmin > 0.0) || !(rj->fmax > rj->fmin) || !std::isfinite(rj->fmax))
+        return fail(SRHMC_ERR_INVALID, "the flux prior needs 0 < fmin < fmax (got %g, %g)", rj->fmin, rj->fmax);
+    if (!(c->cfg.alpha > 1.0)) return fail(SRHMC_ERR_INVALID, "the power-law flux prior needs alpha > 1 (got %g)", c->cfg.alpha);
+    if (!(rj->beta_a > 0.0) || !(rj->beta_b > 0.0) || !std::isfinite(rj->beta_a) || !std::isfinite(rj->beta_b))
+        return fail(SRHMC_ERR_INVALID, "beta_a and beta_b must be positive (got %g, %g)", rj->beta_a, rj->beta_b);
+    if (!(rj->K_split > 0.0) || !std::isfinite(rj->K_split)) return fail(SRHMC_ERR_INVALID, "K_split must be positive (got %g)", rj->K_split);
+    const size_t F = c->cfg.n_fields, S = 3 * (size_t)c->cfg.max_stars;
+    if (a->nstars)
+        for (size_t f = 0; f < F; ++f)
+            if (a->nstars[f] < 0 || a->nstars[f] > c->cfg.max_stars)
+                return fail(SRHMC_ERR_INVALID, "nstars[%zu] = %d is outside 0..max_stars (%d)", f, a->nstars[f], c->cfg.max_stars);
+    if (int rc = srhmc_run_upload(c, a)) return rc;
+    LaunchArgs A;
+    if (int rc = build_run_launch_args(c, a, A)) return rc;
+    A.mode = MODE_RUN_RJ;
+    const size_t rows = (size_t)c->run_rows, L = (size_t)a->niter + 1;
+    // star counts change along the chain: the slots past N of every row and of q_final read back as zeros
+    if (S) {
+        if (a->q_chain) CU_TRY(cudaMemsetAsync(c->qchain.ptr, 0, F * rows * S * 8, c->stream));
+        if (a->p_chain) CU_TRY(cudaMemsetAsync(c->pchain.ptr, 0, F * rows * S * 8, c->stream));
+        CU_TRY(cudaMemsetAsync(c->qout.ptr, 0, F * S * 8, c->stream));
+    }
+    RjParams R;
+    std::memset(&R, 0, sizeof(R));
+    R.cdf0 = pm[0] / psum;
+    R.cdf1 = (pm[0] + pm[1]) / psum;
+    const double e = 1.0 - c->cfg.alpha;
+    R.pl_lo = std::pow(rj->fmin, e);
+    R.pl_span = std::pow(rj->fmax, e) - std::pow(rj->fmin, e);
+    R.K_split = rj->K_split;
+    R.beta_a = rj->beta_a;
+    R.beta_b = rj->beta_b;
+    R.ln_beta = std::lgamma(rj->beta_a) + std::lgamma(rj->beta_b) - std::lgamma(rj->beta_a + rj->beta_b);
+    R.field_stride = (long long)(2 * S + c->threads);  // q and pixel gradient of the iteration's start, merge partial sums
+    if (rj->draws) {
+        if (int rc = upload(c, c->rj_draws, rj->draws, F * L * kRjDraws * 8)) return rc;
+        R.draws = c->rj_draws.as<double>();
+    }
+    if (int rc = c->rj_N.ensure(F * rows * 4)) return rc;
+    if (int rc = c->rj_move.ensure(F * rows)) return rc;
+    if (int rc = c->rj_nfinal.ensure(F * 4)) return rc;
+    if (int rc = c->rj_overflow.ensure(F * 4)) return rc;
+    R.N_chain = c->rj_N.as<int>();
+    R.move_chain = c->rj_move.as<unsigned char>();
+    R.n_final = c->rj_nfinal.as<int>();
+    R.overflow = c->rj_overflow.as<int>();
+    if (int rc = c->scratch.ensure((kRjHeaderDoubles + F * (size_t)R.field_stride) * 8)) return rc;
+    CU_TRY(cudaMemcpyAsync(c->scratch.ptr, &R, sizeof(R), cudaMemcpyHostToDevice, c->stream));
+    // never the one-star kernel: it cannot change a field's star count
+    if (int rc = launch_field(c, A, false)) return rc;
+    if (rj->N_chain) if (int rc = download(c, rj->N_chain, c->rj_N, F * rows * 4)) return rc;
+    if (rj->move_chain) if (int rc = download(c, rj->move_chain, c->rj_move, F * rows)) return rc;
+    if (rj->n_final) if (int rc = download(c, rj->n_final, c->rj_nfinal, F * 4)) return rc;
+    if (rj->overflow) if (int rc = download(c, rj->overflow, c->rj_overflow, F * 4)) return rc;
+    return srhmc_run_download(c, a);
+}
+
 int srhmc_run_single(srhmc_ctx* c, const double* q0, const double* p0, const int32_t* nstars, int32_t nsteps, double dt,
                      double delta, int32_t counter_max, int32_t f_pos, double g_ff2, double beta, double* q_chain,
                      double* p_chain, double* E_chain, double* V_chain, double* T_chain) {
@@ -1278,6 +1356,23 @@ int srhmc_philox_draws_ids(srhmc_ctx* c, uint64_t seed, int32_t niter, int32_t f
     CU_TRY(cudaStreamSynchronize(c->stream));
     c->run_has_normals = false;  // the staging buffers were overwritten
     c->run_has_lnu = false;
+    return 0;
+}
+
+int srhmc_philox_rj_draws(srhmc_ctx* c, uint64_t seed, int32_t niter, int32_t fid_base, int32_t fid_stride, double beta_a,
+                          double beta_b, double* draws) {
+    if (!c) return null_ctx();
+    if (!draws || niter < 0) return fail(SRHMC_ERR_INVALID, "bad argument");
+    if (!(beta_a > 0.0) || !(beta_b > 0.0)) return fail(SRHMC_ERR_INVALID, "beta_a and beta_b must be positive");
+    if (fid_stride == 0) fid_stride = 1;
+    CU_TRY(cudaSetDevice(c->cfg.device));
+    const size_t F = c->cfg.n_fields, L = (size_t)niter + 1, bytes = F * L * kRjDraws * 8;
+    if (int rc = c->rj_draws.ensure(bytes)) return rc;
+    const int e = rj_dump_launch(c->stream, seed, (int)F, (int)L, fid_base, fid_stride, beta_a, beta_b, c->rj_draws.as<double>());
+    if (e != 0) return fail(SRHMC_ERR_CUDA, "reversible-jump draw dump failed: %s", cudaGetErrorString((cudaError_t)e));
+    c->launches += 1;
+    if (int rc = download(c, draws, c->rj_draws, bytes)) return rc;
+    CU_TRY(cudaStreamSynchronize(c->stream));
     return 0;
 }
 

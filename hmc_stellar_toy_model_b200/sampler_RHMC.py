@@ -11,9 +11,12 @@ What runs where
                   global np.random stream is consumed in exactly the reference's order (sampler_RHMC.py:1021-1075:
                   randn(3N), one uniform for np.random.choice, one uniform for the accept test, per iteration), so a
                   script that seeds np.random reproduces the reference's chain step for step.
-  host + device   reversible-jump moves (birth/death, split/merge; sampler_RHMC.py:1084-1445): the trans-dimensional
-                  proposal bookkeeping stays on the host as upstream, every RHMC leg / V / H / T around it runs on the
-                  device (one launch per leg).
+  host + device   reversible-jump moves (birth/death, split/merge; sampler_RHMC.py:1084-1445): by default the
+                  trans-dimensional proposal bookkeeping stays on the host as upstream (the legacy np.random stream, byte
+                  for byte), every RHMC leg / V / H / T around it runs on the device (one launch per leg).
+  device (opt-in) gym.device_seed = <int> (new capability): the whole reversible-jump run is ONE launch of the
+                  crowded-field kernel (RHMCContext.run_rj), proposals included, drawing counter-based Philox; the global
+                  np.random stream is not touched.
   not provided    matplotlib diagnostics (no-ops here), the "naive"/"leap_frog" solvers and run_single_HMC (unused by
                   any script, labelled broken upstream).
 
@@ -337,6 +340,9 @@ class multi_gym(base_class):
         self.A_chain = None
         self.fmin = None
         self.fmax = None
+        #: None: reversible-jump runs draw from the global np.random stream with the proposals on the host (reference
+        #: order).  An int: they run entirely on the device with counter-based Philox draws keyed by this seed.
+        self.device_seed = None
 
     def run_RHMC(self, q_model_0, f_pos=True, delta=1e-6, Niter=100, Nsteps=100, dt=1e-1, save_traj=False,
                  counter_max=1000, verbose=False, q_true=None, schedule_g_ff2=None, N_max=50,
@@ -359,6 +365,8 @@ class multi_gym(base_class):
         L = Niter + 1
 
         if float(P_move[1]) != 0.0 or float(P_move[2]) != 0.0:
+            if self.device_seed is not None:
+                return self._run_RHMC_rj_device(q0, f_pos, delta, counter_max, schedule_g_ff2, schedule_beta)
             return self._run_RHMC_rj(q0, f_pos, delta, counter_max, verbose, schedule_g_ff2, schedule_beta)
 
         # the reference's draws, in the reference's order (sampler_RHMC.py:1022, 1046, 1075)
@@ -496,6 +504,37 @@ class multi_gym(base_class):
                 print("N_objs: %d\n" % self.Nobjs)
                 self.R_accept_report(idx_iter=l, run_window=10)
                 print("\n\n")
+        print("Finished. Final report.")
+        self.R_accept_report(idx_iter=-1, running=False)
+
+    def _run_RHMC_rj_device(self, q0, f_pos, delta, counter_max, schedule_g_ff2, schedule_beta):
+        """The reversible-jump run as one device launch (RHMCContext.run_rj); same attributes, shapes and dtypes as
+        _run_RHMC_rj."""
+        if self.fmin is None or self.fmax is None:
+            raise TypeError("reversible-jump moves need gym.fmin and gym.fmax (sampler_RHMC.py:1200-1210)")
+        sg = None if schedule_g_ff2 is None else np.asarray(schedule_g_ff2, dtype=float)
+        sb = None if schedule_beta is None else np.asarray(schedule_beta, dtype=float)
+        r = self._rj_ctx().run_rj(self._pad(q0), self.Niter, self.Nsteps, self.dt, nstars=[self.Nobjs], delta=delta,
+                                  counter_max=counter_max, f_pos=f_pos, g_ff2=self.g_ff2, beta=self.beta,
+                                  schedule_g_ff2=sg, schedule_beta=sb, seed=int(self.device_seed), P_move=self.P_move,
+                                  fmin=self.fmin, fmax=self.fmax, K_split=self.K_split, beta_a=self.beta_a,
+                                  beta_b=self.beta_b)
+        if r.overflow[0] >= 0:
+            raise ValueError("the proposal of iteration %d needs %d stars but N_max = %d"
+                             % (r.overflow[0], self.N_max + 1, self.N_max))
+        L = self.Niter + 1
+        if sg is not None and sg.size:
+            self.g_ff2 = sg[min(L, sg.size) - 1]
+        if sb is not None and sb.size:
+            self.beta = sb[min(L, sb.size) - 1]
+        self.q_chain, self.p_chain = r.q_chain[0], r.p_chain[0]
+        self.E_chain, self.V_chain, self.T_chain = r.E_chain[0], r.V_chain[0], r.T_chain[0]
+        self.A_chain = r.A_chain[0].astype(bool)
+        self.move_chain = r.move_chain[0].astype(int)
+        self.N_chain = r.N_chain[0].astype(int)
+        self.Nobjs = int(r.n_final[0])
+        self.d = 3 * self.Nobjs
+        self.kernel_ms = r.kernel_ms
         print("Finished. Final report.")
         self.R_accept_report(idx_iter=-1, running=False)
 

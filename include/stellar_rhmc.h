@@ -155,6 +155,26 @@ typedef struct srhmc_run_args {
     const int32_t* field_ids;
 } srhmc_run_args;
 
+/* Reversible-jump part of a chain run (srhmc_run_rj).  Replaces multi_gym.run_RHMC with P_move[1] or P_move[2] nonzero
+ * (sampler_RHMC.py:1009-1198: birth/death and split/merge proposals, sampler_RHMC.py:1200-1445, between two RHMC legs of
+ * nsteps steps each).  Each iteration draws one record of 14 doubles (srhmc_philox_rj_draws): u_move, u_grow, u_a, u_b, u_c,
+ * two split-offset normals, the split share ~ Beta(beta_a, beta_b) and six momentum normals.
+ * Shapes (F = n_fields, L = niter+1, Ls = ceil(L / chain_stride)): draws [F,L,14] or NULL (device Philox, key run.seed);
+ * outputs, each may be NULL: N_chain [F,Ls] star count at the start of each kept iteration, move_chain [F,Ls]
+ * (0 within, 1 birth, 2 death, 3 split, 4 merge), n_final [F], overflow [F] (first iteration whose proposal needed more
+ * than max_stars stars, -1 if none).  alpha and V_prior_const come from the context's srhmc_config. */
+typedef struct srhmc_rj_args {
+    double P_move[3];
+    double fmin, fmax;
+    double K_split;
+    double beta_a, beta_b;
+    const double* draws;
+    int32_t* N_chain;
+    uint8_t* move_chain;
+    int32_t* n_final;
+    int32_t* overflow;
+} srhmc_rj_args;
+
 int srhmc_abi_version(void);
 const char* srhmc_last_error(void);
 int srhmc_device_count(void);
@@ -267,6 +287,19 @@ int srhmc_run(srhmc_ctx* ctx, const srhmc_run_args* args);
 int srhmc_run_upload(srhmc_ctx* ctx, const srhmc_run_args* args);
 int srhmc_run_launch(srhmc_ctx* ctx, const srhmc_run_args* args);
 int srhmc_run_download(srhmc_ctx* ctx, const srhmc_run_args* args);
+
+/* Reversible-jump chains (see srhmc_rj_args): every iteration of every field inside one launch of the CTA-per-field kernel,
+ * the star count of each field changing on the device.  `run` is used as by srhmc_run (q0, nstars, schedules, seed,
+ * injected normals / lnu, chain outputs, chain_stride, field ids); chain rows are zero past 3 * N_chain of their row.
+ * Where the reference raises (a death or split with no star, a merge with fewer than two stars or all pair weights zero,
+ * a proposal needing more than max_stars stars) the jump is rejected with the state unchanged.  P_move = {1, 0, 0}
+ * reproduces srhmc_run bit for bit.  FP64 contexts only. */
+int srhmc_run_rj(srhmc_ctx* ctx, const srhmc_run_args* run, const srhmc_rj_args* rj);
+
+/* The draw records [F, niter+1, 14] srhmc_run_rj consumes for `seed` with the field identity of srhmc_run_args; the split
+ * share depends on beta_a, beta_b. */
+int srhmc_philox_rj_draws(srhmc_ctx* ctx, uint64_t seed, int32_t niter, int32_t field_id_base, int32_t field_id_stride,
+                          double beta_a, double beta_b, double* draws);
 
 /* One long trajectory per field recording V-V0, T-T0 and their sum after every step.  Replaces
  * single_gym.run_single_RHMC(solver="implicit") (sampler_RHMC.py:649-783).
