@@ -462,7 +462,7 @@ class BigFieldRHMC:
     def _step_struct(self, dt, delta, g_ff2, counter_max, f_pos, iteration, seed):
         return _capi.BigStep(dt=float(dt), delta=float(delta), g_ff2=float(g_ff2), counter_max=int(counter_max),
                              f_pos=int(bool(f_pos)), iteration=int(iteration),
-                             fixed_point_mode=int(getattr(self, "fixed_point_mode", 0)), seed=int(seed))
+                             fixed_point_mode=self.fixed_point_mode, seed=int(seed))
 
     def _all(self, name, st):
         for s in self.strips:
@@ -471,9 +471,7 @@ class BigFieldRHMC:
     def evaluate(self, want_V=True, **kw):
         """One gradient (and potential) evaluation at the current star state."""
         st = self._step_struct(kw.get("dt", 0.0), 1e-6, kw.get("g_ff2", 1.0), 1000, kw.get("f_pos", True), 0, 0)
-        if self.multi:
-            self._all("PACK", st)
-            self.comm.gather_ghosts(self.strips)
+        self._ghosts(st)
         self._all("EVAL_V" if want_V else "EVAL", st)
         self._all("ENERGY", st)
         if self.multi:
@@ -488,9 +486,7 @@ class BigFieldRHMC:
         if self.multi:
             self.comm.max_counters(self.strips)
         self._all("QFIX_KICK", st)
-        if self.multi:
-            self._all("PACK", st)
-            self.comm.gather_ghosts(self.strips)
+        self._ghosts(st)
 
     def _ghosts(self, st):
         if self.multi:
@@ -536,9 +532,7 @@ class BigFieldRHMC:
     def steps(self, nsteps, dt, delta=1e-6, counter_max=1000, g_ff2=1.0):
         """nsteps leapfrog steps from the current (q, p) (srhmc_step semantics)."""
         st = self._step_struct(dt, delta, g_ff2, counter_max, True, 0, 0)
-        if self.multi:
-            self._all("PACK", st)
-            self.comm.gather_ghosts(self.strips)
+        self._ghosts(st)
         self._all("EVAL", st)
         self.trajectory(st, nsteps, False)
 
@@ -581,9 +575,7 @@ class BigFieldRHMC:
             s.set_recording(L, chain_stride, want)
         self._rec = rec
         st0 = self._step_struct(dt, delta, g_ff2, counter_max, f_pos, 0, seed)
-        if self.multi:
-            self._all("PACK", st0)
-            self.comm.gather_ghosts(self.strips)
+        self._ghosts(st0)
         self._all("EVAL_V", st0)
         has_sched = schedule_g_ff2 is not None and len(schedule_g_ff2) > 0
         dist_comm = isinstance(self.comm, TorchDistComm)
@@ -606,7 +598,7 @@ class BigFieldRHMC:
             # one captured iteration serves every later run with the same launch parameters (the chain row and the RNG
             # counter come from the device-side iteration counter; the buffers are owned by the strips and never move)
             key = (int(nsteps), float(dt), float(delta), float(g_ff2), int(counter_max), bool(f_pos), int(seed), L,
-                   tuple(s.n for s in self.strips), int(getattr(self, "fixed_point_mode", 0)), want, int(chain_stride))
+                   tuple(s.n for s in self.strips), self.fixed_point_mode, want, int(chain_stride))
             if normals is not None or lnu is not None:
                 key = None  # injected draws live in buffers that are re-allocated per run: always capture afresh
             if key is None or getattr(self, "_graph_key", None) != key:

@@ -358,36 +358,146 @@ __device__ __forceinline__ double dphi_f(const BigParams& P, const MetricFast& m
     return gf + m.tphi;
 }
 
-// (1) p -= h dphi/dq; (2) p fixed point, phase A: iterate to this star's own convergence, record the count
-__global__ void big_kick1_kernel(const BigParams P, const BigStep S, int n, const double* q, double* p, const double* g,
-                                 double* a1, double* a2, int* cnt, const PeerX X) {
-    int local_max = 0;
-    for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += gridDim.x * blockDim.x) {
-        const double f = q[3 * k];
-        const MetricFast m = metric_fast(S.K, f);
-        double pf = p[3 * k] - S.h * dphi_f(P, m, g[3 * k], f);
-        p[3 * k + 1] -= S.h * g[3 * k + 1];
-        p[3 * k + 2] -= S.h * g[3 * k + 2];
-        const double rho = pf, kap = m.kap;
-        a1[3 * k] = rho;      // anchor
-        a2[3 * k] = kap;
-        int c = 0;
-        while (c < S.counter_max) {
-            const double pn = rho - S.h * (((pf * pf) * kap) / 2.0);
-            const bool more = fabs(pf - pn) > S.delta;
-            pf = pn;
-            ++c;
-            if (!more) break;
-        }
-        p[3 * k] = pf;
-        a1[3 * k + 1] = (double)c;  // own count
-        local_max = max(local_max, c);
-    }
-    if (local_max) atomicMax(cnt, local_max);
-    if (X.prod && !S.per_star) peer_max_epilogue(X, cnt);
+// The pieces of RHMC_single_step (sampler_RHMC.py:522-566) for one star.  Every scalar kernel below is composed of them, so a
+// fused phase does the arithmetic of the phases it fuses in the same order (tests/test_bigfield_phases.py).
+struct Star3 {
+    double f, x, y;
+};
+__device__ __forceinline__ Star3 load3(const double* a, int k) { return {a[3 * k], a[3 * k + 1], a[3 * k + 2]}; }
+__device__ __forceinline__ void store3(double* a, int k, const Star3& v) {
+    a[3 * k] = v.f; a[3 * k + 1] = v.x; a[3 * k + 2] = v.y;
 }
 
-// p fixed point phase B (continue to the global count), then (3) q fixed point phase A
+// dV/dq of star k at s: the sum of its footprint partials when the evaluation left them (stored to g on the way), else g
+__device__ __forceinline__ Star3 star_grad(const BigParams& P, int k, const Star3& s, const double* gpart, double* g) {
+    Star3 d;
+    if (gpart) {
+        gsum_star(P, k, s.f, s.x, s.y, gpart, d.f, d.x, d.y);
+        store3(g, k, d);
+    } else {
+        d = load3(g, k);
+    }
+    return d;
+}
+
+// (1), (5): p -= h dphi/dq (dphi = dphi_f for the flux)
+__device__ __forceinline__ void half_kick(const BigStep& S, double dphi, const Star3& g, Star3& p) {
+    p.f = p.f - S.h * dphi;
+    p.x -= S.h * g.x;
+    p.y -= S.h * g.y;
+}
+
+// (6): reflections at f_lim and at the image edges
+__device__ __forceinline__ void reflect(const BigParams& P, const Star3& s, Star3& p) {
+    if (s.f < P.F.f_lim) p.f *= -1.0;
+    if ((s.x < 0.0) || (s.x > P.Rg - 1.0)) p.x *= -1.0;
+    if ((s.y < 0.0) || (s.y > P.C - 1.0)) p.y *= -1.0;
+}
+
+// (2): one iteration of the p fixed point p' = rho - h (p^2 kap)/2
+__device__ __forceinline__ double pfix_iter(const BigStep& S, double rho, double kap, double pf) {
+    return rho - S.h * (((pf * pf) * kap) / 2.0);
+}
+
+// (2), phase A: iterate from rho = pf to this star's own convergence; returns the count
+__device__ __forceinline__ int pfix_own(const BigStep& S, double kap, double& pf) {
+    const double rho = pf;
+    int c = 0;
+    while (c < S.counter_max) {
+        const double pn = pfix_iter(S, rho, kap, pf);
+        const bool more = fabs(pf - pn) > S.delta;
+        pf = pn;
+        ++c;
+        if (!more) break;
+    }
+    return c;
+}
+
+// (3): one iteration of the q fixed point q' = sigma + h (b + p/H(q)).  b = p/H(sigma) is an argument because the kernels
+// compute it in two forms (inv_hff_k / inv_hxx_k and metric_fast) that the compiler may contract differently.
+__device__ __forceinline__ Star3 qfix_iter(const BigStep& S, const Star3& sg, const Star3& b, const Star3& p, const Star3& q) {
+    const double uq = inv_hff_k(S.K, q.f), ihq = inv_hxx_k(S.K, q.f);
+    return {sg.f + S.h * (b.f + p.f * uq), sg.x + S.h * (b.x + p.x * ihq), sg.y + S.h * (b.y + p.y * ihq)};
+}
+
+// (3), phase A: iterate from q = sigma to this star's own convergence; returns the count
+__device__ __forceinline__ int qfix_own(const BigStep& S, const Star3& sg, const Star3& b, const Star3& p, Star3& q) {
+    q = sg;
+    int c = 0;
+    while (c < S.counter_max) {
+        const Star3 nq = qfix_iter(S, sg, b, p, q);
+        const double d = fmax(fabs(q.f - nq.f), fmax(fabs(q.x - nq.x), fabs(q.y - nq.y)));
+        q = nq;
+        ++c;
+        if (!(d > S.delta)) break;
+    }
+    return c;
+}
+
+// own q fixed-point count of star k (phase A, for phase B): n ints past the 3n doubles of a2
+__device__ __forceinline__ int& own_qcount(double* a2, int n, int k) { return reinterpret_cast<int*>(a2 + 3 * (size_t)n)[k]; }
+__device__ __forceinline__ int own_qcount(const double* a2, int n, int k) {
+    return reinterpret_cast<const int*>(a2 + 3 * (size_t)n)[k];
+}
+
+// (4): p -= h dtau/dq at the new q (only the flux momentum changes)
+__device__ __forceinline__ double dtau_kick(const BigStep& S, double qf, double pf) {
+    return pfix_iter(S, pf, metric_fast(S.K, qf).kap, pf);
+}
+
+// Prologue of a position update on the star-parallel evaluation path: the model image of the COMING evaluation is reset to the
+// background here (nobody reads it between the last gather and the next scatter), which saves that path a launch per step
+__device__ __forceinline__ void fill_background(const BigParams& P, double* L, size_t npix) {
+    if (L)
+        for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < npix; i += (size_t)gridDim.x * blockDim.x) L[i] = P.F.B;
+}
+
+// Epilogue of a position update: on the tile path the pair records of the new position for the coming evaluation (bin_star,
+// big_tile.cuh); with peer exchange the boundary-star counts per 1024-star chunk for the ordered ghost packing that follows
+// (integer atomics: exact)
+__device__ __forceinline__ void moved_star(const BigParams& P, int k, const Star3& q, int ntx, int* tcnt, PairRec* tlist,
+                                           int* err, int2* pack_counts, double lo_edge, double hi_edge) {
+    if (tcnt) bin_star(P, ntx, k, q.f, q.x, q.y, true, tcnt, tlist, err);
+    if (pack_counts) {
+        if (q.x < lo_edge) atomicAdd(&pack_counts[k >> 10].x, 1);
+        if (q.x >= hi_edge) atomicAdd(&pack_counts[k >> 10].y, 1);
+    }
+}
+
+// The kicks of the field-wide stop rule, one thread per star, at the current q and gradient:
+//   LAST_HALF   [g = sum of the footprint partials, when the evaluation left them], (5) p -= h dphi/dq, (6) reflections
+//   NEXT_FIRST  (1) p -= h dphi/dq, (2) p fixed point phase A: anchor and own count in a1, kap in a2, maximum count in *cnt
+// <false, true> is KICK1; <true, false> KICK2 and the tail of EVAL_KICK2 / EVAL_V_KICK2; <true, true> EVAL_KICK2_KICK1 (the last
+// half kick of a step and the first one of the next use the same q and the same gradient).
+template <bool LAST_HALF, bool NEXT_FIRST>
+__global__ void big_kick_kernel(const BigParams P, const BigStep S, int n, const double* q, double* p, double* g,
+                                const double* gpart, double* a1, double* a2, int* cnt, const PeerX X) {
+    int local_max = 0;
+    for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += gridDim.x * blockDim.x) {
+        const Star3 s = load3(q, k);
+        const Star3 gr = star_grad(P, k, s, LAST_HALF ? gpart : nullptr, g);
+        const MetricFast m = metric_fast(S.K, s.f);
+        const double dphi = dphi_f(P, m, gr.f, s.f);
+        Star3 pk = load3(p, k);
+        if (LAST_HALF) {
+            half_kick(S, dphi, gr, pk);
+            reflect(P, s, pk);
+        }
+        if (NEXT_FIRST) {
+            half_kick(S, dphi, gr, pk);
+            a1[3 * k] = pk.f;   // anchor
+            a2[3 * k] = m.kap;
+            const int c = pfix_own(S, m.kap, pk.f);
+            a1[3 * k + 1] = (double)c;
+            local_max = max(local_max, c);
+        }
+        store3(p, k, pk);
+    }
+    if (NEXT_FIRST && local_max) atomicMax(cnt, local_max);
+    if (NEXT_FIRST && X.prod && !S.per_star) peer_max_epilogue(X, cnt);
+}
+
+// p fixed point phase B (continue to the field-wide count), then (3) q fixed point phase A: sigma in a1, p/H(sigma) in a2
 __global__ void big_pfix_qfix_kernel(const BigParams P, const BigStep S, int n, double* q, double* p, double* a1, double* a2,
                                      const int* cnt_p, int* cnt_q, const PeerX X) {
     const int target = S.per_star ? 0 : *cnt_p;
@@ -395,80 +505,36 @@ __global__ void big_pfix_qfix_kernel(const BigParams P, const BigStep S, int n, 
     for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += gridDim.x * blockDim.x) {
         double pf = p[3 * k];
         const double rho = a1[3 * k], kap = a2[3 * k];
-        for (int c = (int)a1[3 * k + 1]; c < target; ++c) pf = rho - S.h * (((pf * pf) * kap) / 2.0);
+        for (int c = (int)a1[3 * k + 1]; c < target; ++c) pf = pfix_iter(S, rho, kap, pf);
         p[3 * k] = pf;
-        // q' = sigma + h (p/H(sigma) + p/H(q))
-        const double sf = q[3 * k], sx = q[3 * k + 1], sy = q[3 * k + 2];
-        const double px = p[3 * k + 1], py = p[3 * k + 2];
-        const double u0 = inv_hff_k(S.K, sf), ih0 = inv_hxx_k(S.K, sf);
-        const double bf = pf * u0, bx = px * ih0, by = py * ih0;
-        double qf = sf, qx = sx, qy = sy;
-        int c = 0;
-        while (c < S.counter_max) {
-            const double uq = inv_hff_k(S.K, qf), ihq = inv_hxx_k(S.K, qf);
-            const double nf = sf + S.h * (bf + pf * uq);
-            const double nx = sx + S.h * (bx + px * ihq);
-            const double ny = sy + S.h * (by + py * ihq);
-            const double d = fmax(fabs(qf - nf), fmax(fabs(qx - nx), fabs(qy - ny)));
-            qf = nf; qx = nx; qy = ny;
-            ++c;
-            if (!(d > S.delta)) break;
-        }
-        a1[3 * k] = sf; a1[3 * k + 1] = sx; a1[3 * k + 2] = sy;   // sigma
-        a2[3 * k] = bf; a2[3 * k + 1] = bx; a2[3 * k + 2] = by;   // p/H(sigma)
-        q[3 * k] = qf; q[3 * k + 1] = qx; q[3 * k + 2] = qy;
+        const Star3 sg = load3(q, k), pk = {pf, p[3 * k + 1], p[3 * k + 2]};
+        const double u0 = inv_hff_k(S.K, sg.f), ih0 = inv_hxx_k(S.K, sg.f);
+        const Star3 b = {pf * u0, pk.x * ih0, pk.y * ih0};
+        Star3 qn;
+        const int c = qfix_own(S, sg, b, pk, qn);
+        store3(a1, k, sg);
+        store3(a2, k, b);
+        store3(q, k, qn);
         local_max = max(local_max, c);
-        reinterpret_cast<int*>(a2 + 3 * (size_t)n)[k] = c;   // own count, past the 3n doubles of a2
+        own_qcount(a2, n, k) = c;
     }
     if (local_max) atomicMax(cnt_q, local_max);
     if (X.prod && !S.per_star) peer_max_epilogue(X, cnt_q);
 }
 
-// q fixed point phase B, then (4) p -= h dtau/dq at the new q
-// and -- tile path -- the pair records of the star's final position for the coming evaluation (bin_star, big_tile.cuh)
+// q fixed point phase B, then (4) p -= h dtau/dq at the new q, and the position-update epilogue
 __global__ void big_qfix_kick_kernel(const BigParams P, const BigStep S, int n, double* q, double* p, const double* a1,
                                      const double* a2, const int* cnt_q, int ntx, int* tcnt, PairRec* tlist, int* err,
                                      int2* pack_counts, double lo_edge, double hi_edge, double* Lfill, size_t npix) {
-    // star-parallel evaluation path: the model image of the COMING evaluation is reset to the background here (nobody reads
-    // it between the last gather and the next scatter), which saves that path a launch per leapfrog step
-    if (Lfill)
-        for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < npix; i += (size_t)gridDim.x * blockDim.x) Lfill[i] = P.F.B;
+    fill_background(P, Lfill, npix);
     const int target = S.per_star ? 0 : *cnt_q;
     for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += gridDim.x * blockDim.x) {
-        const double sf = a1[3 * k], sx = a1[3 * k + 1], sy = a1[3 * k + 2];
-        const double bf = a2[3 * k], bx = a2[3 * k + 1], by = a2[3 * k + 2];
-        const double pf = p[3 * k], px = p[3 * k + 1], py = p[3 * k + 2];
-        double qf = q[3 * k], qx = q[3 * k + 1], qy = q[3 * k + 2];
-        for (int c = reinterpret_cast<const int*>(a2 + 3 * (size_t)n)[k]; c < target; ++c) {
-            const double uq = inv_hff_k(S.K, qf), ihq = inv_hxx_k(S.K, qf);
-            qf = sf + S.h * (bf + pf * uq);
-            qx = sx + S.h * (bx + px * ihq);
-            qy = sy + S.h * (by + py * ihq);
-        }
-        q[3 * k] = qf; q[3 * k + 1] = qx; q[3 * k + 2] = qy;
-        const MetricFast m = metric_fast(S.K, qf);
-        p[3 * k] = pf - S.h * (((pf * pf) * m.kap) / 2.0);
-        if (tcnt) bin_star(P, ntx, k, qf, qx, qy, true, tcnt, tlist, err);
-        // boundary-star counts per 1024-star chunk for the ordered ghost packing that follows (integer atomics: exact)
-        if (pack_counts) {
-            if (qx < lo_edge) atomicAdd(&pack_counts[k >> 10].x, 1);
-            if (qx >= hi_edge) atomicAdd(&pack_counts[k >> 10].y, 1);
-        }
-    }
-}
-
-// (5) p -= h dphi/dq at the new q; (6) reflections
-__global__ void big_kick2_kernel(const BigParams P, const BigStep S, int n, const double* q, double* p, const double* g) {
-    for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += gridDim.x * blockDim.x) {
-        const double f = q[3 * k], x = q[3 * k + 1], y = q[3 * k + 2];
-        const MetricFast m = metric_fast(S.K, f);
-        double pf = p[3 * k] - S.h * dphi_f(P, m, g[3 * k], f);
-        double px = p[3 * k + 1] - S.h * g[3 * k + 1];
-        double py = p[3 * k + 2] - S.h * g[3 * k + 2];
-        if (f < P.F.f_lim) pf *= -1.0;
-        if ((x < 0.0) || (x > P.Rg - 1.0)) px *= -1.0;
-        if ((y < 0.0) || (y > P.C - 1.0)) py *= -1.0;
-        p[3 * k] = pf; p[3 * k + 1] = px; p[3 * k + 2] = py;
+        const Star3 sg = load3(a1, k), b = load3(a2, k), pk = load3(p, k);
+        Star3 qn = load3(q, k);
+        for (int c = own_qcount(a2, n, k); c < target; ++c) qn = qfix_iter(S, sg, b, pk, qn);
+        store3(q, k, qn);
+        p[3 * k] = dtau_kick(S, qn.f, pk.f);
+        moved_star(P, k, qn, ntx, tcnt, tlist, err, pack_counts, lo_edge, hi_edge);
     }
 }
 
@@ -476,126 +542,32 @@ __global__ void big_kick2_kernel(const BigParams P, const BigStep S, int n, cons
 // more, so everything between two gradient evaluations is ONE per-star kernel and no iteration count crosses the GPUs:
 //   [FROM_EVAL: g = sum of the footprint partials, (5) last half kick and (6) reflections of the step that just ended]
 //   (1) p -= h dphi/dq, (2) p fixed point, (3) q fixed point -- each to the star's own convergence --,
-//   (4) p -= h dtau/dq at the new q, pair records of the new position, boundary-star counts for the ghost packing.
-// Same expressions, in the same order, as big_tail_kernel / big_kick1_kernel / big_pfix_qfix_kernel / big_qfix_kick_kernel.
+//   (4) p -= h dtau/dq at the new q, and the position-update epilogue.
 template <bool FROM_EVAL>
 __global__ void big_perstar_kernel(const BigParams P, const BigStep S, int n, double* q, double* p, double* g, const double* gpart,
                                    int ntx, int* tcnt, PairRec* tlist, int* err, int2* pack_counts, double lo_edge, double hi_edge,
                                    double* Lfill, size_t npix) {
-    if (Lfill)   // as big_qfix_kick_kernel: background reset of the star-parallel path's model image
-        for (size_t i = blockIdx.x * (size_t)blockDim.x + threadIdx.x; i < npix; i += (size_t)gridDim.x * blockDim.x) Lfill[i] = P.F.B;
+    fill_background(P, Lfill, npix);
     for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += gridDim.x * blockDim.x) {
-        const double sf = q[3 * k], sx = q[3 * k + 1], sy = q[3 * k + 2];
-        double gf, gx, gy;
-        if (FROM_EVAL && gpart) {
-            gsum_star(P, k, sf, sx, sy, gpart, gf, gx, gy);
-            g[3 * k] = gf; g[3 * k + 1] = gx; g[3 * k + 2] = gy;
-        } else {
-            gf = g[3 * k]; gx = g[3 * k + 1]; gy = g[3 * k + 2];
-        }
-        const MetricFast m0 = metric_fast(S.K, sf);
-        const double dphi = dphi_f(P, m0, gf, sf);
-        double pf = p[3 * k], px = p[3 * k + 1], py = p[3 * k + 2];
+        const Star3 sg = load3(q, k);
+        const Star3 gr = star_grad(P, k, sg, FROM_EVAL ? gpart : nullptr, g);
+        const MetricFast m0 = metric_fast(S.K, sg.f);
+        const double dphi = dphi_f(P, m0, gr.f, sg.f);
+        Star3 pk = load3(p, k);
         if (FROM_EVAL) {
-            pf = pf - S.h * dphi;
-            px -= S.h * gx;
-            py -= S.h * gy;
-            if (sf < P.F.f_lim) pf *= -1.0;
-            if ((sx < 0.0) || (sx > P.Rg - 1.0)) px *= -1.0;
-            if ((sy < 0.0) || (sy > P.C - 1.0)) py *= -1.0;
+            half_kick(S, dphi, gr, pk);
+            reflect(P, sg, pk);
         }
-        // (1), (2)
-        pf = pf - S.h * dphi;
-        px -= S.h * gx;
-        py -= S.h * gy;
-        {
-            const double rho = pf, kap = m0.kap;
-            int c = 0;
-            while (c < S.counter_max) {
-                const double pn = rho - S.h * (((pf * pf) * kap) / 2.0);
-                const bool more = fabs(pf - pn) > S.delta;
-                pf = pn;
-                ++c;
-                if (!more) break;
-            }
-        }
-        // (3) q' = sigma + h (p/H(sigma) + p/H(q))
-        const double bf = pf * m0.u, bx = px * m0.ihxx, by = py * m0.ihxx;
-        double qf = sf, qx = sx, qy = sy;
-        {
-            int c = 0;
-            while (c < S.counter_max) {
-                const double uq = inv_hff_k(S.K, qf), ihq = inv_hxx_k(S.K, qf);
-                const double nf = sf + S.h * (bf + pf * uq);
-                const double nx = sx + S.h * (bx + px * ihq);
-                const double ny = sy + S.h * (by + py * ihq);
-                const double d = fmax(fabs(qf - nf), fmax(fabs(qx - nx), fabs(qy - ny)));
-                qf = nf; qx = nx; qy = ny;
-                ++c;
-                if (!(d > S.delta)) break;
-            }
-        }
-        q[3 * k] = qf; q[3 * k + 1] = qx; q[3 * k + 2] = qy;
-        // (4)
-        const MetricFast m = metric_fast(S.K, qf);
-        p[3 * k] = pf - S.h * (((pf * pf) * m.kap) / 2.0);
-        p[3 * k + 1] = px;
-        p[3 * k + 2] = py;
-        if (tcnt) bin_star(P, ntx, k, qf, qx, qy, true, tcnt, tlist, err);
-        if (pack_counts) {
-            if (qx < lo_edge) atomicAdd(&pack_counts[k >> 10].x, 1);
-            if (qx >= hi_edge) atomicAdd(&pack_counts[k >> 10].y, 1);
-        }
+        half_kick(S, dphi, gr, pk);
+        pfix_own(S, m0.kap, pk.f);
+        const Star3 b = {pk.f * m0.u, pk.x * m0.ihxx, pk.y * m0.ihxx};
+        Star3 qn;
+        qfix_own(S, sg, b, pk, qn);
+        store3(q, k, qn);
+        pk.f = dtau_kick(S, qn.f, pk.f);
+        store3(p, k, pk);
+        moved_star(P, k, qn, ntx, tcnt, tlist, err, pack_counts, lo_edge, hi_edge);
     }
-}
-
-// Tail of a leapfrog step in ONE per-star kernel: [tile path: g = sum of the footprint partials (gsum_star)] ->
-// (5) p -= h dphi/dq at the new q -> (6) reflections -> [NEXT: steps (1) and (2, phase A) of the following leapfrog
-// step, which start from the same q and the same gradient].  Same operations in the same order as big_gsum_kernel,
-// big_kick2_kernel and big_kick1_kernel run back to back.
-template <bool NEXT>
-__global__ void big_tail_kernel(const BigParams P, const BigStep S, int n, const double* q, double* p, double* g,
-                                const double* gpart, double* a1, double* a2, int* cnt, const PeerX X) {
-    int local_max = 0;
-    for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += gridDim.x * blockDim.x) {
-        const double f = q[3 * k], x = q[3 * k + 1], y = q[3 * k + 2];
-        double gf, gx, gy;
-        if (gpart) {
-            gsum_star(P, k, f, x, y, gpart, gf, gx, gy);
-            g[3 * k] = gf; g[3 * k + 1] = gx; g[3 * k + 2] = gy;
-        } else {
-            gf = g[3 * k]; gx = g[3 * k + 1]; gy = g[3 * k + 2];
-        }
-        const MetricFast m = metric_fast(S.K, f);
-        const double dphi = dphi_f(P, m, gf, f);
-        double pf = p[3 * k] - S.h * dphi;
-        double px = p[3 * k + 1] - S.h * gx;
-        double py = p[3 * k + 2] - S.h * gy;
-        if (f < P.F.f_lim) pf *= -1.0;
-        if ((x < 0.0) || (x > P.Rg - 1.0)) px *= -1.0;
-        if ((y < 0.0) || (y > P.C - 1.0)) py *= -1.0;
-        if (NEXT) {
-            pf = pf - S.h * dphi;
-            px -= S.h * gx;
-            py -= S.h * gy;
-            const double rho = pf, kap = m.kap;
-            a1[3 * k] = rho;
-            a2[3 * k] = kap;
-            int c = 0;
-            while (c < S.counter_max) {
-                const double pn = rho - S.h * (((pf * pf) * kap) / 2.0);
-                const bool more = fabs(pf - pn) > S.delta;
-                pf = pn;
-                ++c;
-                if (!more) break;
-            }
-            a1[3 * k + 1] = (double)c;
-            local_max = max(local_max, c);
-        }
-        p[3 * k] = pf; p[3 * k + 1] = px; p[3 * k + 2] = py;
-    }
-    if (NEXT && local_max) atomicMax(cnt, local_max);
-    if (NEXT && X.prod && !S.per_star) peer_max_epilogue(X, cnt);
 }
 
 // momentum refresh p = z sqrt(H) (sampler_RHMC.py:1021-1022) with device Philox keyed by the GLOBAL star id, or
@@ -724,7 +696,7 @@ __global__ void big_record_kernel(int n, const double* q, const double* p, const
 // [b kPackChunk, (b+1) kPackChunk); a first kernel counts its matches, the second one starts at the sum of the counts of
 // the blocks before it and compacts with warp ballots.
 constexpr int kPackChunk = 1024;
-static_assert(kPackChunk == 1 << 10, "big_qfix_kick_kernel counts boundary stars per chunk with k >> 10");
+static_assert(kPackChunk == 1 << 10, "moved_star counts boundary stars per chunk with k >> 10");
 
 __global__ void big_pack_count_kernel(int n, const double* q, double lo_edge, double hi_edge, int2* counts) {
     __shared__ int c[2];
@@ -887,7 +859,7 @@ __device__ void ghost_exchange_body(const PeerPtrs peers, int rank, int world, c
 
 // Ordered ghost packing, the exchange and the binning of the received ghosts in ONE kernel: every block compacts its chunk
 // (as big_pack_kernel), the last block to finish runs the exchange body.  The chunk counts come from the position-update
-// kernel (big_qfix_kick_kernel) and are zeroed here for the next step.
+// kernel (moved_star) and are zeroed here for the next step.
 struct GhostX {
     PeerPtrs peers;
     int rank, world;
@@ -946,17 +918,17 @@ struct srhmc_big {
     BBuf D, L, q, p, g, a1, a2, q0, g0, gid, vpart, scalars, gscalars, state, counters, send, recv, err, normals, lnu, E, V, T, A;
     // fused tile evaluation (big_tile.cuh): tile grid over the local rows, per-tile star lists, per-star footprint partials
     BBuf tcnt, tlist, gpart;
-    bool own_binned = false;
+    bool own_binned = false;   // the pair records of the owned stars' current positions are already in the tile lists
     // peer exchange (our own collectives over P2P / IPC mapped memory)
     BBuf peerbox, xepoch, packcnt, xticket;
     bool ghosts_binned = false;   // the ghost exchange kernel has already put the received ghosts into the tile lists
     // With peer exchange the kernel that produces a fixed-point count all-reduces it in its last block, the position-update
     // kernel counts the boundary stars, and packing + ghost exchange + ghost binning are one kernel: 5 kernels per leapfrog
     // step on N ranks.
-    bool pack_counted = false;   // big_qfix_kick_kernel has left this step's chunk counts in packcnt
+    bool pack_counted = false;   // the position-update kernel has left this step's chunk counts in packcnt
     PeerPtrs peers{};
     void* ipc_opened[kMaxWorld] = {};
-    bool peer_enabled = false;  // the pair records of the owned stars' current positions are already in the tile lists
+    bool peer_enabled = false;  // srhmc_big_comm_import has mapped every rank's mailbox: the phases exchange over peer memory
     BBuf epart, tickets;  // per-block energy partials; last-block tickets [0] energy, [1] tile potential
     // sample recording (srhmc_big_set_recording): rows [rec_rows][n][3] of q and/or p in slot order, written at RECORD_E0
     BBuf slot, recq, recp;
@@ -1011,6 +983,83 @@ int refresh_float_data(srhmc_big* b) {
     b->launches += 1;
     const cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return bfail(SRHMC_ERR_CUDA, "float conversion of the data failed: %s", cudaGetErrorString(e));
+    return 0;
+}
+
+// Rows of the boundary lists: an owned star with x < lo_edge can touch the data rows of the rank below, one with x >= hi_edge
+// those of the rank above
+void ghost_edges(const srhmc_big* b, double& lo_edge, double& hi_edge) {
+    const double reach = (double)(b->cfg.nrows_halo + b->P.rad + 1);
+    lo_edge = (b->rank > 0) ? (double)b->P.own_lo + reach : -1e300;
+    hi_edge = (b->rank < b->world - 1) ? (double)b->P.own_hi - reach : 1e300;
+}
+
+// Enqueue the gradient (want_V: and the pixel potential) at the current q on the context's evaluation path: the fused tile
+// kernel (FP64, or FP32 for gradient-only evaluations), the star-centric kernel (very sparse fields) or the star-parallel
+// scatter / pixel / gather kernels.  The first two leave per-star footprint partials, and *gpart points at them; the
+// star-parallel kernels write g, and *gpart is nullptr.
+int enqueue_eval(srhmc_big* b, bool want_V, const double** gpart) {
+    const BigParams& P = b->P;
+    const int n = b->n;
+    cudaStream_t st = b->stream;
+    int* cnt = b->counters.as<int>();
+    const size_t list = 1 + 3 * (size_t)std::max(1, b->cfg.max_ghosts);
+    const double* ga = (b->world > 1 && b->rank > 0) ? b->recv.as<double>() + ((size_t)(b->rank - 1) * 2 + 1) * list : nullptr;
+    const double* gb = (b->world > 1 && b->rank < b->world - 1) ? b->recv.as<double>() + ((size_t)(b->rank + 1) * 2 + 0) * list : nullptr;
+    *gpart = nullptr;
+    if (!b->use_tiles) {
+        const size_t npix = (size_t)P.nrows * P.C;
+        const int pg = (int)std::min<size_t>((npix + 255) / 256, (size_t)kVBlocks);
+        if (!b->L_filled) {
+            big_fill_kernel<<<pg, 256, 0, st>>>(b->L.as<double>(), npix, P.F.B);
+            b->launches += 1;
+        }
+        b->L_filled = false;
+        const int total = n + 2 * std::max(1, b->cfg.max_ghosts);
+        const int sg = std::max(1, std::min((total * 32 + 255) / 256, 16 * b->sm_count));
+        big_scatter_kernel<<<sg, 256, 0, st>>>(P, b->q.as<double>(), n, ga, gb, b->L.as<double>(), b->err.as<int>());
+        big_pixel_kernel<<<pg, 256, 0, st>>>(P, b->D.as<double>(), b->L.as<double>(), want_V, b->vpart.as<double>());
+        if (want_V) big_vsum_kernel<<<1, 256, 0, st>>>(b->vpart.as<double>(), pg, b->scalars.as<double>());
+        const int gg = std::max(1, std::min((n * 32 + 255) / 256, 16 * b->sm_count));
+        big_gather_kernel<<<gg, 256, 0, st>>>(P, b->q.as<double>(), n, b->L.as<double>(), b->g.as<double>());
+        b->launches += want_V ? 4 : 3;
+        return 0;
+    }
+    TileSrc S;
+    S.q = b->q.as<double>(); S.ga = ga; S.gb = gb; S.n_own = n; S.cap = std::max(1, b->cfg.max_ghosts);
+    const int ntiles = b->nty * b->ntx;
+    if (!b->own_binned && n > 0) {
+        big_bin_kernel<<<std::max(1, std::min((n + 255) / 256, 8 * b->sm_count)), 256, 0, st>>>(
+            P, S, b->ntx, 0, n, b->tcnt.as<int>(), b->tlist.as<PairRec>(), b->err.as<int>());
+        b->launches += 1;
+    }
+    if ((ga || gb) && !b->ghosts_binned) {
+        big_bin_kernel<<<std::max(1, std::min((2 * S.cap + 255) / 256, 8 * b->sm_count)), 256, 0, st>>>(
+            P, S, b->ntx, n, n + 2 * S.cap, b->tcnt.as<int>(), b->tlist.as<PairRec>(), b->err.as<int>());
+        b->launches += 1;
+    }
+    b->own_binned = false;  // the tile kernel consumes the lists and re-zeroes the counters
+    b->ghosts_binned = false;
+    if (b->precision == 32 && !want_V) {
+        big_tile32_kernel<<<ntiles, kTileThreads, sizeof(TileSmemF), st>>>(P, S, b->ntx, b->tcnt.as<int>(), b->tlist.as<PairRec>(),
+                                                                           b->gpart.as<double>(), cnt, b->tmapD32);
+    } else if (!want_V && n > 0 && P.rad <= 15 && (b->star_mode == 1 || (b->star_mode < 0 && 2.0 * n <= 3.0 * ntiles))) {
+        // very sparse field (mean tile list below ~1.5 records): one warp per owned star, neighbours from the tile lists
+        // (big_star.cuh: only the patches are read, not every pixel); the lists are
+        // consumed here, so their counters are re-zeroed by a memset node instead of by the tile CTAs
+        const int sgrid = std::max(1, std::min((n + kStarWarps - 1) / kStarWarps, 64 * b->sm_count));
+        const auto star = P.rad <= 12 ? big_star_kernel<25> : big_star_kernel<31>;
+        star<<<sgrid, 32 * kStarWarps, 0, st>>>(P, n, b->q.as<double>(), b->D.as<double>(), b->ntx, b->tcnt.as<int>(),
+                                                b->tlist.as<PairRec>(), b->gpart.as<double>(), cnt);
+        BCU(cudaMemsetAsync(b->tcnt.ptr, 0, (size_t)ntiles * 4, st));
+    } else {
+        const auto tile = want_V ? big_tile_kernel<1> : big_tile_kernel<0>;
+        tile<<<ntiles, kTileThreads, sizeof(TileSmem), st>>>(P, S, b->ntx, b->D.as<double>(), b->tcnt.as<int>(), b->tlist.as<PairRec>(),
+                                                             b->gpart.as<double>(), b->vpart.as<double>(), b->tickets.as<unsigned int>() + 1,
+                                                             b->scalars.as<double>(), cnt, nullptr, 0ull, b->tmapD, b->tma ? 1 : 0);
+    }
+    b->launches += 1;
+    *gpart = b->gpart.as<double>();
     return 0;
 }
 
@@ -1088,7 +1137,7 @@ int srhmc_big_create(const srhmc_big_config* cfg, srhmc_big** out) {
         if ((cfg->cols % 2) == 0) b->tma = encode_tile_map(&b->tmapD, b->D.ptr, cfg->nrows, cfg->cols, 8);
     }
     rc |= b->q.ensure(S * 8); rc |= b->p.ensure(S * 8); rc |= b->g.ensure(S * 8);
-    rc |= b->a1.ensure(S * 8); rc |= b->a2.ensure(S * 8 + (size_t)cfg->max_stars * 4 + 8);
+    rc |= b->a1.ensure(S * 8); rc |= b->a2.ensure(S * 8 + (size_t)cfg->max_stars * 4 + 8);   // a2: then own_qcount
     rc |= b->q0.ensure(S * 8); rc |= b->g0.ensure(S * 8); rc |= b->gid.ensure((size_t)cfg->max_stars * 8);
     rc |= b->slot.ensure((size_t)cfg->max_stars * 4);
     rc |= b->vpart.ensure(std::max<size_t>(kVBlocks, ntiles) * 8); rc |= b->scalars.ensure(kScalars * 8); rc |= b->gscalars.ensure(kScalars * 8); rc |= b->state.ensure(8 * 8);
@@ -1635,11 +1684,9 @@ int srhmc_big_phase(srhmc_big* b, int32_t phase, const srhmc_big_step* s) {
     BigStep S;
     S.h = s->dt / 2.0; S.delta = s->delta; S.g_ff2 = s->g_ff2; S.counter_max = s->counter_max;
     S.per_star = s->fixed_point_mode != 0 ? 1 : 0;
-    S.K.c = (P.F.B / P.F.g0) / P.F.g_ff; S.K.ig2 = 1.0 / s->g_ff2; S.K.ig1 = 1.0 / P.F.g1; S.K.Bg2 = P.F.B / P.F.g2;
-    S.K.igxx = 1.0 / P.F.g_xx; S.K.f_low = P.F.f_low;   // make_metric_k (common.cuh) on the host
+    S.K = make_metric_k(P.F, s->g_ff2);
     const int tb = 128, gs = std::max(1, std::min((n + tb - 1) / tb, 4 * b->sm_count));
     const size_t npix = (size_t)P.nrows * P.C;
-    const size_t list = 1 + 3 * (size_t)std::max(1, b->cfg.max_ghosts);
     int* cnt = b->counters.as<int>();
     cudaStream_t st = b->stream;
     PeerX X;
@@ -1650,26 +1697,38 @@ int srhmc_big_phase(srhmc_big* b, int32_t phase, const srhmc_big_step* s) {
         X.prod = 1;
         X.epoch = b->xepoch.as<unsigned long long>(); X.ticket = b->xticket.as<unsigned int>(); X.err = b->err.as<int>();
     }
-    // per-star stop rule: the whole advance between two evaluations in one kernel (big_perstar_kernel)
-    auto launch_perstar = [&](bool from_eval, const double* gpart_in) -> int {
-        if (b->use_tiles && (b->own_binned || b->ghosts_binned)) {  // records nobody consumed
+    // the kicks of the field-wide stop rule (big_kick_kernel)
+    auto kick = [&](bool last_half, bool next_first, const double* gpart) {
+        const auto kernel = !last_half ? big_kick_kernel<false, true> : next_first ? big_kick_kernel<true, true> : big_kick_kernel<true, false>;
+        kernel<<<gs, tb, 0, st>>>(P, S, n, b->q.as<double>(), b->p.as<double>(), b->g.as<double>(), gpart, b->a1.as<double>(),
+                                  b->a2.as<double>(), cnt, X);
+        b->launches += 1;
+    };
+    // The kernels that move the stars: QFIX_KICK (big_qfix_kick_kernel) and, per-star stop rule, the whole advance between two
+    // evaluations (big_perstar_kernel).  Both leave the new positions' pair records, the boundary counts and the reset model
+    // image for the next evaluation and PACK.
+    auto position_update = [&](bool perstar, bool from_eval, const double* gpart) -> int {
+        if (b->use_tiles && (b->own_binned || b->ghosts_binned)) {  // records nobody consumed (two position updates without an evaluation)
             BCU(cudaMemsetAsync(b->tcnt.ptr, 0, (size_t)b->nty * b->ntx * 4, st));
             b->ghosts_binned = false;
         }
-        if (peer_multi && b->pack_counted) BCU(cudaMemsetAsync(b->packcnt.ptr, 0, b->packcnt.cap, st));
-        const double reach_k = (double)(b->cfg.nrows_halo + P.rad + 1);
-        const double lo_edge_k = (b->rank > 0) ? (double)P.own_lo + reach_k : -1e300;
-        const double hi_edge_k = (b->rank < b->world - 1) ? (double)P.own_hi - reach_k : 1e300;
+        if (peer_multi && b->pack_counted)   // counts nobody consumed (two position updates without a PACK)
+            BCU(cudaMemsetAsync(b->packcnt.ptr, 0, b->packcnt.cap, st));
+        double lo_edge, hi_edge;
+        ghost_edges(b, lo_edge, hi_edge);
         int* tc = b->use_tiles ? b->tcnt.as<int>() : nullptr;
         PairRec* tl = b->use_tiles ? b->tlist.as<PairRec>() : nullptr;
         int2* pc = peer_multi ? b->packcnt.as<int2>() : nullptr;
         double* lf = (!b->use_tiles && n > 0) ? b->L.as<double>() : nullptr;
-        if (from_eval)
-            big_perstar_kernel<true><<<gs, tb, 0, st>>>(P, S, n, b->q.as<double>(), b->p.as<double>(), b->g.as<double>(), gpart_in,
-                                                        b->ntx, tc, tl, b->err.as<int>(), pc, lo_edge_k, hi_edge_k, lf, npix);
-        else
-            big_perstar_kernel<false><<<gs, tb, 0, st>>>(P, S, n, b->q.as<double>(), b->p.as<double>(), b->g.as<double>(), nullptr,
-                                                         b->ntx, tc, tl, b->err.as<int>(), pc, lo_edge_k, hi_edge_k, lf, npix);
+        if (perstar) {
+            const auto kernel = from_eval ? big_perstar_kernel<true> : big_perstar_kernel<false>;
+            kernel<<<gs, tb, 0, st>>>(P, S, n, b->q.as<double>(), b->p.as<double>(), b->g.as<double>(), gpart, b->ntx, tc, tl,
+                                      b->err.as<int>(), pc, lo_edge, hi_edge, lf, npix);
+        } else {
+            big_qfix_kick_kernel<<<gs, tb, 0, st>>>(P, S, n, b->q.as<double>(), b->p.as<double>(), b->a1.as<double>(),
+                                                    b->a2.as<double>(), cnt + 1, b->ntx, tc, tl, b->err.as<int>(), pc, lo_edge,
+                                                    hi_edge, lf, npix);
+        }
         b->L_filled = lf != nullptr;
         b->pack_counted = peer_multi;
         b->own_binned = b->use_tiles;
@@ -1678,13 +1737,12 @@ int srhmc_big_phase(srhmc_big* b, int32_t phase, const srhmc_big_step* s) {
     };
     switch (phase) {
         case SRHMC_BIG_PS_ADVANCE:
-            if (int rc = launch_perstar(false, nullptr)) return rc;
+            if (int rc = position_update(true, false, nullptr)) return rc;
             break;
         case SRHMC_BIG_PACK: {
             // boundary lists for the neighbours: everything that can touch their data rows
-            const double reach = (double)(b->cfg.nrows_halo + P.rad + 1);
-            const double lo_edge = (b->rank > 0) ? (double)P.own_lo + reach : -1e300;
-            const double hi_edge = (b->rank < b->world - 1) ? (double)P.own_hi - reach : 1e300;
+            double lo_edge, hi_edge;
+            ghost_edges(b, lo_edge, hi_edge);
             const int pb = std::max(1, (n + kPackChunk - 1) / kPackChunk);
             if (peer_multi) {
                 if (!b->pack_counted) {   // a PACK that does not follow a position update (first evaluation of a run)
@@ -1692,7 +1750,8 @@ int srhmc_big_phase(srhmc_big* b, int32_t phase, const srhmc_big_step* s) {
                     b->launches += 1;
                 }
                 GhostX G;
-                G.peers = b->peers; G.rank = b->rank; G.world = b->world; G.recv = b->recv.as<double>(); G.list = list;
+                G.peers = b->peers; G.rank = b->rank; G.world = b->world; G.recv = b->recv.as<double>();
+                G.list = 1 + 3 * (size_t)std::max(1, b->cfg.max_ghosts);
                 G.epoch = b->xepoch.as<unsigned long long>(); G.ticket = b->xticket.as<unsigned int>() + 1;
                 G.ntx = b->ntx; G.n_own = n;
                 G.tcnt = b->use_tiles ? b->tcnt.as<int>() : nullptr;
@@ -1716,87 +1775,25 @@ int srhmc_big_phase(srhmc_big* b, int32_t phase, const srhmc_big_step* s) {
         case SRHMC_BIG_EVAL_V_KICK2:
         case SRHMC_BIG_EVAL_KICK2_KICK1:
         case SRHMC_BIG_EVAL_PS_ADVANCE: {
-            const int want_V = (phase == SRHMC_BIG_EVAL_V || phase == SRHMC_BIG_EVAL_V_KICK2) ? 1 : 0;
-            // tail: 0 none, 1 the step's last half kick + reflections, 2 also the next step's first kick + p fixed point A,
-            // 3 (per-star stop rule) the step's end and the whole advance of the next step in one kernel
-            const int tail = phase == SRHMC_BIG_EVAL_PS_ADVANCE ? 3 : (phase == SRHMC_BIG_EVAL_KICK2_KICK1 ? 2 :
-                             ((phase == SRHMC_BIG_EVAL_KICK2 || phase == SRHMC_BIG_EVAL_V_KICK2) ? 1 : 0));
-            const double* ga = (b->world > 1 && b->rank > 0) ? b->recv.as<double>() + ((size_t)(b->rank - 1) * 2 + 1) * list : nullptr;
-            const double* gb = (b->world > 1 && b->rank < b->world - 1) ? b->recv.as<double>() + ((size_t)(b->rank + 1) * 2 + 0) * list : nullptr;
+            // the evaluation, then its tail: the step's last half kick and reflections, and with them either the next step's
+            // first half kick and p fixed point phase A or (per-star stop rule) the whole advance of the next step
+            const bool want_V = phase == SRHMC_BIG_EVAL_V || phase == SRHMC_BIG_EVAL_V_KICK2;
+            const bool last_half = phase != SRHMC_BIG_EVAL && phase != SRHMC_BIG_EVAL_V;
+            const bool next_first = phase == SRHMC_BIG_EVAL_KICK2_KICK1;
+            const bool ps_advance = phase == SRHMC_BIG_EVAL_PS_ADVANCE;
             const double* gpart = nullptr;
-            if (b->use_tiles) {
-                TileSrc S;
-                S.q = b->q.as<double>(); S.ga = ga; S.gb = gb; S.n_own = n; S.cap = std::max(1, b->cfg.max_ghosts);
-                const int ntiles = b->nty * b->ntx;
-                if (!b->own_binned && n > 0) {
-                    big_bin_kernel<<<std::max(1, std::min((n + 255) / 256, 8 * b->sm_count)), 256, 0, st>>>(
-                        P, S, b->ntx, 0, n, b->tcnt.as<int>(), b->tlist.as<PairRec>(), b->err.as<int>());
+            if (int rc = enqueue_eval(b, want_V, &gpart)) return rc;
+            if (!last_half) {
+                if (gpart) {   // no tail sums the footprint partials into g
+                    big_gsum_kernel<<<gs, tb, 0, st>>>(P, b->q.as<double>(), n, gpart, b->g.as<double>());
                     b->launches += 1;
                 }
-                if ((ga || gb) && !b->ghosts_binned) {
-                    big_bin_kernel<<<std::max(1, std::min((2 * S.cap + 255) / 256, 8 * b->sm_count)), 256, 0, st>>>(
-                        P, S, b->ntx, n, n + 2 * S.cap, b->tcnt.as<int>(), b->tlist.as<PairRec>(), b->err.as<int>());
-                    b->launches += 1;
-                }
-                b->own_binned = false;  // the tile kernel consumes the lists and re-zeroes the counters
-                b->ghosts_binned = false;
-                if (b->precision == 32 && !want_V) {
-                    big_tile32_kernel<<<ntiles, kTileThreads, sizeof(TileSmemF), st>>>(P, S, b->ntx, b->tcnt.as<int>(), b->tlist.as<PairRec>(),
-                                                                                       b->gpart.as<double>(), cnt, b->tmapD32);
-                } else if (!want_V && n > 0 && P.rad <= 15 &&
-                           (b->star_mode == 1 || (b->star_mode < 0 && 2.0 * n <= 3.0 * ntiles))) {
-                    // very sparse field (mean tile list below ~1.5 records): one warp per owned star, neighbours from the tile lists
-                    // (big_star.cuh: only the patches are read, not every pixel); the lists are
-                    // consumed here, so their counters are re-zeroed by a memset node instead of by the tile CTAs
-                    const int sgrid = std::max(1, std::min((n + kStarWarps - 1) / kStarWarps, 64 * b->sm_count));
-                    if (P.rad <= 12)
-                        big_star_kernel<25><<<sgrid, 32 * kStarWarps, 0, st>>>(P, n, b->q.as<double>(), b->D.as<double>(), b->ntx,
-                                                                               b->tcnt.as<int>(), b->tlist.as<PairRec>(), b->gpart.as<double>(), cnt);
-                    else
-                        big_star_kernel<31><<<sgrid, 32 * kStarWarps, 0, st>>>(P, n, b->q.as<double>(), b->D.as<double>(), b->ntx,
-                                                                               b->tcnt.as<int>(), b->tlist.as<PairRec>(), b->gpart.as<double>(), cnt);
-                    BCU(cudaMemsetAsync(b->tcnt.ptr, 0, (size_t)ntiles * 4, st));
-                } else if (want_V)
-                    big_tile_kernel<1><<<ntiles, kTileThreads, sizeof(TileSmem), st>>>(P, S, b->ntx, b->D.as<double>(), b->tcnt.as<int>(),
-                        b->tlist.as<PairRec>(), b->gpart.as<double>(), b->vpart.as<double>(),
-                        b->tickets.as<unsigned int>() + 1, b->scalars.as<double>(), cnt, nullptr, 0ull, b->tmapD, b->tma ? 1 : 0);
-                else
-                    big_tile_kernel<0><<<ntiles, kTileThreads, sizeof(TileSmem), st>>>(P, S, b->ntx, b->D.as<double>(), b->tcnt.as<int>(),
-                        b->tlist.as<PairRec>(), b->gpart.as<double>(), b->vpart.as<double>(),
-                        b->tickets.as<unsigned int>() + 1, b->scalars.as<double>(), cnt, nullptr, 0ull, b->tmapD, b->tma ? 1 : 0);
-                b->launches += 1;
-                if (tail == 0) {
-                    big_gsum_kernel<<<gs, tb, 0, st>>>(P, b->q.as<double>(), n, b->gpart.as<double>(), b->g.as<double>());
-                    b->launches += 1;
-                }
-                gpart = b->gpart.as<double>();
+            } else if (ps_advance) {
+                if (int rc = position_update(true, true, gpart)) return rc;
             } else {
-                const int pg = (int)std::min<size_t>((npix + 255) / 256, (size_t)kVBlocks);
-                if (!b->L_filled) {
-                    big_fill_kernel<<<pg, 256, 0, st>>>(b->L.as<double>(), npix, P.F.B);
-                    b->launches += 1;
-                }
-                b->L_filled = false;
-                const int total = n + 2 * std::max(1, b->cfg.max_ghosts);
-                const int sg = std::max(1, std::min((total * 32 + 255) / 256, 16 * b->sm_count));
-                big_scatter_kernel<<<sg, 256, 0, st>>>(P, b->q.as<double>(), n, ga, gb, b->L.as<double>(), b->err.as<int>());
-                big_pixel_kernel<<<pg, 256, 0, st>>>(P, b->D.as<double>(), b->L.as<double>(), want_V, b->vpart.as<double>());
-                if (want_V) big_vsum_kernel<<<1, 256, 0, st>>>(b->vpart.as<double>(), pg, b->scalars.as<double>());
-                const int gg = std::max(1, std::min((n * 32 + 255) / 256, 16 * b->sm_count));
-                big_gather_kernel<<<gg, 256, 0, st>>>(P, b->q.as<double>(), n, b->L.as<double>(), b->g.as<double>());
-                b->launches += want_V ? 4 : 3;
-                if (tail == 2) BCU(cudaMemsetAsync(cnt, 0, 8, st));  // the tile kernel does this on the tile path
+                if (next_first && !b->use_tiles) BCU(cudaMemsetAsync(cnt, 0, 8, st));  // the tile and star kernels zero the counts
+                kick(true, next_first, gpart);
             }
-            if (tail == 1)
-                big_tail_kernel<false><<<gs, tb, 0, st>>>(P, S, n, b->q.as<double>(), b->p.as<double>(), b->g.as<double>(), gpart,
-                                                          b->a1.as<double>(), b->a2.as<double>(), cnt, X);
-            else if (tail == 2)
-                big_tail_kernel<true><<<gs, tb, 0, st>>>(P, S, n, b->q.as<double>(), b->p.as<double>(), b->g.as<double>(), gpart,
-                                                         b->a1.as<double>(), b->a2.as<double>(), cnt, X);
-            else if (tail == 3) {
-                if (int rc = launch_perstar(true, gpart)) return rc;
-            }
-            if (tail == 1 || tail == 2) b->launches += 1;
             break;
         }
         case SRHMC_BIG_RESET_ITER:
@@ -1804,9 +1801,7 @@ int srhmc_big_phase(srhmc_big* b, int32_t phase, const srhmc_big_step* s) {
             break;
         case SRHMC_BIG_KICK1:
             BCU(cudaMemsetAsync(cnt, 0, 8, st));
-            big_kick1_kernel<<<gs, tb, 0, st>>>(P, S, n, b->q.as<double>(), b->p.as<double>(), b->g.as<double>(),
-                                                b->a1.as<double>(), b->a2.as<double>(), cnt, X);
-            b->launches += 1;
+            kick(false, true, nullptr);
             break;
         case SRHMC_BIG_PFIX_QFIX:
             // tiled over peers: the field-wide maximum of the p fixed-point counts was all-reduced by the last block of the
@@ -1815,30 +1810,11 @@ int srhmc_big_phase(srhmc_big* b, int32_t phase, const srhmc_big_step* s) {
                                                     b->a2.as<double>(), cnt, cnt + 1, X);
             b->launches += 1;
             break;
-        case SRHMC_BIG_QFIX_KICK: {
-            if (b->use_tiles && (b->own_binned || b->ghosts_binned)) {  // records nobody consumed (two position updates without an evaluation)
-                BCU(cudaMemsetAsync(b->tcnt.ptr, 0, (size_t)b->nty * b->ntx * 4, st));
-                b->ghosts_binned = false;
-            }
-            if (peer_multi && b->pack_counted)   // counts nobody consumed (two position updates without a PACK)
-                BCU(cudaMemsetAsync(b->packcnt.ptr, 0, b->packcnt.cap, st));
-            const double reach_k = (double)(b->cfg.nrows_halo + P.rad + 1);
-            const double lo_edge_k = (b->rank > 0) ? (double)P.own_lo + reach_k : -1e300;
-            const double hi_edge_k = (b->rank < b->world - 1) ? (double)P.own_hi - reach_k : 1e300;
-            big_qfix_kick_kernel<<<gs, tb, 0, st>>>(P, S, n, b->q.as<double>(), b->p.as<double>(), b->a1.as<double>(),
-                                                    b->a2.as<double>(), cnt + 1, b->ntx, b->use_tiles ? b->tcnt.as<int>() : nullptr,
-                                                    b->use_tiles ? b->tlist.as<PairRec>() : nullptr, b->err.as<int>(),
-                                                    peer_multi ? b->packcnt.as<int2>() : nullptr, lo_edge_k, hi_edge_k,
-                                                    (!b->use_tiles && n > 0) ? b->L.as<double>() : nullptr, npix);
-            b->L_filled = !b->use_tiles && n > 0;
-            b->pack_counted = peer_multi;
-            b->own_binned = b->use_tiles;
-            b->launches += 1;
+        case SRHMC_BIG_QFIX_KICK:
+            if (int rc = position_update(false, false, nullptr)) return rc;
             break;
-        }
         case SRHMC_BIG_KICK2:
-            big_kick2_kernel<<<gs, tb, 0, st>>>(P, S, n, b->q.as<double>(), b->p.as<double>(), b->g.as<double>());
-            b->launches += 1;
+            kick(true, false, nullptr);
             break;
         case SRHMC_BIG_MOMENTUM: {
             const double* z = b->normals.ptr ? b->normals.as<double>() : nullptr;

@@ -15,7 +15,7 @@
 //     does not depend on the order the atomics filled the lists: results stay bit-reproducible run to run;
 //   * rho = D / Lambda - 1 (product-tree reciprocal) and the three residual-weighted sums of the star's own PSF over its own
 //     patch, folded over the lanes with shuffles: the complete pixel gradient of the star, written to footprint slot 0 of
-//     `gpart` (the other slots are zeroed), so big_tail_kernel / big_gsum_kernel consume it unchanged.
+//     `gpart` (the other slots are zeroed), so big_kick_kernel / big_gsum_kernel consume it unchanged.
 // Measured on 8192^2 / 1e5 stars (BASELINE configs[4], 3.6 neighbours per star): 331 us per gradient against 242 us for the
 // tile kernel (ncu: 1850 warp-instructions per star -- 210 per neighbour pass, 220 for the copies' address arithmetic -- at
 // IPC 2.1 with 16 warps per SM), i.e. C5 275 vs 352 M star-steps/s: every neighbour costs two warp-wide exponentials per

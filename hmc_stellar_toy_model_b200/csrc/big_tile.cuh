@@ -14,7 +14,7 @@
 //              (EVAL_V: the last tile to finish sums the per-tile potential partials in tile order); the CTA
 //              re-zeroes its list counter for the next evaluation
 //   gsum       per owned star: sum of its footprint slots in fixed order, scale -> g[3n]; fused into the scalar kernel
-//              that consumes the gradient (big_tail_kernel) or run on its own (big_gsum_kernel)
+//              that consumes the gradient (big_kick_kernel, big_perstar_kernel) or run on its own (big_gsum_kernel)
 //
 // No floating-point atomics anywhere: results are bit-reproducible run to run.
 #pragma once

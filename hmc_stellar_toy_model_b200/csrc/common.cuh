@@ -191,7 +191,7 @@ __device__ __forceinline__ float rcp_fast(float a) { return __frcp_rn(a); }
 struct MetricK {
     double c, ig2, ig1, Bg2, igxx, f_low;
 };
-__device__ __forceinline__ MetricK make_metric_k(const FieldParams& P, double g_ff2) {
+__host__ __device__ __forceinline__ MetricK make_metric_k(const FieldParams& P, double g_ff2) {
     MetricK K;
     K.c = (P.B / P.g0) / P.g_ff;
     K.ig2 = 1.0 / g_ff2;
