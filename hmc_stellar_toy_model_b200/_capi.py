@@ -260,6 +260,8 @@ SIGNATURES = {
     "srhmc_big_read_chains": (C.c_int, [C.c_void_p, C.c_int32, c_double_p, c_double_p, c_double_p, c_uint8_p,
                                         C.POINTER(C.c_double), C.POINTER(C.c_int32)]),
     "srhmc_big_read_scalars": (C.c_int, [C.c_void_p, c_double_p]),
+    "srhmc_big_rj_configure": (C.c_int, [C.c_void_p, C.POINTER(RjArgs), C.c_int32]),
+    "srhmc_big_rj_finish": (C.c_int, [C.c_void_p, C.c_int32, C.POINTER(RjArgs)]),
     "srhmc_big_phase": (C.c_int, [C.c_void_p, C.c_int32, C.POINTER(BigStep)]),
     "srhmc_big_set_recording": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32]),
     "srhmc_big_read_samples": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, c_double_p, c_double_p]),

@@ -25,7 +25,8 @@ from ._capi import check_big as check
 from .utils import mag2flux
 
 PHASE = dict(PACK=0, EVAL=1, EVAL_V=2, KICK1=3, PFIX_QFIX=4, QFIX_KICK=5, KICK2=6, MOMENTUM=7, ENERGY=8, RECORD_E0=9,
-             ACCEPT=10, RESET_ITER=11, EVAL_KICK2=12, EVAL_V_KICK2=13, EVAL_KICK2_KICK1=14, PS_ADVANCE=15, EVAL_PS_ADVANCE=16)
+             ACCEPT=10, RESET_ITER=11, EVAL_KICK2=12, EVAL_V_KICK2=13, EVAL_KICK2_KICK1=14, PS_ADVANCE=15, EVAL_PS_ADVANCE=16,
+             RJ_BEGIN=17, RJ_JUMP=18, RJ_ACCEPT=19)
 
 
 # ----------------------------------------------------------------------------------------------- host-side geometry
@@ -145,6 +146,7 @@ class BigFieldStrip:
             # otherwise stars two strips away could touch the local rows and the neighbour exchange is not enough
             raise ValueError("strips of %d rows are too thin for halo %d / patch radius %d" % (hi - lo, halo, patch_radius))
         self.rows, self.cols, self.rank, self.world, self.device = rows, cols, rank, world, device
+        self.max_stars = max(1, max_stars)
         self.lo, self.hi, self.row0, self.nrows, self.halo, self.rad = lo, hi, row0, nrows, halo, patch_radius
         cfg = _capi.BigConfig(abi_version=_capi.ABI_VERSION, device=device, rows_global=rows, cols=cols, own_lo=lo,
                               own_hi=hi, row0=row0, nrows=nrows, nrows_halo=halo, max_stars=max(1, max_stars),
@@ -217,6 +219,14 @@ class BigFieldStrip:
         check(self._lib.srhmc_big_set_stars(self._h, _capi.dptr(q), mine.ctypes.data_as(C.POINTER(C.c_int64)), len(mine)))
         self.n, self.ids, self.n_global = len(mine), mine, len(q_global)
 
+    def set_table(self, q):
+        """Store the stars [n,3] as a table in the given order (storage index = table index, ids 0..n-1): the layout of
+        reversible-jump runs."""
+        q = np.ascontiguousarray(np.asarray(q, dtype=np.float64).reshape(-1, 3))
+        ids = np.arange(len(q), dtype=np.int64)
+        check(self._lib.srhmc_big_set_stars(self._h, _capi.dptr(q), ids.ctypes.data_as(C.POINTER(C.c_int64)), len(q)))
+        self.n, self.ids, self.n_global = len(q), ids, len(q)
+
     def get_stars(self):
         q, p, g = (np.zeros((self.n, 3)) for _ in range(3))
         check(self._lib.srhmc_big_get_stars(self._h, _capi.dptr(q), _capi.dptr(p), _capi.dptr(g)))
@@ -226,10 +236,32 @@ class BigFieldStrip:
         p = np.ascontiguousarray(p, dtype=np.float64).reshape(self.n, 3)
         check(self._lib.srhmc_big_set_momenta(self._h, _capi.dptr(p)))
 
-    def set_draws(self, normals, lnu, n_iters):
-        z = None if normals is None else np.ascontiguousarray(normals, dtype=np.float64).reshape(n_iters, self.n, 3)
+    def set_draws(self, normals, lnu, n_iters, rows=None):
+        rows = self.n if rows is None else rows
+        z = None if normals is None else np.ascontiguousarray(normals, dtype=np.float64).reshape(n_iters, rows, 3)
         u = None if lnu is None else np.ascontiguousarray(lnu, dtype=np.float64).reshape(n_iters)
         check(self._lib.srhmc_big_set_draws(self._h, _capi.dptr(z), _capi.dptr(u), n_iters))
+
+    def rj_configure(self, rj, n_iters):
+        """Enter reversible-jump mode for the coming n_iters iterations (srhmc_big_rj_configure)."""
+        check(self._lib.srhmc_big_rj_configure(self._h, C.byref(rj), int(n_iters)))
+
+    def rj_finish(self, n_iters):
+        """Leave reversible-jump mode: (N_chain, move_chain, n_final, overflow); the strip then holds the n_final stars."""
+        N = np.zeros(n_iters, dtype=np.int32)
+        mv = np.zeros(n_iters, dtype=np.uint8)
+        nf, ov = C.c_int32(), C.c_int32()
+        out = _capi.RjArgs(N_chain=_capi.iptr(N), move_chain=_capi.bptr(mv), n_final=C.pointer(nf), overflow=C.pointer(ov))
+        check(self._lib.srhmc_big_rj_finish(self._h, int(n_iters), C.byref(out)))
+        self.n = self.n_global = int(nf.value)
+        self.ids = np.arange(self.n, dtype=np.int64)
+        return N, mv, int(nf.value), int(ov.value)
+
+    def read_table_samples(self, nrows, want):
+        """{name: [nrows, max_stars, 3]} of the rows a reversible-jump run recorded (table order, zero past N)."""
+        out = {w: np.empty((int(nrows), self.max_stars, 3)) for w in want}
+        check(self._lib.srhmc_big_read_samples(self._h, 0, int(nrows), _capi.dptr(out.get("q")), _capi.dptr(out.get("p"))))
+        return out
 
     def alloc_chains(self, n_iters):
         check(self._lib.srhmc_big_alloc_chains(self._h, n_iters))
@@ -565,6 +597,7 @@ class BigFieldRHMC:
         L = niter + 1
         want = record_want(want)
         Ls = record_rows(L, chain_stride)
+        self._rj_graph_key = None   # set_recording below may move the buffers run_rj's captured graph writes
         # a change of the recording set-up may move its buffers: no graph captured before it may be replayed after it
         rec = (want, int(chain_stride), L, tuple(s.n for s in self.strips))
         if rec != getattr(self, "_rec", None):
@@ -632,6 +665,101 @@ class BigFieldRHMC:
         for w in want:
             out[w + "_chain"] = self._samples(w, Ls)
         return out
+
+    def run_rj(self, niter, nsteps, dt, *, P_move, fmin, fmax, K_split=1., beta_a=2., beta_b=2., seed=0, draws=None, normals=None,
+               lnu=None, delta=1e-6, counter_max=1000, f_pos=True, g_ff2=1.0, want=("q",), chain_stride=1, use_graph=None):
+        """multi_gym.run_RHMC with birth/death and split/merge moves (P_move[1:] != 0) on an untiled field: the semantics of
+        RHMCContext(patch_radius=r).run_rj for one field (tests/rj_oracle.rj_run with rad = r), the star count on the device.
+        The strip's stars are first re-stored as a table in the order of the list given to set_stars (ids 0..n-1); the
+        momentum of star k is keyed by its table index, the jump record of iteration l by (seed, field 0, l).  draws
+        [niter+1, 14], normals [niter+1, 3 max_stars] and lnu [niter+1] replace the device's draws.  alpha and V_prior_const
+        are the strip's.
+
+        Returns run()'s dict plus N_chain, move_chain (0 within, 1 birth, 2 death, 3 split, 4 merge), n_final, overflow and
+        q_chain / p_chain [ceil((niter+1) / chain_stride), max_stars, 3] in table order, zero past N.  Afterwards the strip
+        holds the n_final stars (get_stars, ids), and a later run() starts from them.  An iteration whose proposal needed more
+        than max_stars stars is rejected; the run then raises ValueError, as the drop-in does, with the result dict as its
+        `result` attribute.  use_graph: one captured
+        iteration replayed niter+1 times (default: on for niter >= 2)."""
+        if self.multi or len(self.strips) != 1:
+            raise ValueError("reversible-jump runs need the whole field on one device (world_size = 1)")
+        if self.fixed_point_mode != 0:
+            raise ValueError("reversible-jump runs use the reference stop rule (fixed_point_mode = 0)")
+        (s,) = self.strips
+        L = niter + 1
+        want = record_want(want)
+        Ls = record_rows(L, chain_stride)
+        q_list = np.empty((s.n, 3))
+        q_list[s.ids] = s.get_stars()[0]
+        s.set_table(q_list)
+        rj = _capi.RjArgs(P_move=(C.c_double * 3)(*[float(x) for x in P_move]), fmin=float(fmin), fmax=float(fmax),
+                          K_split=float(K_split), beta_a=float(beta_a), beta_b=float(beta_b),
+                          draws=_capi.dptr(None if draws is None else np.ascontiguousarray(draws, dtype=np.float64).reshape(L, 14)))
+        s.rj_configure(rj, L)
+        try:
+            s.set_draws(normals, lnu, L, rows=s.max_stars)
+            s.alloc_chains(L)
+            s.set_recording(L, chain_stride, want)
+            self._graph_key = self._rec = None   # run()'s captured graph and recording set-up are not this run's
+            st0 = self._step_struct(dt, delta, g_ff2, counter_max, f_pos, 0, seed)
+            s.phase("EVAL_V", st0)
+            if use_graph is None:
+                use_graph = L >= 3
+            self.replayed_launches = 0
+            if use_graph:
+                import torch
+
+                s.phase("RESET_ITER", st0)
+                # one captured iteration serves every later run_rj with the same launch parameters and buffers
+                key = (int(nsteps), float(dt), float(delta), float(g_ff2), int(counter_max), bool(f_pos), int(seed), L,
+                       tuple(float(x) for x in P_move), float(fmin), float(fmax), float(K_split), float(beta_a),
+                       float(beta_b), want, int(chain_stride))
+                if draws is not None or normals is not None or lnu is not None:
+                    key = None   # injected draws live in buffers that are re-allocated per run: always capture afresh
+                if key is None or getattr(self, "_rj_graph_key", None) != key:
+                    stg = self._step_struct(dt, delta, g_ff2, counter_max, f_pos, -1, seed)
+                    run_stream = torch.cuda.current_stream()
+                    graph = torch.cuda.CUDAGraph()
+                    before = s.launch_count
+                    with torch.cuda.graph(graph, capture_error_mode="thread_local"):
+                        s.adopt_stream(torch.cuda.current_stream().cuda_stream)
+                        self._rj_iteration(stg, nsteps)
+                    s.adopt_stream(run_stream.cuda_stream)
+                    self._rj_graph, self._rj_graph_key = graph, key
+                    self._rj_graph_nodes = s.launch_count - before
+                for _ in range(L):
+                    self._rj_graph.replay()
+                self.replayed_launches = self._rj_graph_nodes * L
+            else:
+                for l in range(L):
+                    self._rj_iteration(self._step_struct(dt, delta, g_ff2, counter_max, f_pos, l, seed), nsteps)
+            out = s.read_chains(L)
+            if want:
+                for w, v in s.read_table_samples(Ls, want).items():
+                    out[w + "_chain"] = v
+        finally:
+            N, mv, n_final, overflow = s.rj_finish(L)
+        out.update(N_chain=N, move_chain=mv, n_final=n_final, overflow=overflow, accept_rate=out["n_accepted"] / float(L))
+        if overflow >= 0:
+            err = ValueError("the proposal of iteration %d needs %d stars but max_stars = %d" % (overflow, s.max_stars + 1,
+                                                                                              s.max_stars))
+            err.result = out   # the chains of the run, overflowing iterations rejected
+            raise err
+        return out
+
+    def _rj_iteration(self, st, nsteps):
+        """One reversible-jump iteration: leg 1, the jump, the gradient at the edited table and leg 2 are enqueued every time;
+        the device skips what the iteration's move does not run."""
+        self._all("MOMENTUM", st)
+        self._all("ENERGY", st)
+        self._all("RECORD_E0", st)
+        self._all("RJ_BEGIN", st)
+        self.trajectory(st, nsteps, True)
+        self._all("RJ_JUMP", st)
+        self._all("EVAL_V", st)
+        self.trajectory(st, nsteps, True)
+        self._all("ENERGY", st)
+        self._all("RJ_ACCEPT", st)
 
     def _samples(self, name, rows, chunk_bytes=256 << 20):
         """Recorded rows of every strip hosted here in global-id order, downloaded in pieces of about `chunk_bytes`."""

@@ -113,12 +113,15 @@ __device__ __forceinline__ bool last_block_ticket(unsigned int* ticket, bool* fl
 #include "big_tile.cuh"
 #include "big_star.cuh"
 #include "big_peaks.cuh"
+#include "big_rj.cuh"
 
 namespace {
 
 // One warp per star (own stars first, then the two ghost lists).  ghost list layout: [0] = count, then f,x,y triples.
+template <bool LIVE>
 __global__ void big_scatter_kernel(const BigParams P, const double* q, int n_own, const double* ghost_a,
-                                   const double* ghost_b, double* L, int* err) {
+                                   const double* ghost_b, double* L, int* err, const int* nd) {
+    if (LIVE) n_own = *nd;
     const int lane = threadIdx.x & 31;
     const long long warp = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const long long nwarps = ((long long)gridDim.x * blockDim.x) >> 5;
@@ -178,7 +181,9 @@ __global__ void big_vsum_kernel(const double* vpart, int nblocks, double* scalar
 }
 
 // One warp per OWNED star: g_f = -sum rho PSF, g_x = -(f/s^2) sum rho dx PSF, g_y likewise (sampler_RHMC.py:404-406).
-__global__ void big_gather_kernel(const BigParams P, const double* q, int n_own, const double* L, double* g) {
+template <bool LIVE>
+__global__ void big_gather_kernel(const BigParams P, const double* q, int n_own, const double* L, double* g, const int* nd) {
+    if (LIVE) n_own = *nd;
     const int lane = threadIdx.x & 31;
     const long long warp = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const long long nwarps = ((long long)gridDim.x * blockDim.x) >> 5;
@@ -469,9 +474,10 @@ __device__ __forceinline__ void moved_star(const BigParams& P, int k, const Star
 //   NEXT_FIRST  (1) p -= h dphi/dq, (2) p fixed point phase A: anchor and own count in a1, kap in a2, maximum count in *cnt
 // <false, true> is KICK1; <true, false> KICK2 and the tail of EVAL_KICK2 / EVAL_V_KICK2; <true, true> EVAL_KICK2_KICK1 (the last
 // half kick of a step and the first one of the next use the same q and the same gradient).
-template <bool LAST_HALF, bool NEXT_FIRST>
+template <bool LAST_HALF, bool NEXT_FIRST, bool LIVE>
 __global__ void big_kick_kernel(const BigParams P, const BigStep S, int n, const double* q, double* p, double* g,
-                                const double* gpart, double* a1, double* a2, int* cnt, const PeerX X) {
+                                const double* gpart, double* a1, double* a2, int* cnt, const PeerX X, const int* nd) {
+    if (LIVE) n = *nd;
     int local_max = 0;
     for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += gridDim.x * blockDim.x) {
         const Star3 s = load3(q, k);
@@ -498,11 +504,13 @@ __global__ void big_kick_kernel(const BigParams P, const BigStep S, int n, const
 }
 
 // p fixed point phase B (continue to the field-wide count), then (3) q fixed point phase A: sigma in a1, p/H(sigma) in a2
+template <bool LIVE>
 __global__ void big_pfix_qfix_kernel(const BigParams P, const BigStep S, int n, double* q, double* p, double* a1, double* a2,
-                                     const int* cnt_p, int* cnt_q, const PeerX X) {
+                                     const int* cnt_p, int* cnt_q, const PeerX X, const int* nd) {
     const int target = S.per_star ? 0 : *cnt_p;
+    const int nk = LIVE ? *nd : n;   // n: the layout of own_qcount
     int local_max = 0;
-    for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += gridDim.x * blockDim.x) {
+    for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < nk; k += gridDim.x * blockDim.x) {
         double pf = p[3 * k];
         const double rho = a1[3 * k], kap = a2[3 * k];
         for (int c = (int)a1[3 * k + 1]; c < target; ++c) pf = pfix_iter(S, rho, kap, pf);
@@ -523,12 +531,14 @@ __global__ void big_pfix_qfix_kernel(const BigParams P, const BigStep S, int n, 
 }
 
 // q fixed point phase B, then (4) p -= h dtau/dq at the new q, and the position-update epilogue
+template <bool LIVE>
 __global__ void big_qfix_kick_kernel(const BigParams P, const BigStep S, int n, double* q, double* p, const double* a1,
                                      const double* a2, const int* cnt_q, int ntx, int* tcnt, PairRec* tlist, int* err,
-                                     int2* pack_counts, double lo_edge, double hi_edge, double* Lfill, size_t npix) {
+                                     int2* pack_counts, double lo_edge, double hi_edge, double* Lfill, size_t npix, const int* nd) {
     fill_background(P, Lfill, npix);
     const int target = S.per_star ? 0 : *cnt_q;
-    for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += gridDim.x * blockDim.x) {
+    const int nk = LIVE ? *nd : n;   // n: the layout of own_qcount
+    for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < nk; k += gridDim.x * blockDim.x) {
         const Star3 sg = load3(a1, k), b = load3(a2, k), pk = load3(p, k);
         Star3 qn = load3(q, k);
         for (int c = own_qcount(a2, n, k); c < target; ++c) qn = qfix_iter(S, sg, b, pk, qn);
@@ -572,12 +582,14 @@ __global__ void big_perstar_kernel(const BigParams P, const BigStep S, int n, do
 
 // momentum refresh p = z sqrt(H) (sampler_RHMC.py:1021-1022) with device Philox keyed by the GLOBAL star id, or
 // injected normals; saves the iteration's start state
+template <bool LIVE>
 __global__ void big_momentum_kernel(const BigParams P, double g_ff2, int n, const double* q, double* p, const double* g,
                                     double* q0, double* g0, const long long* gid, unsigned long long seed, int iter_host,
-                                    const int* iter_dev, const double* normals_all /* [iters,n,3] or nullptr */) {
+                                    const int* iter_dev, const double* normals_all /* [iters,n,3] or nullptr */, const int* nd) {
     const int iter = iter_dev ? *iter_dev : iter_host;
     const double* normals = normals_all ? normals_all + (size_t)iter * n * 3 : nullptr;
-    for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += gridDim.x * blockDim.x) {
+    const int nk = LIVE ? *nd : n;   // n: the row length of the normals
+    for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < nk; k += gridDim.x * blockDim.x) {
         const Metric m = metric_of(P.F, q[3 * k], g_ff2);
         double z[3];
         if (normals) {
@@ -599,10 +611,12 @@ constexpr int kEnergyBlocks = 256;
 
 // scalars[1] = sum (p^2/H + ln|H|)/2, scalars[2] = # stars outside the support, scalars[3] = prior potential
 // (per-block partials, summed in block order by the last block)
+template <bool LIVE>
 __global__ void big_energy_kernel(const BigParams P, double g_ff2, int f_pos, int n, const double* q, const double* p,
-                                  double* part /* [gridDim.x][4] */, unsigned int* ticket, double* scalars) {
+                                  double* part /* [gridDim.x][4] */, unsigned int* ticket, double* scalars, const int* nd) {
     __shared__ double red[4 * 32];
     __shared__ bool is_last;
+    if (LIVE) n = *nd;
     double v[4] = {0, 0, 0, 0};
     for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += gridDim.x * blockDim.x) {
         const double f = q[3 * k], x = q[3 * k + 1], y = q[3 * k + 2];
@@ -677,8 +691,10 @@ __global__ void big_restore_v_kernel(double* local_scalars, const double* state,
 // Sample row of the iteration (RECORD_E0: q before the trajectory, p just drawn by MOMENTUM) when the iteration is a multiple of
 // the stride: row iter / stride, stars in ascending global-id order (slot = rank of the star's id within the strip), so the rows
 // do not depend on the storage order.  One thread per coordinate: coalesced reads, the three coordinates of a star together.
+// With a live count (reversible-jump mode: n = max_stars, slots in table order) the rows are zero past it.
+template <bool LIVE>
 __global__ void big_record_kernel(int n, const double* q, const double* p, const int* slot, int iter_host, const int* iter_dev,
-                                  int stride, int rows, double* rec_q, double* rec_p) {
+                                  int stride, int rows, double* rec_q, double* rec_p, const int* nd) {
     const int iter = iter_dev ? *iter_dev : iter_host;
     if (iter < 0 || iter % stride) return;
     const int r = iter / stride;
@@ -686,8 +702,9 @@ __global__ void big_record_kernel(int n, const double* q, const double* p, const
     const size_t row = (size_t)r * 3 * n;
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < 3 * n; i += gridDim.x * blockDim.x) {
         const size_t o = row + 3 * (size_t)slot[i / 3] + i % 3;
-        if (rec_q) rec_q[o] = q[i];
-        if (rec_p) rec_p[o] = p[i];
+        const bool live = !LIVE || i < 3 * *nd;
+        if (rec_q) rec_q[o] = live ? q[i] : 0.0;
+        if (rec_p) rec_p[o] = live ? p[i] : 0.0;
     }
 }
 
@@ -947,6 +964,13 @@ struct srhmc_big {
     int world = 1, rank = 0;
     bool have_data = false;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
+    // reversible-jump mode (srhmc_big_rj_configure .. srhmc_big_rj_finish, big_rj.cuh): the per-star kernels take their count
+    // from rjst and are launched for max_stars; rj_leg2: the step phases enqueued since RJ_JUMP belong to leg 2
+    bool rj_on = false, rj_leg2 = false;
+    RjParams rjp{};
+    double rj_inv_cell = 0.0;
+    int rj_ncx = 1, rj_ncy = 1;
+    BBuf rjst, rjdraws, rjN, rjmove, rjrow, rjhead, rjnext;
 };
 
 namespace {
@@ -998,9 +1022,9 @@ void ghost_edges(const srhmc_big* b, double& lo_edge, double& hi_edge) {
 // kernel (FP64, or FP32 for gradient-only evaluations), the star-centric kernel (very sparse fields) or the star-parallel
 // scatter / pixel / gather kernels.  The first two leave per-star footprint partials, and *gpart points at them; the
 // star-parallel kernels write g, and *gpart is nullptr.
-int enqueue_eval(srhmc_big* b, bool want_V, const double** gpart) {
+// nd: the live star count on the device (reversible-jump mode, n = max_stars), or nullptr.
+int enqueue_eval(srhmc_big* b, bool want_V, const double** gpart, int n, const int* nd) {
     const BigParams& P = b->P;
-    const int n = b->n;
     cudaStream_t st = b->stream;
     int* cnt = b->counters.as<int>();
     const size_t list = 1 + 3 * (size_t)std::max(1, b->cfg.max_ghosts);
@@ -1017,11 +1041,11 @@ int enqueue_eval(srhmc_big* b, bool want_V, const double** gpart) {
         b->L_filled = false;
         const int total = n + 2 * std::max(1, b->cfg.max_ghosts);
         const int sg = std::max(1, std::min((total * 32 + 255) / 256, 16 * b->sm_count));
-        big_scatter_kernel<<<sg, 256, 0, st>>>(P, b->q.as<double>(), n, ga, gb, b->L.as<double>(), b->err.as<int>());
+        (nd ? big_scatter_kernel<true> : big_scatter_kernel<false>)<<<sg, 256, 0, st>>>(P, b->q.as<double>(), n, ga, gb, b->L.as<double>(), b->err.as<int>(), nd);
         big_pixel_kernel<<<pg, 256, 0, st>>>(P, b->D.as<double>(), b->L.as<double>(), want_V, b->vpart.as<double>());
         if (want_V) big_vsum_kernel<<<1, 256, 0, st>>>(b->vpart.as<double>(), pg, b->scalars.as<double>());
         const int gg = std::max(1, std::min((n * 32 + 255) / 256, 16 * b->sm_count));
-        big_gather_kernel<<<gg, 256, 0, st>>>(P, b->q.as<double>(), n, b->L.as<double>(), b->g.as<double>());
+        (nd ? big_gather_kernel<true> : big_gather_kernel<false>)<<<gg, 256, 0, st>>>(P, b->q.as<double>(), n, b->L.as<double>(), b->g.as<double>(), nd);
         b->launches += want_V ? 4 : 3;
         return 0;
     }
@@ -1029,13 +1053,13 @@ int enqueue_eval(srhmc_big* b, bool want_V, const double** gpart) {
     S.q = b->q.as<double>(); S.ga = ga; S.gb = gb; S.n_own = n; S.cap = std::max(1, b->cfg.max_ghosts);
     const int ntiles = b->nty * b->ntx;
     if (!b->own_binned && n > 0) {
-        big_bin_kernel<<<std::max(1, std::min((n + 255) / 256, 8 * b->sm_count)), 256, 0, st>>>(
-            P, S, b->ntx, 0, n, b->tcnt.as<int>(), b->tlist.as<PairRec>(), b->err.as<int>());
+        (nd ? big_bin_kernel<true> : big_bin_kernel<false>)<<<std::max(1, std::min((n + 255) / 256, 8 * b->sm_count)), 256, 0, st>>>(
+            P, S, b->ntx, 0, n, b->tcnt.as<int>(), b->tlist.as<PairRec>(), b->err.as<int>(), nd);
         b->launches += 1;
     }
     if ((ga || gb) && !b->ghosts_binned) {
-        big_bin_kernel<<<std::max(1, std::min((2 * S.cap + 255) / 256, 8 * b->sm_count)), 256, 0, st>>>(
-            P, S, b->ntx, n, n + 2 * S.cap, b->tcnt.as<int>(), b->tlist.as<PairRec>(), b->err.as<int>());
+        big_bin_kernel<false><<<std::max(1, std::min((2 * S.cap + 255) / 256, 8 * b->sm_count)), 256, 0, st>>>(
+            P, S, b->ntx, n, n + 2 * S.cap, b->tcnt.as<int>(), b->tlist.as<PairRec>(), b->err.as<int>(), nullptr);
         b->launches += 1;
     }
     b->own_binned = false;  // the tile kernel consumes the lists and re-zeroes the counters
@@ -1043,14 +1067,15 @@ int enqueue_eval(srhmc_big* b, bool want_V, const double** gpart) {
     if (b->precision == 32 && !want_V) {
         big_tile32_kernel<<<ntiles, kTileThreads, sizeof(TileSmemF), st>>>(P, S, b->ntx, b->tcnt.as<int>(), b->tlist.as<PairRec>(),
                                                                            b->gpart.as<double>(), cnt, b->tmapD32);
-    } else if (!want_V && n > 0 && P.rad <= 15 && (b->star_mode == 1 || (b->star_mode < 0 && 2.0 * n <= 3.0 * ntiles))) {
+    } else if (!want_V && n > 0 && P.rad <= 15 && (b->star_mode == 1 || (b->star_mode < 0 && 2.0 * b->n <= 3.0 * ntiles))) {
         // very sparse field (mean tile list below ~1.5 records): one warp per owned star, neighbours from the tile lists
         // (big_star.cuh: only the patches are read, not every pixel); the lists are
         // consumed here, so their counters are re-zeroed by a memset node instead of by the tile CTAs
         const int sgrid = std::max(1, std::min((n + kStarWarps - 1) / kStarWarps, 64 * b->sm_count));
-        const auto star = P.rad <= 12 ? big_star_kernel<25> : big_star_kernel<31>;
+        const auto star = P.rad <= 12 ? (nd ? big_star_kernel<25, true> : big_star_kernel<25, false>)
+                                      : (nd ? big_star_kernel<31, true> : big_star_kernel<31, false>);
         star<<<sgrid, 32 * kStarWarps, 0, st>>>(P, n, b->q.as<double>(), b->D.as<double>(), b->ntx, b->tcnt.as<int>(),
-                                                b->tlist.as<PairRec>(), b->gpart.as<double>(), cnt);
+                                                b->tlist.as<PairRec>(), b->gpart.as<double>(), cnt, nd);
         BCU(cudaMemsetAsync(b->tcnt.ptr, 0, (size_t)ntiles * 4, st));
     } else {
         const auto tile = want_V ? big_tile_kernel<1> : big_tile_kernel<0>;
@@ -1171,7 +1196,7 @@ int srhmc_big_destroy(srhmc_big* b) {
     BBuf* all[] = {&b->D, &b->L, &b->q, &b->p, &b->g, &b->a1, &b->a2, &b->q0, &b->g0, &b->gid, &b->vpart, &b->scalars, &b->gscalars, &b->state,
                    &b->counters, &b->send, &b->recv, &b->err, &b->normals, &b->lnu, &b->E, &b->V, &b->T, &b->A,
                    &b->tcnt, &b->tlist, &b->gpart, &b->epart, &b->tickets, &b->xepoch, &b->packcnt, &b->xticket, &b->D32,
-                   &b->slot, &b->recq, &b->recp};
+                   &b->slot, &b->recq, &b->recp, &b->rjst, &b->rjdraws, &b->rjN, &b->rjmove, &b->rjrow, &b->rjhead, &b->rjnext};
     for (BBuf* x : all) x->release();
     for (int r = 0; r < kMaxWorld; ++r)
         if (b->ipc_opened[r]) cudaIpcCloseMemHandle(b->ipc_opened[r]);
@@ -1265,8 +1290,8 @@ int srhmc_big_mock_data(srhmc_big* b, const double* q_true, int32_t n, uint64_t 
         TileSrc S;
         S.q = nullptr; S.ga = truth.as<double>(); S.gb = nullptr; S.n_own = 0; S.cap = std::max(1, n);
         if (n)
-            big_bin_kernel<<<std::max(1, std::min((n + 255) / 256, 8 * b->sm_count)), 256, 0, st>>>(
-                b->P, S, b->ntx, 0, n, b->tcnt.as<int>(), b->tlist.as<PairRec>(), b->err.as<int>());
+            big_bin_kernel<false><<<std::max(1, std::min((n + 255) / 256, 8 * b->sm_count)), 256, 0, st>>>(
+                b->P, S, b->ntx, 0, n, b->tcnt.as<int>(), b->tlist.as<PairRec>(), b->err.as<int>(), nullptr);
         big_tile_kernel<2><<<(int)ntiles, kTileThreads, sizeof(TileSmem), st>>>(b->P, S, b->ntx, nullptr, b->tcnt.as<int>(), b->tlist.as<PairRec>(),
                                                                                 nullptr, nullptr, nullptr, nullptr, nullptr, b->D.as<double>(), seed,
                                                                                 b->tmapD, 0);
@@ -1423,14 +1448,16 @@ int srhmc_big_buffers(srhmc_big* b, srhmc_big_buffers_t* out) {
 }
 
 int srhmc_big_set_draws(srhmc_big* b, const double* normals, const double* lnu, int32_t n_iters) {
-    // normals [n_iters, n, 3] for the owned stars (parity mode) and lnu [n_iters]; either may be NULL (device Philox)
+    // normals [n_iters, n, 3] for the owned stars (parity mode; reversible-jump mode: [n_iters, max_stars, 3] in table order)
+    // and lnu [n_iters]; either may be NULL (device Philox)
     if (!b || n_iters < 0) return bfail(SRHMC_ERR_INVALID, "bad argument");
     BCU(cudaSetDevice(b->cfg.device));
     b->normals.release();
     b->lnu.release();
-    if (normals && b->n && n_iters) {
-        if (int rc = b->normals.ensure((size_t)n_iters * b->n * 24)) return rc;
-        BCU(cudaMemcpyAsync(b->normals.ptr, normals, (size_t)n_iters * b->n * 24, cudaMemcpyHostToDevice, b->stream));
+    const int rown = b->rj_on ? b->cfg.max_stars : b->n;
+    if (normals && rown && n_iters) {
+        if (int rc = b->normals.ensure((size_t)n_iters * rown * 24)) return rc;
+        BCU(cudaMemcpyAsync(b->normals.ptr, normals, (size_t)n_iters * rown * 24, cudaMemcpyHostToDevice, b->stream));
     }
     if (lnu && n_iters) {
         if (int rc = b->lnu.ensure((size_t)n_iters * 8)) return rc;
@@ -1452,6 +1479,95 @@ int srhmc_big_alloc_chains(srhmc_big* b, int32_t n_iters) {
     BCU(cudaMemsetAsync(b->T.ptr, 0, (size_t)n_iters * 8, b->stream));
     BCU(cudaMemsetAsync(b->A.ptr, 0, (size_t)n_iters, b->stream));
     BCU(cudaMemsetAsync(b->state.ptr, 0, 64, b->stream));
+    return 0;
+}
+
+int srhmc_big_rj_configure(srhmc_big* b, const srhmc_rj_args* rj, int32_t n_iters) {
+    if (!b || !rj) return bfail(SRHMC_ERR_INVALID, "null argument");
+    if (n_iters < 1) return bfail(SRHMC_ERR_INVALID, "n_iters must be >= 1");
+    if (b->world > 1)
+        return bfail(SRHMC_ERR_INVALID, "reversible-jump runs need the whole field on one device: this context is a strip of %d", b->world);
+    if (b->precision != 64) return bfail(SRHMC_ERR_INVALID, "reversible-jump runs need precision 64");
+    const double* pm = rj->P_move;
+    for (int i = 0; i < 3; ++i)
+        if (!(pm[i] >= 0.0) || !std::isfinite(pm[i])) return bfail(SRHMC_ERR_INVALID, "P_move[%d] = %g is not a finite probability", i, pm[i]);
+    const double psum = (pm[0] + pm[1]) + pm[2];
+    if (!(psum > 0.0)) return bfail(SRHMC_ERR_INVALID, "P_move sums to 0");
+    if (!(rj->fmin > 0.0) || !(rj->fmax > rj->fmin) || !std::isfinite(rj->fmax))
+        return bfail(SRHMC_ERR_INVALID, "the flux prior needs 0 < fmin < fmax (got %g, %g)", rj->fmin, rj->fmax);
+    if (!(b->cfg.alpha > 1.0)) return bfail(SRHMC_ERR_INVALID, "the power-law flux prior needs alpha > 1 (got %g)", b->cfg.alpha);
+    // the merge's cell-list cut-off needs a bounded Beta density
+    if (!(rj->beta_a >= 1.0) || !(rj->beta_b >= 1.0) || !std::isfinite(rj->beta_a) || !std::isfinite(rj->beta_b))
+        return bfail(SRHMC_ERR_INVALID, "beta_a and beta_b must be >= 1 (got %g, %g)", rj->beta_a, rj->beta_b);
+    if (!(rj->K_split > 0.0) || !std::isfinite(rj->K_split)) return bfail(SRHMC_ERR_INVALID, "K_split must be positive (got %g)", rj->K_split);
+    BCU(cudaSetDevice(b->cfg.device));
+    const int cap = b->cfg.max_stars;
+    const double cell = rj_merge_cell(rj->K_split);
+    b->rj_ncx = std::max(1, (int)std::ceil(b->P.Rg / cell));
+    b->rj_ncy = std::max(1, (int)std::ceil(b->P.C / cell));
+    b->rj_inv_cell = 1.0 / cell;
+    int rc = b->rjst.ensure(sizeof(BigRj)) | b->rjN.ensure((size_t)n_iters * 4) | b->rjmove.ensure((size_t)n_iters) |
+             b->rjrow.ensure((size_t)cap * 8) | b->rjnext.ensure((size_t)cap * 4) |
+             b->rjhead.ensure(((size_t)b->rj_ncx * b->rj_ncy + 1) * 4);
+    if (rj->draws) rc |= b->rjdraws.ensure((size_t)n_iters * kRjDraws * 8);
+    if (rc) {
+        cudaGetLastError();
+        return bfail(SRHMC_ERR_CUDA, "cannot allocate the reversible-jump buffers");
+    }
+    RjParams& R = b->rjp;
+    std::memset(&R, 0, sizeof(R));
+    R.cdf0 = pm[0] / psum;
+    R.cdf1 = (pm[0] + pm[1]) / psum;
+    const double e = 1.0 - b->cfg.alpha;
+    R.pl_lo = std::pow(rj->fmin, e);
+    R.pl_span = std::pow(rj->fmax, e) - std::pow(rj->fmin, e);
+    R.K_split = rj->K_split;
+    R.beta_a = rj->beta_a;
+    R.beta_b = rj->beta_b;
+    R.ln_beta = std::lgamma(rj->beta_a) + std::lgamma(rj->beta_b) - std::lgamma(rj->beta_a + rj->beta_b);
+    if (rj->draws) {
+        BCU(cudaMemcpyAsync(b->rjdraws.ptr, rj->draws, (size_t)n_iters * kRjDraws * 8, cudaMemcpyHostToDevice, b->stream));
+        R.draws = b->rjdraws.as<double>();
+    }
+    // table order: storage index = table index = Philox key of the momentum = slot of a recorded row, for every slot a birth
+    // can fill
+    std::vector<int64_t> ids(cap);
+    std::vector<int32_t> slots(cap);
+    std::iota(ids.begin(), ids.end(), (int64_t)0);
+    std::iota(slots.begin(), slots.end(), 0);
+    BigRj st0;
+    std::memset(&st0, 0, sizeof(st0));
+    st0.N = st0.n1 = st0.n2 = b->n;   // the evaluation that starts a run sees every star
+    st0.overflow = -1;
+    BCU(cudaMemcpyAsync(b->gid.ptr, ids.data(), (size_t)cap * 8, cudaMemcpyHostToDevice, b->stream));
+    BCU(cudaMemcpyAsync(b->slot.ptr, slots.data(), (size_t)cap * 4, cudaMemcpyHostToDevice, b->stream));
+    BCU(cudaMemcpyAsync(b->rjst.ptr, &st0, sizeof(st0), cudaMemcpyHostToDevice, b->stream));
+    BCU(cudaMemsetAsync(b->rjN.ptr, 0, (size_t)n_iters * 4, b->stream));
+    BCU(cudaMemsetAsync(b->rjmove.ptr, 0, (size_t)n_iters, b->stream));
+    BCU(cudaStreamSynchronize(b->stream));
+    b->sorted_ids.assign(ids.begin(), ids.begin() + b->n);
+    b->rj_on = true;
+    b->rj_leg2 = false;
+    return 0;
+}
+
+int srhmc_big_rj_finish(srhmc_big* b, int32_t n_iters, const srhmc_rj_args* out) {
+    if (!b) return bfail(SRHMC_ERR_INVALID, "null context");
+    if (!b->rj_on) return bfail(SRHMC_ERR_STATE, "srhmc_big_rj_configure has not been called");
+    if (n_iters < 0 || (size_t)n_iters * 4 > b->rjN.cap) return bfail(SRHMC_ERR_INVALID, "n_iters exceeds the configured run");
+    BCU(cudaSetDevice(b->cfg.device));
+    BigRj st;
+    BCU(cudaMemcpyAsync(&st, b->rjst.ptr, sizeof(st), cudaMemcpyDeviceToHost, b->stream));
+    if (out && out->N_chain) BCU(cudaMemcpyAsync(out->N_chain, b->rjN.ptr, (size_t)n_iters * 4, cudaMemcpyDeviceToHost, b->stream));
+    if (out && out->move_chain) BCU(cudaMemcpyAsync(out->move_chain, b->rjmove.ptr, (size_t)n_iters, cudaMemcpyDeviceToHost, b->stream));
+    BCU(cudaStreamSynchronize(b->stream));
+    if (out && out->n_final) *out->n_final = st.N;
+    if (out && out->overflow) *out->overflow = st.overflow;
+    b->n = st.N;
+    b->sorted_ids.resize(st.N);
+    for (int k = 0; k < st.N; ++k) b->sorted_ids[k] = k;
+    b->rj_on = false;
+    b->rj_leg2 = false;
     return 0;
 }
 
@@ -1495,7 +1611,8 @@ int srhmc_big_set_recording(srhmc_big* b, int32_t n_iters, int32_t stride, int32
     if (std::adjacent_find(b->sorted_ids.begin(), b->sorted_ids.end()) != b->sorted_ids.end())
         return bfail(SRHMC_ERR_STATE, "an owned global id appears twice: the sample rows need distinct ids");
     const int rows = (int)((n_iters + (int64_t)stride - 1) / stride);
-    const size_t bytes = std::max<size_t>(1, (size_t)rows * b->n * 24);
+    const int width = b->rj_on ? b->cfg.max_stars : b->n;   // reversible-jump rows: max_stars slots in table order
+    const size_t bytes = std::max<size_t>(1, (size_t)rows * width * 24);
     BCU(cudaStreamSynchronize(b->stream));
     BBuf* want[2] = {want_q ? &b->recq : nullptr, want_p ? &b->recp : nullptr};
     BBuf* drop[2] = {want_q ? nullptr : &b->recq, want_p ? nullptr : &b->recp};
@@ -1507,12 +1624,12 @@ int srhmc_big_set_recording(srhmc_big* b, int32_t n_iters, int32_t stride, int32
             b->recq.release();
             b->recp.release();
             b->rec_rows = 0;
-            return bfail(SRHMC_ERR_CUDA, "cannot allocate %zu bytes for %d sample rows of %d stars", bytes, rows, b->n);
+            return bfail(SRHMC_ERR_CUDA, "cannot allocate %zu bytes for %d sample rows of %d stars", bytes, rows, width);
         }
     }
     b->rec_rows = rows;
     b->rec_stride = stride;
-    b->rec_n = b->n;
+    b->rec_n = width;
     return 0;
 }
 
@@ -1680,7 +1797,14 @@ int srhmc_big_phase(srhmc_big* b, int32_t phase, const srhmc_big_step* s) {
     if (!b->have_data) return bfail(SRHMC_ERR_STATE, "srhmc_big_set_data has not been called");
     BCU(cudaSetDevice(b->cfg.device));
     const BigParams& P = b->P;
-    const int n = b->n;
+    if (b->rj_on && s->fixed_point_mode != 0)
+        return bfail(SRHMC_ERR_INVALID, "reversible-jump mode runs the reference stop rule only (fixed_point_mode = 0)");
+    // reversible-jump mode: every per-star kernel is launched for max_stars and reads its count on the device -- the live
+    // count, or (the step phases) the count of the leg, 0 when the device skips it
+    const int n = b->rj_on ? b->cfg.max_stars : b->n;
+    BigRj* rjst = b->rj_on ? b->rjst.as<BigRj>() : nullptr;
+    const int* nd_live = rjst ? &rjst->N : nullptr;
+    const int* nd_step = rjst ? (b->rj_leg2 ? &rjst->n2 : &rjst->n1) : nullptr;
     BigStep S;
     S.h = s->dt / 2.0; S.delta = s->delta; S.g_ff2 = s->g_ff2; S.counter_max = s->counter_max;
     S.per_star = s->fixed_point_mode != 0 ? 1 : 0;
@@ -1699,9 +1823,12 @@ int srhmc_big_phase(srhmc_big* b, int32_t phase, const srhmc_big_step* s) {
     }
     // the kicks of the field-wide stop rule (big_kick_kernel)
     auto kick = [&](bool last_half, bool next_first, const double* gpart) {
-        const auto kernel = !last_half ? big_kick_kernel<false, true> : next_first ? big_kick_kernel<true, true> : big_kick_kernel<true, false>;
+        const auto kernel = nd_step ? (!last_half ? big_kick_kernel<false, true, true> : next_first ? big_kick_kernel<true, true, true>
+                                                                                                 : big_kick_kernel<true, false, true>)
+                                    : (!last_half ? big_kick_kernel<false, true, false> : next_first ? big_kick_kernel<true, true, false>
+                                                                                                  : big_kick_kernel<true, false, false>);
         kernel<<<gs, tb, 0, st>>>(P, S, n, b->q.as<double>(), b->p.as<double>(), b->g.as<double>(), gpart, b->a1.as<double>(),
-                                  b->a2.as<double>(), cnt, X);
+                                  b->a2.as<double>(), cnt, X, nd_step);
         b->launches += 1;
     };
     // The kernels that move the stars: QFIX_KICK (big_qfix_kick_kernel) and, per-star stop rule, the whole advance between two
@@ -1725,9 +1852,9 @@ int srhmc_big_phase(srhmc_big* b, int32_t phase, const srhmc_big_step* s) {
             kernel<<<gs, tb, 0, st>>>(P, S, n, b->q.as<double>(), b->p.as<double>(), b->g.as<double>(), gpart, b->ntx, tc, tl,
                                       b->err.as<int>(), pc, lo_edge, hi_edge, lf, npix);
         } else {
-            big_qfix_kick_kernel<<<gs, tb, 0, st>>>(P, S, n, b->q.as<double>(), b->p.as<double>(), b->a1.as<double>(),
+            (nd_step ? big_qfix_kick_kernel<true> : big_qfix_kick_kernel<false>)<<<gs, tb, 0, st>>>(P, S, n, b->q.as<double>(), b->p.as<double>(), b->a1.as<double>(),
                                                     b->a2.as<double>(), cnt + 1, b->ntx, tc, tl, b->err.as<int>(), pc, lo_edge,
-                                                    hi_edge, lf, npix);
+                                                    hi_edge, lf, npix, nd_step);
         }
         b->L_filled = lf != nullptr;
         b->pack_counted = peer_multi;
@@ -1782,10 +1909,10 @@ int srhmc_big_phase(srhmc_big* b, int32_t phase, const srhmc_big_step* s) {
             const bool next_first = phase == SRHMC_BIG_EVAL_KICK2_KICK1;
             const bool ps_advance = phase == SRHMC_BIG_EVAL_PS_ADVANCE;
             const double* gpart = nullptr;
-            if (int rc = enqueue_eval(b, want_V, &gpart)) return rc;
+            if (int rc = enqueue_eval(b, want_V, &gpart, n, nd_step)) return rc;
             if (!last_half) {
                 if (gpart) {   // no tail sums the footprint partials into g
-                    big_gsum_kernel<<<gs, tb, 0, st>>>(P, b->q.as<double>(), n, gpart, b->g.as<double>());
+                    (nd_step ? big_gsum_kernel<true> : big_gsum_kernel<false>)<<<gs, tb, 0, st>>>(P, b->q.as<double>(), n, gpart, b->g.as<double>(), nd_step);
                     b->launches += 1;
                 }
             } else if (ps_advance) {
@@ -1806,8 +1933,8 @@ int srhmc_big_phase(srhmc_big* b, int32_t phase, const srhmc_big_step* s) {
         case SRHMC_BIG_PFIX_QFIX:
             // tiled over peers: the field-wide maximum of the p fixed-point counts was all-reduced by the last block of the
             // kernel that produced it
-            big_pfix_qfix_kernel<<<gs, tb, 0, st>>>(P, S, n, b->q.as<double>(), b->p.as<double>(), b->a1.as<double>(),
-                                                    b->a2.as<double>(), cnt, cnt + 1, X);
+            (nd_step ? big_pfix_qfix_kernel<true> : big_pfix_qfix_kernel<false>)<<<gs, tb, 0, st>>>(P, S, n, b->q.as<double>(), b->p.as<double>(), b->a1.as<double>(),
+                                                    b->a2.as<double>(), cnt, cnt + 1, X, nd_step);
             b->launches += 1;
             break;
         case SRHMC_BIG_QFIX_KICK:
@@ -1818,21 +1945,22 @@ int srhmc_big_phase(srhmc_big* b, int32_t phase, const srhmc_big_step* s) {
             break;
         case SRHMC_BIG_MOMENTUM: {
             const double* z = b->normals.ptr ? b->normals.as<double>() : nullptr;
-            big_momentum_kernel<<<gs, tb, 0, st>>>(P, s->g_ff2, n, b->q.as<double>(), b->p.as<double>(), b->g.as<double>(),
+            (nd_live ? big_momentum_kernel<true> : big_momentum_kernel<false>)<<<gs, tb, 0, st>>>(P, s->g_ff2, n, b->q.as<double>(), b->p.as<double>(), b->g.as<double>(),
                                                    b->q0.as<double>(), b->g0.as<double>(), b->gid.as<long long>(), s->seed,
-                                                   s->iteration, s->iteration < 0 ? cnt + 2 : nullptr, z);
+                                                   s->iteration, s->iteration < 0 ? cnt + 2 : nullptr, z, nd_live);
             b->launches += 1;
             break;
         }
         case SRHMC_BIG_ENERGY:
-            big_energy_kernel<<<std::max(1, std::min((n + 255) / 256, kEnergyBlocks)), 256, 0, st>>>(
+            (nd_live ? big_energy_kernel<true> : big_energy_kernel<false>)<<<std::max(1, std::min((n + 255) / 256, kEnergyBlocks)), 256, 0, st>>>(
                 P, s->g_ff2, s->f_pos, n, b->q.as<double>(), b->p.as<double>(), b->epart.as<double>(),
-                b->tickets.as<unsigned int>(), b->scalars.as<double>());
+                b->tickets.as<unsigned int>(), b->scalars.as<double>(), nd_live);
             b->launches += 1;
             break;
         case SRHMC_BIG_RECORD_E0:
         case SRHMC_BIG_ACCEPT: {
             const int ph = phase == SRHMC_BIG_ACCEPT ? 1 : 0;
+            if (ph == 1 && b->rj_on) return bfail(SRHMC_ERR_STATE, "reversible-jump mode ends an iteration with RJ_ACCEPT");
             // single rank: the global sums are the local ones; otherwise the caller has all-reduced `scalars` into
             // `global_scalars` on this stream before this phase
             if (b->world == 1) {
@@ -1856,11 +1984,50 @@ int srhmc_big_phase(srhmc_big* b, int32_t phase, const srhmc_big_step* s) {
             if (ph == 0 && b->rec_rows > 0) {   // sample row of this iteration (srhmc_big_set_recording)
                 if (b->rec_n != n) return bfail(SRHMC_ERR_STATE, "the stars changed since srhmc_big_set_recording");
                 if (n > 0) {
-                    big_record_kernel<<<std::max(1, std::min((3 * n + 255) / 256, 4 * b->sm_count)), 256, 0, st>>>(
+                    (nd_live ? big_record_kernel<true> : big_record_kernel<false>)<<<std::max(1, std::min((3 * n + 255) / 256, 4 * b->sm_count)), 256, 0, st>>>(
                         n, b->q.as<double>(), b->p.as<double>(), b->slot.as<int>(), s->iteration, s->iteration < 0 ? cnt + 2 : nullptr,
-                        b->rec_stride, b->rec_rows, b->recq.as<double>(), b->recp.as<double>());
+                        b->rec_stride, b->rec_rows, b->recq.as<double>(), b->recp.as<double>(), nd_live);
                     b->launches += 1;
                 }
+            }
+            break;
+        }
+        case SRHMC_BIG_RJ_BEGIN:
+        case SRHMC_BIG_RJ_JUMP:
+        case SRHMC_BIG_RJ_ACCEPT: {
+            if (!b->rj_on) return bfail(SRHMC_ERR_STATE, "srhmc_big_rj_configure has not been called");
+            int* iter_dev = s->iteration < 0 ? cnt + 2 : nullptr;
+            const int cap = b->cfg.max_stars;
+            const int eg = std::max(1, std::min((3 * cap + 255) / 256, 4 * b->sm_count));
+            if (phase == SRHMC_BIG_RJ_BEGIN) {
+                big_rj_begin_kernel<<<1, 32, 0, st>>>(b->rjp, rjst, cap, s->seed, s->iteration, iter_dev, b->rjN.as<int>(),
+                                                      b->rjmove.as<unsigned char>());
+                b->launches += 1;
+                b->rj_leg2 = false;
+            } else if (phase == SRHMC_BIG_RJ_JUMP) {
+                // merge cell lists, row sums, the proposal (also keeps leg 1's pixel potential), the edited table out of place
+                // into a1 / a2 (free between two leapfrog steps) and back; every kernel returns at once unless its move runs
+                BCU(cudaMemsetAsync(b->rjhead.ptr, 0xFF, b->rjhead.cap, st));
+                const int mg = std::max(1, std::min((cap + 255) / 256, 8 * b->sm_count));
+                big_rj_merge_bin_kernel<<<mg, 256, 0, st>>>(rjst, b->q.as<double>(), b->rj_inv_cell, b->rj_ncx, b->rj_ncy,
+                                                           b->rjhead.as<int>(), b->rjnext.as<int>());
+                big_rj_merge_rows_kernel<<<mg, 256, 0, st>>>(b->rjp, rjst, b->q.as<double>(), b->rj_inv_cell, b->rj_ncx, b->rj_ncy,
+                                                            b->rjhead.as<int>(), b->rjnext.as<int>(), b->rjrow.as<double>());
+                big_rj_propose_kernel<<<1, kRjThreads, 0, st>>>(P, b->rjp, s->g_ff2, rjst, b->q.as<double>(), b->p.as<double>(),
+                                                               b->rjrow.as<double>(), b->scalars.as<double>(), b->rj_inv_cell,
+                                                               b->rj_ncx, b->rj_ncy, b->rjhead.as<int>(), b->rjnext.as<int>());
+                big_rj_edit_kernel<<<eg, 256, 0, st>>>(rjst, b->q.as<double>(), b->p.as<double>(), b->a1.as<double>(), b->a2.as<double>());
+                big_rj_commit_kernel<<<eg, 256, 0, st>>>(rjst, b->a1.as<double>(), b->a2.as<double>(), b->q.as<double>(), b->p.as<double>());
+                b->launches += 5;
+                b->rj_leg2 = true;
+            } else {
+                big_rj_accept_kernel<<<gs, tb, 0, st>>>(rjst, b->scalars.as<double>(), b->state.as<double>(), s->seed, s->iteration,
+                                                       iter_dev, b->lnu.ptr ? b->lnu.as<double>() : nullptr, b->q.as<double>(),
+                                                       b->p.as<double>(), b->g.as<double>(), b->q0.as<double>(), b->g0.as<double>(),
+                                                       b->A.ptr ? b->A.as<unsigned char>() : nullptr);
+                big_rj_finish_kernel<<<1, 1, 0, st>>>(rjst, b->scalars.as<double>(), b->state.as<double>(), iter_dev);
+                b->launches += 2;
+                b->rj_leg2 = false;
             }
             break;
         }

@@ -129,7 +129,13 @@ __device__ __forceinline__ bool merge_conflict(const double* q, const double* ma
     return !(d2 > dr2 || fabs(__dsub_rn(mag[i], mag[j])) > dmag_tol);
 }
 
-// magnitude, state and cell list of every seed (lists are linked through `next`; head[ncx * ncy] is the non-finite list)
+// puts item i at (x, y) at the head of its cell's list (linked through `next`; head[ncx * ncy] is the non-finite list)
+__device__ __forceinline__ void merge_cell_insert(int i, double x, double y, double inv_cell, int ncx, int ncy, int* head, int* next) {
+    const int c = merge_wild(x, y) ? ncx * ncy : merge_cell_1d(x, inv_cell, ncx) * ncy + merge_cell_1d(y, inv_cell, ncy);
+    next[i] = atomicExch(&head[c], i);
+}
+
+// magnitude, state and cell list of every seed
 __global__ void big_merge_bin_kernel(int n, const double* q, const unsigned char* alive, double flux_to_count, double inv_cell,
                                      int ncx, int ncy, double* mag, int* head, int* next, unsigned char* state, int* n_open) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -140,9 +146,7 @@ __global__ void big_merge_bin_kernel(int n, const double* q, const unsigned char
     }
     // flux2mag (utils.py:27-28) of f / flux_to_count
     mag[i] = __dsub_rn(22.5, __dmul_rn(2.5, log10(q[3 * i] / flux_to_count)));
-    const double x = q[3 * i + 1], y = q[3 * i + 2];
-    const int c = merge_wild(x, y) ? ncx * ncy : merge_cell_1d(x, inv_cell, ncx) * ncy + merge_cell_1d(y, inv_cell, ncy);
-    next[i] = atomicExch(&head[c], i);
+    merge_cell_insert(i, q[3 * i + 1], q[3 * i + 2], inv_cell, ncx, ncy, head, next);
     state[i] = kMergeOpen;
     atomicAdd(n_open, 1);
 }

@@ -43,10 +43,11 @@ __device__ __forceinline__ PairRec ldg_rec(const PairRec* p) {
     return r;
 }
 
-template <int NR>   // rows / columns of the largest patch: 2 rad + 1 <= NR <= 31
+template <int NR, bool LIVE>   // rows / columns of the largest patch: 2 rad + 1 <= NR <= 31; LIVE: the star count is *nd
 __global__ void __launch_bounds__(32 * kStarWarps, 4)
 big_star_kernel(const BigParams P, int n_own, const double* __restrict__ q, const double* __restrict__ D, int ntx,
-                const int* __restrict__ cnt, const PairRec* __restrict__ list, double* __restrict__ gpart, int* fp_counters) {
+                const int* __restrict__ cnt, const PairRec* __restrict__ list, double* __restrict__ gpart, int* fp_counters,
+                const int* nd /* live stars (reversible-jump mode), or nullptr: n_own */) {
     __shared__ double s_d[kStarWarps][NR][32];  // data patch: lane c copies and reads column j0 + c only
     __shared__ double2 s_row[kStarWarps][32];   // own star: {ex, ex dx} of row i0 + r
     __shared__ double s_nex[kStarWarps][32];    // current neighbour: ex of row i0 + r (0 outside its patch)
@@ -54,6 +55,7 @@ big_star_kernel(const BigParams P, int n_own, const double* __restrict__ q, cons
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     // the fixed-point iteration counters of the leapfrog step are free between its last reader and the next step
     if (fp_counters && blockIdx.x == 0 && threadIdx.x < 2) fp_counters[threadIdx.x] = 0;
+    if (LIVE) n_own = *nd;
     for (int k = blockIdx.x * kStarWarps + warp; k < n_own; k += gridDim.x * kStarWarps) {
         const double f = q[3 * k], x = q[3 * k + 1], y = q[3 * k + 2];
         double* out = gpart + (size_t)k * 12;

@@ -109,7 +109,10 @@ __device__ __forceinline__ void bin_star(const BigParams& P, int ntx, int sid, d
 }
 
 // sources [sid0, sid1): own stars are [0, n_own), the ghost lists follow (tile_source)
-__global__ void big_bin_kernel(const BigParams P, const TileSrc S, int ntx, int sid0, int sid1, int* cnt, PairRec* list, int* err) {
+template <bool LIVE>
+__global__ void big_bin_kernel(const BigParams P, const TileSrc S, int ntx, int sid0, int sid1, int* cnt, PairRec* list, int* err,
+                               const int* nd /* live owned stars: sid1 */) {
+    if (LIVE) sid1 = *nd;
     for (int sid = sid0 + blockIdx.x * blockDim.x + threadIdx.x; sid < sid1; sid += gridDim.x * blockDim.x) {
         const double* src = tile_source(S, sid);
         if (!src) continue;
@@ -654,7 +657,9 @@ __device__ __forceinline__ void gsum_star(const BigParams& P, int k, double f, d
     gy = -sy * P.inv_s2;
 }
 
-__global__ void big_gsum_kernel(const BigParams P, const double* q, int n_own, const double* gpart, double* g) {
+template <bool LIVE>
+__global__ void big_gsum_kernel(const BigParams P, const double* q, int n_own, const double* gpart, double* g, const int* nd) {
+    if (LIVE) n_own = *nd;
     for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < n_own; k += gridDim.x * blockDim.x)
         gsum_star(P, k, q[3 * k], q[3 * k + 1], q[3 * k + 2], gpart, g[3 * k], g[3 * k + 1], g[3 * k + 2]);
 }

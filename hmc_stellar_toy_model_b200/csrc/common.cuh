@@ -171,6 +171,12 @@ __device__ __forceinline__ Metric metric_of(const FieldParams& P, double f, doub
     return m;
 }
 
+// One star's share of the two sums of T = (sum p^2/H + sum ln|H|)/2 (sampler_RHMC.py:353-363)
+__device__ __forceinline__ void kinetic_terms(const Metric& m, double pf, double px, double py, double& quad, double& logdet) {
+    quad += pf * pf / m.Hff + px * px / m.Hxx + py * py / m.Hxx;
+    logdet += log(fabs(m.Hff)) + 2.0 * log(fabs(m.Hxx));
+}
+
 // ------------------------------------------------------------------ arithmetic helpers
 // 1/a for normal positive a: MUFU.RCP64H seed (~2^-20) + one cubic step -> ~2^-60 relative error.
 __device__ __forceinline__ double rcp_fast(double a) {

@@ -611,12 +611,6 @@ struct Energies {
     double V, T;
 };
 
-// One star's share of the two sums of T = (sum p^2/H + sum ln|H|)/2 (sampler_RHMC.py:353-363)
-__device__ __forceinline__ void kinetic_terms(const Metric& m, double pf, double px, double py, double& quad, double& logdet) {
-    quad += pf * pf / m.Hff + px * px / m.Hxx + py * py / m.Hxx;
-    logdet += log(fabs(m.Hff)) + 2.0 * log(fabs(m.Hxx));
-}
-
 // two CTA-wide maxima of the fixed-point iteration counts (rhmc_step): a corner of the reduction scratch that block_sum
 // (at most 7 values wide here) never touches
 template <typename T>

@@ -12,7 +12,7 @@
 // than two stars or all pair weights zero, a proposal needing more than Nmax stars) the jump is rejected with the state
 // unchanged; the first iteration whose proposal needed more than Nmax stars is reported in RjParams.overflow.
 #pragma once
-#include "rj_draws.cuh"
+#include "rj_moves.cuh"
 
 namespace srhmc {
 
@@ -21,48 +21,11 @@ constexpr int kRjRec = 192;               // the iteration's draw record, kRjDra
 constexpr int kRjBc = kRjRec + kRjDraws;  // proposal broadcast: [0] merge pick, [1] log ratio, [2..7] row A, [8..13] row B
 constexpr int kRjStart = kRjBc + 14;      // E0, V and N of the iteration's start (3 doubles, red[220, 223))
 static_assert(kRjStart + 3 <= 224, "the reversible-jump slots must stay below fp_count_slots");
-enum RjStatus : int { RJ_OK = 0, RJ_REFUSED = 1, RJ_OVERFLOW = 2 };
 
-// ln of the Beta(a, b) density (scipy.stats.beta.logpdf)
-__device__ __forceinline__ double beta_logpdf(const RjParams& R, double x) {
-    return (R.beta_a - 1.0) * log(x) + (R.beta_b - 1.0) * log1p(-x) - R.ln_beta;
-}
-
-// Merge weight of the ordered pair (i, j) (drop-in _merge_weights): Beta density of the share f_j / (f_i + f_j), zero
-// within 1e-6 of one half, times the Gaussian split kernel at the pair's separation
+// Merge weight of the ordered pair (i, j) of the table (merge_weight_of, rj_moves.cuh)
 template <typename T>
 __device__ __forceinline__ double merge_weight(const Ctx<T>& c, const RjParams& R, int i, int j) {
-    const double fi = c.q[3 * i], fj = c.q[3 * j];
-    const double share = fj / (fi + fj);
-    // outside (0, 1) (a flux at or below 0, possible with f_pos = 0) the Beta density is 0, as scipy's BETA.pdf gives it
-    if (!(share > 0.0 && share < 1.0) || fabs(share - 0.5) < 1e-6) return 0.0;
-    const double dr = c.q[3 * i + 1] - c.q[3 * j + 1], dc = c.q[3 * i + 2] - c.q[3 * j + 2];
-    const double k2 = R.K_split * R.K_split;
-    return exp(beta_logpdf(R, share)) * (exp(-(dr * dr + dc * dc) / (2.0 * k2)) / (2.0 * CUDART_PI * k2));
-}
-
-// 0 within, 1 birth, 2 death, 3 split, 4 merge (gym.move_types) from u_move (np.random.choice's rule) and u_grow
-__device__ __forceinline__ int rj_move_code(const RjParams& R, const double* rec) {
-    const int move = rec[0] < R.cdf0 ? 0 : (rec[0] < R.cdf1 ? 1 : 2);
-    const bool grow = rec[1] < 0.5;
-    return move == 0 ? 0 : (move == 1 ? (grow ? 1 : 2) : (grow ? 3 : 4));
-}
-
-// T(p, H(q)) of one star
-template <typename T>
-__device__ __forceinline__ double star_T(const Ctx<T>& c, const double* q3, const double* p3) {
-    double quad = 0.0, logdet = 0.0;
-    kinetic_terms(metric_of(*c.P, q3[0], c.g_ff2), p3[0], p3[1], p3[2], quad, logdet);
-    return (quad + logdet) / 2.0;
-}
-
-// p3 = z sqrt(H(q3)): the momentum of a proposed star
-template <typename T>
-__device__ __forceinline__ void draw_momentum(const Ctx<T>& c, const double* q3, const double* z, double* p3) {
-    const Metric m = metric_of(*c.P, q3[0], c.g_ff2);
-    p3[0] = z[0] * sqrt(m.Hff);
-    p3[1] = z[1] * sqrt(m.Hxx);
-    p3[2] = z[2] * sqrt(m.Hxx);
+    return merge_weight_of(R, c.q + 3 * i, c.q + 3 * j);
 }
 
 // Removes rows d0 and d1 (-1: none) of q and p keeping the order of the others (np.delete).  Rows only move down, so a
@@ -107,7 +70,7 @@ static __device__ __noinline__ int rj_propose(const FieldParams& P, double* q, d
     const int tid = threadIdx.x, nt = blockDim.x;
     double* bc = c.red + kRjBc;
     int d0 = -1, d1 = -1;
-    if (code == 2) d0 = min((int)floor(rec[2] * n), n - 1);
+    if (code == 2) d0 = rj_index(rec, n);
     if (code == 4) {
         // weights of all n^2 ordered pairs: thread t sums the flat indices [t m, (t + 1) m) in order, thread 0 adds the
         // partial sums in thread order and picks the first flat index i n + j whose cumulative weight exceeds u W
@@ -156,33 +119,21 @@ static __device__ __noinline__ int rj_propose(const FieldParams& P, double* q, d
         double lr = 0.0;
         if (code == 1) {
             // newborn: row, column and flux from the prior, momentum from H of the newborn
-            rowB[1] = rec[2] * (P.R - 2.0) + 1.0;
-            rowB[2] = rec[3] * (P.C - 2.0) + 1.0;
-            rowB[0] = exp(log(R.pl_lo + rec[4] * R.pl_span) / (1.0 - P.alpha));
-            draw_momentum(c, rowB, rec + 8, rowB + 3);
-            lr = P.alpha * log(rowB[0]) - 3.0 / 2.0 + star_T(c, rowB, rowB + 3) + P.Vpc;
+            rj_newborn(R, P.R, P.C, P.alpha, rec, rowB);
+            draw_momentum(P, g_ff2, rowB, rec + 8, rowB + 3);
+            lr = rj_lr_birth(P, rowB[0], star_T(P, g_ff2, rowB, rowB + 3));
         } else if (code == 2) {
-            const double* qv = c.q + 3 * d0;
-            lr = -P.alpha * log(qv[0]) + 3.0 / 2.0 - star_T(c, qv, c.p + 3 * d0) - P.Vpc;
+            lr = rj_lr_death(P, c.q[3 * d0], star_T(P, g_ff2, c.q + 3 * d0, c.p + 3 * d0));
         } else if (code == 3) {
             // the parent becomes child one in place, child two is appended
-            const int par = min((int)floor(rec[2] * n), n - 1);
+            const int par = rj_index(rec, n);
             const double fp = c.q[3 * par], rp = c.q[3 * par + 1], cp = c.q[3 * par + 2];
             const double off_r = rec[5] * K, off_c = rec[6] * K, share = rec[7];
-            rowA[0] = share * fp;
-            rowA[1] = rp + (1.0 - share) * off_r;
-            rowA[2] = cp + (1.0 - share) * off_c;
-            rowB[0] = (1.0 - share) * fp;
-            rowB[1] = rp - share * off_r;
-            rowB[2] = cp - share * off_c;
-            draw_momentum(c, rowA, rec + 8, rowA + 3);
-            draw_momentum(c, rowB, rec + 11, rowB + 3);
-            double quad = 0.0, logdet = 0.0;
-            kinetic_terms(metric_of(P, rowA[0], c.g_ff2), rowA[3], rowA[4], rowA[5], quad, logdet);
-            kinetic_terms(metric_of(P, rowB[0], c.g_ff2), rowB[3], rowB[4], rowB[5], quad, logdet);
-            const double T_children = (quad + logdet) / 2.0;
-            lr = (-3.0 / 2.0) + log(fp) - beta_logpdf(R, share) + kernel_norm + ((off_r * off_r + off_c * off_c) / (2.0 * k2)) +
-                 T_children - star_T(c, c.q + 3 * par, c.p + 3 * par);
+            rj_children(fp, rp, cp, off_r, off_c, share, rowA, rowB);
+            draw_momentum(P, g_ff2, rowA, rec + 8, rowA + 3);
+            draw_momentum(P, g_ff2, rowB, rec + 11, rowB + 3);
+            lr = rj_lr_split(R, kernel_norm, fp, share, off_r, off_c, pair_T(P, g_ff2, rowA, rowA + 3, rowB, rowB + 3),
+                             star_T(P, g_ff2, c.q + 3 * par, c.p + 3 * par));
             bc[0] = (double)par;
         } else {
             // merge of the ordered pair (one, two): the merged star uses the share f_one / (f_one + f_two)
@@ -190,16 +141,10 @@ static __device__ __noinline__ int rj_propose(const FieldParams& P, double* q, d
             const double* b = c.q + 3 * d1;
             const double share = a[0] / (a[0] + b[0]);
             const double gap2 = (a[1] - b[1]) * (a[1] - b[1]) + (a[2] - b[2]) * (a[2] - b[2]);
-            rowB[0] = a[0] + b[0];
-            rowB[1] = share * a[1] + (1.0 - share) * b[1];
-            rowB[2] = share * a[2] + (1.0 - share) * b[2];
-            double quad = 0.0, logdet = 0.0;
-            kinetic_terms(metric_of(P, a[0], c.g_ff2), c.p[3 * d0], c.p[3 * d0 + 1], c.p[3 * d0 + 2], quad, logdet);
-            kinetic_terms(metric_of(P, b[0], c.g_ff2), c.p[3 * d1], c.p[3 * d1 + 1], c.p[3 * d1 + 2], quad, logdet);
-            const double T_pair = (quad + logdet) / 2.0;
-            draw_momentum(c, rowB, rec + 8, rowB + 3);
-            lr = (3.0 / 2.0) - log(rowB[0]) + beta_logpdf(R, share) - kernel_norm - (gap2 / (2.0 * k2)) - T_pair +
-                 star_T(c, rowB, rowB + 3);
+            rj_merged(a, b, share, rowB);
+            const double T_pair = pair_T(P, g_ff2, a, c.p + 3 * d0, b, c.p + 3 * d1);
+            draw_momentum(P, g_ff2, rowB, rec + 8, rowB + 3);
+            lr = rj_lr_merge(R, kernel_norm, rowB[0], share, gap2, T_pair, star_T(P, g_ff2, rowB, rowB + 3));
         }
         bc[1] = lr;
     }

@@ -414,7 +414,11 @@ typedef enum srhmc_big_phase_id {
     SRHMC_BIG_EVAL_KICK2_KICK1 = 14, /* EVAL, KICK2 and the KICK1 of the following leapfrog step (same q, same gradient) */
     /* per-star stop rule (srhmc_big_step.fixed_point_mode = 1): steps 1-4 of a7 couple no stars, so they are one kernel */
     SRHMC_BIG_PS_ADVANCE = 15,       /* KICK1, both fixed points to each star's own convergence, p -= h dtau/dq, binning */
-    SRHMC_BIG_EVAL_PS_ADVANCE = 16   /* EVAL, KICK2 and the PS_ADVANCE of the following leapfrog step */
+    SRHMC_BIG_EVAL_PS_ADVANCE = 16,  /* EVAL, KICK2 and the PS_ADVANCE of the following leapfrog step */
+    /* reversible-jump mode (srhmc_big_rj_configure): RJ_BEGIN after RECORD_E0, leg 1, RJ_JUMP, EVAL_V, leg 2, ENERGY, RJ_ACCEPT */
+    SRHMC_BIG_RJ_BEGIN = 17,         /* the iteration's draw record and move; refusals that depend on N alone; N / move rows */
+    SRHMC_BIG_RJ_JUMP = 18,          /* on a jump: the proposal, the table edit in place (order kept), p = -p, the log ratio */
+    SRHMC_BIG_RJ_ACCEPT = 19         /* ln u < -dE (+ log ratio); restore q, g, V and N on rejection; p = -p after a jump */
 } srhmc_big_phase_id;
 
 typedef struct srhmc_big_step {
@@ -474,6 +478,23 @@ int srhmc_big_comm_import(srhmc_big* b, const void* ipc_handles, void* const* ra
 /* Parity mode: normals [n_iters, n, 3] for the owned stars and/or lnu [n_iters]; NULL -> device Philox (seed). */
 int srhmc_big_set_draws(srhmc_big* b, const double* normals, const double* lnu, int32_t n_iters);
 int srhmc_big_alloc_chains(srhmc_big* b, int32_t n_iters);
+/* Reversible-jump chains on one large field (multi_gym.run_RHMC with P_move[1:] != 0, srhmc_run_rj's semantics with a
+ * patch-limited PSF): the star count lives on the device, so one captured graph of an iteration serves every count.  From
+ * this call until srhmc_big_rj_finish the stars are a table in the order srhmc_big_set_stars gave them (the ids must be
+ * 0..n-1 in that order); a death or merge removes rows keeping the others' order, a newborn, second child or merged star is
+ * appended.  Every per-star kernel is launched for max_stars and reads the count on the device.  The momentum of star k is
+ * keyed by the table index k (field id 0), the record of iteration l is rj_record(seed, 0, l, beta_a, beta_b) unless
+ * rj->draws [n_iters, 14] is given; srhmc_big_set_draws then takes normals [n_iters, max_stars, 3].  Recorded rows are
+ * [max_stars][3] in table order, zero past N.  An iteration is MOMENTUM, ENERGY, RECORD_E0, RJ_BEGIN, nsteps leapfrog steps,
+ * RJ_JUMP, EVAL_V, nsteps leapfrog steps, ENERGY, RJ_ACCEPT; the device skips the second leg of a within-model iteration and
+ * both legs of a refused jump (a death or split with no star, a merge with fewer than two stars or all weights zero, a
+ * proposal needing more than max_stars stars).  Refuses (SRHMC_ERR_INVALID) a strip of a tiled field, precision 32 and
+ * beta_a or beta_b below 1; the phases refuse fixed_point_mode = 1.  The output pointers of rj are not used here. */
+int srhmc_big_rj_configure(srhmc_big* b, const srhmc_rj_args* rj, int32_t n_iters);
+/* Ends reversible-jump mode after the run: out->N_chain [n_iters] (N at the start of each iteration), out->move_chain
+ * [n_iters], out->n_final [1] and out->overflow [1] (first iteration whose proposal needed more than max_stars stars, -1 if
+ * none), each may be NULL.  The context then holds the n_final stars of the table, ids 0..n_final-1. */
+int srhmc_big_rj_finish(srhmc_big* b, int32_t n_iters, const srhmc_rj_args* out);
 int srhmc_big_read_chains(srhmc_big* b, int32_t n_iters, double* E, double* V, double* T, uint8_t* A, double* n_accepted,
                           int32_t* error_flag /* 1: an owned star left the local data window; 2: ghost list overflow;
                                                     3: tile list overflow; 4: peer exchange timed out */);
