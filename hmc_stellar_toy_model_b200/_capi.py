@@ -266,6 +266,13 @@ SIGNATURES = {
     "srhmc_big_set_recording": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32]),
     "srhmc_big_read_samples": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, c_double_p, c_double_p]),
     "srhmc_big_convergence_stats": (C.c_int, [C.POINTER(C.c_void_p), C.c_int32, C.c_int32, C.c_int32, c_double_p, c_double_p]),
+    "srhmc_big_set_chains": (C.c_int, [C.c_void_p, C.c_int32]),
+    "srhmc_big_set_chain_stars": (C.c_int, [C.c_void_p, C.c_int32, c_double_p, C.POINTER(C.c_int64), C.c_int32]),
+    "srhmc_big_get_chain_stars": (C.c_int, [C.c_void_p, C.c_int32, c_double_p, c_double_p, c_double_p]),
+    "srhmc_big_read_chain_rows": (C.c_int, [C.c_void_p, C.c_int32, c_double_p, c_double_p, c_double_p, c_uint8_p, c_double_p,
+                                            C.POINTER(C.c_int32)]),
+    "srhmc_big_read_chain_samples": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, c_double_p, c_double_p]),
+    "srhmc_big_chain_convergence_stats": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, c_double_p, c_double_p]),
     "srhmc_big_find_peaks": (C.c_int, [C.c_void_p, C.POINTER(BigPeaksArgs)]),
 }
 

@@ -45,6 +45,25 @@ def tile_order(q, cols, tile=64):
     return np.argsort(key, kind="stable").astype(np.int64)
 
 
+def chain_starts(q, chains, cols):
+    """Storage of K chains of one whole field: q [N,3] (every chain starts there) or [K,N,3] (chain c starts at q[c]) ->
+    (q_store [K,N,3], ids [K,N], slots [K,N]).  Chain c is stored in the 64x64-tile order of its own start (tile_order): chains
+    started from different catalogues sort differently, and the tile kernel sums each tile's stars in id order, so this keeps
+    chain c equal to a one-chain engine started from q[c].  ids[c] is the global id of each stored star; slots[c] the column
+    of each stored star in a recorded row (the rank of its id), the same ascending-id columns for every chain."""
+    q = np.asarray(q, dtype=np.float64)
+    if q.ndim == 3:
+        if q.shape[0] != chains or q.shape[2] != 3:
+            raise ValueError("per-chain starts must be [K=%d, N, 3], got %s" % (chains, q.shape))
+    else:
+        q = q.reshape(-1, 3)
+        q = np.broadcast_to(q, (chains,) + q.shape)
+    ids = np.stack([tile_order(q[c], cols) for c in range(chains)]).reshape(chains, q.shape[1])
+    q_store = np.ascontiguousarray(np.take_along_axis(q, ids[:, :, None], axis=1))
+    slots = np.argsort(np.argsort(ids, axis=1, kind="stable"), axis=1, kind="stable")
+    return q_store, ids, slots
+
+
 def strip_bounds(rows: int, world: int):
     """Owned row ranges [lo, hi) of `world` equal-height strips (the last one takes the remainder)."""
     base = rows // world
@@ -136,7 +155,10 @@ class BigFieldStrip:
     """One rank's strip: thin wrapper over the srhmc_big_* entry points."""
 
     def __init__(self, *, rows, cols, rank, world, device, max_stars, max_ghosts, patch_radius, halo, psf_fwhm_pix,
-                 B_count, f_lim, f_low, g0, g1, g2, g_xx, g_ff, use_prior=False, alpha=2.0, V_prior_const=0.0):
+                 B_count, f_lim, f_low, g0, g1, g2, g_xx, g_ff, use_prior=False, alpha=2.0, V_prior_const=0.0, chains=1):
+        """chains: K chains of the same field in this context (srhmc_big_set_chains: world = 1, FP64, device draws; every
+        evaluation on the tile kernel).  With K > 1 set_stars takes [N,3] or [K,N,3], ids is [K,N] and the per-star arrays
+        gain a leading chain axis."""
         self._lib = _capi.load_library()
         lo, hi = strip_bounds(rows, world)[rank]
         row0, nrows = data_window(rows, lo, hi, halo)
@@ -160,6 +182,19 @@ class BigFieldStrip:
         self.n_global = 0
         self.ids = np.zeros(0, dtype=np.int64)
         self._views = None
+        self.chains = 1
+        self.layout = 0
+        if chains != 1:
+            self.set_chains(chains)
+
+    def set_chains(self, k):
+        """K chains of this field (srhmc_big_set_chains); every chain's stars are cleared.  k = 1 returns to the one-chain
+        engine on the evaluation path chosen at creation."""
+        check(self._lib.srhmc_big_set_chains(self._h, int(k)))
+        self.chains = int(k)
+        self.layout += 1   # the per-chain buffers moved: no graph captured before may be replayed
+        self.n = self.n_global = 0
+        self.ids = np.zeros((0,) if k == 1 else (k, 0), dtype=np.int64)
 
     def close(self):
         if getattr(self, "_h", None):
@@ -207,7 +242,16 @@ class BigFieldStrip:
         return out
 
     def set_stars(self, q_global):
-        """Take the stars of the global list [N,3] (f, x, y) whose row coordinate falls in this strip."""
+        """Take the stars of the global list [N,3] (f, x, y) whose row coordinate falls in this strip.  K > 1 chains (whole
+        field): [N,3] starts every chain there, [K,N,3] chain c at q_global[c] (chain_starts)."""
+        if self.chains > 1:
+            q, ids, _ = chain_starts(q_global, self.chains, self.cols)
+            for c in range(self.chains):
+                idc = np.ascontiguousarray(ids[c])
+                check(self._lib.srhmc_big_set_chain_stars(self._h, c, _capi.dptr(q[c]), idc.ctypes.data_as(C.POINTER(C.c_int64)),
+                                                          idc.size))
+            self.n, self.ids, self.n_global = ids.shape[1], ids, ids.shape[1]
+            return
         q_global = np.asarray(q_global, dtype=np.float64).reshape(-1, 3)
         mine = np.nonzero(owner_of(q_global[:, 1], self.rows, self.world) == self.rank)[0].astype(np.int64)
         # stars are stored in 64x64-tile order (row-major over the tiles, stable inside a tile): consecutive warps of the
@@ -228,6 +272,12 @@ class BigFieldStrip:
         self.n, self.ids, self.n_global = len(q), ids, len(q)
 
     def get_stars(self):
+        """(q, p, grad) in storage order: [n,3] each, [K,n,3] with K > 1 chains."""
+        if self.chains > 1:
+            q, p, g = (np.zeros((self.chains, self.n, 3)) for _ in range(3))
+            for c in range(self.chains):
+                check(self._lib.srhmc_big_get_chain_stars(self._h, c, _capi.dptr(q[c]), _capi.dptr(p[c]), _capi.dptr(g[c])))
+            return q, p, g
         q, p, g = (np.zeros((self.n, 3)) for _ in range(3))
         check(self._lib.srhmc_big_get_stars(self._h, _capi.dptr(q), _capi.dptr(p), _capi.dptr(g)))
         return q, p, g
@@ -267,12 +317,21 @@ class BigFieldStrip:
         check(self._lib.srhmc_big_alloc_chains(self._h, n_iters))
 
     def read_chains(self, n_iters):
-        E, V, T = (np.zeros(n_iters) for _ in range(3))
-        A = np.zeros(n_iters, dtype=np.uint8)
-        nacc = C.c_double()
+        """E / V / T / A_chain [n_iters] and n_accepted; with K > 1 chains [K, n_iters] and [K]."""
         err = C.c_int32()
-        check(self._lib.srhmc_big_read_chains(self._h, n_iters, _capi.dptr(E), _capi.dptr(V), _capi.dptr(T),
-                                              _capi.bptr(A), C.byref(nacc), C.byref(err)))
+        if self.chains > 1:
+            E, V, T = (np.zeros((self.chains, n_iters)) for _ in range(3))
+            A = np.zeros((self.chains, n_iters), dtype=np.uint8)
+            nacc = np.zeros(self.chains)
+            check(self._lib.srhmc_big_read_chain_rows(self._h, n_iters, _capi.dptr(E), _capi.dptr(V), _capi.dptr(T),
+                                                      _capi.bptr(A), _capi.dptr(nacc), C.byref(err)))
+        else:
+            E, V, T = (np.zeros(n_iters) for _ in range(3))
+            A = np.zeros(n_iters, dtype=np.uint8)
+            acc = C.c_double()
+            check(self._lib.srhmc_big_read_chains(self._h, n_iters, _capi.dptr(E), _capi.dptr(V), _capi.dptr(T),
+                                                  _capi.bptr(A), C.byref(acc), C.byref(err)))
+            nacc = float(acc.value)
         if err.value == 1:
             raise RuntimeError("an owned star drifted out of the local data window (halo %d rows): re-partition "
                                "more often or enlarge the halo" % self.halo)
@@ -282,17 +341,22 @@ class BigFieldStrip:
             raise RuntimeError("more than 1024 stars touch one 64x64 tile: the fused tile evaluation cannot hold the list")
         if err.value == 4:
             raise RuntimeError("peer exchange timed out: a rank of the tiling never delivered its contribution")
-        return dict(E_chain=E, V_chain=V, T_chain=T, A_chain=A, n_accepted=float(nacc.value))
+        return dict(E_chain=E, V_chain=V, T_chain=T, A_chain=A, n_accepted=nacc)
 
     def set_recording(self, n_iters, stride=1, want=()):
         """Record the sample rows of the coming run (see srhmc_big_set_recording); want=() turns recording off."""
         want = record_want(want)
         check(self._lib.srhmc_big_set_recording(self._h, int(n_iters), int(stride), int("q" in want), int("p" in want)))
 
-    def read_samples(self, row0, nrows, want=("q",)):
-        """{name: [nrows, n, 3]} of recorded rows [row0, row0 + nrows), stars in slot order (`slot_ids(self.ids)`)."""
+    def read_samples(self, row0, nrows, want=("q",), chain=None):
+        """{name: [nrows, n, 3]} of recorded rows [row0, row0 + nrows), stars in slot order (`slot_ids(self.ids)`); with
+        K > 1 chains those of chain `chain`."""
         want = record_want(want)
         out = {w: np.empty((int(nrows), self.n, 3)) for w in want}
+        if self.chains > 1:
+            check(self._lib.srhmc_big_read_chain_samples(self._h, int(chain), int(row0), int(nrows), _capi.dptr(out.get("q")),
+                                                         _capi.dptr(out.get("p"))))
+            return out
         check(self._lib.srhmc_big_read_samples(self._h, int(row0), int(nrows), _capi.dptr(out.get("q")),
                                                _capi.dptr(out.get("p"))))
         return out
@@ -491,6 +555,15 @@ class BigFieldRHMC:
         self.multi = self.strips[0].world > 1
         self.fixed_point_mode = int(fixed_point_mode)
 
+    @property
+    def chains(self):
+        """K: the chains of the field each strip holds (BigFieldStrip(chains=K))."""
+        return self.strips[0].chains
+
+    def _one_chain(self, what):
+        if self.chains > 1:
+            raise ValueError("%s runs one chain: this engine holds %d (K chains run through run())" % (what, self.chains))
+
     def _step_struct(self, dt, delta, g_ff2, counter_max, f_pos, iteration, seed):
         return _capi.BigStep(dt=float(dt), delta=float(delta), g_ff2=float(g_ff2), counter_max=int(counter_max),
                              f_pos=int(bool(f_pos)), iteration=int(iteration),
@@ -502,6 +575,7 @@ class BigFieldRHMC:
 
     def evaluate(self, want_V=True, **kw):
         """One gradient (and potential) evaluation at the current star state."""
+        self._one_chain("evaluate")
         st = self._step_struct(kw.get("dt", 0.0), 1e-6, kw.get("g_ff2", 1.0), 1000, kw.get("f_pos", True), 0, 0)
         self._ghosts(st)
         self._all("EVAL_V" if want_V else "EVAL", st)
@@ -563,6 +637,7 @@ class BigFieldRHMC:
 
     def steps(self, nsteps, dt, delta=1e-6, counter_max=1000, g_ff2=1.0):
         """nsteps leapfrog steps from the current (q, p) (srhmc_step semantics)."""
+        self._one_chain("steps")
         st = self._step_struct(dt, delta, g_ff2, counter_max, True, 0, 0)
         self._ghosts(st)
         self._all("EVAL", st)
@@ -593,17 +668,24 @@ class BigFieldRHMC:
 
         use_graph: capture ONE Metropolis iteration (all its phases and, when tiled, its NCCL collectives) into a CUDA
         graph and replay it niter+1 times -- the chain row and RNG counter then come from a device-side iteration
-        counter.  Default: on for an untiled field without a g_ff2 schedule."""
+        counter.  Default: on for an untiled field without a g_ff2 schedule.
+
+        K > 1 chains (BigFieldStrip(chains=K)): chain c draws from Philox field c (chain 0 is the one-chain run), every
+        launch covers the K chains; E / V / T / A_chain are [K, L], n_accepted and accept_rate [K], q_chain / p_chain
+        [K, Ls, N_global, 3].  Injected normals / lnu need one chain."""
+        if self.chains > 1 and (normals is not None or lnu is not None):
+            raise ValueError("injected normals / lnu need one chain: K = %d chains draw from Philox fields 0..K-1" % self.chains)
         L = niter + 1
         want = record_want(want)
         Ls = record_rows(L, chain_stride)
         self._rj_graph_key = None   # set_recording below may move the buffers run_rj's captured graph writes
         # a change of the recording set-up may move its buffers: no graph captured before it may be replayed after it
-        rec = (want, int(chain_stride), L, tuple(s.n for s in self.strips))
+        rec = (want, int(chain_stride), L, tuple((s.n, s.layout) for s in self.strips))
         if rec != getattr(self, "_rec", None):
             self._graph_key = None
         for s in self.strips:
-            s.set_draws(None if normals is None else np.asarray(normals)[:, s.ids, :], lnu, L)
+            if s.chains == 1:
+                s.set_draws(None if normals is None else np.asarray(normals)[:, s.ids, :], lnu, L)
             s.alloc_chains(L)
             s.set_recording(L, chain_stride, want)
         self._rec = rec
@@ -681,6 +763,7 @@ class BigFieldRHMC:
         than max_stars stars is rejected; the run then raises ValueError, as the drop-in does, with the result dict as its
         `result` attribute.  use_graph: one captured
         iteration replayed niter+1 times (default: on for niter >= 2)."""
+        self._one_chain("run_rj")
         if self.multi or len(self.strips) != 1:
             raise ValueError("reversible-jump runs need the whole field on one device (world_size = 1)")
         if self.fixed_point_mode != 0:
@@ -762,8 +845,19 @@ class BigFieldRHMC:
         self._all("RJ_ACCEPT", st)
 
     def _samples(self, name, rows, chunk_bytes=256 << 20):
-        """Recorded rows of every strip hosted here in global-id order, downloaded in pieces of about `chunk_bytes`."""
+        """Recorded rows of every strip hosted here in global-id order, downloaded in pieces of about `chunk_bytes`
+        ([K, rows, N_global, 3] with K > 1 chains)."""
         n_global = self.strips[0].n_global
+        if self.chains > 1:
+            (s,) = self.strips
+            out = np.full((self.chains, rows, n_global, 3), np.nan)
+            step = max(1, chunk_bytes // max(1, 24 * s.n))
+            for c in range(self.chains):
+                cols = slot_ids(s.ids[c])
+                for r0 in range(0, rows, step):
+                    nr = min(step, rows - r0)
+                    out[c][r0:r0 + nr, cols, :] = s.read_samples(r0, nr, (name,), chain=c)[name]
+            return out
         out = np.full((rows, n_global, 3), np.nan)
         for s in self.strips:
             cols = slot_ids(s.ids)
@@ -775,12 +869,21 @@ class BigFieldRHMC:
 
     def energies(self):
         """(V, T) at the last EVAL_V + ENERGY of the strips hosted here (all of them, or world_size = 1)."""
+        self._one_chain("energies")
         sc = sum(s.read_scalars() for s in self.strips)
         V = np.inf if sc[2] > 0 else sc[0] + sc[3]
         return float(V), float(sc[1])
 
     def stars(self, n_global):
-        """(q, p, grad) of the stars hosted by this process scattered into global-id order (NaN elsewhere)."""
+        """(q, p, grad) of the stars hosted by this process scattered into global-id order (NaN elsewhere); [K, N, 3] each
+        with K > 1 chains."""
+        if self.chains > 1:
+            (s,) = self.strips
+            q, p, g = (np.full((self.chains, n_global, 3), np.nan) for _ in range(3))
+            a, b, c = s.get_stars()
+            for k in range(self.chains):
+                q[k, s.ids[k]], p[k, s.ids[k]], g[k, s.ids[k]] = a[k], b[k], c[k]
+            return q, p, g
         q = np.full((n_global, 3), np.nan)
         p = np.full((n_global, 3), np.nan)
         g = np.full((n_global, 3), np.nan)
@@ -794,8 +897,20 @@ def convergence_stats(engines, thin_rate=5, warm_up_num=0):
     """utils.convergence_stats (split-chain R-hat and n_eff, the reference's quirks kept) over the q rows that K >= 2 runs of
     the same field recorded on the device (`run(..., want=("q",))`): each engine is one chain, all hosted on one device with
     the same tiling and row count (different seeds or starts).  One variable-parallel kernel per strip; returns (R, n_eff),
-    each [N_global, 3] in global-id order, NaN for stars hosted by other processes."""
+    each [N_global, 3] in global-id order, NaN for stars hosted by other processes.  `engines` may also be ONE engine of
+    K >= 2 chains (BigFieldStrip(chains=K)): the statistics then cover its own chains."""
+    if isinstance(engines, BigFieldRHMC):
+        engines = [engines]
     engines = list(engines)
+    if len(engines) == 1 and engines[0].chains > 1:
+        (s,) = engines[0].strips
+        r, ne = np.empty(3 * s.n), np.empty(3 * s.n)
+        check(s._lib.srhmc_big_chain_convergence_stats(s._h, int(thin_rate), int(warm_up_num), _capi.dptr(r), _capi.dptr(ne)))
+        R = np.full((s.n_global, 3), np.nan)
+        n_eff = np.full((s.n_global, 3), np.nan)
+        cols = slot_ids(s.ids[0])
+        R[cols], n_eff[cols] = r.reshape(-1, 3), ne.reshape(-1, 3)
+        return R, n_eff
     if len(engines) < 2:
         raise ValueError("convergence statistics need at least two chains (utils.py:94)")
     nstrips = len(engines[0].strips)

@@ -68,11 +68,28 @@ struct BigParams {
     int use_prior;
     double inv2s2, inv_s2, norm;
     FieldParams F;          // constants for metric_of (B, g0.., f_low, f_lim, alpha, Vpc)
+    // Chain axis (srhmc_big_set_chains): chain c = blockIdx.y of a launch works on slice c of every per-chain buffer.  The
+    // slices' lengths in elements; a one-chain launch has blockIdx.y = 0 and never needs them.
+    struct {
+        long long M;        // max_stars: q, p, g, a1, q0, g0 hold 3 M doubles per chain, a2 4 M + 1, gpart 12 M; gid, slot M
+        long long tiles;    // tcnt: tiles ints per chain; tlist: tiles kTileMaxList records
+        long long vpart;    // pixel-potential partials
+        long long rows;     // E, V, T, A: the iterations of srhmc_big_alloc_chains
+        long long rec;      // recorded q / p rows: rec_rows 3 rec_n doubles
+    } X;
 };
 
 constexpr int kMaxRad = 15;
 constexpr int kScalars = 8;   // [0] V partial, [1] T partial, [2] bad count, [3] spare ... (doubles)
 constexpr int kVBlocks = 1024;
+constexpr int kStateLen = 8;  // doubles of a chain's state: [0] E0, [1] pixel potential at the start, [2] accepted, [3] count
+constexpr int kMaxChains = 64;
+
+// Slice of chain blockIdx.y of a per-chain buffer whose chains are `stride` elements apart (null stays null)
+template <typename T>
+__device__ __forceinline__ T* chain_slice(T* p, long long stride) {
+    return p ? p + blockIdx.y * stride : p;
+}
 
 // ------------------------------------------------------------------------------------------------ pixel kernels
 __global__ void big_fill_kernel(double* L, size_t n, double B) {
@@ -478,6 +495,10 @@ template <bool LAST_HALF, bool NEXT_FIRST, bool LIVE>
 __global__ void big_kick_kernel(const BigParams P, const BigStep S, int n, const double* q, double* p, double* g,
                                 const double* gpart, double* a1, double* a2, int* cnt, const PeerX X, const int* nd) {
     if (LIVE) n = *nd;
+    q += blockIdx.y * 3 * P.X.M; p += blockIdx.y * 3 * P.X.M; g += blockIdx.y * 3 * P.X.M; a1 += blockIdx.y * 3 * P.X.M;
+    a2 += blockIdx.y * (4 * P.X.M + 1);
+    gpart = chain_slice(gpart, 12 * P.X.M);
+    cnt += blockIdx.y;
     int local_max = 0;
     for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += gridDim.x * blockDim.x) {
         const Star3 s = load3(q, k);
@@ -507,6 +528,10 @@ __global__ void big_kick_kernel(const BigParams P, const BigStep S, int n, const
 template <bool LIVE>
 __global__ void big_pfix_qfix_kernel(const BigParams P, const BigStep S, int n, double* q, double* p, double* a1, double* a2,
                                      const int* cnt_p, int* cnt_q, const PeerX X, const int* nd) {
+    q += blockIdx.y * 3 * P.X.M; p += blockIdx.y * 3 * P.X.M; a1 += blockIdx.y * 3 * P.X.M;
+    a2 += blockIdx.y * (4 * P.X.M + 1);
+    cnt_p += blockIdx.y;
+    cnt_q += blockIdx.y;
     const int target = S.per_star ? 0 : *cnt_p;
     const int nk = LIVE ? *nd : n;   // n: the layout of own_qcount
     int local_max = 0;
@@ -536,6 +561,11 @@ __global__ void big_qfix_kick_kernel(const BigParams P, const BigStep S, int n, 
                                      const double* a2, const int* cnt_q, int ntx, int* tcnt, PairRec* tlist, int* err,
                                      int2* pack_counts, double lo_edge, double hi_edge, double* Lfill, size_t npix, const int* nd) {
     fill_background(P, Lfill, npix);
+    q += blockIdx.y * 3 * P.X.M; p += blockIdx.y * 3 * P.X.M; a1 += blockIdx.y * 3 * P.X.M;
+    a2 += blockIdx.y * (4 * P.X.M + 1);
+    cnt_q += blockIdx.y;
+    tcnt = chain_slice(tcnt, P.X.tiles);
+    tlist = chain_slice(tlist, P.X.tiles * kTileMaxList);
     const int target = S.per_star ? 0 : *cnt_q;
     const int nk = LIVE ? *nd : n;   // n: the layout of own_qcount
     for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < nk; k += gridDim.x * blockDim.x) {
@@ -558,6 +588,10 @@ __global__ void big_perstar_kernel(const BigParams P, const BigStep S, int n, do
                                    int ntx, int* tcnt, PairRec* tlist, int* err, int2* pack_counts, double lo_edge, double hi_edge,
                                    double* Lfill, size_t npix) {
     fill_background(P, Lfill, npix);
+    q += blockIdx.y * 3 * P.X.M; p += blockIdx.y * 3 * P.X.M; g += blockIdx.y * 3 * P.X.M;
+    gpart = chain_slice(gpart, 12 * P.X.M);
+    tcnt = chain_slice(tcnt, P.X.tiles);
+    tlist = chain_slice(tlist, P.X.tiles * kTileMaxList);
     for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += gridDim.x * blockDim.x) {
         const Star3 sg = load3(q, k);
         const Star3 gr = star_grad(P, k, sg, FROM_EVAL ? gpart : nullptr, g);
@@ -589,13 +623,17 @@ __global__ void big_momentum_kernel(const BigParams P, double g_ff2, int n, cons
     const int iter = iter_dev ? *iter_dev : iter_host;
     const double* normals = normals_all ? normals_all + (size_t)iter * n * 3 : nullptr;
     const int nk = LIVE ? *nd : n;   // n: the row length of the normals
+    // chain c draws from Philox field c (chain 0: the one-chain engine's field 0)
+    q += blockIdx.y * 3 * P.X.M; p += blockIdx.y * 3 * P.X.M; g += blockIdx.y * 3 * P.X.M;
+    q0 += blockIdx.y * 3 * P.X.M; g0 += blockIdx.y * 3 * P.X.M;
+    gid += blockIdx.y * P.X.M;
     for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < nk; k += gridDim.x * blockDim.x) {
         const Metric m = metric_of(P.F, q[3 * k], g_ff2);
         double z[3];
         if (normals) {
             z[0] = normals[3 * k]; z[1] = normals[3 * k + 1]; z[2] = normals[3 * k + 2];
         } else {
-            philox_normals3(seed, 0u, (uint32_t)iter, (uint32_t)gid[k], z);
+            philox_normals3(seed, blockIdx.y, (uint32_t)iter, (uint32_t)gid[k], z);
         }
         p[3 * k] = z[0] * sqrt(m.Hff);
         p[3 * k + 1] = z[1] * sqrt(m.Hxx);
@@ -617,6 +655,10 @@ __global__ void big_energy_kernel(const BigParams P, double g_ff2, int f_pos, in
     __shared__ double red[4 * 32];
     __shared__ bool is_last;
     if (LIVE) n = *nd;
+    q += blockIdx.y * 3 * P.X.M; p += blockIdx.y * 3 * P.X.M;
+    part += blockIdx.y * 4 * kEnergyBlocks;
+    ticket += blockIdx.y * 2;
+    scalars += blockIdx.y * kScalars;
     double v[4] = {0, 0, 0, 0};
     for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += gridDim.x * blockDim.x) {
         const double f = q[3 * k], x = q[3 * k + 1], y = q[3 * k + 2];
@@ -645,14 +687,20 @@ __global__ void big_energy_kernel(const BigParams P, double g_ff2, int f_pos, in
 }
 
 // E = V + T from the (all-reduced) scalars: slot 4 <- E (kept as E0 when `first`), accept test otherwise
-__global__ void big_accept_kernel(int phase /*0: record E0, 1: accept*/, const double* scalars /* global sums */,
+__global__ void big_accept_kernel(const BigParams P, int phase /*0: record E0, 1: accept*/, const double* scalars /* global sums */,
                                   const double* local_scalars, double* state,
                                   unsigned long long seed, int iter_host, const int* iter_dev, const double* lnu_in, int n,
                                   double* q, double* g,
                                   const double* q0, const double* g0, double* E_chain, double* V_chain, double* T_chain,
                                   unsigned char* A_chain) {
-    // every thread evaluates the same scalars; thread 0 of block 0 writes the records
+    // every thread evaluates the same scalars; thread 0 of block 0 writes the records.  Chain c (blockIdx.y) takes log u
+    // from Philox field c.
     const int iter = iter_dev ? *iter_dev : iter_host;
+    scalars += blockIdx.y * kScalars; local_scalars += blockIdx.y * kScalars;
+    state += blockIdx.y * kStateLen;
+    q += blockIdx.y * 3 * P.X.M; g += blockIdx.y * 3 * P.X.M; q0 += blockIdx.y * 3 * P.X.M; g0 += blockIdx.y * 3 * P.X.M;
+    E_chain = chain_slice(E_chain, P.X.rows); V_chain = chain_slice(V_chain, P.X.rows); T_chain = chain_slice(T_chain, P.X.rows);
+    A_chain = chain_slice(A_chain, P.X.rows);
     const double V = (scalars[2] > 0.0) ? CUDART_INF : scalars[0] + scalars[3];
     const double T = scalars[1];
     const double E = V + T;
@@ -667,7 +715,7 @@ __global__ void big_accept_kernel(int phase /*0: record E0, 1: accept*/, const d
         return;
     }
     const double dE = E - state[0];
-    const double lnu = lnu_in ? lnu_in[iter] : philox_lnu(seed, 0u, (uint32_t)iter);
+    const double lnu = lnu_in ? lnu_in[iter] : philox_lnu(seed, blockIdx.y, (uint32_t)iter);
     const bool accept = (dE < 0.0) || (lnu < -dE);
     if (!accept) {
         for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < 3 * n; i += gridDim.x * blockDim.x) {
@@ -682,10 +730,11 @@ __global__ void big_accept_kernel(int phase /*0: record E0, 1: accept*/, const d
     }
 }
 // the pixel potential must follow the state on rejection: separate tiny kernel so that it runs after every block of
-// big_accept_kernel has read scalars[0]
+// big_accept_kernel has read scalars[0].  Thread c restores chain c; the shared iteration counter advances once.
 __global__ void big_restore_v_kernel(double* local_scalars, const double* state, int* iter_dev) {
-    if (state[2] == 0.0) local_scalars[0] = state[1];
-    if (iter_dev) *iter_dev += 1;  // the next replay of a captured iteration works on the next chain row
+    const int c = threadIdx.x;
+    if (state[kStateLen * c + 2] == 0.0) local_scalars[kScalars * c] = state[kStateLen * c + 1];
+    if (iter_dev && c == 0) *iter_dev += 1;  // the next replay of a captured iteration works on the next chain row
 }
 
 // Sample row of the iteration (RECORD_E0: q before the trajectory, p just drawn by MOMENTUM) when the iteration is a multiple of
@@ -693,12 +742,14 @@ __global__ void big_restore_v_kernel(double* local_scalars, const double* state,
 // do not depend on the storage order.  One thread per coordinate: coalesced reads, the three coordinates of a star together.
 // With a live count (reversible-jump mode: n = max_stars, slots in table order) the rows are zero past it.
 template <bool LIVE>
-__global__ void big_record_kernel(int n, const double* q, const double* p, const int* slot, int iter_host, const int* iter_dev,
-                                  int stride, int rows, double* rec_q, double* rec_p, const int* nd) {
+__global__ void big_record_kernel(const BigParams P, int n, const double* q, const double* p, const int* slot, int iter_host,
+                                  const int* iter_dev, int stride, int rows, double* rec_q, double* rec_p, const int* nd) {
     const int iter = iter_dev ? *iter_dev : iter_host;
     if (iter < 0 || iter % stride) return;
     const int r = iter / stride;
     if (r >= rows) return;
+    q += blockIdx.y * 3 * P.X.M; p += blockIdx.y * 3 * P.X.M; slot += blockIdx.y * P.X.M;
+    rec_q = chain_slice(rec_q, P.X.rec); rec_p = chain_slice(rec_p, P.X.rec);
     const size_t row = (size_t)r * 3 * n;
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < 3 * n; i += gridDim.x * blockDim.x) {
         const size_t o = row + 3 * (size_t)slot[i / 3] + i % 3;
@@ -953,6 +1004,14 @@ struct srhmc_big {
     int rec_rows = 0, rec_stride = 1, rec_n = 0;
     int nty = 0, ntx = 0;
     bool use_tiles = false;
+    bool use_tiles_created = false;   // the evaluation path srhmc_big_create chose (srhmc_big_set_chains(1) returns to it)
+    // chain axis (srhmc_big_set_chains): K chains of this field, each with its own slice of the per-chain buffers (P.X) and
+    // its own stars (chain_n, chain_ids: sorted ids per chain); chains_ok: the chains' id sets were checked equal since the
+    // last srhmc_big_set_chain_stars, and n / sorted_ids are theirs
+    int chains = 1;
+    std::vector<int> chain_n;
+    std::vector<std::vector<int64_t>> chain_ids;
+    bool chains_ok = true;
     int precision = 64;        // 32: gradient-only evaluations run the FP32 tile kernel on a float copy of the data
     BBuf D32;
     CUtensorMap tmapD32{};
@@ -1052,6 +1111,23 @@ int enqueue_eval(srhmc_big* b, bool want_V, const double** gpart, int n, const i
     TileSrc S;
     S.q = b->q.as<double>(); S.ga = ga; S.gb = gb; S.n_own = n; S.cap = std::max(1, b->cfg.max_ghosts);
     const int ntiles = b->nty * b->ntx;
+    const int K = b->chains;
+    if (K > 1) {   // every chain on the tile kernel (srhmc_big_set_chains): one launch of each kernel covers them all
+        if (!b->own_binned && n > 0) {
+            big_bin_kernel<false><<<dim3(std::max(1, std::min((n + 255) / 256, 8 * b->sm_count)), K), 256, 0, st>>>(
+                P, S, b->ntx, 0, n, b->tcnt.as<int>(), b->tlist.as<PairRec>(), b->err.as<int>(), nullptr);
+            b->launches += 1;
+        }
+        b->own_binned = false;
+        const auto tile = want_V ? big_tile_kernel<1, true> : big_tile_kernel<0, true>;
+        tile<<<dim3(ntiles, K), kTileThreads, sizeof(TileSmem), st>>>(P, S, b->ntx, b->D.as<double>(), b->tcnt.as<int>(),
+                                                                     b->tlist.as<PairRec>(), b->gpart.as<double>(), b->vpart.as<double>(),
+                                                                     b->tickets.as<unsigned int>() + 1, b->scalars.as<double>(), cnt,
+                                                                     nullptr, 0ull, b->tmapD, b->tma ? 1 : 0);
+        b->launches += 1;
+        *gpart = b->gpart.as<double>();
+        return 0;
+    }
     if (!b->own_binned && n > 0) {
         (nd ? big_bin_kernel<true> : big_bin_kernel<false>)<<<std::max(1, std::min((n + 255) / 256, 8 * b->sm_count)), 256, 0, st>>>(
             P, S, b->ntx, 0, n, b->tcnt.as<int>(), b->tlist.as<PairRec>(), b->err.as<int>(), nd);
@@ -1085,6 +1161,24 @@ int enqueue_eval(srhmc_big* b, bool want_V, const double** gpart, int n, const i
     }
     b->launches += 1;
     *gpart = b->gpart.as<double>();
+    return 0;
+}
+
+// an entry point that takes one chain's arrays, on a context of K > 1 chains
+int refuse_chains(const srhmc_big* b, const char* instead) {
+    return bfail(SRHMC_ERR_STATE, "this context holds %d chains: use %s", b->chains, instead);
+}
+
+// K > 1: every chain must carry the same star ids (the columns of the recorded rows line up across chains); n and
+// sorted_ids become theirs.  Checked once after a change of a chain's stars.
+int chains_agree(srhmc_big* b) {
+    if (b->chains_ok) return 0;
+    for (int c = 1; c < b->chains; ++c)
+        if (b->chain_n[c] != b->chain_n[0] || b->chain_ids[c] != b->chain_ids[0])
+            return bfail(SRHMC_ERR_STATE, "chain %d holds other star ids than chain 0: the chains of a context carry the same stars", c);
+    b->n = b->chain_n[0];
+    b->sorted_ids = b->chain_ids[0];
+    b->chains_ok = true;
     return 0;
 }
 
@@ -1143,6 +1237,10 @@ int srhmc_big_create(const srhmc_big_config* cfg, srhmc_big** out) {
         if (!std::strcmp(e, "tile")) b->use_tiles = true;
         else if (!std::strcmp(e, "scatter")) b->use_tiles = false;
     }
+    b->use_tiles_created = b->use_tiles;
+    P.X.M = cfg->max_stars;
+    P.X.tiles = (long long)ntiles;
+    P.X.vpart = (long long)std::max<size_t>(kVBlocks, ntiles);
     int rc = 0;
     rc |= b->D.ensure(npix * 8);
     if (!b->use_tiles) rc |= b->L.ensure(npix * 8);
@@ -1245,6 +1343,7 @@ int srhmc_big_set_data(srhmc_big* b, const double* D_local) {
 int srhmc_big_set_precision(srhmc_big* b, int32_t precision) {
     // 32: gradient-only evaluations through the FP32 tile kernel (float copy of the data, TMA); 64: everything FP64
     if (!b || (precision != 32 && precision != 64)) return bfail(SRHMC_ERR_INVALID, "precision must be 64 or 32");
+    if (precision == 32 && b->chains > 1) return bfail(SRHMC_ERR_STATE, "K chains run the FP64 tile kernel: precision 32 needs one chain");
     BCU(cudaSetDevice(b->cfg.device));
     if (precision == 32) {
         if (!b->use_tiles || !b->tma)
@@ -1284,7 +1383,7 @@ int srhmc_big_mock_data(srhmc_big* b, const double* q_true, int32_t n, uint64_t 
     const double cnt = (double)n;
     cudaError_t e = cudaMemcpyAsync(truth.ptr, &cnt, 8, cudaMemcpyHostToDevice, st);
     if (e == cudaSuccess && n) e = cudaMemcpyAsync(truth.as<double>() + 1, q_true, (size_t)n * 24, cudaMemcpyHostToDevice, st);
-    if (e == cudaSuccess) e = cudaMemsetAsync(b->tcnt.ptr, 0, ntiles * 4, st);
+    if (e == cudaSuccess) e = cudaMemsetAsync(b->tcnt.ptr, 0, b->tcnt.cap, st);   // every chain's lists
     b->own_binned = false;
     if (e == cudaSuccess) {
         TileSrc S;
@@ -1315,9 +1414,17 @@ int srhmc_big_mock_data(srhmc_big* b, const double* q_true, int32_t n, uint64_t 
 }
 
 int srhmc_big_set_stars(srhmc_big* b, const double* q, const int64_t* global_ids, int32_t n) {
+    if (!b) return bfail(SRHMC_ERR_INVALID, "null argument");
+    if (b->chains > 1) return refuse_chains(b, "srhmc_big_set_chain_stars");
+    return srhmc_big_set_chain_stars(b, 0, q, global_ids, n);
+}
+
+int srhmc_big_set_chain_stars(srhmc_big* b, int32_t chain, const double* q, const int64_t* global_ids, int32_t n) {
     if (!b || (n > 0 && (!q || !global_ids))) return bfail(SRHMC_ERR_INVALID, "null argument");
     if (n < 0 || n > b->cfg.max_stars) return bfail(SRHMC_ERR_INVALID, "%d stars exceed max_stars = %d", n, b->cfg.max_stars);
+    if (chain < 0 || chain >= b->chains) return bfail(SRHMC_ERR_INVALID, "chain %d outside the context's %d chains", chain, b->chains);
     BCU(cudaSetDevice(b->cfg.device));
+    const size_t M = (size_t)b->cfg.max_stars;
     // slot of a star = rank of its id among the strip's ids: the position of its column in a recorded sample row
     std::vector<int32_t> order(n), slots(n);
     std::iota(order.begin(), order.end(), 0);
@@ -1328,13 +1435,13 @@ int srhmc_big_set_stars(srhmc_big* b, const double* q, const int64_t* global_ids
         sorted[r] = global_ids[order[r]];
     }
     if (n) {
-        BCU(cudaMemcpyAsync(b->q.ptr, q, (size_t)n * 24, cudaMemcpyHostToDevice, b->stream));
-        BCU(cudaMemcpyAsync(b->gid.ptr, global_ids, (size_t)n * 8, cudaMemcpyHostToDevice, b->stream));
-        BCU(cudaMemcpyAsync(b->slot.ptr, slots.data(), (size_t)n * 4, cudaMemcpyHostToDevice, b->stream));
+        BCU(cudaMemcpyAsync(b->q.as<double>() + chain * 3 * M, q, (size_t)n * 24, cudaMemcpyHostToDevice, b->stream));
+        BCU(cudaMemcpyAsync(b->gid.as<int64_t>() + chain * M, global_ids, (size_t)n * 8, cudaMemcpyHostToDevice, b->stream));
+        BCU(cudaMemcpyAsync(b->slot.as<int32_t>() + chain * M, slots.data(), (size_t)n * 4, cudaMemcpyHostToDevice, b->stream));
     }
-    BCU(cudaMemsetAsync(b->p.ptr, 0, 3 * (size_t)b->cfg.max_stars * 8, b->stream));
+    BCU(cudaMemsetAsync(b->p.as<double>() + chain * 3 * M, 0, 3 * M * 8, b->stream));
     if (b->own_binned || b->ghosts_binned) {  // records of the previous positions
-        BCU(cudaMemsetAsync(b->tcnt.ptr, 0, (size_t)b->nty * b->ntx * 4, b->stream));
+        BCU(cudaMemsetAsync(b->tcnt.ptr, 0, (size_t)b->chains * b->nty * b->ntx * 4, b->stream));
         b->own_binned = false;
         b->ghosts_binned = false;
     }
@@ -1343,25 +1450,96 @@ int srhmc_big_set_stars(srhmc_big* b, const double* q, const int64_t* global_ids
         b->pack_counted = false;
     }
     BCU(cudaStreamSynchronize(b->stream));
-    b->n = n;
-    b->sorted_ids.swap(sorted);
+    if (b->chains == 1) {
+        b->n = n;
+        b->sorted_ids.swap(sorted);
+        return 0;
+    }
+    b->chain_n[chain] = n;
+    b->chain_ids[chain].swap(sorted);
+    b->chains_ok = false;
     return 0;
 }
 
 int srhmc_big_get_stars(srhmc_big* b, double* q, double* p, double* grad) {
     if (!b) return bfail(SRHMC_ERR_INVALID, "null context");
+    if (b->chains > 1) return refuse_chains(b, "srhmc_big_get_chain_stars");
+    return srhmc_big_get_chain_stars(b, 0, q, p, grad);
+}
+
+int srhmc_big_get_chain_stars(srhmc_big* b, int32_t chain, double* q, double* p, double* grad) {
+    if (!b) return bfail(SRHMC_ERR_INVALID, "null context");
+    if (chain < 0 || chain >= b->chains) return bfail(SRHMC_ERR_INVALID, "chain %d outside the context's %d chains", chain, b->chains);
     BCU(cudaSetDevice(b->cfg.device));
-    if (b->n) {
-        if (q) BCU(cudaMemcpyAsync(q, b->q.ptr, (size_t)b->n * 24, cudaMemcpyDeviceToHost, b->stream));
-        if (p) BCU(cudaMemcpyAsync(p, b->p.ptr, (size_t)b->n * 24, cudaMemcpyDeviceToHost, b->stream));
-        if (grad) BCU(cudaMemcpyAsync(grad, b->g.ptr, (size_t)b->n * 24, cudaMemcpyDeviceToHost, b->stream));
+    const size_t n = b->chains > 1 ? (size_t)b->chain_n[chain] : (size_t)b->n, off = (size_t)chain * 3 * b->cfg.max_stars;
+    if (n) {
+        if (q) BCU(cudaMemcpyAsync(q, b->q.as<double>() + off, n * 24, cudaMemcpyDeviceToHost, b->stream));
+        if (p) BCU(cudaMemcpyAsync(p, b->p.as<double>() + off, n * 24, cudaMemcpyDeviceToHost, b->stream));
+        if (grad) BCU(cudaMemcpyAsync(grad, b->g.as<double>() + off, n * 24, cudaMemcpyDeviceToHost, b->stream));
     }
     BCU(cudaStreamSynchronize(b->stream));
     return 0;
 }
 
+int srhmc_big_set_chains(srhmc_big* b, int32_t k) {
+    if (!b) return bfail(SRHMC_ERR_INVALID, "null context");
+    if (k < 1 || k > kMaxChains) return bfail(SRHMC_ERR_INVALID, "%d chains: a context holds 1..%d", k, kMaxChains);
+    if (k > 1 && b->world > 1)
+        return bfail(SRHMC_ERR_INVALID, "K chains need the whole field on one device: this context is a strip of %d", b->world);
+    if (k > 1 && b->precision != 64) return bfail(SRHMC_ERR_STATE, "K chains run the FP64 tile kernel: the context is at precision 32");
+    if (b->rj_on) return bfail(SRHMC_ERR_STATE, "the context is in reversible-jump mode (srhmc_big_rj_finish first)");
+    BCU(cudaSetDevice(b->cfg.device));
+    BCU(cudaStreamSynchronize(b->stream));
+    // K > 1 always runs the tile kernel (the scatter path would need K model images); one chain returns to the created path
+    const bool tiles = k > 1 || b->use_tiles_created;
+    const size_t K = (size_t)k, M = (size_t)b->cfg.max_stars, NT = (size_t)b->P.X.tiles, S = 3 * M;
+    BBuf* per[] = {&b->q, &b->p, &b->g, &b->a1, &b->a2, &b->q0, &b->g0, &b->gid, &b->slot, &b->gpart, &b->tcnt, &b->tlist,
+                   &b->vpart, &b->scalars, &b->gscalars, &b->state, &b->counters, &b->epart, &b->tickets, &b->E, &b->V, &b->T,
+                   &b->A, &b->recq, &b->recp, &b->normals, &b->lnu};
+    for (BBuf* x : per) x->release();
+    int rc = 0;
+    rc |= b->q.ensure(K * S * 8); rc |= b->p.ensure(K * S * 8); rc |= b->g.ensure(K * S * 8); rc |= b->a1.ensure(K * S * 8);
+    rc |= b->a2.ensure(K * (4 * M + 1) * 8); rc |= b->q0.ensure(K * S * 8); rc |= b->g0.ensure(K * S * 8);
+    rc |= b->gid.ensure(K * M * 8); rc |= b->slot.ensure(K * M * 4);
+    rc |= b->vpart.ensure(K * (size_t)b->P.X.vpart * 8);
+    rc |= b->scalars.ensure(K * kScalars * 8); rc |= b->gscalars.ensure(K * kScalars * 8); rc |= b->state.ensure(K * kStateLen * 8);
+    rc |= b->counters.ensure((2 * K + 2) * 4); rc |= b->epart.ensure(K * kEnergyBlocks * 4 * 8); rc |= b->tickets.ensure(K * 2 * 4);
+    if (tiles) {
+        rc |= b->tcnt.ensure(K * NT * 4);
+        rc |= b->tlist.ensure(K * NT * (size_t)kTileMaxList * sizeof(PairRec));
+        rc |= b->gpart.ensure(K * 12 * M * 8);
+    }
+    if (rc) {
+        cudaGetLastError();
+        return bfail(SRHMC_ERR_CUDA, "cannot allocate the buffers of %d chains of %zu stars", k, M);
+    }
+    BCU(cudaMemset(b->scalars.ptr, 0, b->scalars.cap));
+    BCU(cudaMemset(b->gscalars.ptr, 0, b->gscalars.cap));
+    BCU(cudaMemset(b->state.ptr, 0, b->state.cap));
+    BCU(cudaMemset(b->counters.ptr, 0, b->counters.cap));
+    BCU(cudaMemset(b->tickets.ptr, 0, b->tickets.cap));
+    if (tiles) BCU(cudaMemset(b->tcnt.ptr, 0, b->tcnt.cap));
+    if (k > 1) {
+        BCU(cudaFuncSetAttribute(big_tile_kernel<0, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(TileSmem)));
+        BCU(cudaFuncSetAttribute(big_tile_kernel<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(TileSmem)));
+        if (!b->tma && (b->cfg.cols % 2) == 0) b->tma = encode_tile_map(&b->tmapD, b->D.ptr, b->cfg.nrows, b->cfg.cols, 8);
+    }
+    b->use_tiles = tiles;
+    b->chains = k;
+    b->chain_n.assign(K, 0);
+    b->chain_ids.assign(K, std::vector<int64_t>());
+    b->chains_ok = true;
+    b->n = 0;
+    b->sorted_ids.clear();
+    b->rec_rows = 0;
+    b->P.X.rows = b->P.X.rec = 0;
+    b->own_binned = b->ghosts_binned = b->pack_counted = b->L_filled = false;
+    return 0;
+}
+
 int srhmc_big_set_momenta(srhmc_big* b, const double* p) {
     if (!b || !p) return bfail(SRHMC_ERR_INVALID, "null argument");
+    if (b->chains > 1) return refuse_chains(b, "the device's momentum draws (srhmc_big_set_chain_stars starts every chain at p = 0)");
     BCU(cudaSetDevice(b->cfg.device));
     if (b->n) BCU(cudaMemcpyAsync(b->p.ptr, p, (size_t)b->n * 24, cudaMemcpyHostToDevice, b->stream));
     BCU(cudaStreamSynchronize(b->stream));
@@ -1451,6 +1629,7 @@ int srhmc_big_set_draws(srhmc_big* b, const double* normals, const double* lnu, 
     // normals [n_iters, n, 3] for the owned stars (parity mode; reversible-jump mode: [n_iters, max_stars, 3] in table order)
     // and lnu [n_iters]; either may be NULL (device Philox)
     if (!b || n_iters < 0) return bfail(SRHMC_ERR_INVALID, "bad argument");
+    if (b->chains > 1) return refuse_chains(b, "the device's Philox draws (chain c draws from field c)");
     BCU(cudaSetDevice(b->cfg.device));
     b->normals.release();
     b->lnu.release();
@@ -1470,20 +1649,23 @@ int srhmc_big_set_draws(srhmc_big* b, const double* normals, const double* lnu, 
 int srhmc_big_alloc_chains(srhmc_big* b, int32_t n_iters) {
     if (!b || n_iters < 1) return bfail(SRHMC_ERR_INVALID, "bad argument");
     BCU(cudaSetDevice(b->cfg.device));
-    if (int rc = b->E.ensure((size_t)n_iters * 8)) return rc;
-    if (int rc = b->V.ensure((size_t)n_iters * 8)) return rc;
-    if (int rc = b->T.ensure((size_t)n_iters * 8)) return rc;
-    if (int rc = b->A.ensure((size_t)n_iters)) return rc;
-    BCU(cudaMemsetAsync(b->E.ptr, 0, (size_t)n_iters * 8, b->stream));
-    BCU(cudaMemsetAsync(b->V.ptr, 0, (size_t)n_iters * 8, b->stream));
-    BCU(cudaMemsetAsync(b->T.ptr, 0, (size_t)n_iters * 8, b->stream));
-    BCU(cudaMemsetAsync(b->A.ptr, 0, (size_t)n_iters, b->stream));
-    BCU(cudaMemsetAsync(b->state.ptr, 0, 64, b->stream));
+    const size_t rows = (size_t)b->chains * n_iters;   // [chain][iteration]
+    if (int rc = b->E.ensure(rows * 8)) return rc;
+    if (int rc = b->V.ensure(rows * 8)) return rc;
+    if (int rc = b->T.ensure(rows * 8)) return rc;
+    if (int rc = b->A.ensure(rows)) return rc;
+    BCU(cudaMemsetAsync(b->E.ptr, 0, rows * 8, b->stream));
+    BCU(cudaMemsetAsync(b->V.ptr, 0, rows * 8, b->stream));
+    BCU(cudaMemsetAsync(b->T.ptr, 0, rows * 8, b->stream));
+    BCU(cudaMemsetAsync(b->A.ptr, 0, rows, b->stream));
+    BCU(cudaMemsetAsync(b->state.ptr, 0, (size_t)b->chains * kStateLen * 8, b->stream));
+    b->P.X.rows = n_iters;
     return 0;
 }
 
 int srhmc_big_rj_configure(srhmc_big* b, const srhmc_rj_args* rj, int32_t n_iters) {
     if (!b || !rj) return bfail(SRHMC_ERR_INVALID, "null argument");
+    if (b->chains > 1) return refuse_chains(b, "one chain per context for reversible-jump runs (srhmc_big_set_chains(b, 1))");
     if (n_iters < 1) return bfail(SRHMC_ERR_INVALID, "n_iters must be >= 1");
     if (b->world > 1)
         return bfail(SRHMC_ERR_INVALID, "reversible-jump runs need the whole field on one device: this context is a strip of %d", b->world);
@@ -1574,6 +1756,7 @@ int srhmc_big_rj_finish(srhmc_big* b, int32_t n_iters, const srhmc_rj_args* out)
 int srhmc_big_read_chains(srhmc_big* b, int32_t n_iters, double* E, double* V, double* T, uint8_t* A, double* n_accepted,
                           int32_t* error_flag) {
     if (!b) return bfail(SRHMC_ERR_INVALID, "null context");
+    if (b->chains > 1) return refuse_chains(b, "srhmc_big_read_chain_rows");
     BCU(cudaSetDevice(b->cfg.device));
     if (E) BCU(cudaMemcpyAsync(E, b->E.ptr, (size_t)n_iters * 8, cudaMemcpyDeviceToHost, b->stream));
     if (V) BCU(cudaMemcpyAsync(V, b->V.ptr, (size_t)n_iters * 8, cudaMemcpyDeviceToHost, b->stream));
@@ -1585,6 +1768,30 @@ int srhmc_big_read_chains(srhmc_big* b, int32_t n_iters, double* E, double* V, d
     BCU(cudaMemcpyAsync(&err, b->err.ptr, 4, cudaMemcpyDeviceToHost, b->stream));
     BCU(cudaStreamSynchronize(b->stream));
     if (n_accepted) *n_accepted = st[3];
+    if (error_flag) *error_flag = err;
+    return 0;
+}
+
+int srhmc_big_read_chain_rows(srhmc_big* b, int32_t n_iters, double* E, double* V, double* T, uint8_t* A, double* n_accepted,
+                              int32_t* error_flag) {
+    if (!b) return bfail(SRHMC_ERR_INVALID, "null context");
+    if (n_iters < 0 || n_iters > b->P.X.rows) return bfail(SRHMC_ERR_INVALID, "%d iterations, %lld allocated", n_iters, b->P.X.rows);
+    BCU(cudaSetDevice(b->cfg.device));
+    const int K = b->chains;
+    const size_t L = (size_t)n_iters, rows = (size_t)b->P.X.rows;
+    for (int c = 0; c < K && L; ++c) {
+        if (E) BCU(cudaMemcpyAsync(E + c * L, b->E.as<double>() + c * rows, L * 8, cudaMemcpyDeviceToHost, b->stream));
+        if (V) BCU(cudaMemcpyAsync(V + c * L, b->V.as<double>() + c * rows, L * 8, cudaMemcpyDeviceToHost, b->stream));
+        if (T) BCU(cudaMemcpyAsync(T + c * L, b->T.as<double>() + c * rows, L * 8, cudaMemcpyDeviceToHost, b->stream));
+        if (A) BCU(cudaMemcpyAsync(A + c * L, b->A.as<uint8_t>() + c * rows, L, cudaMemcpyDeviceToHost, b->stream));
+    }
+    std::vector<double> st((size_t)K * kStateLen);
+    int err = 0;
+    BCU(cudaMemcpyAsync(st.data(), b->state.ptr, st.size() * 8, cudaMemcpyDeviceToHost, b->stream));
+    BCU(cudaMemcpyAsync(&err, b->err.ptr, 4, cudaMemcpyDeviceToHost, b->stream));
+    BCU(cudaStreamSynchronize(b->stream));
+    if (n_accepted)
+        for (int c = 0; c < K; ++c) n_accepted[c] = st[(size_t)c * kStateLen + 3];
     if (error_flag) *error_flag = err;
     return 0;
 }
@@ -1608,11 +1815,12 @@ int srhmc_big_set_recording(srhmc_big* b, int32_t n_iters, int32_t stride, int32
         return 0;
     }
     if (n_iters < 1 || stride < 1) return bfail(SRHMC_ERR_INVALID, "n_iters and stride must be >= 1");
+    if (int rc = chains_agree(b)) return rc;
     if (std::adjacent_find(b->sorted_ids.begin(), b->sorted_ids.end()) != b->sorted_ids.end())
         return bfail(SRHMC_ERR_STATE, "an owned global id appears twice: the sample rows need distinct ids");
     const int rows = (int)((n_iters + (int64_t)stride - 1) / stride);
     const int width = b->rj_on ? b->cfg.max_stars : b->n;   // reversible-jump rows: max_stars slots in table order
-    const size_t bytes = std::max<size_t>(1, (size_t)rows * width * 24);
+    const size_t bytes = std::max<size_t>(1, (size_t)b->chains * rows * width * 24);   // [chain][row][star][3]
     BCU(cudaStreamSynchronize(b->stream));
     BBuf* want[2] = {want_q ? &b->recq : nullptr, want_p ? &b->recp : nullptr};
     BBuf* drop[2] = {want_q ? nullptr : &b->recq, want_p ? nullptr : &b->recp};
@@ -1630,16 +1838,24 @@ int srhmc_big_set_recording(srhmc_big* b, int32_t n_iters, int32_t stride, int32
     b->rec_rows = rows;
     b->rec_stride = stride;
     b->rec_n = width;
+    b->P.X.rec = (long long)rows * width * 3;
     return 0;
 }
 
 int srhmc_big_read_samples(srhmc_big* b, int32_t row0, int32_t nrows, double* q, double* p) {
     if (!b) return bfail(SRHMC_ERR_INVALID, "null context");
+    if (b->chains > 1) return refuse_chains(b, "srhmc_big_read_chain_samples");
+    return srhmc_big_read_chain_samples(b, 0, row0, nrows, q, p);
+}
+
+int srhmc_big_read_chain_samples(srhmc_big* b, int32_t chain, int32_t row0, int32_t nrows, double* q, double* p) {
+    if (!b) return bfail(SRHMC_ERR_INVALID, "null context");
+    if (chain < 0 || chain >= b->chains) return bfail(SRHMC_ERR_INVALID, "chain %d outside the context's %d chains", chain, b->chains);
     if (row0 < 0 || nrows < 0 || (int64_t)row0 + nrows > b->rec_rows)
         return bfail(SRHMC_ERR_INVALID, "rows [%d, %d) outside the %d recorded rows", row0, row0 + nrows, b->rec_rows);
     if ((q && !b->recq.ptr) || (p && !b->recp.ptr)) return bfail(SRHMC_ERR_STATE, "%s was not recorded", (q && !b->recq.ptr) ? "q" : "p");
     BCU(cudaSetDevice(b->cfg.device));
-    const size_t row = (size_t)b->rec_n * 24, off = (size_t)row0 * row, bytes = (size_t)nrows * row;
+    const size_t row = (size_t)b->rec_n * 24, off = (size_t)chain * b->P.X.rec * 8 + (size_t)row0 * row, bytes = (size_t)nrows * row;
     if (q && bytes) BCU(cudaMemcpyAsync(q, b->recq.as<unsigned char>() + off, bytes, cudaMemcpyDeviceToHost, b->stream));
     if (p && bytes) BCU(cudaMemcpyAsync(p, b->recp.as<unsigned char>() + off, bytes, cudaMemcpyDeviceToHost, b->stream));
     BCU(cudaStreamSynchronize(b->stream));
@@ -1655,6 +1871,8 @@ int srhmc_big_convergence_stats(srhmc_big* const* chains, int32_t k, int32_t thi
     for (int32_t c = 0; c < k; ++c) {
         const srhmc_big* b = chains[c];
         if (!b) return bfail(SRHMC_ERR_INVALID, "chain %d is null", c);
+        if (b->chains > 1)
+            return bfail(SRHMC_ERR_INVALID, "chain %d is a context of %d chains: use srhmc_big_chain_convergence_stats", c, b->chains);
         if (!b->recq.ptr || b->rec_rows == 0) return bfail(SRHMC_ERR_STATE, "chain %d has no recorded q rows", c);
         if (b->cfg.device != c0->cfg.device) return bfail(SRHMC_ERR_INVALID, "chain %d is on device %d, chain 0 on %d", c, b->cfg.device, c0->cfg.device);
         if (b->rec_rows != c0->rec_rows || b->rec_stride != c0->rec_stride)
@@ -1680,6 +1898,34 @@ int srhmc_big_convergence_stats(srhmc_big* const* chains, int32_t k, int32_t thi
     cudaError_t e = (cudaError_t)conv_stats_var_launch(st, x, k, c0->rec_rows, d, thin_rate, warm_up_num, out.as<double>(),
                                                        out.as<double>() + d);
     chains[0]->launches += 1;
+    if (e == cudaSuccess) e = cudaMemcpyAsync(R, out.ptr, (size_t)d * 8, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(n_eff, out.as<double>() + d, (size_t)d * 8, cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+    out.release();
+    if (e != cudaSuccess) return bfail(SRHMC_ERR_CUDA, "chain statistics failed: %s", cudaGetErrorString(e));
+    return 0;
+}
+
+int srhmc_big_chain_convergence_stats(srhmc_big* b, int32_t thin_rate, int32_t warm_up_num, double* R, double* n_eff) {
+    if (!b || !R || !n_eff) return bfail(SRHMC_ERR_INVALID, "null argument");
+    const int k = b->chains;
+    if (k < 2) return bfail(SRHMC_ERR_INVALID, "convergence statistics need at least two chains (utils.py:94), got %d", k);
+    if (k > kMaxStatsChains) return bfail(SRHMC_ERR_INVALID, "at most %d chains, got %d", kMaxStatsChains, k);
+    if (!b->recq.ptr || b->rec_rows == 0) return bfail(SRHMC_ERR_STATE, "the chains have no recorded q rows");
+    const int d = 3 * b->rec_n;
+    if (int rc = check_stats_args(k, b->rec_rows, d, 1, thin_rate, warm_up_num)) return bfail(rc, "%s", srhmc_last_error());
+    BCU(cudaSetDevice(b->cfg.device));
+    const double* x[kMaxStatsChains];
+    for (int c = 0; c < k; ++c) x[c] = b->recq.as<double>() + (size_t)c * b->P.X.rec;   // K rows of one recording buffer
+    BBuf out;
+    if (int rc = out.ensure(2 * (size_t)d * 8)) {
+        cudaGetLastError();
+        return bfail(rc, "cannot allocate the statistics output (%d variables)", d);
+    }
+    cudaStream_t st = b->stream;
+    cudaError_t e = (cudaError_t)conv_stats_var_launch(st, x, k, b->rec_rows, d, thin_rate, warm_up_num, out.as<double>(),
+                                                       out.as<double>() + d);
+    b->launches += 1;
     if (e == cudaSuccess) e = cudaMemcpyAsync(R, out.ptr, (size_t)d * 8, cudaMemcpyDeviceToHost, st);
     if (e == cudaSuccess) e = cudaMemcpyAsync(n_eff, out.as<double>() + d, (size_t)d * 8, cudaMemcpyDeviceToHost, st);
     if (e == cudaSuccess) e = cudaStreamSynchronize(st);
@@ -1795,8 +2041,12 @@ int srhmc_big_find_peaks(srhmc_big* b, const srhmc_big_peaks_args* a) {
 int srhmc_big_phase(srhmc_big* b, int32_t phase, const srhmc_big_step* s) {
     if (!b || !s) return bfail(SRHMC_ERR_INVALID, "null argument");
     if (!b->have_data) return bfail(SRHMC_ERR_STATE, "srhmc_big_set_data has not been called");
+    if (int rc = chains_agree(b)) return rc;
     BCU(cudaSetDevice(b->cfg.device));
     const BigParams& P = b->P;
+    // chain axis: every per-star launch covers the K chains (gridDim.y = K); chain c's fixed-point counts are cnt[c] and
+    // cnt[K + c], the shared iteration counter cnt[2 K]
+    const int K = b->chains;
     if (b->rj_on && s->fixed_point_mode != 0)
         return bfail(SRHMC_ERR_INVALID, "reversible-jump mode runs the reference stop rule only (fixed_point_mode = 0)");
     // reversible-jump mode: every per-star kernel is launched for max_stars and reads its count on the device -- the live
@@ -1827,7 +2077,7 @@ int srhmc_big_phase(srhmc_big* b, int32_t phase, const srhmc_big_step* s) {
                                                                                                  : big_kick_kernel<true, false, true>)
                                     : (!last_half ? big_kick_kernel<false, true, false> : next_first ? big_kick_kernel<true, true, false>
                                                                                                   : big_kick_kernel<true, false, false>);
-        kernel<<<gs, tb, 0, st>>>(P, S, n, b->q.as<double>(), b->p.as<double>(), b->g.as<double>(), gpart, b->a1.as<double>(),
+        kernel<<<dim3(gs, K), tb, 0, st>>>(P, S, n, b->q.as<double>(), b->p.as<double>(), b->g.as<double>(), gpart, b->a1.as<double>(),
                                   b->a2.as<double>(), cnt, X, nd_step);
         b->launches += 1;
     };
@@ -1836,7 +2086,7 @@ int srhmc_big_phase(srhmc_big* b, int32_t phase, const srhmc_big_step* s) {
     // image for the next evaluation and PACK.
     auto position_update = [&](bool perstar, bool from_eval, const double* gpart) -> int {
         if (b->use_tiles && (b->own_binned || b->ghosts_binned)) {  // records nobody consumed (two position updates without an evaluation)
-            BCU(cudaMemsetAsync(b->tcnt.ptr, 0, (size_t)b->nty * b->ntx * 4, st));
+            BCU(cudaMemsetAsync(b->tcnt.ptr, 0, (size_t)K * b->nty * b->ntx * 4, st));
             b->ghosts_binned = false;
         }
         if (peer_multi && b->pack_counted)   // counts nobody consumed (two position updates without a PACK)
@@ -1849,11 +2099,11 @@ int srhmc_big_phase(srhmc_big* b, int32_t phase, const srhmc_big_step* s) {
         double* lf = (!b->use_tiles && n > 0) ? b->L.as<double>() : nullptr;
         if (perstar) {
             const auto kernel = from_eval ? big_perstar_kernel<true> : big_perstar_kernel<false>;
-            kernel<<<gs, tb, 0, st>>>(P, S, n, b->q.as<double>(), b->p.as<double>(), b->g.as<double>(), gpart, b->ntx, tc, tl,
+            kernel<<<dim3(gs, K), tb, 0, st>>>(P, S, n, b->q.as<double>(), b->p.as<double>(), b->g.as<double>(), gpart, b->ntx, tc, tl,
                                       b->err.as<int>(), pc, lo_edge, hi_edge, lf, npix);
         } else {
-            (nd_step ? big_qfix_kick_kernel<true> : big_qfix_kick_kernel<false>)<<<gs, tb, 0, st>>>(P, S, n, b->q.as<double>(), b->p.as<double>(), b->a1.as<double>(),
-                                                    b->a2.as<double>(), cnt + 1, b->ntx, tc, tl, b->err.as<int>(), pc, lo_edge,
+            (nd_step ? big_qfix_kick_kernel<true> : big_qfix_kick_kernel<false>)<<<dim3(gs, K), tb, 0, st>>>(P, S, n, b->q.as<double>(), b->p.as<double>(), b->a1.as<double>(),
+                                                    b->a2.as<double>(), cnt + K, b->ntx, tc, tl, b->err.as<int>(), pc, lo_edge,
                                                     hi_edge, lf, npix, nd_step);
         }
         b->L_filled = lf != nullptr;
@@ -1912,7 +2162,7 @@ int srhmc_big_phase(srhmc_big* b, int32_t phase, const srhmc_big_step* s) {
             if (int rc = enqueue_eval(b, want_V, &gpart, n, nd_step)) return rc;
             if (!last_half) {
                 if (gpart) {   // no tail sums the footprint partials into g
-                    (nd_step ? big_gsum_kernel<true> : big_gsum_kernel<false>)<<<gs, tb, 0, st>>>(P, b->q.as<double>(), n, gpart, b->g.as<double>(), nd_step);
+                    (nd_step ? big_gsum_kernel<true> : big_gsum_kernel<false>)<<<dim3(gs, K), tb, 0, st>>>(P, b->q.as<double>(), n, gpart, b->g.as<double>(), nd_step);
                     b->launches += 1;
                 }
             } else if (ps_advance) {
@@ -1924,17 +2174,17 @@ int srhmc_big_phase(srhmc_big* b, int32_t phase, const srhmc_big_step* s) {
             break;
         }
         case SRHMC_BIG_RESET_ITER:
-            BCU(cudaMemsetAsync(cnt + 2, 0, 4, st));
+            BCU(cudaMemsetAsync(cnt + 2 * K, 0, 4, st));
             break;
         case SRHMC_BIG_KICK1:
-            BCU(cudaMemsetAsync(cnt, 0, 8, st));
+            BCU(cudaMemsetAsync(cnt, 0, 8 * K, st));
             kick(false, true, nullptr);
             break;
         case SRHMC_BIG_PFIX_QFIX:
             // tiled over peers: the field-wide maximum of the p fixed-point counts was all-reduced by the last block of the
             // kernel that produced it
-            (nd_step ? big_pfix_qfix_kernel<true> : big_pfix_qfix_kernel<false>)<<<gs, tb, 0, st>>>(P, S, n, b->q.as<double>(), b->p.as<double>(), b->a1.as<double>(),
-                                                    b->a2.as<double>(), cnt, cnt + 1, X, nd_step);
+            (nd_step ? big_pfix_qfix_kernel<true> : big_pfix_qfix_kernel<false>)<<<dim3(gs, K), tb, 0, st>>>(P, S, n, b->q.as<double>(), b->p.as<double>(), b->a1.as<double>(),
+                                                    b->a2.as<double>(), cnt, cnt + K, X, nd_step);
             b->launches += 1;
             break;
         case SRHMC_BIG_QFIX_KICK:
@@ -1945,14 +2195,14 @@ int srhmc_big_phase(srhmc_big* b, int32_t phase, const srhmc_big_step* s) {
             break;
         case SRHMC_BIG_MOMENTUM: {
             const double* z = b->normals.ptr ? b->normals.as<double>() : nullptr;
-            (nd_live ? big_momentum_kernel<true> : big_momentum_kernel<false>)<<<gs, tb, 0, st>>>(P, s->g_ff2, n, b->q.as<double>(), b->p.as<double>(), b->g.as<double>(),
+            (nd_live ? big_momentum_kernel<true> : big_momentum_kernel<false>)<<<dim3(gs, K), tb, 0, st>>>(P, s->g_ff2, n, b->q.as<double>(), b->p.as<double>(), b->g.as<double>(),
                                                    b->q0.as<double>(), b->g0.as<double>(), b->gid.as<long long>(), s->seed,
-                                                   s->iteration, s->iteration < 0 ? cnt + 2 : nullptr, z, nd_live);
+                                                   s->iteration, s->iteration < 0 ? cnt + 2 * K : nullptr, z, nd_live);
             b->launches += 1;
             break;
         }
         case SRHMC_BIG_ENERGY:
-            (nd_live ? big_energy_kernel<true> : big_energy_kernel<false>)<<<std::max(1, std::min((n + 255) / 256, kEnergyBlocks)), 256, 0, st>>>(
+            (nd_live ? big_energy_kernel<true> : big_energy_kernel<false>)<<<dim3(std::max(1, std::min((n + 255) / 256, kEnergyBlocks)), K), 256, 0, st>>>(
                 P, s->g_ff2, s->f_pos, n, b->q.as<double>(), b->p.as<double>(), b->epart.as<double>(),
                 b->tickets.as<unsigned int>(), b->scalars.as<double>(), nd_live);
             b->launches += 1;
@@ -1964,28 +2214,28 @@ int srhmc_big_phase(srhmc_big* b, int32_t phase, const srhmc_big_step* s) {
             // single rank: the global sums are the local ones; otherwise the caller has all-reduced `scalars` into
             // `global_scalars` on this stream before this phase
             if (b->world == 1) {
-                BCU(cudaMemcpyAsync(b->gscalars.ptr, b->scalars.ptr, kScalars * 8, cudaMemcpyDeviceToDevice, st));
+                BCU(cudaMemcpyAsync(b->gscalars.ptr, b->scalars.ptr, (size_t)K * kScalars * 8, cudaMemcpyDeviceToDevice, st));
             } else if (b->peer_enabled) {  // sum of the energy partials over the ranks, in rank order on every rank
                 big_xchg_small_kernel<<<1, 32, 0, st>>>(b->peers, b->rank, b->world, kScalars, b->scalars.as<double>(),
                                                         b->gscalars.as<double>(), b->xepoch.as<unsigned long long>(), b->err.as<int>());
                 b->launches += 1;
             }
-            big_accept_kernel<<<gs, tb, 0, st>>>(ph, b->gscalars.as<double>(), b->scalars.as<double>(), b->state.as<double>(), s->seed, s->iteration,
-                                                 s->iteration < 0 ? cnt + 2 : nullptr,
+            big_accept_kernel<<<dim3(gs, K), tb, 0, st>>>(P, ph, b->gscalars.as<double>(), b->scalars.as<double>(), b->state.as<double>(), s->seed, s->iteration,
+                                                 s->iteration < 0 ? cnt + 2 * K : nullptr,
                                                  b->lnu.ptr ? b->lnu.as<double>() : nullptr, n, b->q.as<double>(),
                                                  b->g.as<double>(), b->q0.as<double>(), b->g0.as<double>(),
                                                  b->E.ptr ? b->E.as<double>() : nullptr, b->V.ptr ? b->V.as<double>() : nullptr,
                                                  b->T.ptr ? b->T.as<double>() : nullptr,
                                                  b->A.ptr ? b->A.as<unsigned char>() : nullptr);
             if (ph == 1)
-                big_restore_v_kernel<<<1, 1, 0, st>>>(b->scalars.as<double>(), b->state.as<double>(),
-                                                      s->iteration < 0 ? cnt + 2 : nullptr);
+                big_restore_v_kernel<<<1, K, 0, st>>>(b->scalars.as<double>(), b->state.as<double>(),
+                                                      s->iteration < 0 ? cnt + 2 * K : nullptr);
             b->launches += 1 + ph;
             if (ph == 0 && b->rec_rows > 0) {   // sample row of this iteration (srhmc_big_set_recording)
                 if (b->rec_n != n) return bfail(SRHMC_ERR_STATE, "the stars changed since srhmc_big_set_recording");
                 if (n > 0) {
-                    (nd_live ? big_record_kernel<true> : big_record_kernel<false>)<<<std::max(1, std::min((3 * n + 255) / 256, 4 * b->sm_count)), 256, 0, st>>>(
-                        n, b->q.as<double>(), b->p.as<double>(), b->slot.as<int>(), s->iteration, s->iteration < 0 ? cnt + 2 : nullptr,
+                    (nd_live ? big_record_kernel<true> : big_record_kernel<false>)<<<dim3(std::max(1, std::min((3 * n + 255) / 256, 4 * b->sm_count)), K), 256, 0, st>>>(
+                        P, n, b->q.as<double>(), b->p.as<double>(), b->slot.as<int>(), s->iteration, s->iteration < 0 ? cnt + 2 * K : nullptr,
                         b->rec_stride, b->rec_rows, b->recq.as<double>(), b->recp.as<double>(), nd_live);
                     b->launches += 1;
                 }

@@ -113,8 +113,12 @@ template <bool LIVE>
 __global__ void big_bin_kernel(const BigParams P, const TileSrc S, int ntx, int sid0, int sid1, int* cnt, PairRec* list, int* err,
                                const int* nd /* live owned stars: sid1 */) {
     if (LIVE) sid1 = *nd;
+    TileSrc Sc = S;   // chain blockIdx.y: its stars into its own lists
+    Sc.q = chain_slice(S.q, 3 * P.X.M);
+    cnt += blockIdx.y * P.X.tiles;
+    list += blockIdx.y * P.X.tiles * kTileMaxList;
     for (int sid = sid0 + blockIdx.x * blockDim.x + threadIdx.x; sid < sid1; sid += gridDim.x * blockDim.x) {
-        const double* src = tile_source(S, sid);
+        const double* src = tile_source(Sc, sid);
         if (!src) continue;
         bin_star(P, ntx, sid, src[0], src[1], src[2], sid < S.n_own, cnt, list, err);
     }
@@ -226,9 +230,20 @@ __device__ __forceinline__ void cp_async8(void* smem, const void* gmem) {
 __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
 __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_group 0;" ::: "memory"); }
 
+// blockIdx.y read where it is used: the chain tile kernel applies its chain offsets at each use, so that no offset pointer
+// is held in a register across the kernel (asm volatile: the read is neither hoisted nor merged)
+__device__ __forceinline__ unsigned chain_at_use() {
+    unsigned y;
+    asm volatile("mov.u32 %0, %%ctaid.y;" : "=r"(y));
+    return y;
+}
+
 // MODE 0: gradient; 1: gradient + pixel potential; 2: mock data -- the rendered model of the tile is Poisson-sampled
-// (poisson.cuh, counter = global pixel index) into Dout and nothing else happens
-template <int MODE>
+// (poisson.cuh, counter = global pixel index) into Dout and nothing else happens.
+// CHAINS: the launch covers the context's chains, chain c = blockIdx.y with its own lists, partials, ticket and fixed-point
+// counters (counter j of chain c at fp_counters[j K + c]); the shared data tile is the same for every chain.  A template flag
+// so that the one-chain instantiations keep their code.
+template <int MODE, bool CHAINS = false>
 __global__ void __launch_bounds__(kTileThreads, 4) big_tile_kernel(const BigParams P, const TileSrc S, int ntx,
                                                                 const double* __restrict__ D,
                                                                 int* __restrict__ cnt,
@@ -238,6 +253,8 @@ __global__ void __launch_bounds__(kTileThreads, 4) big_tile_kernel(const BigPara
                                                                 unsigned long long mock_seed,
                                                                 const __grid_constant__ CUtensorMap tmapD, int use_tma) {
     constexpr bool WANT_V = MODE == 1;
+    // chain offsets are applied where each buffer is used (offset pointers held across the kernel cost registers)
+    const int tile = CHAINS ? (int)(chain_at_use() * P.X.tiles) + blockIdx.x : blockIdx.x;   // this chain's list of this tile
     extern __shared__ __align__(128) unsigned char tile_smem_raw[];
     TileSmem& sm = *reinterpret_cast<TileSmem*>(tile_smem_raw);
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -284,13 +301,13 @@ __global__ void __launch_bounds__(kTileThreads, 4) big_tile_kernel(const BigPara
     // ---- the tile's pair list, ranked by star id so that every sum below has a fixed order.  The first kTileRecs records
     //      are fetched speculatively together with the count (one trip to L2 instead of two dependent ones); they carry
     //      the star's (f, x, y), so no third trip follows.
-    list += (size_t)blockIdx.x * kTileMaxList;
+    list += (size_t)tile * kTileMaxList;
     PairRec spec;
     spec.sid = 0; spec.box = 0; spec.f = spec.x = spec.y = 0.0;
     if (tid < kTileRecs) spec = ld_rec(&list[tid]);
-    const int nl = min(cnt[blockIdx.x], kTileMaxList);  // an overflow was flagged when the list was filled
+    const int nl = min(cnt[tile], kTileMaxList);  // an overflow was flagged when the list was filled
     // the fixed-point iteration counters of the leapfrog step are free between its last reader and the next step
-    if (fp_counters && blockIdx.x == 0 && tid < 2) fp_counters[tid] = 0;
+    if (fp_counters && blockIdx.x == 0 && tid < 2) fp_counters[CHAINS ? tid * gridDim.y + blockIdx.y : tid] = 0;
     // guard entries of the factor tables stay zero for the whole launch; the 32 body entries are rewritten per pair
     for (int k = tid; k < kTileChunk * 4 * kTabPad; k += kTileThreads) {
         const int pair = k / (4 * kTabPad), e = k % (4 * kTabPad), side = e / kTabPad, g = e % kTabPad;
@@ -316,7 +333,7 @@ __global__ void __launch_bounds__(kTileThreads, 4) big_tile_kernel(const BigPara
         sm.order[r] = (unsigned short)k;
     }
     __syncthreads();
-    if (tid == 0) cnt[blockIdx.x] = 0;  // every thread has read the count: ready for the next evaluation's binning
+    if (tid == 0) cnt[CHAINS ? (int)(chain_at_use() * P.X.tiles) + blockIdx.x : blockIdx.x] = 0;  // every thread has read the count: ready for the next evaluation's binning
     // record with the s-th smallest star id
     auto rec_at = [&](int s) -> PairRec {
         const int k = sm.order[s];
@@ -407,7 +424,7 @@ __global__ void __launch_bounds__(kTileThreads, 4) big_tile_kernel(const BigPara
     if (WANT_V) {
         double a1[1] = {v};
         block_sum<1>(a1, sm.red);
-        if (tid == 0) vpart[blockIdx.x] = a1[0];
+        if (tid == 0) vpart[CHAINS ? chain_at_use() * P.X.vpart + blockIdx.x : blockIdx.x] = a1[0];
     }
     __syncthreads();
 
@@ -451,11 +468,18 @@ __global__ void __launch_bounds__(kTileThreads, 4) big_tile_kernel(const BigPara
             yv += __shfl_xor_sync(0xffffffffu, yv, 2);
             yv += __shfl_xor_sync(0xffffffffu, yv, 1);
             // lane 0: sum sf, lane 8: sum sx, lane 16: sum sy
-            if ((lane & 7) == 0 && lane < 24) gpart[((size_t)rec.sid * 4 + (rec.box >> 24)) * 3 + (lane >> 3)] = yv;
+            if ((lane & 7) == 0 && lane < 24)
+                gpart[((size_t)(CHAINS ? rec.sid + chain_at_use() * P.X.M : rec.sid) * 4 + (rec.box >> 24)) * 3 + (lane >> 3)] = yv;
         }
     }
     // ---- pixel potential: the last tile to finish sums the per-tile partials in tile order -> scalars[0]
     if (WANT_V) {
+        if (CHAINS) {
+            const unsigned c = chain_at_use();
+            ticket += c * 2;
+            vpart += c * P.X.vpart;
+            scalars += c * kScalars;
+        }
         if (last_block_ticket(ticket, &sm.is_last)) {
             double w[1] = {0.0};
             for (int b = tid; b < (int)gridDim.x; b += kTileThreads) w[0] += __ldcg(vpart + b);
@@ -660,6 +684,8 @@ __device__ __forceinline__ void gsum_star(const BigParams& P, int k, double f, d
 template <bool LIVE>
 __global__ void big_gsum_kernel(const BigParams P, const double* q, int n_own, const double* gpart, double* g, const int* nd) {
     if (LIVE) n_own = *nd;
+    q += blockIdx.y * 3 * P.X.M; g += blockIdx.y * 3 * P.X.M;
+    gpart += blockIdx.y * 12 * P.X.M;
     for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < n_own; k += gridDim.x * blockDim.x)
         gsum_star(P, k, q[3 * k], q[3 * k + 1], q[3 * k + 2], gpart, g[3 * k], g[3 * k + 1], g[3 * k + 2]);
 }

@@ -517,6 +517,28 @@ int srhmc_big_read_samples(srhmc_big* b, int32_t row0, int32_t nrows, double* q,
 int srhmc_big_convergence_stats(srhmc_big* const* chains, int32_t k, int32_t thin_rate, int32_t warm_up_num, double* R,
                                 double* n_eff);
 
+/* K chains of one field in one context (world_size = 1, precision 64, not in reversible-jump mode).  Every chain carries the
+ * same star ids with its own values and is independent of the others: its own fixed-point stop rule (the maximum over its
+ * own stars), energies, Metropolis test and restore.  Chain c draws from Philox field c -- philox_normals3(seed, c, iter, id)
+ * and philox_lnu(seed, c, iter) -- so chain 0 is the one-chain engine's chain.  The data window, step parameters, seed,
+ * iteration counter and error flag are shared; one launch of each kernel covers every chain (gridDim.y = K), so a phase
+ * enqueues as many kernels for K chains as for one.  K > 1 always evaluates on the FP64 tile kernel.
+ * srhmc_big_set_chains (re)allocates the per-chain buffers and clears every chain's stars (recording and chain rows too);
+ * k = 1 returns to the evaluation path srhmc_big_create chose.  With K > 1 the one-chain calls (set_stars, get_stars,
+ * set_momenta, set_draws, read_chains, read_samples, rj_configure) return SRHMC_ERR_STATE; device draws only. */
+int srhmc_big_set_chains(srhmc_big* b, int32_t k /* 1..64 */);
+/* The stars of chain `chain` ([n,3] in the chain's own storage order, ids [n]); momenta zero.  The first phase or recording
+ * set-up after a change refuses chains whose id sets differ. */
+int srhmc_big_set_chain_stars(srhmc_big* b, int32_t chain, const double* q, const int64_t* global_ids, int32_t n);
+int srhmc_big_get_chain_stars(srhmc_big* b, int32_t chain, double* q, double* p, double* grad /* each [n,3], may be NULL */);
+/* E, V, T [K, n_iters], A [K, n_iters], n_accepted [K] (any may be NULL); error_flag as srhmc_big_read_chains */
+int srhmc_big_read_chain_rows(srhmc_big* b, int32_t n_iters, double* E, double* V, double* T, uint8_t* A, double* n_accepted,
+                              int32_t* error_flag);
+/* srhmc_big_read_samples for chain `chain`: rows in the chain's ascending-id slot order, the same columns for every chain */
+int srhmc_big_read_chain_samples(srhmc_big* b, int32_t chain, int32_t row0, int32_t nrows, double* q, double* p);
+/* srhmc_big_convergence_stats over the context's own K chains (2..16) from their recorded q rows */
+int srhmc_big_chain_convergence_stats(srhmc_big* b, int32_t thin_rate, int32_t warm_up_num, double* R, double* n_eff);
+
 /* lightsource_gym.find_peaks (samplers.py:129-254) on the context's image: every seed descends on a pure-background model
  * (B_count) with every potential and gradient evaluated over its (2 patch_radius + 1)^2 window, clipped to the image; it
  * stops when V on the window of its new position changes by less than 1e-9 relative (V at the old position re-evaluated on
